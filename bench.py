@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: IQL gradient steps/sec, summed over ensemble members.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
 
 One bench *step* = one fused engine call that runs ``inner`` IQL updates
 (replay sample + V/Q/actor update + Polyak + LR schedule) for every one of the
@@ -16,6 +16,12 @@ the NCCL all-gather of the per-step loss scalars.
 oracle/_ref by __graft_entry__.build()) on the host cores -- one member, all threads and one
 thread, 1M-row buffer, a bounded number of steps -- and the same code with device="cuda"
 (`torch_eager_b200`: what a user of the reference gets on this GPU today).
+
+`--dump-outputs DIR` writes what the last timed step computed, as float32 .npy files: ``losses.npy`` (the [S, inner, 3]
+losses the engine call returns), ``params.npy`` and ``target.npy`` (the parameter and Q-target arenas of all S members
+after that call).  An array above 4 Mi elements is replaced by a fixed, seeded sample of 4 Mi of its flattened elements,
+so a dump stays under 64 MB.  Inputs depend only on the arguments, so two builds run with the same arguments can be
+compared file by file.  Multi-GPU runs dump rank 0's members.
 """
 import argparse
 import json
@@ -64,6 +70,23 @@ def flops_per_step(w):
 
 def gather_bytes_per_step(w):
     return w["B"] * (2 * w["S"] + w["A"] + 2) * 4
+
+
+DUMP_MAX_ELEMS = 1 << 22  # per array: three float32 arrays stay under 64 MB
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each array as out_dir/<name>.npy in float32; one above DUMP_MAX_ELEMS becomes a seeded sample of its
+    flattened elements (the same positions on every run with the same shape)."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a, dtype=np.float32)
+        if a.size > DUMP_MAX_ELEMS:
+            pick = np.sort(np.random.default_rng(0).choice(a.size, DUMP_MAX_ELEMS, replace=False))
+            a = a.reshape(-1)[pick]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 class ClockSampler:
@@ -455,6 +478,8 @@ def run_ours(args, w, rank, world, local_rank, collect=None):
         ms = float(t.item())
     final = losses.cpu().numpy()
     assert np.isfinite(final).all(), "non-finite losses in the timed region"
+    if args.dump_outputs and rank == 0:  # before the e2e leg below trains the same engine further
+        dump_outputs(args.dump_outputs, {"losses": final, "params": eng.params.cpu(), "target": eng.target.cpu()})
     total_steps = world * S_local * inner * args.steps
     value = total_steps / (ms * 1e-3)
 
@@ -479,7 +504,7 @@ def run_ours(args, w, rank, world, local_rank, collect=None):
     for _ in range(3):
         e2e_step()
     sync_all()
-    e2e_steps = max(2, args.steps)
+    e2e_steps = args.steps
     e0.record()
     for _ in range(e2e_steps):
         e2e_step()
@@ -655,7 +680,13 @@ def main():
     ap.add_argument("--fast-init", action="store_true")
     ap.add_argument("--all-configs", action="store_true",
                     help="N = 1: run every BASELINE.json workload back to back and print ONE line with the table")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's losses, parameters and Q targets to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.all_configs):
+        ap.error("--dump-outputs needs --impl ours and a single workload")
     w = dict(WORKLOADS[args.workload])
     if args.members:
         w["members"] = args.members

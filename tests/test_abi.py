@@ -146,18 +146,17 @@ def test_train_config_fields_match_reference_dataclasses():
     from jsrl_corl_b200.jsrl_utils import JsrlTrainConfig
     from oracle.ref_loader import load_reference_iql, reference_available
 
-    if not reference_available():
-        pytest.skip("reference tree not present (GPU box)")
-
     def fields(cls):
         return {f.name: f.default for f in dataclasses.fields(cls) if f.default is not dataclasses.MISSING}
 
-    assert fields(J.TrainConfig) == fields(load_reference_iql("finetune").TrainConfig)
-    assert fields(J.OfflineTrainConfig) == fields(load_reference_iql("offline").TrainConfig)
     assert set(fields(J.TrainConfig)) < set(f.name for f in dataclasses.fields(JsrlTrainConfig))
     # offline variant: a Dropout module exists whenever dropout is not None (even 0.0): keys 0,3,6
     pol = J.GaussianPolicy(4, 2, 1.0, 16, 2, dropout=0.0, dropout_when_not_none=True)
     assert [k for k in pol.state_dict() if k.endswith("weight")] == ["net.net.0.weight", "net.net.3.weight", "net.net.6.weight"]
+    if not reference_available():
+        pytest.skip("needs the original jsrl-CORL source under JSRL_REFERENCE_ROOT; no stored outputs of it exist for this comparison")
+    assert fields(J.TrainConfig) == fields(load_reference_iql("finetune").TrainConfig)
+    assert fields(J.OfflineTrainConfig) == fields(load_reference_iql("offline").TrainConfig)
     ref_pol = load_reference_iql("offline").GaussianPolicy(4, 2, 1.0, 16, 2, dropout=0.0)
     assert list(pol.state_dict().keys()) == list(ref_pol.state_dict().keys())
     ref_fin = load_reference_iql("finetune").GaussianPolicy(4, 2, 1.0, 16, 2, dropout=0.0)

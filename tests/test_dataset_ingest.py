@@ -25,7 +25,7 @@ def test_preprocessing_functions_match_the_reference():
     from oracle.ref_loader import load_reference_iql, reference_available
 
     if not reference_available():
-        pytest.skip("reference files not staged")
+        pytest.skip("needs the original jsrl-CORL source under JSRL_REFERENCE_ROOT; no stored outputs of it exist for this comparison")
     ref = load_reference_iql("finetune")
     from jsrl_corl_b200 import iql as ours
 

@@ -150,7 +150,8 @@ def _load_reference_jsrl():
 def test_curriculum_differential_against_reference(capsys):
     ref = _load_reference_jsrl()
     if ref is None:
-        pytest.skip("reference jsrl_utils.py not importable here")
+        pytest.skip("needs the original jsrl-CORL finetune/jsrl_utils.py importable under JSRL_REFERENCE_ROOT; "
+                    "no stored outputs of it exist for this comparison")
     rng = np.random.RandomState(0)
     for trial in range(40):
         kw = dict(n_curriculum_stages=int(rng.randint(1, 8)), tolerance=float(rng.choice([0.0, 0.05, 0.3])),

@@ -71,7 +71,7 @@ def test_oracle_against_live_reference():
     from oracle.ref_loader import load_reference_iql, reference_available
 
     if not reference_available():
-        pytest.skip("reference tree not present (GPU box)")
+        pytest.skip("needs the original jsrl-CORL source under JSRL_REFERENCE_ROOT; no stored outputs of it exist for this comparison")
     import torch
 
     ref = load_reference_iql("offline")
