@@ -140,7 +140,9 @@ int iql_set_counters(iql_engine* e, int32_t member, const iql_counters* c);
 
 /* Engine options (no counterpart in the reference: they select between equivalent B200 code paths and exist for
  * tests and measurements).  IQL_OPT_STEP_PATH must be set before iql_bind_state. */
-#define IQL_OPT_STEP_PATH 1  /* 0 auto (default; = 1 today), 1 one kernel per phase + adam_polyak, 2 chained backward + fused optimizer (bind fails where unsupported) */
+#define IQL_OPT_STEP_PATH 1  /* 0 auto (default): 4 where it is supported and the ensemble has >= 8 members or >= 3 hidden layers, else 1;
+                              1 one kernel per phase + adam_polyak; 2 chained backward + fused optimizer; 3 is not assigned;
+                              4 chained backward (gradients only) + adam_polyak.  2 and 4: bind fails where unsupported */
 #define IQL_OPT_KEEP_GRADS 2 /* != 0: the chained backward also stores the hidden / input weight gradients to `grads` */
 int iql_set_option(iql_engine* e, int32_t key, int64_t value);
 /* Which code path serves this handle (after iql_bind_state).  IQL_INFO_TENSOR_CORE_PATH == 0 under
@@ -149,7 +151,8 @@ int iql_set_option(iql_engine* e, int32_t key, int64_t value);
  * math_mode="tf32" was asked for with strict=True. */
 #define IQL_INFO_TENSOR_CORE_PATH 1
 #define IQL_INFO_FUSED_FORWARD 2
-#define IQL_INFO_CHAINED_BACKWARD 3
+#define IQL_INFO_CHAINED_BACKWARD 3       /* IQL_OPT_STEP_PATH 2: chained backward with the optimizer in its epilogue */
+#define IQL_INFO_CHAINED_BACKWARD_GRADS 4 /* chained backward storing the gradients, adam_polyak after it (4, or auto) */
 int iql_get_info(const iql_engine* e, int32_t key, int64_t* out);
 int iql_get_counters(iql_engine* e, int32_t member, iql_counters* out, void* stream);
 /* replaces: copy.deepcopy(self.qf) iql.py:464,584,598 (q_target <- qf) */
@@ -273,7 +276,7 @@ int64_t iql_last_launch_count(const iql_engine* e);
  * words written, < 0 when tracing is off or `max_words` is too small. */
 int iql_debug_fused_trace(long long* out, int32_t max_words);
 /* IQL_STEP_TRACE=1 (with IQL_B200_DEBUG=1): per-launch start / end globaltimer stamps of the step's kernels
- * (tools/step_trace.py); reset != 0 arms the slots, otherwise copies [12][2] stamps (ns) to `out`. */
+ * (tools/step_trace.py); reset != 0 arms the slots, otherwise copies [13][2] stamps (ns) to `out`. */
 int iql_debug_step_trace(iql_engine* e, int32_t reset, unsigned long long* out, int32_t max_words, void* stream);
 /* IQL_CHAIN_TRACE=1: globaltimer stamps of CTA pair 0 of the last bwd_chain launch (tools/chain_trace.py) */
 int iql_debug_chain_trace(long long* out, int32_t max_words);

@@ -21,8 +21,8 @@ SAMPLE_PHILOX, SAMPLE_INDICES, SAMPLE_PRELOADED = 0, 1, 2
 NET_Q1, NET_Q2, NET_V, NET_ACTOR = 0, 1, 2, 3
 KIND_WEIGHT, KIND_BIAS, KIND_LOG_STD = 0, 1, 2
 OPT_STEP_PATH, OPT_KEEP_GRADS = 1, 2
-INFO_TENSOR_CORE_PATH, INFO_FUSED_FORWARD, INFO_CHAINED_BACKWARD = 1, 2, 3
-STEP_PATHS = {"auto": 0, "phases": 1, "chain": 2}
+INFO_TENSOR_CORE_PATH, INFO_FUSED_FORWARD, INFO_CHAINED_BACKWARD, INFO_CHAINED_BACKWARD_GRADS = 1, 2, 3, 4
+STEP_PATHS = {"auto": 0, "phases": 1, "chain": 2, "chain_grads": 4}
 
 
 class Config(C.Structure):

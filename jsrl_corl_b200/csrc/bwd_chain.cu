@@ -26,6 +26,13 @@
 // the producers wait on it (acquire.cluster + fence.proxy.async) before the first load that depends on it.
 // W_l is overwritten by the wgrad_l epilogue only after the MMAs of dgrad_l (issued earlier, completed in order) have
 // consumed the shared-memory copy of the old W_l.
+//
+// Gradient-only mode (grads_only, IQL_OPT_STEP_PATH = 4): the wgrad epilogues store the FP32 weight gradients from the
+// staging tile to the grads arena (16-byte stores, exact zeros in the row padding of the input layer, as the per-phase
+// kernels write them) and the task-end small-parameter pass is skipped; adam_polyak_kernel runs after the launch.
+// The epilogue streams at the HBM rate of a plain store instead of the 72 % the in-epilogue optimizer reaches
+// (DESIGN.md section 8), and the chain keeps what it is good at: one launch for the hidden-layer backward, every dZ
+// read back from L2 by the pair that wrote it.
 #include <cuda.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -49,7 +56,7 @@ constexpr int C_EPI_WARPS = 16, C_CGROUPS = 4;
 constexpr int C_STG_BYTES = 5120;  // per-warp staging: 32 x 36 floats (transposing epilogue) or a swizzled 32 x 32 box
 constexpr int C_AUX_BYTES = 4 * 256 * 4;  // bias-gradient sums [4 lane quarters][256]
 constexpr int C_PEER_SLOTS = 3;
-constexpr int C_EPI_SMEM = C_EPI_WARPS * C_STG_BYTES + C_AUX_BYTES + C_PEER_SLOTS * 256 * 4;
+constexpr int C_EPI_SMEM = C_EPI_WARPS * C_STG_BYTES + C_AUX_BYTES + C_PEER_SLOTS * 4 * 256 * 4;
 constexpr int C_SMEM = C_RING + C_EPI_SMEM + 1024 /*align*/ + 512 /*barriers*/;
 constexpr int C_THREADS = 576;
 constexpr int C_MAX_PHASES = 2 * FUSED_MAX_LAYERS;
@@ -69,7 +76,8 @@ struct ChainPhase {
 };
 
 struct ChainParams {
-  int n_phases, n_dgrad, n_tasks, keep_grads;
+  int n_phases, n_dgrad, n_tasks, keep_grads, grads_only;
+  int db_tile_order;  // gradient-only: bias gradients in the summation order of the single-CTA per-phase dgrad
   ChainPhase ph[C_MAX_PHASES];
   // parameters the phases do not cover (biases, output layer, log_std), per network slot (V, q1, q2, actor):
   // flat ranges [lo, hi) inside a member block, multiples of 4 floats
@@ -137,17 +145,21 @@ __device__ __forceinline__ void adam_rows(const StepCtx& ctx, const float* __res
 __device__ __forceinline__ void fence_proxy_async_all() { asm volatile("fence.proxy.async;" ::: "memory"); }
 
 // (18 warps = 5 on two of the four schedulers: 16384 / 5 / 32 = 102 registers per thread at most -> ptxas settles on 96)
+// GRADS_ONLY: gradient-only instance (ChainParams::grads_only), compiled without the optimizer code
+template <bool GRADS_ONLY>
 __global__ void __launch_bounds__(C_THREADS, 1)
 bwd_chain_kernel(const GemmProb* __restrict__ probs, const CUtensorMap* __restrict__ maps, const CUtensorMap* __restrict__ cmaps,
                  const ChainParams cp, const StepCtx ctx, float* __restrict__ params, float* __restrict__ exp_avg,
                  float* __restrict__ exp_avg_sq, float* __restrict__ target, float* __restrict__ grads) {
   extern __shared__ uint8_t smem_raw[];
+  // step timeline: gradient-only instance only (the stamp registers push the fused-optimizer instance into spills)
+  if (GRADS_ONLY) stamp_begin(ctx.stamps, ST_CHAIN);
   const uint32_t raw = smem_u32(smem_raw);
   const uint32_t base = (raw + 1023u) & ~1023u;
   uint8_t* smem = smem_raw + (base - raw);
   uint8_t* epi_smem = smem + C_RING;
   float* csum_s = reinterpret_cast<float*>(epi_smem + C_EPI_WARPS * C_STG_BYTES);            // [4][256]
-  float* peer_csum = reinterpret_cast<float*>(epi_smem + C_EPI_WARPS * C_STG_BYTES + C_AUX_BYTES);  // [3][256]
+  float* peer_csum = reinterpret_cast<float*>(epi_smem + C_EPI_WARPS * C_STG_BYTES + C_AUX_BYTES);  // [3][4][256]
   // barriers: full[4] empty[4] tfull[2] tempty[2] csfull[3] gready | tmem slot
   const uint32_t bars = base + C_RING + C_EPI_SMEM;
   const uint32_t full0 = bars, empty0 = bars + 8 * C_STAGES, tfull0 = bars + 16 * C_STAGES, tempty0 = tfull0 + 16;
@@ -342,17 +354,33 @@ bwd_chain_kernel(const GemmProb* __restrict__ probs, const CUtensorMap* __restri
             mbar_arrive_cluster(gready_own);
             mbar_arrive_cluster(gready_peer);
           }
-          // bias gradient: add the lane quarters, then the two CTAs (fixed order)
+          // bias gradient: add the lane quarters, then the two CTAs (fixed order).  db_tile_order: the order of the
+          // per-phase dgrad when it runs one CTA per problem (both 128-row M tiles in one CTA, quarter q of the second
+          // tile added to quarter q of the first, then the quarters), so that the bias gradients match it bit for bit
           asm volatile("bar.sync 1, 512;" ::: "memory");
-          if (et < 256) {
-            float own = ((csum_s[et] + csum_s[256 + et]) + csum_s[512 + et]) + csum_s[768 + et];
+          if (GRADS_ONLY && cp.db_tile_order && et < 256) {
             const uint32_t cslot = dcount % C_PEER_SLOTS, par = (dcount / C_PEER_SLOTS) & 1u;
+            float* pc = &peer_csum[cslot * 4 * 256 + et];
             if (rank != 0) {
-              st_cluster_f32(mapa_u32(smem_u32(&peer_csum[cslot * 256 + et]), 0), own);
+#pragma unroll
+              for (int qq = 0; qq < 4; ++qq) st_cluster_f32(mapa_u32(smem_u32(pc + qq * 256), 0), csum_s[qq * 256 + et]);
               mbar_arrive_cluster(mapa_u32(csfull0 + 8 * cslot, 0));
             } else {
               mbar_wait_cluster(csfull0 + 8 * cslot, par);
-              own += peer_csum[cslot * 256 + et];
+              float own = csum_s[et] + pc[0];
+#pragma unroll
+              for (int qq = 1; qq < 4; ++qq) own += csum_s[qq * 256 + et] + pc[qq * 256];
+              if (p.dbias != nullptr && et < p.N) p.dbias[et] = own;
+            }
+          } else if (et < 256) {
+            float own = ((csum_s[et] + csum_s[256 + et]) + csum_s[512 + et]) + csum_s[768 + et];
+            const uint32_t cslot = dcount % C_PEER_SLOTS, par = (dcount / C_PEER_SLOTS) & 1u;
+            if (rank != 0) {
+              st_cluster_f32(mapa_u32(smem_u32(&peer_csum[cslot * 4 * 256 + et]), 0), own);
+              mbar_arrive_cluster(mapa_u32(csfull0 + 8 * cslot, 0));
+            } else {
+              mbar_wait_cluster(csfull0 + 8 * cslot, par);
+              own += peer_csum[cslot * 4 * 256 + et];
               if (p.dbias != nullptr && et < p.N) p.dbias[et] = own;
             }
           }
@@ -360,7 +388,7 @@ bwd_chain_kernel(const GemmProb* __restrict__ probs, const CUtensorMap* __restri
           if (tracer) ctrace(cp, 2, task_it, pi, 3);
           ++dcount;
         } else {
-          // ---- weight gradient: transpose through the staging tile, optimizer on the way out ----
+          // ---- weight gradient: transpose through the staging tile, optimizer (or the gradient store) on the way out ----
           const int64_t i0 = (int64_t)(p.C - grads) - (int64_t)p.member * ctx.P;  // flat offset of W_l in the member block
           const int ld = p.ldc, ncols = p.N;
           const MemberScalars* sc = ctx.scalars + p.member;
@@ -378,7 +406,7 @@ bwd_chain_kernel(const GemmProb* __restrict__ probs, const CUtensorMap* __restri
           const int n_units = wide ? 2 : (2 * n_chunks - ch + C_CGROUPS - 1) / C_CGROUPS;
           // the optimizer state this warp is about to stream does not depend on the accumulator: pull it into L2 while
           // the MMAs of the phase still run (one 128-byte line per lane = row, per array and unit)
-          if (!(cp.dbg & 4)) {
+          if (!GRADS_ONLY && !(cp.dbg & 4)) {
             for (int un = 0; un < n_units; ++un) {
               const int wu = ch + un * C_CGROUPS;
               const int c = wide ? wu : (wu >> 1);
@@ -415,7 +443,24 @@ bwd_chain_kernel(const GemmProb* __restrict__ probs, const CUtensorMap* __restri
                               __uint_as_float(r[4 * j + 3]));
             __syncwarp();
             const int col = c * 32 + lc;
-            if (col < ld) {
+            if (GRADS_ONLY && col < ld) {
+              // lane octet lr, row group i: row 4 i + lr of the half, 32 consecutive columns = one 128-byte line
+#pragma unroll 1
+              for (int half = h_lo; half < h_hi; ++half) {
+#pragma unroll
+                for (int i = 0; i < 4; ++i) {
+                  const int rl = half * 16 + 4 * i + lr;
+                  float4 g4 = *reinterpret_cast<const float4*>(&stg[rl * 36 + lc]);
+                  if (col + 3 >= ncols) {  // row padding of the input-layer weights: exact zeros
+                    if (col >= ncols) g4.x = 0.f;
+                    if (col + 1 >= ncols) g4.y = 0.f;
+                    if (col + 2 >= ncols) g4.z = 0.f;
+                    g4.w = 0.f;
+                  }
+                  *reinterpret_cast<float4*>(grads + mo + i0 + (int64_t)(row_base + rl) * ld + col) = g4;
+                }
+              }
+            } else if (!GRADS_ONLY && col < ld) {
               const int istep = 4 * ld;  // row group i is 4 rows further
 #pragma unroll 1
               for (int half = h_lo; half < h_hi; ++half) {
@@ -444,6 +489,7 @@ bwd_chain_kernel(const GemmProb* __restrict__ probs, const CUtensorMap* __restri
         }
       }
       if (tracer) ctrace(cp, 2, task_it, cp.n_phases, 0);
+      if (GRADS_ONLY) continue;
       // ---- small parameters of the task (biases, output layer, log_std): leader CTA, gradients from the grads arena;
       // the segments are laid end to end over the 512 threads so that all their loads are in flight together ----
       asm volatile("bar.sync 1, 512;" ::: "memory");
@@ -483,6 +529,7 @@ bwd_chain_kernel(const GemmProb* __restrict__ probs, const CUtensorMap* __restri
   __syncwarp();
   cluster_sync();
   if (warp == 1) asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
+  if (GRADS_ONLY) stamp_end(ctx.stamps, ST_CHAIN);
 }
 
 }  // namespace
@@ -521,12 +568,17 @@ int bwd_chain_wgrad0_tile_n(int k0) { return k0 <= 64 ? 64 : (k0 <= 128 ? 128 : 
 
 void launch_bwd_chain(const BwdChainArgs& a, const StepCtx& ctx, cudaStream_t st) {
   static bool attr[64] = {};
-  if (first_use_on_device(attr)) cudaFuncSetAttribute(bwd_chain_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, C_SMEM);
+  if (first_use_on_device(attr)) {
+    cudaFuncSetAttribute(bwd_chain_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, C_SMEM);
+    cudaFuncSetAttribute(bwd_chain_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, C_SMEM);
+  }
   ChainParams cp;
   memset(&cp, 0, sizeof(cp));
   cp.n_phases = a.n_phases;
   cp.n_tasks = a.n_tasks;
   cp.keep_grads = a.keep_grads;
+  cp.grads_only = a.grads_only;
+  cp.db_tile_order = a.db_tile_order;
   int dg = 0;
   for (int i = 0; i < a.n_phases; ++i) {
     ChainPhase& ph = cp.ph[i];
@@ -561,7 +613,7 @@ void launch_bwd_chain(const BwdChainArgs& a, const StepCtx& ctx, cudaStream_t st
     if (n_sm <= 0) n_sm = 148;
   }
   const int workers = a.n_tasks < n_sm / 2 ? a.n_tasks : n_sm / 2;
-  launch_pdl(bwd_chain_kernel, dim3(2 * workers), dim3(C_THREADS), C_SMEM, st, 2, a.probs, (const CUtensorMap*)a.maps,
+  launch_pdl(a.grads_only ? bwd_chain_kernel<true> : bwd_chain_kernel<false>, dim3(2 * workers), dim3(C_THREADS), C_SMEM, st, 2, a.probs, (const CUtensorMap*)a.maps,
              (const CUtensorMap*)a.cmaps, cp, ctx, a.params, a.exp_avg, a.exp_avg_sq, a.target, a.grads);
 }
 

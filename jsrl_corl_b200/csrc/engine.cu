@@ -24,6 +24,10 @@
 using namespace iql;
 
 static thread_local std::string g_create_error;
+// "auto" runs the chained backward (gradients only, IQL_OPT_STEP_PATH = 4) from this many members on with two hidden
+// layers, and from one member on with three or more (each extra layer is two more per-phase launches): measured
+// crossover against the per-phase backward on the B200 (profiles/r03_summary.md)
+static constexpr int CHAIN_GRADS_MIN_MEMBERS = 8;
 
 // Optional per-launch instrumentation of one update step (iql_profile_step).
 struct StepTimer {
@@ -106,7 +110,9 @@ struct iql_engine {
   std::vector<char> h_maps_store;
   // chained backward + optimizer (bwd_chain.cu): phase list, CTA-pair tensor maps, small-parameter ranges
   bool chain = false;
-  int step_path = 0;             // iql_set_option(IQL_OPT_STEP_PATH): 0 auto, 1 per-phase kernels, 2 chained backward (required)
+  bool chain_grads = false;      // the chain stores the weight gradients; adam_polyak_kernel runs after it
+  int step_path = 0;             // iql_set_option(IQL_OPT_STEP_PATH): 0 auto, 1 per-phase kernels, 2 chained backward +
+                                 // optimizer, 4 chained backward (gradients) + adam_polyak_kernel (2 and 4 required)
   int keep_grads = 0;            // iql_set_option(IQL_OPT_KEEP_GRADS): the chained backward also stores the weight gradients
   BwdChainArgs chain_args;
   char* d_maps_chain = nullptr;
@@ -383,7 +389,9 @@ extern "C" int iql_set_hparams(iql_engine* e, int32_t member, const iql_hparams*
 extern "C" int iql_set_option(iql_engine* e, int32_t key, int64_t value) {
   if (!e) return IQL_ERR_INVALID;
   if (key == IQL_OPT_STEP_PATH) {
-    if (value < 0 || value > 2) return fail(e, IQL_ERR_INVALID, "iql_set_option: IQL_OPT_STEP_PATH must be 0 (auto), 1 (per-phase kernels) or 2 (chained backward)");
+    if (value < 0 || value > 4 || value == 3)
+      return fail(e, IQL_ERR_INVALID, "iql_set_option: IQL_OPT_STEP_PATH must be 0 (auto), 1 (per-phase kernels), 2 (chained backward + "
+                                      "optimizer) or 4 (chained backward, optimizer in its own kernel)");
     if (e->bound && e->step_path != (int)value) return fail(e, IQL_ERR_STATE, "iql_set_option: IQL_OPT_STEP_PATH must be set before iql_bind_state");
     e->step_path = (int)value;
     return IQL_OK;
@@ -403,7 +411,8 @@ extern "C" int iql_get_info(const iql_engine* e, int32_t key, int64_t* out) {
   switch (key) {
     case IQL_INFO_TENSOR_CORE_PATH: *out = tc ? 1 : 0; return IQL_OK;   // 0: the FP32 CUDA-core kernels run this shape
     case IQL_INFO_FUSED_FORWARD: *out = e->bound && e->fused_fwd ? 1 : 0; return IQL_OK;
-    case IQL_INFO_CHAINED_BACKWARD: *out = e->bound && e->chain ? 1 : 0; return IQL_OK;
+    case IQL_INFO_CHAINED_BACKWARD: *out = e->bound && e->chain && !e->chain_grads ? 1 : 0; return IQL_OK;
+    case IQL_INFO_CHAINED_BACKWARD_GRADS: *out = e->bound && e->chain && e->chain_grads ? 1 : 0; return IQL_OK;
     default: return IQL_ERR_INVALID;
   }
 }
@@ -764,13 +773,17 @@ extern "C" int iql_bind_state(iql_engine* e, float* params, float* exp_avg, floa
     else
       e->h_maps_pol.clear();
   }
-  // ---- chained backward + optimizer: phase list and CTA-pair maps ----
-  e->chain = false;
+  // ---- chained backward: phase list and CTA-pair maps ----
+  e->chain = e->chain_grads = false;
   e->h_maps_chain.clear();
-  // opt-in (IQL_OPT_STEP_PATH = 2): measured on the 64-member ensemble the chained backward streams the optimizer state
-  // at 72 % of the HBM peak against 99 % for adam_polyak_kernel and ends up 10 % behind the per-phase kernels
-  // (DESIGN.md section 8); "auto" therefore keeps one kernel per phase
-  if (tc_mode && e->step_path == 2 && e->fw_splits == 1 &&
+  // IQL_OPT_STEP_PATH = 2 (opt-in): optimizer in the wgrad epilogue.  Measured on the 64-member ensemble it streams the
+  // optimizer state at 72 % of the HBM peak against 99 % for adam_polyak_kernel and ends up 10 % behind the per-phase
+  // kernels (DESIGN.md section 8).  IQL_OPT_STEP_PATH = 4: the chain computes the gradients only and adam_polyak_kernel
+  // follows.  "auto" takes 4 from CHAIN_GRADS_MIN_MEMBERS members on, or with 3+ hidden layers: below that the
+  // per-phase kernels' narrow dgrad units spread a two-layer step of few tasks over more SMs (DESIGN.md section 8).
+  const bool want_chain = e->step_path == 2 || e->step_path == 4 ||
+                          (e->step_path == 0 && (S >= CHAIN_GRADS_MIN_MEMBERS || e->cfg.n_hidden >= 3));
+  if (tc_mode && want_chain && e->fw_splits == 1 &&
       bwd_chain_supported(e->cfg.batch_size, e->cfg.hidden_dim, e->cfg.n_hidden, e->fused_fwd)) {
     const int L = e->cfg.n_hidden, ntask = 4 * S;
     BwdChainArgs& ca = e->chain_args;
@@ -791,6 +804,7 @@ extern "C" int iql_bind_state(iql_engine* e, float* params, float* exp_avg, floa
       const Phase& pw = e->bwd_phases[2 * (L - l)];      // dW_l = dZ_l^T H_l
       const Phase& px = e->bwd_phases[2 * (L - l) + 1];  // dZ_{l-1} = (dZ_l W_l) * [H_l > 0]
       if (!px.rowepi || px.mode != 1 || pw.mode != 2) { ok = false; break; }
+      ca.db_tile_order = px.cta2 ? 0 : 1;  // bias gradients summed as the per-phase dgrad of this shape sums them
       add_phase(0, px, 256, e->cfg.hidden_dim, L - 1 - l);
       add_phase(1, pw, 256, e->cfg.batch_size, L - 1 - l);
     }
@@ -819,9 +833,10 @@ extern "C" int iql_bind_state(iql_engine* e, float* params, float* exp_avg, floa
       }
     }
     e->chain = ok;
+    e->chain_grads = ok && e->step_path != 2;
     if (!ok) e->h_maps_chain.clear();
   }
-  if (e->step_path == 2 && !e->chain)
+  if ((e->step_path == 2 || e->step_path == 4) && !e->chain)
     return fail(e, IQL_ERR_INVALID, "iql_bind_state: IQL_OPT_STEP_PATH = chained backward, but this shape / math mode does not support it "
                                     "(needs tf32, hidden 256, batch 256, 2..4 hidden layers)");
   if (!e->side) {  // optional: without it the backward simply stays on one stream
@@ -964,6 +979,35 @@ extern "C" int iql_load_batch(iql_engine* e, int32_t member, const float* states
   CUDA_TRY(e, cudaGetLastError());
   e->preloaded[member] = 1;
   return IQL_OK;
+}
+
+// The chained backward (bwd_chain.cu) after the output-layer backward: hidden dgrad / wgrad chain and input-layer wgrad,
+// plus Adam + Polyak in the wgrad epilogues unless the engine runs it gradient-only.  With `tm`, the work of the launch
+// goes to the timer's last slot.
+static void launch_chain(iql_engine* e, const StepCtx& ctx, cudaStream_t st, StepTimer* tm) {
+  if (tm) {  // operands read once; dZ written; the weight gradients written (gradient-only) or the optimizer state streamed
+    double fl = 0, by = 0;
+    for (size_t i = 2; i < e->bwd_phases.size(); ++i) {
+      const Phase& q = e->bwd_phases[i];
+      for (int j = 0; j < q.count; ++j) {
+        const GemmProb& g = e->h_probs[q.first + j];
+        fl += 2.0 * g.M * g.N * g.K;
+        by += 4.0 * ((double)g.M * g.K + (double)g.N * g.K + (q.mode == 1 || e->chain_grads ? (double)g.M * g.N : 0.0));
+      }
+    }
+    if (!e->chain_grads)  // p, m, v in and out + shadows
+      by += e->cfg.n_members * 4.0 * ((6.0 + 1.0) * e->layout.param_floats + 3.0 * e->layout.q_floats);
+    tm->flops.back() = fl;
+    tm->bytes.back() = by;
+  }
+  BwdChainArgs ca = e->chain_args;
+  ca.probs = e->d_probs;
+  ca.maps = e->d_maps_chain;
+  ca.cmaps = e->d_maps_c;
+  ca.keep_grads = e->keep_grads;
+  ca.grads_only = e->chain_grads ? 1 : 0;
+  ca.params = e->params; ca.exp_avg = e->exp_avg; ca.exp_avg_sq = e->exp_avg_sq; ca.target = e->target; ca.grads = e->grads;
+  launch_bwd_chain(ca, ctx, st);
 }
 
 // one update step for all members; returns number of launches
@@ -1162,7 +1206,7 @@ static int enqueue_step(iql_engine* e, StepCtx& ctx, bool gather, cudaStream_t s
   const bool two_streams = tf32 && !tm && !no_side && e->side != nullptr;
   int forks = 0;
   // chained backward: the output-layer backward (phases 0, 1) runs as before, everything after it -- hidden dgrad /
-  // wgrad chain, input-layer wgrad, Adam + Polyak -- is ONE launch on CTA pairs
+  // wgrad chain, input-layer wgrad (+ Adam + Polyak unless gradient-only) -- is ONE launch on CTA pairs
   const bool chain = e->chain && tf32 && last_ok && e->bwd_phases.size() >= 3 && e->bwd_phases[0].kind == PH_LAST_WGRAD &&
                      e->bwd_phases[1].kind == PH_LAST_DGRAD;
   for (size_t i = 0; i < e->bwd_phases.size(); ++i) {
@@ -1195,6 +1239,13 @@ static int enqueue_step(iql_engine* e, StepCtx& ctx, bool gather, cudaStream_t s
       run_phase(ph, n1, n2);
     }
   }
+  // chained backward (gradients only): the chain reads nothing the side stream writes (loss kernel: logged losses,
+  // log_std gradient, Adam scalars; row-split reduction: dW_L, db_L), so it starts right after the output-layer backward
+  if (chain && e->chain_grads) {
+    if (tm) tm->mark("bwd_chain_grads", 0, 0);
+    launch_chain(e, ctx, st, tm);
+    ++launches;
+  }
   if (forks > 0 || loss_on_side || lb_on_side) cudaStreamWaitEvent(st_main, e->ev_side, 0);  // join before the optimizer
   // Adam: read g, p, m, v + target; write p, m, v + target (+ the TF32 shadow copies in tcgen05 mode)
   if (tm) {
@@ -1216,9 +1267,9 @@ static int enqueue_step(iql_engine* e, StepCtx& ctx, bool gather, cudaStream_t s
     }
     tm->mark("adam_polyak", 0, S_d * 4.0 * (7.0 * e->layout.param_floats + 2.0 * e->layout.q_floats + shadow_p + shadow_t));
   }
-  // (chained backward: its input-layer weight-gradient phase still reads the gathered rows, so the next step's gather
-  // cannot run beside it; the caller then gathers at the top of every step)
-  const bool fork_gather = gather_next && !tm && e->side != nullptr && !chain;
+  // (chained backward + optimizer: its input-layer weight-gradient phase still reads the gathered rows, so the next
+  // step's gather cannot run beside it; the caller then gathers at the top of every step)
+  const bool fork_gather = gather_next && !tm && e->side != nullptr && !(chain && !e->chain_grads);
   if (fork_gather) {
     StepCtx next = ctx;
     next.k = ctx.k + 1;
@@ -1229,29 +1280,9 @@ static int enqueue_step(iql_engine* e, StepCtx& ctx, bool gather, cudaStream_t s
     ++launches;
   }
   ctx.unbias_out = (ctx.k == ctx.K - 1) ? 1 : 0;  // the call's last optimizer launch leaves plain fp32 in the arenas
-  if (chain) {
-    if (tm) {
-      double fl = 0, by = 0;
-      for (size_t i = 2; i < e->bwd_phases.size(); ++i) {
-        const Phase& q = e->bwd_phases[i];
-        for (int j = 0; j < q.count; ++j) {
-          const GemmProb& g = e->h_probs[q.first + j];
-          fl += 2.0 * g.M * g.N * g.K;
-          by += 4.0 * ((double)g.M * g.K + (double)g.N * g.K + (q.mode == 1 ? (double)g.M * g.N : 0.0));
-        }
-      }
-      by += S_d * 4.0 * ((6.0 + 1.0) * e->layout.param_floats + 3.0 * e->layout.q_floats);  // p, m, v in and out + shadows
-      tm->label.back() = "bwd_chain";
-      tm->flops.back() = fl;
-      tm->bytes.back() = by;
-    }
-    BwdChainArgs ca = e->chain_args;
-    ca.probs = e->d_probs;
-    ca.maps = e->d_maps_chain;
-    ca.cmaps = e->d_maps_c;
-    ca.keep_grads = e->keep_grads;
-    ca.params = e->params; ca.exp_avg = e->exp_avg; ca.exp_avg_sq = e->exp_avg_sq; ca.target = e->target; ca.grads = e->grads;
-    launch_bwd_chain(ca, ctx, st);
+  if (chain && !e->chain_grads) {
+    if (tm) tm->label.back() = "bwd_chain";
+    launch_chain(e, ctx, st, tm);
   } else {
     launch_adam(ctx, e->params, e->exp_avg, e->exp_avg_sq, e->target, e->grads, st);
     if (ctx.advance_k > 0) ctx.advance_k = -1;  // consumed: the optimizer launch advanced the counters
@@ -1295,8 +1326,8 @@ extern "C" int iql_train_steps(iql_engine* e, int32_t k_steps, int32_t sample_mo
   ctx.idx_out = idx_out;
   const bool gather = sample_mode != IQL_SAMPLE_PRELOADED;
   static const bool no_overlap_gather = dbg_getenv("IQL_B200_NO_GATHER_AHEAD") != nullptr || dbg_getenv("IQL_B200_NO_SIDE_STREAM") != nullptr;
-  // (not with the chained backward: its last phase still reads the gathered rows, see enqueue_step)
-  const bool overlap_gather = !no_overlap_gather && e->side != nullptr && st != nullptr && !e->chain;
+  // (not with the chained backward + optimizer: its last phase still reads the gathered rows, see enqueue_step)
+  const bool overlap_gather = !no_overlap_gather && e->side != nullptr && st != nullptr && !(e->chain && !e->chain_grads);
   // the legacy default stream cannot be captured; the facade runs the engine on its own stream
   // Graphs: the K-step Philox loop, and the single preloaded step of the drop-in `train(batch)` path (its ~11
   // launches would otherwise be launch-latency bound).  Keyed by K, negative for the preloaded variant.

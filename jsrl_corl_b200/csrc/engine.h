@@ -149,7 +149,7 @@ struct WorkspaceLayout {
 
 // launch slots of the step timeline (tools/step_trace.py)
 enum StampSlot : int { ST_REFRESH = 0, ST_GATHER, ST_FWD, ST_POLHEAD, ST_LOSS, ST_LASTBWD, ST_LBREDUCE, ST_WGRAD, ST_DGRAD, ST_FWGRAD, ST_ADAM,
-                       ST_ADVANCE, ST_COUNT };
+                       ST_ADVANCE, ST_CHAIN, ST_COUNT };
 
 // forward pass ids
 enum Pass : int { PASS_V_NEXT = 0, PASS_V = 1, PASS_TQ1 = 2, PASS_TQ2 = 3, PASS_Q1 = 4, PASS_Q2 = 5, PASS_PI = 6, N_PASS = 7 };

@@ -51,12 +51,15 @@ void launch_fused_fwd(const FusedFwdArgs& a, const StepCtx& ctx, cudaStream_t st
 // Chained backward + optimizer (bwd_chain.cu): one CTA pair per (member, trainable net) runs the hidden-layer dgrad /
 // wgrad phases back to back and applies Adam + Polyak in the wgrad epilogues.  Hidden width 256, batch 256,
 // 2..FUSED_MAX_LAYERS hidden layers, fused forward on (it writes the ReLU sign bits the dgrad phases mask with).
+// grads_only: the wgrad epilogues store the weight gradients to the grads arena instead and the optimizer runs as
+// adam_polyak_kernel after the launch.
 struct BwdChainArgs {
   const GemmProb* probs;  // the engine's device problem table (base)
   const void* maps;       // chain tensor maps, CTA-pair boxes: per phase 2 per task (A, B)
   const void* cmaps;      // store maps of the backward outputs, indexed by absolute problem index
-  int n_phases, n_tasks, keep_grads;
-  int kind[2 * FUSED_MAX_LAYERS];         // 0 dgrad, 1 wgrad + optimizer
+  int n_phases, n_tasks, keep_grads, grads_only;
+  int db_tile_order;  // grads_only: bias-gradient summation order of the single-CTA dgrad (the per-phase dgrad is not on CTA pairs)
+  int kind[2 * FUSED_MAX_LAYERS];         // 0 dgrad, 1 wgrad (+ optimizer unless grads_only)
   int prob_first[2 * FUSED_MAX_LAYERS];   // first problem of the phase (task i uses prob_first + i)
   int map_first[2 * FUSED_MAX_LAYERS];    // first map of the phase inside `maps` (in maps)
   int tile_n[2 * FUSED_MAX_LAYERS], k[2 * FUSED_MAX_LAYERS], wait_dgrads[2 * FUSED_MAX_LAYERS];

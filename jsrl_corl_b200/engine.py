@@ -100,7 +100,8 @@ class EnsembleEngine:
         # FP32 CUDA-core kernels -- reported here, and refused when the caller insists on tensor cores
         self.paths = {"tensor_cores": bool(self.info(_lib.INFO_TENSOR_CORE_PATH)),
                       "fused_forward": bool(self.info(_lib.INFO_FUSED_FORWARD)),
-                      "chained_backward": bool(self.info(_lib.INFO_CHAINED_BACKWARD))}
+                      "chained_backward": bool(self.info(_lib.INFO_CHAINED_BACKWARD)),
+                      "chained_backward_grads": bool(self.info(_lib.INFO_CHAINED_BACKWARD_GRADS))}
         if math_mode == "tf32" and strict_tf32 and not self.paths["tensor_cores"]:
             raise ValueError(f"math_mode='tf32' with strict_tf32: batch {batch_size} / hidden {hidden_dim} is outside the tcgen05 "
                              "kernels (batch % 128 == 0 and hidden % 256 == 0 required); the FP32 kernels would run")

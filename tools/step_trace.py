@@ -17,7 +17,7 @@ from jsrl_corl_b200 import IQLEnsemble, ReplayBuffer, _lib
 from jsrl_corl_b200.synthetic import synthetic_dataset
 
 SLOTS = ["refresh", "gather", "fused_fwd", "policy_head", "loss", "last_bwd", "lb_reduce", "hidden_wgrad", "hidden_dgrad", "first_wgrad",
-         "adam_polyak", "advance"]
+         "adam_polyak", "advance", "bwd_chain"]
 
 
 def main():
