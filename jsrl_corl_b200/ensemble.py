@@ -153,7 +153,11 @@ class IQLEnsemble:
     def load_member_state_dict(self, m: int, sd: Dict[str, Any]):
         """Inverse of ``member_state_dict``; also accepts checkpoints written by
         the reference.  As in the reference (iql.py:584) the target network is
-        re-cloned from qf."""
+        re-cloned from qf.  The Adam betas and eps come from the optimizer groups,
+        which the engine requires to agree (one set per member)."""
+        groups = [sd[key]["param_groups"][0] for key in ("q_optimizer", "v_optimizer", "actor_optimizer")]
+        if any(tuple(g["betas"]) != tuple(groups[0]["betas"]) or g["eps"] != groups[0]["eps"] for g in groups[1:]):
+            raise NotImplementedError("the three Adam optimizers must share betas and eps")
         e = self.engine
         drop = self.actor_dropout > 0.0
         e.load_params(m, {"qf": sd["qf"], "vf": sd["vf"], "actor": sd["actor"]}, dropout_keys=drop, sync_target=True)
@@ -173,7 +177,8 @@ class IQLEnsemble:
                     m2[grp][n].zero_()
             steps[grp] = step
         sched = sd.get("actor_lr_schedule") or {}
-        kw = dict(qf_lr=sd["q_optimizer"]["param_groups"][0]["lr"], vf_lr=sd["v_optimizer"]["param_groups"][0]["lr"])
+        kw = dict(qf_lr=groups[0]["lr"], vf_lr=groups[1]["lr"], adam_beta1=float(groups[0]["betas"][0]),
+                  adam_beta2=float(groups[0]["betas"][1]), adam_eps=float(groups[0]["eps"]))
         if sched:
             kw.update(actor_lr=sched["base_lrs"][0], cosine_t_max=int(sched["T_max"]), lr_eta_min=float(sched["eta_min"]))
         else:

@@ -58,6 +58,7 @@ class OracleConfig:
     max_steps: Optional[int] = 1000000  # CosineAnnealingLR T_max; None = no schedule
     adam_betas: tuple = (0.9, 0.999)
     adam_eps: float = 1e-8
+    lr_eta_min: float = 0.0  # CosineAnnealingLR eta_min
 
 
 def mlp_layer_names(n_hidden: int, dropout: bool) -> List[int]:
@@ -96,7 +97,10 @@ class _Adam:
             g = grads[k].astype(dt, copy=False)
             m = self.exp_avg[k]
             v = self.exp_avg_sq[k]
-            m += w1 * (g - m)  # lerp_
+            if self.beta1 > 0.5:  # lerp_: torch evaluates weights >= 0.5 from the end point (exact g at beta1 = 0)
+                m += w1 * (g - m)
+            else:
+                m[...] = g - (g - m) * (dt(1) - w1)
             v *= dt(self.beta2)
             v += dt(1 - self.beta2) * g * g  # addcmul_
             denom = np.sqrt(v) / dt(bc2_sqrt) + dt(self.eps)
@@ -238,9 +242,9 @@ class NumpyIQL:
         for k in self.q_target:  # soft_update iql.py:72-74: (1-tau)*t + tau*s
             self.q_target[k] = dt(1 - tau) * self.q_target[k] + dt(tau) * self.qf[k]
         self.a_opt.step(a_grads)
-        if cfg.max_steps is not None:  # CosineAnnealingLR.step(), recursive form, eta_min = 0
+        if cfg.max_steps is not None:  # CosineAnnealingLR.step(), recursive form
             self.sched_epoch += 1
-            self.a_opt.lr = cosine_recursive_lr(self.a_opt.lr, cfg.actor_lr, self.sched_epoch, cfg.max_steps)
+            self.a_opt.lr = cosine_recursive_lr(self.a_opt.lr, cfg.actor_lr, self.sched_epoch, cfg.max_steps, cfg.lr_eta_min)
         return {"value_loss": float(v_loss), "q_loss": float(q_loss), "actor_loss": float(actor_loss)}
 
     def state(self) -> Dict[str, Dict[str, np.ndarray]]:

@@ -84,6 +84,30 @@ class Golden:
                             m["discount"], m["tau"], m["lr"], m["lr"], m["lr"], m["max_steps"])
 
 
+def oracle_from_state(cfg, tree, moments=None, steps=None, sched_epoch=0, total_it=0, actor_lr=None, dtype=np.float32):
+    """A NumpyIQL that continues a learner from a given state rather than from its initial one.
+
+    tree: {"qf", "vf", "actor"[, "q_target"]} weights; moments: {grp: {name: (exp_avg, exp_avg_sq)}}; steps: Adam step
+    counts {"qf", "vf", "actor"}; sched_epoch: CosineAnnealingLR.last_epoch.  The current actor lr is the closed form of
+    the schedule at that epoch unless `actor_lr` is given (e.g. the value a reference run stored)."""
+    from oracle.iql_numpy import NumpyIQL, cosine_closed_form_lr
+
+    orc = NumpyIQL(cfg, tree, dtype)
+    steps = steps or {}
+    for grp, o in (("qf", orc.q_opt), ("vf", orc.v_opt), ("actor", orc.a_opt)):
+        o.step_count = int(steps.get(grp, 0))
+        for name, (m, v) in (moments or {}).get(grp, {}).items():
+            o.exp_avg[name][...] = m
+            o.exp_avg_sq[name][...] = v
+    orc.sched_epoch = int(sched_epoch)
+    if actor_lr is not None:
+        orc.a_opt.lr = float(actor_lr)
+    elif cfg.max_steps is not None:
+        orc.a_opt.lr = cosine_closed_form_lr(cfg.actor_lr, orc.sched_epoch, cfg.max_steps, cfg.lr_eta_min)
+    orc.total_it = int(total_it)
+    return orc
+
+
 def batch_from(data, idx):
     return [data["observations"][idx], data["actions"][idx], data["rewards"][idx][:, None],
             data["next_observations"][idx], data["terminals"][idx].astype(np.float32)[:, None]]
@@ -144,17 +168,6 @@ class LateSnapshot(Golden):
         return out
 
     def load_into_oracle(self, dtype=np.float32):
-        from oracle.iql_numpy import NumpyIQL
-
-        tree = self.tree(self.pre)
-        orc = NumpyIQL(self.oracle_config(), tree, dtype)
-        opt = self.opt(self.pre)
-        for grp, o in (("qf", orc.q_opt), ("vf", orc.v_opt), ("actor", orc.a_opt)):
-            o.step_count = self.at
-            for name, (m, v) in opt[grp].items():
-                o.exp_avg[name][...] = m
-                o.exp_avg_sq[name][...] = v
-        orc.sched_epoch = int(self.z[f"{self.pre}/sched_epoch"])
-        orc.a_opt.lr = float(self.z[f"{self.pre}/actor_lr"])
-        orc.total_it = self.at
-        return orc
+        return oracle_from_state(self.oracle_config(), self.tree(self.pre), self.opt(self.pre),
+                                 {"qf": self.at, "vf": self.at, "actor": self.at}, int(self.z[f"{self.pre}/sched_epoch"]),
+                                 self.at, actor_lr=float(self.z[f"{self.pre}/actor_lr"]), dtype=dtype)

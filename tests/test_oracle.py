@@ -97,6 +97,68 @@ def test_oracle_against_live_reference():
             assert abs(lr[k] - lo[k]) <= 2e-5 * abs(lr[k]) + 1e-8
 
 
+@pytest.mark.parametrize("betas,eps", [((0.8, 0.99), 1e-8), ((0.0, 0.999), 1e-8), ((0.9, 0.999), 1e-6)])
+def test_oracle_adam_non_default_settings_match_torch(betas, eps):
+    """The oracle's Adam with betas / eps other than torch's defaults (ensemble members may each have their own)
+    against torch.optim.Adam (single-tensor path), float64, 20 steps with fixed per-step gradients."""
+    import torch
+    from oracle.iql_numpy import _Adam
+
+    rng = np.random.RandomState(4)
+    shapes = {"w": (5, 3), "b": (5,)}
+    init = {k: rng.standard_normal(s) for k, s in shapes.items()}
+    grads = [{k: rng.standard_normal(s) * 10.0 ** rng.uniform(-4, 1) for k, s in shapes.items()} for _ in range(20)]
+    params = {k: v.copy() for k, v in init.items()}
+    orc = _Adam(params, 1e-3, betas, eps, np.float64)
+    tp = {k: torch.tensor(v, dtype=torch.float64, requires_grad=True) for k, v in init.items()}
+    opt = torch.optim.Adam(list(tp.values()), lr=1e-3, betas=betas, eps=eps, foreach=False)
+    for g in grads:
+        orc.step(g)
+        for k, t in tp.items():
+            t.grad = torch.from_numpy(g[k])
+        opt.step()
+        for k, t in tp.items():
+            st = opt.state[t]
+            np.testing.assert_allclose(params[k], t.detach().numpy(), rtol=1e-12, atol=0)
+            np.testing.assert_allclose(orc.exp_avg[k], st["exp_avg"].numpy(), rtol=1e-12, atol=0)
+            np.testing.assert_allclose(orc.exp_avg_sq[k], st["exp_avg_sq"].numpy(), rtol=1e-12, atol=0)
+    assert orc.step_count == 20
+
+
+def test_oracle_cosine_schedule_with_eta_min_matches_torch():
+    """CosineAnnealingLR(T_max=3, eta_min=1e-5) over 10 epochs (past T_max twice, through the recursive form's
+    special branch) against the oracle's recursive form, standalone and as NumpyIQL applies it after each step."""
+    import torch
+    from oracle.iql_numpy import OracleConfig, cosine_recursive_lr
+
+    base, t_max, eta_min = 3e-4, 3, 1e-5
+    p = torch.zeros(1, dtype=torch.float64, requires_grad=True)
+    opt = torch.optim.Adam([p], lr=base)
+    sched = torch.optim.lr_scheduler.CosineAnnealingLR(opt, T_max=t_max, eta_min=eta_min)
+    S, A, H, L, B = 3, 2, 8, 2, 4
+    rng = np.random.RandomState(0)
+    init = {
+        "qf": {f"q{i}.net.{j}.{w}": rng.standard_normal(s) * 0.3 for i in (1, 2) for j, s_w, s_b in
+               ((0, (H, S + A), (H,)), (2, (H, H), (H,)), (4, (1, H), (1,))) for w, s in (("weight", s_w), ("bias", s_b))},
+        "vf": {f"v.net.{j}.{w}": rng.standard_normal(s) * 0.3 for j, s_w, s_b in
+               ((0, (H, S), (H,)), (2, (H, H), (H,)), (4, (1, H), (1,))) for w, s in (("weight", s_w), ("bias", s_b))},
+        "actor": {"log_std": np.zeros(A), **{f"net.net.{j}.{w}": rng.standard_normal(s) * 0.3 for j, s_w, s_b in
+                  ((0, (H, S), (H,)), (2, (H, H), (H,)), (4, (A, H), (A,))) for w, s in (("weight", s_w), ("bias", s_b))}},
+    }
+    orc = NumpyIQL(OracleConfig(S, A, H, L, actor_lr=base, max_steps=t_max, lr_eta_min=eta_min), init, np.float64)
+    lr = base
+    for epoch in range(1, 11):
+        opt.step()
+        sched.step()
+        lr = cosine_recursive_lr(lr, base, epoch, t_max, eta_min)
+        want = opt.param_groups[0]["lr"]
+        assert abs(lr - want) <= 1e-12 * abs(want), (epoch, lr, want)
+        batch = [rng.standard_normal((B, S)), rng.uniform(-1, 1, (B, A)), rng.standard_normal((B, 1)),
+                 rng.standard_normal((B, S)), np.zeros((B, 1))]
+        orc.train(batch)
+        assert orc.sched_epoch == epoch and abs(orc.a_opt.lr - want) <= 1e-12 * abs(want), (epoch, orc.a_opt.lr, want)
+
+
 @pytest.mark.parametrize("name", ["hopper_late_999", "antmaze_late_999"])
 def test_oracle_one_step_from_late_reference_snapshot(name):
     """Late-trajectory regime (Adam step 1000, bias corrections ~ 1, cosine LR ~ 0, saturated exp(beta adv) clamp for
