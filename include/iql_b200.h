@@ -254,6 +254,39 @@ int iql_act_host(iql_engine* e, int32_t member, const float* host_state, float m
  * mean + std * N(0, 1) on the host and clamps max_action * sample.  Same launch / mailbox as iql_act_host. */
 int iql_act_host_gaussian(iql_engine* e, int32_t member, const float* host_state, float* host_mean, float* host_std,
                           void* stream, void* caller_stream);
+
+/* ---- the online phase of an ensemble (one env step of S members at once) ---------------------------------------- */
+/* Per-member action source of iql_act_host_members */
+#define IQL_ACT_SKIP 0         /* the member gets nothing; its rows of host_out / host_std are left untouched          */
+#define IQL_ACT_LEARNER 1      /* eval-mode action of the member's learner: clamp(max_action * tanh(MLP(s)))          */
+#define IQL_ACT_LEARNER_DIST 2 /* Gaussian learner: mean = tanh(MLP(s)) (unscaled) and std = exp(clamp(log_std, -20, 2)) */
+#define IQL_ACT_GUIDE 3        /* eval-mode action of the member's guide (the arena bound by iql_bind_guide)          */
+/* Bind a second [S][param_floats] parameter arena with this handle's layout as the members' guides (JSRL's guide
+ * policy: in practice the frozen offline ensemble's parameter arena, zero-copy).  The engine only reads it.  NULL
+ * unbinds.  16-byte aligned device memory. */
+int iql_bind_guide(iql_engine* e, const float* guide_params);
+/* replaces: GaussianPolicy.act / DeterministicPolicy.act (iql.py:371-379, 403-413) behind jsrl_utils.learner_or_guide_action
+ * (jsrl_utils.py:547-622), for every member of the ensemble in ONE launch: host_states [S][state_dim], host_source [S]
+ * IQL_ACT_* codes.  host_out [S][action_dim] receives the action (or the mean of IQL_ACT_LEARNER_DIST), host_std
+ * [S][action_dim] the std of IQL_ACT_LEARNER_DIST members (may be NULL when no member asks for it).  Skipped members
+ * cost no CTA.  Every active member's result is bit-identical to iql_act_host / iql_act_host_gaussian on the same
+ * weights.  Observations travel through an engine-owned pinned, device-mapped block (no state_dim limit), results
+ * come back through pinned memory with one flag word per member: no copies, no stream synchronisation.  Launched on
+ * `caller_stream`, ordered behind the host steps like iql_act_host.  Refused (IQL_ERR_INVALID): a guide code with no
+ * guide bound, the distribution code on a deterministic policy, unknown codes. */
+int iql_act_host_members(iql_engine* e, const float* host_states, const int8_t* host_source, float max_action,
+                         float* host_out, float* host_std, void* stream, void* caller_stream);
+/* replaces: ReplayBuffer.add_transition (iql.py:180-196) for every member in ONE launch: member m's transition
+ * (host_states [S][state_dim], host_actions [S][action_dim], host_rewards [S], host_next_states [S][state_dim],
+ * host_dones [S], all host memory) is packed in the iql_row_layout layout, padding zeroed, and written at row
+ * host_pointers[m] of the rows bound to member m by iql_bind_replay; host_pointers[m] == -1: no insert for m.
+ * The packed rows travel through an engine-owned pinned, device-mapped block (any row width): two slots used in
+ * turn, each reused only once the kernel has marked it consumed, so the call returns without waiting for the launch
+ * and the caller may reuse its arrays at once.  Launched on `caller_stream`.  Refused (IQL_ERR_INVALID): a pointer
+ * outside [0, capacity), an inserting member with no binding, two inserting members bound to the same rows. */
+int iql_replay_insert_members_host(iql_engine* e, const float* host_states, const float* host_actions,
+                                   const float* host_rewards, const float* host_next_states, const float* host_dones,
+                                   const int64_t* host_pointers, void* stream, void* caller_stream);
 /* Self-test hook for the tcgen05 TF32 GEMM building block (no reference
  * counterpart): C[M,N] = op(A) op(B), mode 0 NT (A[M,K], B[N,K]), 1 NN (A[M,K],
  * B[K,N]), 2 TN (A[K,M], B[K,N]); M multiple of 256, N <= 256 or a multiple of

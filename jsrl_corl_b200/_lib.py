@@ -23,6 +23,8 @@ KIND_WEIGHT, KIND_BIAS, KIND_LOG_STD = 0, 1, 2
 OPT_STEP_PATH, OPT_KEEP_GRADS = 1, 2
 INFO_TENSOR_CORE_PATH, INFO_FUSED_FORWARD, INFO_CHAINED_BACKWARD, INFO_CHAINED_BACKWARD_GRADS = 1, 2, 3, 4
 STEP_PATHS = {"auto": 0, "phases": 1, "chain": 2, "chain_grads": 4}
+ACT_SKIP, ACT_LEARNER, ACT_LEARNER_DIST, ACT_GUIDE = 0, 1, 2, 3
+ACT_SOURCES = {"skip": ACT_SKIP, "learner": ACT_LEARNER, "learner_dist": ACT_LEARNER_DIST, "guide": ACT_GUIDE}
 
 
 class Config(C.Structure):
@@ -113,6 +115,9 @@ SYMBOLS = {
     "iql_act": (C.c_int, [_P, C.c_int32, _P, C.c_int64, C.c_float, _P, _P]),
     "iql_act_host": (C.c_int, [_P, C.c_int32, _P, C.c_float, _P, _P, _P]),
     "iql_act_host_gaussian": (C.c_int, [_P, C.c_int32, _P, _P, _P, _P, _P]),
+    "iql_bind_guide": (C.c_int, [_P, _P]),
+    "iql_act_host_members": (C.c_int, [_P, _P, _P, C.c_float, _P, _P, _P, _P]),
+    "iql_replay_insert_members_host": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "iql_last_launch_count": (C.c_int64, [_P]),
     "iql_debug_fused_trace": (C.c_int, [_P, C.c_int32]),
     "iql_debug_chain_trace": (C.c_int, [_P, C.c_int32]),

@@ -155,6 +155,13 @@ struct iql_engine {
   cudaStream_t host_step_stream = nullptr;  // the caller's stream the last host step was launched on
   bool host_step_stream_set = false;
   cudaEvent_t ev_in = nullptr, ev_out = nullptr;
+  // online phase of an ensemble (iql_act_host_members / iql_replay_insert_members_host)
+  const float* guide = nullptr;  // [S][P] guide parameter arena (iql_bind_guide), read only
+  char* h_actm = nullptr;        // pinned, device-mapped: states [S][state_dim] | ids [S] | codes [S] | results [S][2A] | flags [S]
+  char* h_ins = nullptr;         // pinned, device-mapped: 2 slots of rows [S][RF] | ids [S] | pointers [S] | consumed [S]
+  int ins_slot = 0;              // slot the next insert call fills
+  int ins_n[2] = {0, 0};         // rows launched from each slot (their consumed words are awaited before the slot is refilled)
+  cudaStream_t ins_stream[2] = {nullptr, nullptr};
 };
 
 static int fail(iql_engine* e, int code, const std::string& msg) {
@@ -343,6 +350,8 @@ extern "C" void iql_destroy(iql_engine* e) {
   if (e->ev_out) cudaEventDestroy(e->ev_out);
   if (e->h_mail) cudaFreeHost(e->h_mail);
   if (e->h_act) cudaFreeHost(e->h_act);
+  if (e->h_actm) cudaFreeHost(e->h_actm);
+  if (e->h_ins) cudaFreeHost(e->h_ins);  // synchronises with the device: no insert launch still reads the slots
   if (e->d_stamps) cudaFree(e->d_stamps);
   delete e;
 }
@@ -1642,6 +1651,173 @@ static int act_host_impl(iql_engine* e, int32_t member, const float* host_state,
   for (int i = 0; i < A; ++i) host_action[i] = reinterpret_cast<volatile float*>(e->h_act)[i];
   if (host_std)
     for (int i = 0; i < A; ++i) host_std[i] = reinterpret_cast<volatile float*>(e->h_act)[A + i];
+  return IQL_OK;
+}
+
+// ---------------------------------------------------------------------------
+// Online phase of an ensemble: one act launch and one ring-insert launch per env step for all members
+// ---------------------------------------------------------------------------
+static size_t align16(size_t n) { return (n + 15) & ~(size_t)15; }
+
+// the caller's stream waits for the stream of the last host step when the two differ (as in act_host_impl)
+static int order_behind_host_step(iql_engine* e, cudaStream_t cur) {
+  if (e->host_step_stream_set && e->host_step_stream != cur) {
+    CUDA_TRY(e, cudaEventRecord(e->ev_in, e->host_step_stream));
+    CUDA_TRY(e, cudaStreamWaitEvent(cur, e->ev_in, 0));
+  }
+  return IQL_OK;
+}
+
+extern "C" int iql_bind_guide(iql_engine* e, const float* guide_params) {
+  if (!e) return IQL_ERR_INVALID;
+  if ((uintptr_t)guide_params & 15) return fail(e, IQL_ERR_INVALID, "iql_bind_guide: the guide arena must be 16-byte aligned");
+  e->guide = guide_params;
+  return IQL_OK;
+}
+
+extern "C" int iql_act_host_members(iql_engine* e, const float* host_states, const int8_t* host_source, float max_action,
+                                    float* host_out, float* host_std, void* stream, void* caller_stream) {
+  if (!e) return IQL_ERR_INVALID;
+  if (!host_states || !host_source || !host_out) return fail(e, IQL_ERR_INVALID, "iql_act_host_members: null states, sources or output");
+  if (!e->bound) return fail(e, IQL_ERR_STATE, "iql_act_host_members: state not bound");
+  const int S = e->cfg.n_members, Sd = e->cfg.state_dim, A = e->cfg.action_dim, L = e->cfg.n_hidden;
+  int n = 0;
+  for (int m = 0; m < S; ++m) {
+    const int c = host_source[m];
+    if (c < IQL_ACT_SKIP || c > IQL_ACT_GUIDE) return fail(e, IQL_ERR_INVALID, "iql_act_host_members: unknown source code " + std::to_string(c));
+    if (c == IQL_ACT_GUIDE && !e->guide) return fail(e, IQL_ERR_INVALID, "iql_act_host_members: a member asks for its guide, but no guide is bound (iql_bind_guide)");
+    if (c == IQL_ACT_LEARNER_DIST && e->cfg.deterministic)
+      return fail(e, IQL_ERR_INVALID, "iql_act_host_members: the distribution code needs a Gaussian policy; this one is deterministic");
+    if (c == IQL_ACT_LEARNER_DIST && !host_std) return fail(e, IQL_ERR_INVALID, "iql_act_host_members: null std with distribution members");
+    n += c != IQL_ACT_SKIP;
+  }
+  if (n == 0) return IQL_OK;
+  const size_t off_ids = align16(sizeof(float) * (size_t)S * Sd), off_codes = off_ids + align16(sizeof(int32_t) * S);
+  const size_t off_mail = off_codes + align16(sizeof(int32_t) * S), off_flags = off_mail + align16(sizeof(float) * (size_t)S * 2 * A);
+  if (!e->h_actm) {
+    if (!host_events(e) || cudaHostAlloc((void**)&e->h_actm, off_flags + sizeof(uint32_t) * S, cudaHostAllocMapped) != cudaSuccess) {
+      cudaGetLastError();
+      e->h_actm = nullptr;
+      return fail(e, IQL_ERR_CUDA, "iql_act_host_members: pinned block / event allocation failed");
+    }
+  }
+  float* states = (float*)e->h_actm;
+  int32_t* ids = (int32_t*)(e->h_actm + off_ids);
+  int32_t* codes = (int32_t*)(e->h_actm + off_codes);
+  float* mail = (float*)(e->h_actm + off_mail);
+  volatile uint32_t* flags = (volatile uint32_t*)(e->h_actm + off_flags);
+  // the previous call returned only after every flag of its launch was raised: the block is free to refill
+  memcpy(states, host_states, sizeof(float) * (size_t)S * Sd);
+  int j = 0;
+  for (int m = 0; m < S; ++m)
+    if (host_source[m] != IQL_ACT_SKIP) {
+      ids[j] = m;
+      codes[j] = host_source[m];
+      flags[m] = 0u;
+      ++j;
+    }
+  std::atomic_thread_fence(std::memory_order_seq_cst);
+  cudaStream_t cur = (cudaStream_t)caller_stream;
+  (void)stream;
+  int rc = order_behind_host_step(e, cur);
+  if (rc != IQL_OK) return rc;
+  rc = flush_tables(e, cur);
+  if (rc != IQL_OK) return rc;
+  StepCtx ctx = make_ctx(e);
+  launch_act_members(ctx, e->params, e->guide, e->d_act_off, e->d_act_off + (L + 1), states, ids, codes, n, max_action, mail,
+                     (uint32_t*)flags, cur);
+  CUDA_TRY(e, cudaGetLastError());
+  for (int i = 0; i < n; ++i) {
+    rc = spin_flag(e, flags + ids[i], cur, "iql_act_host_members");
+    if (rc != IQL_OK) return rc;
+  }
+  for (int i = 0; i < n; ++i) {
+    const int m = ids[i];
+    const volatile float* row = mail + (size_t)m * 2 * A;
+    for (int k = 0; k < A; ++k) host_out[(size_t)m * A + k] = row[k];
+    if (codes[i] == IQL_ACT_LEARNER_DIST)
+      for (int k = 0; k < A; ++k) host_std[(size_t)m * A + k] = row[A + k];
+  }
+  return IQL_OK;
+}
+
+extern "C" int iql_replay_insert_members_host(iql_engine* e, const float* host_states, const float* host_actions,
+                                              const float* host_rewards, const float* host_next_states, const float* host_dones,
+                                              const int64_t* host_pointers, void* stream, void* caller_stream) {
+  if (!e) return IQL_ERR_INVALID;
+  if (!host_states || !host_actions || !host_rewards || !host_next_states || !host_dones || !host_pointers)
+    return fail(e, IQL_ERR_INVALID, "iql_replay_insert_members_host: null argument");
+  if (!e->bound) return fail(e, IQL_ERR_STATE, "iql_replay_insert_members_host: state not bound");
+  const int S = e->cfg.n_members;
+  const iql_row_layout& lay = e->layout.row;
+  const int Sd = lay.state_dim, A = lay.action_dim, RF = lay.row_floats;
+  std::vector<std::pair<const float*, int>> rings;
+  for (int m = 0; m < S; ++m) {
+    const int64_t p = host_pointers[m];
+    if (p == -1) continue;
+    const ReplayBinding& b = e->h_replay[m];
+    if (!b.rows) return fail(e, IQL_ERR_INVALID, "iql_replay_insert_members_host: member " + std::to_string(m) + " has no replay binding");
+    if (p < 0 || p >= b.capacity)
+      return fail(e, IQL_ERR_INVALID, "iql_replay_insert_members_host: pointer " + std::to_string(p) + " of member " + std::to_string(m) +
+                                          " is outside [0, " + std::to_string(b.capacity) + ")");
+    rings.emplace_back(b.rows, m);
+  }
+  const int n = (int)rings.size();
+  if (n == 0) return IQL_OK;
+  std::sort(rings.begin(), rings.end());
+  for (int i = 1; i < n; ++i)
+    if (rings[i].first == rings[i - 1].first)
+      return fail(e, IQL_ERR_INVALID, "iql_replay_insert_members_host: members " + std::to_string(rings[i - 1].second) + " and " +
+                                          std::to_string(rings[i].second) + " share one ring; members must not see each other's transitions");
+  const size_t off_ids = align16(sizeof(float) * (size_t)S * RF), off_ptr = off_ids + align16(sizeof(int32_t) * S);
+  const size_t off_cons = off_ptr + align16(sizeof(int64_t) * S), slot_bytes = align16(off_cons + sizeof(uint32_t) * S);
+  if (!e->h_ins) {
+    if (!host_events(e) || cudaHostAlloc((void**)&e->h_ins, 2 * slot_bytes, cudaHostAllocMapped) != cudaSuccess) {
+      cudaGetLastError();
+      e->h_ins = nullptr;
+      return fail(e, IQL_ERR_CUDA, "iql_replay_insert_members_host: pinned block / event allocation failed");
+    }
+    e->ins_n[0] = e->ins_n[1] = 0;
+  }
+  const int s = e->ins_slot;
+  char* slot = e->h_ins + s * slot_bytes;
+  float* rows = (float*)slot;
+  int32_t* ids = (int32_t*)(slot + off_ids);
+  int64_t* ptrs = (int64_t*)(slot + off_ptr);
+  volatile uint32_t* consumed = (volatile uint32_t*)(slot + off_cons);
+  // guard: the launch that last read this slot must have consumed every row of it (it was issued two calls ago, so
+  // this almost never waits; it is a spin on pinned words, not a stream synchronisation)
+  for (int i = 0; i < e->ins_n[s]; ++i) {
+    int rc = spin_flag(e, consumed + i, e->ins_stream[s], "iql_replay_insert_members_host");
+    if (rc != IQL_OK) return rc;
+  }
+  int i = 0;
+  for (int m = 0; m < S; ++m) {
+    if (host_pointers[m] == -1) continue;
+    float* r = rows + (size_t)i * RF;
+    memset(r, 0, sizeof(float) * RF);
+    memcpy(r + lay.off_state, host_states + (size_t)m * Sd, sizeof(float) * Sd);
+    memcpy(r + lay.off_action, host_actions + (size_t)m * A, sizeof(float) * A);
+    memcpy(r + lay.off_next_state, host_next_states + (size_t)m * Sd, sizeof(float) * Sd);
+    r[lay.off_reward] = host_rewards[m];
+    r[lay.off_done] = host_dones[m];
+    ids[i] = m;
+    ptrs[i] = host_pointers[m];
+    consumed[i] = 0u;
+    ++i;
+  }
+  std::atomic_thread_fence(std::memory_order_seq_cst);
+  cudaStream_t cur = (cudaStream_t)caller_stream;
+  (void)stream;
+  int rc = order_behind_host_step(e, cur);
+  if (rc != IQL_OK) return rc;
+  rc = flush_tables(e, cur);
+  if (rc != IQL_OK) return rc;
+  launch_insert_members(e->d_replay, RF, rows, ids, ptrs, n, (uint32_t*)consumed, cur);
+  CUDA_TRY(e, cudaGetLastError());
+  e->ins_n[s] = n;
+  e->ins_stream[s] = cur;
+  e->ins_slot = s ^ 1;
   return IQL_OK;
 }
 

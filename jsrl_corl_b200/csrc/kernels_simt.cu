@@ -668,6 +668,45 @@ void launch_act(const StepCtx& ctx, const float* actor_block, int n_members, con
                                                                    b_off, states, max_action, out);
 }
 
+// every active member of an ensemble in one launch (iql_act_host_members): CTA i serves member ids[i] with the learner
+// arena or the guide arena; the observations are read from device-mapped pinned memory, the results go to the member's
+// mailbox row [2A] (action or mean | std) followed by the member's flag word.  act_body is the single-observation body
+// unchanged, so every member's result is bit-identical to act_host_kernel's.
+__global__ void __launch_bounds__(ACT_THREADS) act_members_kernel(int S, int A, int H, int L, const float* __restrict__ params,
+                                                                  const float* __restrict__ guide, int64_t P,
+                                                                  const int64_t* __restrict__ w_off,
+                                                                  const int64_t* __restrict__ b_off, int64_t log_std_off,
+                                                                  const float* states, const int32_t* ids, const int32_t* codes,
+                                                                  float max_action, float* mail, uint32_t* flags) {
+  extern __shared__ float sm[];
+  const int width = ((H > S ? H : S) + 3) & ~3;
+  float* res = sm + 2 * width;  // [A]
+  const int m = ids[blockIdx.x], code = codes[blockIdx.x];
+  const float* block = (code == IQL_ACT_GUIDE ? guide : params) + (int64_t)m * P;
+  const bool dist = code == IQL_ACT_LEARNER_DIST;
+  act_body(S, A, H, L, block, w_off, b_off, states + (int64_t)m * S, dist ? 1.0f : max_action, res, sm);
+  __syncthreads();
+  if (threadIdx.x < 32) {
+    float* row = mail + (int64_t)m * 2 * A;
+    for (int i = threadIdx.x; i < A; i += 32) {
+      reinterpret_cast<volatile float*>(row)[i] = res[i];
+      if (dist) reinterpret_cast<volatile float*>(row)[A + i] = expf(fminf(fmaxf(block[log_std_off + i], -20.0f), 2.0f));
+    }
+    __threadfence_system();
+    __syncwarp();
+    if (threadIdx.x == 0) reinterpret_cast<volatile uint32_t*>(flags)[m] = 1u;
+  }
+}
+
+void launch_act_members(const StepCtx& ctx, const float* params, const float* guide, const int64_t* w_off, const int64_t* b_off,
+                        const float* states, const int32_t* ids, const int32_t* codes, int n, float max_action, float* mail,
+                        uint32_t* flags, cudaStream_t st) {
+  const int width = ((ctx.H > ctx.S_dim ? ctx.H : ctx.S_dim) + 3) & ~3;
+  act_members_kernel<<<n, ACT_THREADS, (2 * width + ctx.A_dim) * sizeof(float), st>>>(
+      ctx.S_dim, ctx.A_dim, ctx.H, ctx.L, params, guide, ctx.P, w_off, b_off, ctx.deterministic ? 0 : ctx.log_std_off, states,
+      ids, codes, max_action, mail, flags);
+}
+
 int act_host_state_max() { return ACT_STATE_MAX; }
 
 void launch_act_host(const StepCtx& ctx, const float* actor_block, const int64_t* w_off, const int64_t* b_off,

@@ -133,6 +133,31 @@ __global__ void replay_insert_byval_kernel(float* __restrict__ rows, int RF, int
   for (int c = threadIdx.x; c < RF; c += blockDim.x) rows[pointer * RF + c] = row.v[c];
 }
 
+// add_transition of S members at once (iql_replay_insert_members_host): CTA i copies the packed row i of the
+// device-mapped pinned input slot to row pointers[i] of the ring bound to member ids[i], then marks its part of the slot
+// consumed.  Every load of the slot has returned once the CTA passes the barrier (each value was stored), so the host
+// may overwrite the row as soon as the word is raised -- the guard never waits for the rest of the stream.
+__global__ void replay_insert_members_kernel(const ReplayBinding* __restrict__ replay, int RF, const float* rows,
+                                             const int32_t* ids, const int64_t* pointers, uint32_t* consumed) {
+  const int i = blockIdx.x;
+  const int m = ids[i];
+  const int64_t p = pointers[i];
+  float* dst = const_cast<float*>(replay[m].rows) + p * RF;
+  const float* src = rows + (int64_t)i * RF;
+  for (int c = threadIdx.x; c < RF; c += blockDim.x) dst[c] = src[c];
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    __threadfence_system();
+    reinterpret_cast<volatile uint32_t*>(consumed)[i] = 1u;
+  }
+}
+
+void launch_insert_members(const ReplayBinding* replay, int RF, const float* rows, const int32_t* ids, const int64_t* pointers,
+                           int n, uint32_t* consumed, cudaStream_t st) {
+  const int threads = RF < 256 ? ((RF + 31) / 32) * 32 : 256;
+  replay_insert_members_kernel<<<n, threads, 0, st>>>(replay, RF, rows, ids, pointers, consumed);
+}
+
 // ---- sample: Philox (or given) indices + vectorised row gather ------------
 // One thread per float4 of a row; the RF/4 lanes of a row are adjacent, so the
 // row read is a single coalesced burst.  The row is then scattered to the five

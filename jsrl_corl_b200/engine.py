@@ -479,3 +479,89 @@ class EnsembleEngine:
                 guard.__exit__(None, None, None)
         self.act_calls += 1
         return self._act_out.copy(), self._act_std.copy()
+
+    # ------------------------------------------------------------------
+    # online phase of an ensemble: every member's act / ring insert of one env step in one launch each
+    # ------------------------------------------------------------------
+    def bind_guide(self, params: Optional[torch.Tensor]):
+        """Bind a [n_members, param_floats] parameter arena with this engine's layout as the members' guides
+        (`iql_bind_guide`; the engine reads it zero-copy and never writes it).  None unbinds."""
+        if params is None:
+            _lib.check(self._L.iql_bind_guide(self._h, None), self._h, "iql_bind_guide")
+            self._guide_ref = None
+            return
+        if params.device != self.device or params.dtype != torch.float32 or not params.is_contiguous() or \
+                tuple(params.shape) != (self.n_members, self.layout.param_floats):
+            raise ValueError(f"the guide arena must be a contiguous float32 [{self.n_members}, {self.layout.param_floats}] "
+                             "tensor on the engine's device")
+        _lib.check(self._L.iql_bind_guide(self._h, params.data_ptr()), self._h, "iql_bind_guide")
+        self._guide_ref = params
+
+    def _ensure_stream_raw(self):
+        if getattr(self, "_stream_raw", None) is None:
+            self._stream_raw = self.stream.cuda_stream
+
+    def act_members_host(self, states: np.ndarray, source, max_action: float = 1.0, out: Optional[np.ndarray] = None,
+                         std: Optional[np.ndarray] = None):
+        """One env step of every member's policy in one launch (`iql_act_host_members`).  ``states`` [S, state_dim],
+        ``source`` [S] IQL_ACT_* codes (int) or names ("skip", "learner", "learner_dist", "guide").  Returns
+        ``(out, std)``: out [S, action_dim] holds the eval-mode action of "learner" / "guide" members and the unscaled
+        mean of "learner_dist" members, std [S, action_dim] the std of the latter (None when there are none).  Rows of
+        skipped members are left as they were in ``out`` / ``std`` (NaN when the arrays are allocated here)."""
+        S, A = self.n_members, self.action_dim
+        src = np.asarray([_lib.ACT_SOURCES[s] if isinstance(s, str) else int(s) for s in source], dtype=np.int8) \
+            if not (isinstance(source, np.ndarray) and source.dtype == np.int8) else source
+        if src.shape != (S,):
+            raise ValueError(f"source must have one entry per member ({S})")
+        st = np.ascontiguousarray(states, dtype=np.float32)
+        if st.shape != (S, self.state_dim):
+            raise ValueError(f"states must be [{S}, {self.state_dim}]")
+        if out is None:
+            out = np.full((S, A), np.nan, dtype=np.float32)
+        if std is None and (src == _lib.ACT_LEARNER_DIST).any():
+            std = np.full((S, A), np.nan, dtype=np.float32)
+        for arr in (out, std):
+            if arr is not None and (arr.shape != (S, A) or arr.dtype != np.float32 or not arr.flags.c_contiguous):
+                raise ValueError(f"out / std must be C-contiguous float32 [{S}, {A}]")
+        self._ensure_stream_raw()
+        switch = torch._C._cuda_getDevice() != self._dev_index
+        if switch:
+            guard = torch.cuda.device(self.device)
+            guard.__enter__()
+        try:
+            rc = self._L.iql_act_host_members(self._h, st.ctypes.data, src.ctypes.data, float(max_action), out.ctypes.data,
+                                              std.ctypes.data if std is not None else None, self._stream_raw,
+                                              torch._C._cuda_getCurrentRawStream(self._dev_index))
+            if rc:
+                _lib.check(rc, self._h, "iql_act_host_members")
+        finally:
+            if switch:
+                guard.__exit__(None, None, None)
+        self.act_calls += 1
+        return out, std
+
+    def insert_members_host(self, states: np.ndarray, actions: np.ndarray, rewards: np.ndarray, next_states: np.ndarray,
+                            dones: np.ndarray, pointers: np.ndarray):
+        """`ReplayBuffer.add_transition` of every member in one launch (`iql_replay_insert_members_host`): member m's
+        transition goes to row ``pointers[m]`` of the rows bound to m (``-1``: no insert).  Host arrays [S, state_dim],
+        [S, action_dim], [S], [S, state_dim], [S]; the call copies them, so they may be reused when it returns.  Only
+        the engine-side write happens here -- ``IQLEnsemble.add_transitions`` keeps the buffers' pointers."""
+        S = self.n_members
+        f = lambda x, shape: np.ascontiguousarray(x, dtype=np.float32).reshape(shape)  # noqa: E731
+        s, a = f(states, (S, self.state_dim)), f(actions, (S, self.action_dim))
+        r, s2, d = f(rewards, (S,)), f(next_states, (S, self.state_dim)), f(dones, (S,))
+        p = np.ascontiguousarray(pointers, dtype=np.int64).reshape(S)
+        self._ensure_stream_raw()
+        switch = torch._C._cuda_getDevice() != self._dev_index
+        if switch:
+            guard = torch.cuda.device(self.device)
+            guard.__enter__()
+        try:
+            rc = self._L.iql_replay_insert_members_host(self._h, s.ctypes.data, a.ctypes.data, r.ctypes.data, s2.ctypes.data,
+                                                        d.ctypes.data, p.ctypes.data, self._stream_raw,
+                                                        torch._C._cuda_getCurrentRawStream(self._dev_index))
+            if rc:
+                _lib.check(rc, self._h, "iql_replay_insert_members_host")
+        finally:
+            if switch:
+                guard.__exit__(None, None, None)

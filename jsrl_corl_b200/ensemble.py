@@ -50,6 +50,7 @@ class IQLEnsemble:
                                      deterministic, math_mode, device, max_steps_per_call, step_path=step_path)
         self.n_members = n_members
         self.actor_dropout = actor_dropout
+        self.guide: Optional["IQLEnsemble"] = None  # set_guide
         self.seeds = list(seeds) if seeds is not None else list(range(n_members))
         if len(self.seeds) != n_members:
             raise ValueError("need one seed per member")
@@ -104,6 +105,58 @@ class IQLEnsemble:
         if idx.shape != (e.n_members, e.batch_size):
             raise ValueError(f"indices must be [{e.n_members}, {e.batch_size}]")
         return np.asarray(e.host_step(host_indices=idx.ctypes.data), dtype=np.float32).reshape(e.n_members, 3)
+
+    # ---- the online phase: guide, batched act, batched ring insert ------------
+    def set_guide(self, other: Optional["IQLEnsemble"]):
+        """Make ``other``'s members the guides of this ensemble's members (JSRL's guide policy, jsrl_utils.py:285-323):
+        member m's guide is ``other``'s member m, read zero-copy from its parameter arena.  Shapes, policy type and
+        parameter layout must be identical.  Keeps a reference to ``other``; None unbinds."""
+        if other is None:
+            self.engine.bind_guide(None)
+            self.guide = None
+            return
+        a, b = self.engine, other.engine
+        shape = lambda e: (e.n_members, e.state_dim, e.action_dim, e.hidden_dim, e.n_hidden, e.deterministic)  # noqa: E731
+        if shape(a) != shape(b):
+            raise ValueError(f"guide ensemble shape {shape(b)} differs from this ensemble's {shape(a)} "
+                             "(members, state_dim, action_dim, hidden_dim, n_hidden, deterministic)")
+        lay = lambda e: (e.layout.param_floats, [(t.net, t.layer, t.kind, t.rows, t.cols, t.ld, t.offset) for t in e.tensors])  # noqa: E731
+        if lay(a) != lay(b):
+            raise ValueError("guide ensemble has a different parameter layout")
+        if b.device != a.device:
+            raise ValueError("guide ensemble lives on another device")
+        a.bind_guide(b.params)
+        self.guide = other
+
+    def act(self, states: np.ndarray, source, max_action: float = 1.0, out: Optional[np.ndarray] = None,
+            std: Optional[np.ndarray] = None):
+        """Every member's action for one env step in one launch: ``source[m]`` is "skip", "learner" (eval-mode
+        action), "learner_dist" (Gaussian mean and std, sampled by the caller) or "guide" (eval-mode action of the
+        guide set with ``set_guide``), or the matching IQL_ACT_* code.  Returns ``(out, std)`` as
+        ``EnsembleEngine.act_members_host``."""
+        return self.engine.act_members_host(states, source, max_action, out, std)
+
+    def add_transitions(self, states, actions, rewards, next_states, dones, mask=None):
+        """``ReplayBuffer.add_transition`` (iql.py:180-196) for every member whose ``mask`` entry is true (all when
+        None), into the member's own bound buffer, in one launch.  Advances each buffer's ``_pointer`` / ``_size`` as
+        ``add_transition`` does and raises its IndexError for a buffer loaded to the brim -- before anything is
+        written.  Members sharing one buffer cannot insert in the same call."""
+        S = self.n_members
+        bufs = getattr(self, "_buffers", None)
+        if bufs is None:
+            raise RuntimeError("add_transitions: no replay buffers bound (bind_replay)")
+        mask = np.ones(S, dtype=bool) if mask is None else np.asarray(mask, dtype=bool).reshape(S)
+        pointers = np.full(S, -1, dtype=np.int64)
+        for m in np.flatnonzero(mask):
+            rb = bufs[m]
+            if not 0 <= rb._pointer < rb._buffer_size:
+                raise IndexError(f"index {rb._pointer} is out of bounds for dimension 0 with size {rb._buffer_size}")
+            pointers[m] = rb._pointer
+        self.engine.insert_members_host(states, actions, rewards, next_states, dones, pointers)
+        for m in np.flatnonzero(mask):
+            rb = bufs[m]
+            rb._pointer = (rb._pointer + 1) % rb._buffer_size
+            rb._size = min(rb._size + 1, rb._buffer_size)
 
     # ---- checkpoints in the reference layout --------------------------------
     def member_state_dict(self, m: int) -> Dict[str, Any]:

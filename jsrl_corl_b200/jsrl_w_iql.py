@@ -17,6 +17,7 @@ from typing import Callable, Dict, Optional, Tuple
 import numpy as np
 import torch
 
+from . import _lib as _lib_codes
 from . import jsrl_utils as jsrl
 from .iql import (DeterministicPolicy, GaussianPolicy, ReplayBuffer, is_goal_reached, modify_reward_online)
 
@@ -209,3 +210,329 @@ def train_loop(config, env, eval_env, replay_buffer: Optional[ReplayBuffer], sta
                 log(eval_log, trainer.total_it)
                 history.append(dict(eval_log, t=t))
     return trainer, config, history
+
+
+# ---------------------------------------------------------------------------
+# S members through the whole JSRL run at once (the reference's process-per-seed launchers, ray_trainer.py)
+# ---------------------------------------------------------------------------
+# fields every member of an ensemble run must share: the loop runs all members in lockstep (batch size, iteration
+# counts, evaluation points), `horizon_fn` is a module global of jsrl_utils, and the policy type / dropout / online
+# buffer rule fix the engine shape and the update gate
+ENSEMBLE_SHARED_FIELDS = ("batch_size", "offline_iterations", "online_iterations", "eval_freq", "n_episodes", "horizon_fn",
+                          "iql_deterministic", "actor_dropout", "new_online_buffer")
+
+
+def check_ensemble_configs(configs):
+    """Refuse (ValueError) configs whose shared fields differ, and (NotImplementedError) the options the ensemble
+    loop does not cover.  Touches no device."""
+    if len(configs) == 0:
+        raise ValueError("ensemble_train_loop needs at least one config")
+    for f in ENSEMBLE_SHARED_FIELDS:
+        vals = [getattr(c, f) for c in configs]
+        if any(v != vals[0] for v in vals[1:]):
+            raise ValueError(f"ensemble_train_loop: `{f}` must be the same for every member, got {vals}")
+    c0 = configs[0]
+    for c in configs:
+        if getattr(c, "guide_heuristic_fn", None) is not None:
+            raise NotImplementedError("ensemble_train_loop: heuristic guides are host functions of one env; the ensemble's "
+                                      "guides are its offline members (use train_loop)")
+        if getattr(c, "pretrained_policy_path", None) is not None:
+            raise NotImplementedError("ensemble_train_loop: pretrained guides (pretrained_policy_path) are not supported; "
+                                      "the guides are the members trained in the offline phase")
+    if c0.horizon_fn == "variance":
+        raise NotImplementedError("ensemble_train_loop: the `variance` horizon needs a value network per member on the host")
+    if c0.horizon_fn not in jsrl.HORIZON_FNS:
+        raise ValueError(f"unknown horizon_fn {c0.horizon_fn!r}")
+    if c0.actor_dropout:
+        raise NotImplementedError("ensemble_train_loop: training-mode act with active actor dropout has no engine kernel "
+                                  "(the single-learner path falls back to stock torch there)")
+
+
+def member_networks(config, state_dim: int, action_dim: int, max_action: float):
+    """Initial networks of one member: ``torch.manual_seed(config.seed)``, then the offline TwinQ / ValueFunction /
+    policy and the online learner's, in the reference's construction order (jsrl_utils.py:219-282), the learner's
+    drawn right after the offline ones.  The global torch RNG is left as it was.  Returns ((q, v, actor), (q, v,
+    actor)) as CPU modules with the class-default 2x256 networks of ``make_actor``."""
+    from .iql import TwinQ, ValueFunction
+
+    cls = DeterministicPolicy if config.iql_deterministic else GaussianPolicy
+    with torch.random.fork_rng(devices=[]):
+        torch.manual_seed(config.seed)
+        nets = []
+        for _ in range(2):
+            nets.append((TwinQ(state_dim, action_dim), ValueFunction(state_dim),
+                         cls(state_dim, action_dim, max_action, dropout=config.actor_dropout)))
+    return nets[0], nets[1]
+
+
+def _member_hparams(c, t_max: int) -> Dict:
+    return dict(beta=c.beta, iql_tau=c.iql_tau, discount=c.discount, tau=c.tau, vf_lr=c.vf_lr, qf_lr=c.qf_lr,
+                actor_lr=c.actor_lr, cosine_t_max=int(t_max))
+
+
+def _build_ensemble(configs, nets, state_dim, action_dim, t_max, device):
+    from .ensemble import IQLEnsemble
+
+    c0 = configs[0]
+    ens = IQLEnsemble(len(configs), state_dim, action_dim, 256, 2, c0.batch_size, deterministic=c0.iql_deterministic,
+                      device=device, max_steps_per_call=max(1, min(256, int(c0.eval_freq))), seeds=[c.seed for c in configs],
+                      hparams=[_member_hparams(c, t_max) for c in configs], init=False)
+    for m, (q, v, actor) in enumerate(nets):
+        ens.engine.load_params(m, {"qf": q.state_dict(), "vf": v.state_dict(), "actor": actor.state_dict()})
+    return ens
+
+
+@torch.no_grad()
+def ensemble_eval_actor(envs, ensemble, use_guide: bool, configs, max_action: float):
+    """``eval_actor`` for every member at once: member m plays ``n_episodes`` episodes on ``envs[m]`` with
+    ``ensemble``'s member m as the learner and, with ``use_guide``, the guide bound by ``set_guide`` as the guide.
+    All members step in lockstep with one act launch per step; members whose episodes are over are skipped.  Each
+    member's episodes are exactly those ``eval_actor`` plays for it alone (the horizon function reads and
+    ``config.ep_agent_type`` is written per member).  Returns one (returns, success rate, horizon, mean agent type)
+    tuple per member."""
+    S = len(configs)
+    hfn = jsrl.HORIZON_FNS[jsrl.horizon_str]["horizon_fn"]
+    n_ep = configs[0].n_episodes
+    states = np.zeros((S, ensemble.engine.state_dim), dtype=np.float32)
+    source = np.zeros(S, dtype=np.int8)
+    out = np.zeros((S, ensemble.engine.action_dim), dtype=np.float32)
+    ep = [0] * S
+    live = [n_ep > 0] * S
+    fresh = [True] * S
+    raw_state = [None] * S
+    acc = [dict(returns=[], successes=[], horizons=[], agent_types=[]) for _ in range(S)]
+    cur = [None] * S
+    while any(live):
+        for m in range(S):
+            source[m] = 0
+            if not live[m]:
+                continue
+            c = configs[m]
+            if fresh[m]:
+                raw_state[m] = _reset(envs[m], c.seed if ep[m] == 0 else None)
+                cur[m] = dict(ts=0, ret=0.0, goal=False, horizons=[], types=[])
+                fresh[m] = False
+            e = cur[m]
+            c.ep_agent_type = 0 if e["ts"] == 0 else np.mean(e["types"])
+            use_learner, horizon = hfn(e["ts"], raw_state[m], envs[m], c)
+            if not use_guide:
+                use_learner = True
+            e["horizons"].append(horizon)
+            e["types"].append(1 if use_learner else 0)
+            states[m] = np.asarray(raw_state[m], dtype=np.float32).reshape(-1)
+            source[m] = _lib_codes.ACT_LEARNER if use_learner else _lib_codes.ACT_GUIDE
+        ensemble.act(states, source, max_action, out=out)
+        for m in range(S):
+            if not source[m]:
+                continue
+            c, e = configs[m], cur[m]
+            raw_state[m], reward, done, info = _step(envs[m], out[m].copy())
+            e["ret"] += reward
+            e["ts"] += 1
+            e["goal"] = e["goal"] or is_goal_reached(reward, info)
+            if done:
+                a = acc[m]
+                a["successes"].append(float(e["goal"]))
+                a["returns"].append(e["ret"])
+                probing = (not use_guide) and c.max_init_horizon
+                a["horizons"].append(np.max(e["horizons"]) if probing else jsrl.accumulate(e["horizons"]))
+                a["agent_types"].append(np.mean(e["types"]))
+                ep[m] += 1
+                fresh[m] = True
+                live[m] = ep[m] < n_ep
+    results = []
+    for m in range(S):
+        a, c = acc[m], configs[m]
+        horizon = np.max(a["horizons"]) if ((not use_guide) and c.max_init_horizon) else np.mean(a["horizons"])
+        results.append((np.asarray(a["returns"]), float(np.mean(a["successes"])), horizon, float(np.mean(a["agent_types"]))))
+    return results
+
+
+def ensemble_train_loop(configs, envs, eval_envs, replay_buffers, state_dim: int, action_dim: int, max_action: float,
+                        max_steps: int, log: Optional[Callable[[int, Dict, int], None]] = None, reward_mod_dicts=None,
+                        is_env_with_goal: bool = False):
+    """``train_loop`` for S members at once, one ``JsrlTrainConfig`` per member (seed, IQL / Adam hyper-parameters,
+    curriculum, tolerance, noise and checkpoint path may differ; ``ENSEMBLE_SHARED_FIELDS`` may not).
+
+    Offline: one ``IQLEnsemble`` (cosine schedule with T_max = offline_iterations) trained in K-step calls that end at
+    the evaluation points, on indices drawn from each member's own ``np.random.RandomState(seed)``.  Switch: a
+    guide-only evaluation gives each member's initial horizon, the offline ensemble becomes the guide (``set_guide``,
+    its arena read zero-copy) and a fresh learner ensemble starts (no schedule, total_it = offline_iterations, the
+    guide's networks copied when there is a single curriculum stage), each member with its own online ring.  Online,
+    per env step for all members: the horizon functions on the host, ONE act launch, exploration noise or the
+    Gaussian sample from each member's own ``torch.Generator(seed)``, S env steps, ONE ring-insert launch and ONE
+    logged update.  ``train_loop``'s quirks are kept per member.  ``log(member, dict, step)`` receives what
+    ``train_loop``'s ``log`` receives.  Returns (learner ensemble, configs, one eval history per member); the guide
+    ensemble is ``learner.guide``."""
+    check_ensemble_configs(configs)
+    S = len(configs)
+    if not (len(envs) == len(eval_envs) == S):
+        raise ValueError("need one env and one eval env per member")
+    if isinstance(replay_buffers, ReplayBuffer):
+        replay_buffers = [replay_buffers] * S
+    if len(replay_buffers) != S:
+        raise ValueError("need one replay buffer or one per member")
+    reward_mod_dicts = reward_mod_dicts if reward_mod_dicts is not None else [None] * S
+    if not configs[0].new_online_buffer:
+        rows = [rb.rows.data_ptr() for rb in replay_buffers]
+        if len(set(rows)) != S:
+            raise ValueError("new_online_buffer=False: every member needs its own buffer (members must not see each "
+                             "other's transitions)")
+    log = log or (lambda m, d, step: None)
+    c0 = configs[0]
+    B, off, on, eval_freq = int(c0.batch_size), int(c0.offline_iterations), int(c0.online_iterations), int(c0.eval_freq)
+    gaussian = not c0.iql_deterministic
+    jsrl.horizon_str = c0.horizon_fn
+    device = c0.device
+    for c in configs:
+        c.discrete = False
+        if c.checkpoints_path is not None:
+            os.makedirs(c.checkpoints_path, exist_ok=True)
+    nets = [member_networks(c, state_dim, action_dim, max_action) for c in configs]
+    index_rng = [np.random.RandomState(c.seed) for c in configs]
+    noise_rng = [torch.Generator().manual_seed(int(c.seed)) for c in configs]
+    histories = [[] for _ in range(S)]
+    eval_successes = [[] for _ in range(S)]
+    states = [_reset(envs[m], configs[m].seed) for m in range(S)]
+
+    def evaluate(t, ens, use_guide, total_it):
+        if not use_guide:
+            for c in configs:
+                c.curriculum_stage = np.nan
+        results = ensemble_eval_actor(eval_envs, ens, use_guide, configs, max_action)
+        for m, c in enumerate(configs):
+            scores, success, c.mean_horizon_reached, c.eval_mean_agent_type = results[m]
+            score = float(scores.mean())
+            norm_fn = getattr(eval_envs[m], "get_normalized_score", None) if c.normalize_reward else None
+            if norm_fn is not None:
+                score = float(norm_fn(score))
+            eval_log = {}
+            if is_env_with_goal:
+                eval_successes[m].append(success)
+                eval_log["eval/regret"] = float(np.mean(1 - np.array(eval_successes[m])))
+                eval_log["eval/success_rate"] = success
+            if t >= off:
+                configs[m] = c = jsrl.horizon_update_callback(c, score)
+                eval_log = jsrl.add_jsrl_metrics(eval_log, c)
+            if norm_fn is not None:
+                eval_log["eval/d4rl_normalized_score"] = score * 100.0
+            else:
+                eval_log["eval/score"] = score
+            if c.checkpoints_path is not None:
+                torch.save(ens.member_state_dict(m), os.path.join(c.checkpoints_path, f"checkpoint_{t}.pt"))
+            log(m, eval_log, total_it)
+            histories[m].append(dict(eval_log, t=t))
+
+    # ---- offline phase: K-step calls between evaluation points ----
+    offline = _build_ensemble(configs, [n[0] for n in nets], state_dim, action_dim, off, device)
+    offline.bind_replay(list(replay_buffers))
+    first = 0 if not c0.new_online_buffer else min(B, off)  # train_loop's gate `t >= batch_size` on the global t
+    t, done_steps = first, 0
+    while t < off:
+        stop = min(off, (t // eval_freq + 1) * eval_freq, t + offline.engine.max_steps_per_call)
+        K = stop - t
+        idx = np.empty((S, K, B), dtype=np.int64)
+        for m, rb in enumerate(replay_buffers):
+            high = rb._high()
+            for k in range(K):
+                idx[m, k] = index_rng[m].randint(0, high, size=B)
+        losses = offline.train_steps(K, mode="indices", indices=torch.from_numpy(idx)).cpu().numpy()
+        for k in range(K):
+            done_steps += 1
+            for m in range(S):
+                log(m, {"value_loss": float(losses[m, k, 0]), "q_loss": float(losses[m, k, 1]),
+                        "actor_loss": float(losses[m, k, 2]), "offline_iter": t + k}, done_steps)
+        t = stop
+        if t % eval_freq == 0:
+            evaluate(t - 1, offline, False, done_steps)
+    if on <= 0:
+        return offline, configs, histories
+
+    # ---- switch to online: guide-only probe, guide binding, fresh learners, online rings ----
+    for c in configs:
+        c.curriculum_stage = np.nan
+    probe = ensemble_eval_actor(envs, offline, False, configs, max_action)
+    learner = _build_ensemble(configs, [n[1] for n in nets], state_dim, action_dim, 0, device)
+    for m, c in enumerate(configs):
+        if c.n_curriculum_stages == 1:  # the guide's trained networks, fresh optimizers (get_learning_agent)
+            learner.engine.load_params(m, offline.engine.param_views(m))
+        learner.engine.set_counters(m, total_it=off)
+    learner.set_guide(offline)
+    for m, c in enumerate(configs):
+        configs[m] = jsrl.prepare_finetuning(probe[m][2], c)
+    online_buffers = [jsrl.get_online_buffer(c, replay_buffers[m], state_dim, action_dim) for m, c in enumerate(configs)]
+    learner.bind_replay(online_buffers)
+    states = [_reset(envs[m]) for m in range(S)]
+
+    hfn = jsrl.HORIZON_FNS[jsrl.horizon_str]["horizon_fn"]
+    A = action_dim
+    obs = np.zeros((S, state_dim), dtype=np.float32)
+    next_obs = np.zeros((S, state_dim), dtype=np.float32)
+    act_out = np.zeros((S, A), dtype=np.float32)
+    act_std = np.zeros((S, A), dtype=np.float32) if gaussian else None
+    actions = np.zeros((S, A), dtype=np.float32)
+    rewards = np.zeros(S, dtype=np.float32)
+    real_dones = np.zeros(S, dtype=np.float32)
+    source = np.zeros(S, dtype=np.int8)
+    learner_code = _lib_codes.ACT_LEARNER_DIST if gaussian else _lib_codes.ACT_LEARNER
+    use = [False] * S
+    ep_ret, ep_step, goal = [0.0] * S, [0] * S, [False] * S
+    ep_types = [[] for _ in range(S)]
+    train_successes = [[] for _ in range(S)]
+    total_it = off
+    for t in range(off, off + on):
+        online_logs = [{} for _ in range(S)]
+        for m, c in enumerate(configs):
+            if ep_step[m] == 0:
+                ep_types[m] = []
+                c.ep_agent_type = 0
+            else:
+                c.ep_agent_type = np.mean(ep_types[m])
+            use[m], _ = hfn(ep_step[m], states[m], envs[m], c)
+            obs[m] = np.asarray(states[m], dtype=np.float32).reshape(-1)
+            source[m] = learner_code if use[m] else _lib_codes.ACT_GUIDE
+        learner.act(obs, source, max_action, out=act_out, std=act_std)
+        for m, c in enumerate(configs):
+            ep_types[m].append(1 if use[m] else 0)
+            a = act_out[m].copy()
+            if use[m] and gaussian:  # GaussianPolicy.act in training mode: mean + std * N(0, 1), scaled and clipped
+                sample = a + act_std[m] * torch.randn(A, generator=noise_rng[m]).numpy()
+                a = np.clip(max_action * sample, -max_action, max_action).astype(np.float32)
+            elif use[m]:  # deterministic learner: exploration noise
+                noise = (torch.randn(A, generator=noise_rng[m]) * c.expl_noise).clamp(-c.noise_clip, c.noise_clip)
+                a = a + noise.numpy()
+            a = np.clip(max_action * a, -max_action, max_action).astype(np.float32).flatten()
+            next_state, reward, done, info = _step(envs[m], a)
+            ep_step[m] += 1
+            goal[m] = goal[m] or is_goal_reached(reward, info)
+            ep_ret[m] += reward
+            real_dones[m] = float(bool(done and ep_step[m] < max_steps))  # time-outs are not terminals
+            if c.normalize_reward and reward_mod_dicts[m] is not None:
+                reward = modify_reward_online(reward, c.env, **reward_mod_dicts[m])
+            actions[m] = a
+            rewards[m] = reward
+            next_obs[m] = np.asarray(next_state, dtype=np.float32).reshape(-1)
+            states[m] = next_state
+            if done:
+                states[m] = _reset(envs[m])
+                lg = online_logs[m]
+                if is_env_with_goal:
+                    train_successes[m].append(goal[m])
+                    lg["train/regret"] = float(np.mean(1 - np.array(train_successes[m])))
+                    lg["train/is_success"] = float(goal[m])
+                lg.update({"train/episode_return": ep_ret[m], "train/mean_ep_agent_type": float(np.mean(ep_types[m])),
+                           "train/episode_length": ep_step[m]})
+                ep_ret[m], ep_step[m], goal[m] = 0.0, 0, False
+        learner.add_transitions(obs, actions, rewards, next_obs, real_dones)
+        if t >= B or not c0.new_online_buffer:
+            idx = np.stack([index_rng[m].randint(0, online_buffers[m]._high(), size=B) for m in range(S)])
+            losses = learner.train_step_logged(idx)
+            total_it += 1
+            for m in range(S):
+                log_dict = {"value_loss": float(losses[m, 0]), "q_loss": float(losses[m, 1]), "actor_loss": float(losses[m, 2]),
+                            "online_iter": t - off}
+                log_dict.update(online_logs[m])
+                log(m, log_dict, total_it)
+            if (t + 1) % eval_freq == 0:
+                evaluate(t, learner, True, total_it)
+    return learner, configs, histories
