@@ -142,7 +142,9 @@ int iql_set_counters(iql_engine* e, int32_t member, const iql_counters* c);
  * tests and measurements).  IQL_OPT_STEP_PATH must be set before iql_bind_state. */
 #define IQL_OPT_STEP_PATH 1  /* 0 auto (default): 4 where it is supported and the ensemble has >= 8 members or >= 3 hidden layers, else 1;
                               1 one kernel per phase + adam_polyak; 2 chained backward + fused optimizer; 3 is not assigned;
-                              4 chained backward (gradients only) + adam_polyak.  2 and 4: bind fails where unsupported */
+                              4 chained backward (gradients only) + adam_polyak.  2 and 4: bind fails where unsupported --
+                              the chain needs tf32, hidden 256, batch 256, 2..4 hidden layers, action_dim <= 24 and
+                              state_dim + action_dim <= 256; auto takes 1 outside that */
 #define IQL_OPT_KEEP_GRADS 2 /* != 0: the chained backward also stores the hidden / input weight gradients to `grads` */
 int iql_set_option(iql_engine* e, int32_t key, int64_t value);
 /* Which code path serves this handle (after iql_bind_state).  IQL_INFO_TENSOR_CORE_PATH == 0 under

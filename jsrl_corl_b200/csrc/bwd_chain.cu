@@ -558,10 +558,10 @@ extern "C" int iql_debug_chain_trace(long long* out, int32_t max_words) {
   return C_TRACE_WORDS;
 }
 
-bool bwd_chain_supported(int batch, int hidden, int n_hidden, bool fused_fwd) {
+bool bwd_chain_supported(int batch, int hidden, int n_hidden, int k0, bool fused_fwd) {
   chain_trace_buffer();
   return fused_fwd && batch == 2 * C_TILE_M && hidden == 256 && n_hidden >= 2 && n_hidden <= FUSED_MAX_LAYERS &&
-         umma_phase_supported(1, batch, hidden);
+         k0 <= 256 && umma_phase_supported(1, batch, hidden);
 }
 
 int bwd_chain_wgrad0_tile_n(int k0) { return k0 <= 64 ? 64 : (k0 <= 128 ? 128 : 256); }

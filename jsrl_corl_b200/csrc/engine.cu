@@ -68,6 +68,15 @@ struct Phase {
 };
 enum { PH_GENERIC = 0, PH_FIRST_FWD = 1, PH_OUT_FWD = 2, PH_LAST_WGRAD = 3, PH_LAST_DGRAD = 4, PH_FIRST_WGRAD = 5 };
 
+// The output-layer backward runs on the skinny kernels (last_bwd_v4 / last_bwd_kernel<24>, the output-layer operand in
+// shared memory) up to 24 actions; wider heads take two generic GEMMs.  The chained backward starts from the skinny
+// kernels' outputs, so bind time and every step must agree on this rule.
+static bool last_bwd_skinny_ok(int batch, int action_dim) {
+  static const bool no_skinny = dbg_getenv("IQL_B200_NO_SKINNY") != nullptr;
+  const int apad = action_dim <= 1 ? 1 : (action_dim <= 8 ? 8 : 24);
+  return !no_skinny && action_dim <= 24 && ((size_t)batch * apad + 256 * apad) * 4 <= 200 * 1024;
+}
+
 struct iql_engine {
   iql_config cfg;
   iql_layout layout;
@@ -792,8 +801,9 @@ extern "C" int iql_bind_state(iql_engine* e, float* params, float* exp_avg, floa
   // per-phase kernels' narrow dgrad units spread a two-layer step of few tasks over more SMs (DESIGN.md section 8).
   const bool want_chain = e->step_path == 2 || e->step_path == 4 ||
                           (e->step_path == 0 && (S >= CHAIN_GRADS_MIN_MEMBERS || e->cfg.n_hidden >= 3));
-  if (tc_mode && want_chain && e->fw_splits == 1 &&
-      bwd_chain_supported(e->cfg.batch_size, e->cfg.hidden_dim, e->cfg.n_hidden, e->fused_fwd)) {
+  if (tc_mode && want_chain && e->fw_splits == 1 && last_bwd_skinny_ok(e->cfg.batch_size, e->cfg.action_dim) &&
+      bwd_chain_supported(e->cfg.batch_size, e->cfg.hidden_dim, e->cfg.n_hidden, e->cfg.state_dim + e->cfg.action_dim,
+                          e->fused_fwd)) {
     const int L = e->cfg.n_hidden, ntask = 4 * S;
     BwdChainArgs& ca = e->chain_args;
     memset(&ca, 0, sizeof(ca));
@@ -847,7 +857,8 @@ extern "C" int iql_bind_state(iql_engine* e, float* params, float* exp_avg, floa
   }
   if ((e->step_path == 2 || e->step_path == 4) && !e->chain)
     return fail(e, IQL_ERR_INVALID, "iql_bind_state: IQL_OPT_STEP_PATH = chained backward, but this shape / math mode does not support it "
-                                    "(needs tf32, hidden 256, batch 256, 2..4 hidden layers)");
+                                    "(needs tf32, hidden 256, batch 256, 2..4 hidden layers, action_dim <= 24, "
+                                    "state_dim + action_dim <= 256)");
   if (!e->side) {  // optional: without it the backward simply stays on one stream
     if (cudaStreamCreateWithFlags(&e->side, cudaStreamNonBlocking) != cudaSuccess ||
         cudaEventCreateWithFlags(&e->ev_fork, cudaEventDisableTiming) != cudaSuccess ||
@@ -1040,11 +1051,10 @@ static int enqueue_step(iql_engine* e, StepCtx& ctx, bool gather, cudaStream_t s
   // the skinny-layer kernels keep one operand in shared memory; fall back to the generic GEMM when it does not fit
   static const bool no_skinny = dbg_getenv("IQL_B200_NO_SKINNY") != nullptr;
   auto kpad = [](int k) { return k <= 24 ? 24 : (k <= 40 ? 40 : 72); };
-  auto apad = [](int a) { return a <= 1 ? 1 : (a <= 8 ? 8 : 24); };
   const bool first_ok = !no_skinny && K0 <= 72;
   const bool first_wgrad_ok = first_ok && ((size_t)B * kpad(K0) + 512 * (kpad(K0) + 1)) * 4 <= 200 * 1024;
   const bool out_ok = !no_skinny && A <= 64 && (size_t)(A <= 1 ? 1 : (A <= 8 ? 8 : (A <= 24 ? 24 : 64))) * H * 4 <= 200 * 1024;
-  const bool last_ok = !no_skinny && A <= 24 && ((size_t)B * apad(A) + 256 * apad(A)) * 4 <= 200 * 1024;
+  const bool last_ok = last_bwd_skinny_ok(B, A);
   static const bool no_side = dbg_getenv("IQL_B200_NO_SIDE_STREAM") != nullptr;
   const bool loss_recomputed = last_ok && e->bwd_phases.size() >= 2 &&
                                last_bwd_recomputes_loss_grads(H, A, e->bwd_phases[0].count * e->lb_splits, B / e->lb_splits) &&
@@ -1215,9 +1225,9 @@ static int enqueue_step(iql_engine* e, StepCtx& ctx, bool gather, cudaStream_t s
   const bool two_streams = tf32 && !tm && !no_side && e->side != nullptr;
   int forks = 0;
   // chained backward: the output-layer backward (phases 0, 1) runs as before, everything after it -- hidden dgrad /
-  // wgrad chain, input-layer wgrad (+ Adam + Polyak unless gradient-only) -- is ONE launch on CTA pairs
-  const bool chain = e->chain && tf32 && last_ok && e->bwd_phases.size() >= 3 && e->bwd_phases[0].kind == PH_LAST_WGRAD &&
-                     e->bwd_phases[1].kind == PH_LAST_DGRAD;
+  // wgrad chain, input-layer wgrad (+ Adam + Polyak unless gradient-only) -- is ONE launch on CTA pairs.  Bind time set
+  // e->chain only for shapes it serves (tf32, skinny output-layer backward, 2L + 1 phases), so what it reports runs.
+  const bool chain = e->chain;
   for (size_t i = 0; i < e->bwd_phases.size(); ++i) {
     if (chain && i >= 2) break;
     const Phase& ph = e->bwd_phases[i];

@@ -67,7 +67,8 @@ struct BwdChainArgs {
   long long seg_lo[4][FUSED_MAX_LAYERS + 2], seg_hi[4][FUSED_MAX_LAYERS + 2];
   float *params, *exp_avg, *exp_avg_sq, *target, *grads;
 };
-bool bwd_chain_supported(int batch, int hidden, int n_hidden, bool fused_fwd);
+// k0 = state_dim + action_dim: the input-layer wgrad phase runs one N tile per task, at most 256 wide
+bool bwd_chain_supported(int batch, int hidden, int n_hidden, int k0, bool fused_fwd);
 int bwd_chain_wgrad0_tile_n(int k0);
 void launch_bwd_chain(const BwdChainArgs& a, const StepCtx& ctx, cudaStream_t st);
 // bias gradients of a wgrad phase: dbias[m] = sum_k A[k][m]

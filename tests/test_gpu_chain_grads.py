@@ -72,8 +72,8 @@ def test_chain_grads_k_fusion_and_launch_count():
 
 def test_auto_selects_chain_grads_by_members_and_depth():
     """auto: a two-layer single learner keeps the per-phase backward, the 64-member ensemble and a three-layer single
-    learner run the gradient-only chain; a shape the chain does not support stays per-phase under auto and is refused
-    when the chain is asked for."""
+    learner run the gradient-only chain; a shape the chain does not support (batch, input width, action width) stays
+    per-phase under auto and is refused when a chain is asked for."""
     from jsrl_corl_b200 import EnsembleEngine
 
     single = EnsembleEngine(1, 17, 6, 256, 2, 256, False, "tf32", "cuda", 4)
@@ -86,3 +86,10 @@ def test_auto_selects_chain_grads_by_members_and_depth():
     assert not wide.paths["chained_backward_grads"]
     with pytest.raises(ValueError, match="chained backward"):
         EnsembleEngine(2, 11, 3, 256, 2, 512, True, "tf32", "cuda", 4, step_path="chain_grads")
+    # input width past one 256-column wgrad tile (K0 = 257, 306) and output-layer heads past the skinny backward (the
+    # adroit door / hammer / relocate shapes, A = 26..30): per-phase under auto, refused when a chain is asked for
+    for S_dim, A in ((251, 6), (300, 6), (39, 28), (46, 26), (39, 30)):
+        assert not EnsembleEngine(64, S_dim, A, 256, 2, 256, False, "tf32", "cuda", 4).paths["chained_backward_grads"]
+        for step_path in ("chain_grads", "chain"):
+            with pytest.raises(ValueError, match="action_dim <= 24, state_dim \\+ action_dim <= 256"):
+                EnsembleEngine(8, S_dim, A, 256, 2, 256, False, "tf32", "cuda", 4, step_path=step_path)
