@@ -157,6 +157,18 @@ int iql_set_option(iql_engine* e, int32_t key, int64_t value);
 #define IQL_INFO_CHAINED_BACKWARD_GRADS 4 /* chained backward storing the gradients, adam_polyak after it (4, or auto) */
 int iql_get_info(const iql_engine* e, int32_t key, int64_t* out);
 int iql_get_counters(iql_engine* e, int32_t member, iql_counters* out, void* stream);
+/* Per-member batch sizes (a batch-size axis of a hyper-parameter sweep, ray_hyperparam.py).  host_sizes[S] in HOST
+ * memory, 1 <= B_m <= batch_size (default: every B_m = batch_size).  Member m trains on rows [0, B_m) of the engine's
+ * batch: the gather writes zero rows past B_m and reads no index there, the losses and their gradients are means over
+ * B_m rows, and the kernels still run on all batch_size rows (the shapes, tiles and kernel paths of the handle stay
+ * those of batch_size).  In IQL_SAMPLE_PHILOX mode row b < B_m draws the index it draws at any batch size; idx_out
+ * holds -1 past B_m.  Index entries past B_m (iql_train_steps, iql_train_host_step) are never read or checked.  Read by
+ * the kernels at run time: a change takes effect at the next call without recapturing its graph.  iql_load_batch
+ * refuses a member whose B_m != batch_size (IQL_ERR_STATE).  IQL_ERR_INVALID: a null pointer or a size out of range
+ * (nothing is changed then). */
+int iql_set_batch_sizes(iql_engine* e, const int32_t* host_sizes);
+/* host_out[S]: the current B_m of every member. */
+int iql_get_batch_sizes(iql_engine* e, int32_t* host_out);
 /* replaces: copy.deepcopy(self.qf) iql.py:464,584,598 (q_target <- qf) */
 int iql_sync_target(iql_engine* e, int32_t member, void* stream);
 
@@ -210,7 +222,7 @@ int iql_replay_sample_host(const float* rows, const iql_row_layout* lay, int64_t
 int iql_bind_replay(iql_engine* e, int32_t member, const float* rows, int64_t capacity, int64_t size);
 int iql_set_replay_size(iql_engine* e, int32_t member, int64_t size);
 /* Stage an externally sampled batch for member (drop-in `train(batch)` path):
- * dense [B,S],[B,A],[B] or [B,1],[B,S],[B] or [B,1]. */
+ * dense [B,S],[B,A],[B] or [B,1],[B,S],[B] or [B,1].  IQL_ERR_STATE for a member whose B_m != B. */
 int iql_load_batch(iql_engine* e, int32_t member, const float* states, const float* actions,
                    const float* rewards, const float* next_states, const float* dones,
                    void* stream);

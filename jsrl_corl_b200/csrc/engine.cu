@@ -340,7 +340,11 @@ extern "C" int iql_create(const iql_config* cfg, iql_engine** out) {
   def.vf_lr = def.qf_lr = def.actor_lr = 3e-4;
   def.adam_beta1 = 0.9; def.adam_beta2 = 0.999; def.adam_eps = 1e-8;
   def.cosine_t_max = 1000000;
-  for (int m = 0; m < S; ++m) { def.seed = (uint64_t)m; iql_set_hparams(e, m, &def); }
+  for (int m = 0; m < S; ++m) {
+    e->h_scalars[m].batch = cfg->batch_size;
+    def.seed = (uint64_t)m;
+    iql_set_hparams(e, m, &def);
+  }
   const char* g = dbg_getenv("IQL_B200_GRAPHS");
   if (g && g[0] == '0') e->use_graphs = false;
   *out = e;
@@ -383,7 +387,9 @@ extern "C" int iql_set_hparams(iql_engine* e, int32_t member, const iql_hparams*
   if (hp->cosine_t_max < 0) return fail(e, IQL_ERR_INVALID, "iql_set_hparams: cosine_t_max must be >= 0");
   e->h_hparams[member] = *hp;
   MemberScalars& s = e->h_scalars[member];
+  const int32_t batch = s.batch;  // set by iql_set_batch_sizes, not a hyper-parameter of iql_hparams
   memset(&s, 0, sizeof(s));
+  s.batch = batch;
   s.beta = (float)hp->beta;
   s.iql_tau = (float)hp->iql_tau;
   s.discount = (float)hp->discount;
@@ -446,6 +452,24 @@ extern "C" int iql_get_counters(iql_engine* e, int32_t member, iql_counters* out
   (void)stream;  // the host shadow advances in lock-step with the device copy
   if (!e || !out || member < 0 || member >= e->cfg.n_members) return fail(e, IQL_ERR_INVALID, "iql_get_counters: bad member or null");
   *out = e->h_counters[member];
+  return IQL_OK;
+}
+
+extern "C" int iql_set_batch_sizes(iql_engine* e, const int32_t* host_sizes) {
+  if (!e || !host_sizes) return fail(e, IQL_ERR_INVALID, "iql_set_batch_sizes: null argument");
+  const int S = e->cfg.n_members;
+  for (int m = 0; m < S; ++m)
+    if (host_sizes[m] < 1 || host_sizes[m] > e->cfg.batch_size)
+      return fail(e, IQL_ERR_INVALID, "iql_set_batch_sizes: member " + std::to_string(m) + " has batch size " +
+                                          std::to_string(host_sizes[m]) + ", outside [1, " + std::to_string(e->cfg.batch_size) + "]");
+  for (int m = 0; m < S; ++m) e->h_scalars[m].batch = host_sizes[m];
+  e->scalars_dirty = true;  // uploaded with the scalars before the next launch; the graphs read the table at run time
+  return IQL_OK;
+}
+
+extern "C" int iql_get_batch_sizes(iql_engine* e, int32_t* host_out) {
+  if (!e || !host_out) return fail(e, IQL_ERR_INVALID, "iql_get_batch_sizes: null argument");
+  for (int m = 0; m < e->cfg.n_members; ++m) host_out[m] = e->h_scalars[m].batch;
   return IQL_OK;
 }
 
@@ -993,6 +1017,8 @@ extern "C" int iql_load_batch(iql_engine* e, int32_t member, const float* states
   if (!e || member < 0 || member >= e->cfg.n_members) return fail(e, IQL_ERR_INVALID, "iql_load_batch: bad member");
   if (!e->bound) return fail(e, IQL_ERR_STATE, "iql_load_batch: state not bound");
   if (!states || !actions || !rewards || !next_states || !dones) return fail(e, IQL_ERR_INVALID, "iql_load_batch: null batch tensor");
+  if (e->h_scalars[member].batch != e->cfg.batch_size)
+    return fail(e, IQL_ERR_STATE, "iql_load_batch: the member's batch size (iql_set_batch_sizes) differs from the engine's");
   StepCtx ctx = make_ctx(e);
   float* xrow = e->d_ws_f + (int64_t)member * e->wl.member_floats + e->wl.xrow;
   launch_load_batch(ctx, member, xrow, states, actions, rewards, next_states, dones, (cudaStream_t)stream);
@@ -1481,7 +1507,7 @@ extern "C" int iql_train_host_step(iql_engine* e, const int64_t* host_indices, f
   if (gather)
     for (int m = 0; m < S; ++m) {
       const int64_t cap = e->h_replay[m].capacity;
-      for (int b = 0; b < B; ++b) {
+      for (int b = 0; b < e->h_scalars[m].batch; ++b) {  // entries past B_m are never read
         const int64_t i = host_indices[(size_t)m * B + b];
         if (i < 0 || i >= cap) return fail(e, IQL_ERR_INVALID, "iql_train_host_step: index outside the bound replay buffer");
         mail_idx[(size_t)m * B + b] = i;

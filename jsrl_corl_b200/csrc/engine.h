@@ -50,7 +50,10 @@ struct MemberScalars {
   float adam_eps;
   float drop_scale;        // (float)(1/(1-p))
   uint32_t drop_threshold; // floor(p * 2^32); 0 = no dropout
-  uint32_t pad0;
+  // B_m (iql_set_batch_sizes), 1 <= B_m <= B: the member trains on rows [0, B_m) of the engine batch.  Every kernel runs
+  // on all B rows; the gather writes zero rows past B_m, and the loss (loss_kernel, loss_row_grads) skips them and
+  // divides by B_m, so their output-layer gradients -- and hence every gradient they feed -- are exact zeros.
+  int32_t batch;
   double adam_beta1_d, adam_beta2_d;
   double vf_lr, qf_lr, actor_lr, lr_eta_min;
   int64_t cosine_t_max;

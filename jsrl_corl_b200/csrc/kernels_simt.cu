@@ -184,15 +184,19 @@ __device__ __forceinline__ void gather_body(const StepCtx& ctx, float* __restric
   if (t >= ctx.B * Q) return;
   const int b = t / Q, q = t - b * Q;
   const ReplayBinding rb = ctx.replay[m];
-  int64_t idx;
-  if (ctx.indices) {
-    idx = ctx.indices[((int64_t)m * ctx.K + ctx.k) * ctx.B + b];
-  } else {
-    const uint64_t step = (uint64_t)(ctx.counters[m].sample_step + ctx.k);
-    idx = philox_index(ctx.scalars[m].seed, step, (uint32_t)b, (uint64_t)rb.size);
+  // rows past the member's batch B_m are zeros (a finite forward whatever the history) and read no index
+  const bool pad = b >= ctx.scalars[m].batch;
+  int64_t idx = -1;
+  if (!pad) {
+    if (ctx.indices) {
+      idx = ctx.indices[((int64_t)m * ctx.K + ctx.k) * ctx.B + b];
+    } else {
+      const uint64_t step = (uint64_t)(ctx.counters[m].sample_step + ctx.k);
+      idx = philox_index(ctx.scalars[m].seed, step, (uint32_t)b, (uint64_t)rb.size);
+    }
   }
   if (q == 0 && ctx.idx_out) ctx.idx_out[((int64_t)m * ctx.K + ctx.k) * ctx.B + b] = idx;
-  const float4 v = __ldg(reinterpret_cast<const float4*>(rb.rows + idx * RF) + q);
+  const float4 v = pad ? make_float4(0.f, 0.f, 0.f, 0.f) : __ldg(reinterpret_cast<const float4*>(rb.rows + idx * RF) + q);
   float* wm = ws + m * ws_member_floats;
   reinterpret_cast<float4*>(wm + xrow_off + (int64_t)b * RF)[q] = v;
   if (ctx.xhi_off) {  // TF32 hi / lo split of the row for the 3xTF32 input layer
@@ -311,7 +315,10 @@ __global__ void __launch_bounds__(256) loss_kernel(StepCtx ctx, float* __restric
   float* gy = w + wl.gy;
   float* gpi = w + wl.gpi;
   const MemberScalars sc = ctx.scalars[m];
-  const float inv_b = 1.0f / (float)B;
+  // the member's own batch: means over rows [0, B_m); pad rows are skipped (exp(beta * adv) of a zero row may overflow)
+  // and get exact-zero output gradients
+  const int Bm = sc.batch;
+  const float inv_b = 1.0f / (float)Bm;
   const float w_neg = fabsf(sc.iql_tau - 1.0f), w_pos = fabsf(sc.iql_tau);
   const float* log_std = params + m * ctx.P + ctx.log_std_off;
   constexpr float HALF_LOG_2PI = 0.9189385332046727f;
@@ -323,9 +330,15 @@ __global__ void __launch_bounds__(256) loss_kernel(StepCtx ctx, float* __restric
   float v_acc = 0.f, q1_acc = 0.f, q2_acc = 0.f, a_acc = 0.f;
   for (int b0 = 0; b0 < B; b0 += blockDim.x) {  // uniform trip count: every lane takes part in the shuffles
     const int b = b0 + threadIdx.x;
-    const bool valid = b < B;
+    const bool valid = b < Bm;
+    const bool pad = !valid && b < B;
     float adv = 0.f, e = 0.f, eb = 0.f;
     const float* xr = xrow + (int64_t)(valid ? b : 0) * RF;
+    if (pad) {
+      gy[0 * B + b] = 0.f;
+      gy[1 * B + b] = 0.f;
+      gy[2 * B + b] = 0.f;
+    }
     if (valid) {
       const float next_v = yq[PASS_V_NEXT * B + b];
       const float v = yq[PASS_V * B + b];
@@ -370,6 +383,8 @@ __global__ void __launch_bounds__(256) loss_kernel(StepCtx ctx, float* __restric
           dls = eb * (1.0f - diff * diff / var);
         }
         gpi[(int64_t)b * Ald + a] = gmu * (1.0f - mu * mu);
+      } else if (pad) {
+        gpi[(int64_t)b * Ald + a] = 0.f;
       }
       if (gauss && a < LOSS_MAX_A) {
         dls = warp_sum(dls);

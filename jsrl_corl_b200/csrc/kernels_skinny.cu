@@ -364,13 +364,14 @@ __device__ __forceinline__ void loss_row_grads(const StepCtx& ctx, const MemberS
                                                const WorkspaceLayout& wl, const float* __restrict__ log_std, int t, int b,
                                                float* g) {
   const int B = ctx.B, RF = ctx.row.row_floats;
+#pragma unroll
+  for (int a = 0; a < AMAX; ++a) g[a] = 0.f;
+  if (b >= sc.batch) return;  // pad row of a member with B_m < B: zero gradient (loss_kernel)
   const float* yq = w + wl.yq;
-  const float inv_b = 1.0f / (float)B;
+  const float inv_b = 1.0f / (float)sc.batch;
   const float v = yq[PASS_V * B + b];
   const float tq = fminf(yq[PASS_TQ1 * B + b], yq[PASS_TQ2 * B + b]);
   const float adv = tq - v;
-#pragma unroll
-  for (int a = 0; a < AMAX; ++a) g[a] = 0.f;
   if (t == 0) {  // V (expectile)
     const float w_neg = fabsf(sc.iql_tau - 1.0f), w_pos = fabsf(sc.iql_tau);
     const float wt = adv < 0.f ? w_neg : w_pos;

@@ -108,6 +108,7 @@ class EnsembleEngine:
         self.act_calls = 0
         self._act_in = self._act_out = self._act_in_dev = self._act_std = None
         self._hparams = [self._default_hparams(m) for m in range(n_members)]
+        self._batch_sizes = [batch_size] * n_members
         self._replay_refs: Dict[int, torch.Tensor] = {}
         self._idx_stage: Dict[int, torch.Tensor] = {}
         self._host_losses = None
@@ -147,6 +148,21 @@ class EnsembleEngine:
 
     def get_hparams(self, member: int) -> HParams:
         return self._hparams[member]
+
+    def set_batch_sizes(self, sizes):
+        """Per-member batch sizes B_m, 1 <= B_m <= batch_size (`iql_set_batch_sizes`): member m trains on rows
+        [0, B_m) of every sampled batch, and index entries past B_m are ignored.  Takes effect at the next call, also
+        on an already captured graph."""
+        arr = np.ascontiguousarray(sizes, dtype=np.int32).reshape(-1)
+        if arr.shape != (self.n_members,):
+            raise ValueError(f"need one batch size per member ({self.n_members}), got {arr.shape[0]}")
+        _lib.check(self._L.iql_set_batch_sizes(self._h, arr.ctypes.data), self._h, "iql_set_batch_sizes")
+        self._batch_sizes = arr.tolist()
+
+    @property
+    def batch_sizes(self) -> List[int]:
+        """The members' batch sizes B_m (a copy; the per-step host loop reads it without a library call)."""
+        return list(self._batch_sizes)
 
     def get_counters(self, member: int) -> Counters:
         c = Counters()
@@ -349,7 +365,8 @@ class EnsembleEngine:
                     dropout_masks: Optional[torch.Tensor] = None, return_indices: bool = False,
                     out: Optional[torch.Tensor] = None):
         """Run K update steps for all members; returns losses [S, K, 3]
-        (value_loss, q_loss, actor_loss) on the device, asynchronously."""
+        (value_loss, q_loss, actor_loss) on the device, asynchronously.  `indices` [S, K, B]: entries past a
+        member's batch size B_m are ignored; `return_indices` gives -1 there."""
         S, B = self.n_members, self.batch_size
         smode = {"philox": _lib.SAMPLE_PHILOX, "indices": _lib.SAMPLE_INDICES, "preloaded": _lib.SAMPLE_PRELOADED}[mode]
         idx_ptr = None

@@ -45,9 +45,21 @@ class IQLEnsemble:
                  batch_size: int = 256, deterministic: bool = False, actor_dropout: float = 0.0,
                  math_mode: str = "tf32", device="cuda", max_steps_per_call: int = 256,
                  seeds: Optional[Sequence[int]] = None, hparams: Optional[Sequence[Dict[str, Any]]] = None,
-                 init: bool = True, step_path: str = "auto"):
+                 init: bool = True, step_path: str = "auto", batch_sizes: Optional[Sequence[int]] = None):
+        """``batch_size`` is the engine's batch B: it sizes the workspace and picks the kernels.  ``batch_sizes``: one
+        batch size per member, each in [1, B] (default: all B); member m then trains on B_m rows of every batch, as if
+        it were an ensemble of batch B_m, while the kernels still run B rows (see ``EnsembleEngine.set_batch_sizes``)."""
+        if batch_sizes is not None:
+            batch_sizes = [int(b) for b in batch_sizes]
+            if len(batch_sizes) != n_members:
+                raise ValueError(f"batch_sizes needs one entry per member ({n_members}), got {len(batch_sizes)}")
+            bad = [b for b in batch_sizes if not 1 <= b <= batch_size]
+            if bad:
+                raise ValueError(f"batch_sizes must lie in [1, batch_size={batch_size}], got {bad}")
         self.engine = EnsembleEngine(n_members, state_dim, action_dim, hidden_dim, n_hidden, batch_size,
                                      deterministic, math_mode, device, max_steps_per_call, step_path=step_path)
+        if batch_sizes is not None:
+            self.engine.set_batch_sizes(batch_sizes)
         self.n_members = n_members
         self.actor_dropout = actor_dropout
         self.guide: Optional["IQLEnsemble"] = None  # set_guide
@@ -96,11 +108,14 @@ class IQLEnsemble:
         """ONE update step of every member with the losses on the host when it returns ([S, 3] float32:
         value_loss, q_loss, actor_loss) -- the ensemble form of the reference's `log_dict = trainer.train(batch)`
         (offline/iql.py:631-635), for loops that log or branch on the losses every step.  ``indices``: [S, B] int64 rows of
-        the bound buffers (drawn here with numpy, like `ReplayBuffer.sample`, when omitted).  Runs through
-        `iql_train_host_step`: one graph launch, the call returns while the backward of the step is still running."""
+        the bound buffers (member m's first B_m drawn here with numpy, like `ReplayBuffer.sample(B_m)`, when omitted;
+        entries past B_m are ignored).  Runs through `iql_train_host_step`: one graph launch, the call returns while the
+        backward of the step is still running."""
         e = self.engine
         if indices is None:
-            indices = np.stack([np.random.randint(0, rb._high(), size=e.batch_size) for rb in self._buffers])
+            indices = np.zeros((e.n_members, e.batch_size), dtype=np.int64)
+            for m, (rb, bm) in enumerate(zip(self._buffers, e._batch_sizes)):
+                indices[m, :bm] = np.random.randint(0, rb._high(), size=bm)
         idx = np.ascontiguousarray(indices, dtype=np.int64)
         if idx.shape != (e.n_members, e.batch_size):
             raise ValueError(f"indices must be [{e.n_members}, {e.batch_size}]")
