@@ -169,6 +169,22 @@ int iql_get_counters(iql_engine* e, int32_t member, iql_counters* out, void* str
 int iql_set_batch_sizes(iql_engine* e, const int32_t* host_sizes);
 /* host_out[S]: the current B_m of every member. */
 int iql_get_batch_sizes(iql_engine* e, int32_t* host_out);
+/* Members that train (the early stopping of a hyper-parameter search, ray_hyperparam.py's ASHA scheduler).
+ * host_ids[n]: member indices in HOST memory, any order, any non-empty subset; default: every member.  Retiring and
+ * resuming are the same call.  The problem tables, tensor maps and chained-backward tasks are rebuilt over the listed
+ * members only, so the others launch no CTA in any step, and every path choice that depends on the member count (auto
+ * chained backward, CTA pairs, narrow dgrad tiles, the fused forward's wide epilogue, the tensor-core policy head) is
+ * re-made from n; the workspace split chosen at iql_create (row-split output-layer backward, K-split input-layer
+ * weight gradient) stays.  Inactive members are frozen: parameters, moments, target, gradients, counters and B_m keep
+ * every bit, and a resumed member continues as if no time had passed.  They still serve iql_act*, inserts,
+ * iql_sync_target and the tensor views.  Their iql_train_steps loss rows are NaN and their idx_out rows -1; their
+ * iql_train_host_step / iql_host_step_wait losses are NaN; their index entries are never read or checked.  A host step
+ * still in flight is collected first (its losses are dropped).  Host cost: the tensor maps are encoded again, and the
+ * captured graphs are dropped.  IQL_ERR_INVALID: null ids, n < 1, an id out of range or listed twice (nothing changes);
+ * IQL_ERR_STATE: before iql_bind_state. */
+int iql_set_active_members(iql_engine* e, int32_t n, const int32_t* host_ids);
+/* host_mask[S]: 1 for the members that train, 0 for the others. */
+int iql_get_active_members(iql_engine* e, int8_t* host_mask);
 /* replaces: copy.deepcopy(self.qf) iql.py:464,584,598 (q_target <- qf) */
 int iql_sync_target(iql_engine* e, int32_t member, void* stream);
 

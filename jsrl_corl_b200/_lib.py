@@ -98,6 +98,8 @@ SYMBOLS = {
     "iql_get_counters": (C.c_int, [_P, C.c_int32, C.POINTER(Counters), _P]),
     "iql_set_batch_sizes": (C.c_int, [_P, _P]),
     "iql_get_batch_sizes": (C.c_int, [_P, _P]),
+    "iql_set_active_members": (C.c_int, [_P, C.c_int32, _P]),
+    "iql_get_active_members": (C.c_int, [_P, _P]),
     "iql_sync_target": (C.c_int, [_P, C.c_int32, _P]),
     "iql_replay_row_layout": (C.c_int, [C.c_int32, C.c_int32, C.POINTER(RowLayout)]),
     "iql_replay_pack": (C.c_int, [_P, C.POINTER(RowLayout), C.c_int64, C.c_int64, _P, _P, _P, _P, _P, _P]),

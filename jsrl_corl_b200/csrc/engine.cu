@@ -107,6 +107,7 @@ struct iql_engine {
   int64_t* d_act_off = nullptr;  // [2][L+1]
   float* d_loss_ring = nullptr;
   AdamScalars* d_adam_sc = nullptr;  // [S][3], written by the loss kernel, read by the optimizer kernel
+  int32_t* d_active = nullptr;   // [S] device copy of `active` (the first active.size() entries)
   float* d_wshadow = nullptr;    // [S][P]  TF32-rounded params  (tcgen05 mode)
   float* d_tshadow = nullptr;    // [S][PQ] TF32-rounded target
   float* d_wshadow_lo = nullptr; // lo parts (first-layer ranges) for the 3xTF32 input layer
@@ -146,6 +147,10 @@ struct iql_engine {
   std::vector<Phase> fwd_phases, bwd_phases;
   bool bound = false, tables_dirty = true, scalars_dirty = true, counters_dirty = true, replay_dirty = true;
   std::vector<char> preloaded;
+  // members that train (iql_set_active_members), ascending.  The problem tables, tensor maps and chain tasks hold these
+  // members only, and every bind-time choice that depends on the member count is made from active.size().
+  std::vector<int32_t> active;
+  std::vector<char> is_active;   // [S]
   int64_t last_launches = 0;
   std::string err;
   // CUDA graphs of the K-step sequence, keyed by K (Philox sampling mode only)
@@ -295,6 +300,7 @@ static void build_layout(iql_engine* e) {
   tab(sizeof(int64_t) * 2 * (L + 1));
   tab(sizeof(float) * 3 * (int64_t)S * c.max_steps_per_call);
   tab(sizeof(AdamScalars) * 3 * S);
+  tab(sizeof(int32_t) * S);
   if (c.math_mode == IQL_MATH_TF32_TCGEN05) {
     tab(sizeof(float) * (int64_t)S * e->layout.param_floats);
     tab(sizeof(float) * (int64_t)S * e->layout.q_floats);
@@ -334,6 +340,9 @@ extern "C" int iql_create(const iql_config* cfg, iql_engine** out) {
   e->h_counters.assign(S, iql_counters{0, 0, 0, 0, 0, 0});
   e->h_replay.assign(S, ReplayBinding{nullptr, 0, 0});
   e->preloaded.assign(S, 0);
+  e->active.resize(S);
+  for (int m = 0; m < S; ++m) e->active[m] = m;
+  e->is_active.assign(S, 1);
   iql_hparams def;
   memset(&def, 0, sizeof(def));
   def.beta = 3.0; def.iql_tau = 0.7; def.discount = 0.99; def.tau = 0.005;
@@ -475,7 +484,7 @@ extern "C" int iql_get_batch_sizes(iql_engine* e, int32_t* host_out) {
 
 static void build_problems(iql_engine* e) {
   const iql_config& c = e->cfg;
-  const int S = c.n_members, L = c.n_hidden, H = c.hidden_dim, B = c.batch_size;
+  const int Sa = (int)e->active.size(), L = c.n_hidden, H = c.hidden_dim, B = c.batch_size;
   const int ROW = e->layout.row.row_floats;
   const WorkspaceLayout& wl = e->wl;
   const int64_t P = e->layout.param_floats, PQ = e->layout.q_floats;
@@ -509,7 +518,7 @@ static void build_problems(iql_engine* e) {
     Phase ph; ph.mode = 0; ph.first = (int)e->h_probs.size(); ph.maxM = B; ph.maxN = 0; ph.K = 0; ph.umma_ok = false;
     // pass-major order: the six scalar-head passes of all members first, the policy pass last
     for (int f = 0; f < N_PASS; ++f)
-      for (int m = 0; m < S; ++m) {
+      for (const int m : e->active) {
         const PassDef& pd = passes[f];
         const float* blk = pd.tgt ? e->target + (int64_t)m * PQ : e->params + (int64_t)m * P;
         GemmProb p = blank();
@@ -553,7 +562,7 @@ static void build_problems(iql_engine* e) {
     Phase pw; pw.mode = 2; pw.first = (int)e->h_probs.size(); pw.maxM = 0; pw.maxN = 0; pw.K = B; pw.umma_ok = (l < L);
     pw.epi = EPI_NONE;
     pw.kind = (l == L) ? PH_LAST_WGRAD : (l == 0 ? PH_FIRST_WGRAD : PH_GENERIC);
-    for (int m = 0; m < S; ++m)
+    for (const int m : e->active)
       for (int t = 0; t < 4; ++t) {
         const int net = tr[t].net, f = tr[t].pass;
         const PassDef& pd = passes[f];
@@ -581,7 +590,7 @@ static void build_problems(iql_engine* e) {
     Phase px; px.mode = 1; px.first = (int)e->h_probs.size(); px.maxM = B; px.maxN = H; px.K = (l < L) ? H : 0; px.umma_ok = (l < L);
     px.epi = EPI_DRELU;
     px.kind = (l == L) ? PH_LAST_DGRAD : PH_GENERIC;
-    for (int m = 0; m < S; ++m)
+    for (const int m : e->active)
       for (int t = 0; t < 4; ++t) {
         const int net = tr[t].net, f = tr[t].pass;
         GemmProb p = blank();
@@ -616,9 +625,9 @@ static void build_problems(iql_engine* e) {
     const Phase pw0 = e->bwd_phases[0], pn0 = e->bwd_phases[1], pv0 = e->bwd_phases[2];
     for (int which = 0; which < 3; ++which)
       for (int s_ = 0; s_ < sp; ++s_)
-        for (int m = 0; m < S; ++m)
+        for (int mi = 0; mi < Sa; ++mi)
           for (int t = 0; t < 4; ++t) {
-            const int i = m * 4 + t;
+            const int m = e->active[mi], i = mi * 4 + t;  // position of (member, net) in the phase
             float* scr = wsm(m) + wl.lb_scratch + ((int64_t)t * sp + s_) * wl.lb_stride;
             GemmProb p;
             if (which == 0) {  // dgrad: rows [s Bs, (s + 1) Bs)
@@ -649,9 +658,10 @@ static void build_problems(iql_engine* e) {
     pf.first = (int)e->h_probs.size();
     pf.K = Bs;
     for (int s_ = 0; s_ < sp; ++s_)
-      for (int m = 0; m < S; ++m)
+      for (int mi = 0; mi < Sa; ++mi)
         for (int t = 0; t < 4; ++t) {
-          GemmProb p = e->h_probs[p0.first + m * 4 + t];
+          const int m = e->active[mi];
+          GemmProb p = e->h_probs[p0.first + mi * 4 + t];
           float* scr = wsm(m) + wl.fw_scratch + ((int64_t)t * sp + s_) * wl.fw_stride;
           p.A += (int64_t)s_ * Bs * p.lda;
           p.B += (int64_t)s_ * Bs * p.ldb;
@@ -667,42 +677,13 @@ static void build_problems(iql_engine* e) {
   }
 }
 
-extern "C" int iql_bind_state(iql_engine* e, float* params, float* exp_avg, float* exp_avg_sq, float* target,
-                              float* grads, void* workspace, size_t workspace_bytes) {
-  if (!e) return IQL_ERR_INVALID;
-  if (!params || !exp_avg || !exp_avg_sq || !target || !grads || !workspace)
-    return fail(e, IQL_ERR_INVALID, "iql_bind_state: null device pointer");
-  if ((int64_t)workspace_bytes < e->layout.workspace_bytes) return fail(e, IQL_ERR_INVALID, "iql_bind_state: workspace too small");
-  const uintptr_t all = (uintptr_t)params | (uintptr_t)exp_avg | (uintptr_t)exp_avg_sq | (uintptr_t)target |
-                        (uintptr_t)grads | (uintptr_t)workspace;
-  if (all & 127) return fail(e, IQL_ERR_INVALID, "iql_bind_state: pointers must be 128-byte aligned");
-  e->params = params; e->exp_avg = exp_avg; e->exp_avg_sq = exp_avg_sq; e->target = target; e->grads = grads;
-  e->ws = (char*)workspace; e->ws_bytes = workspace_bytes;
-  const int S = e->cfg.n_members, L = e->cfg.n_hidden;
-  const int64_t nprob = (int64_t)S * ((L + 1) * N_PASS + 4 * (L + 1) + 4 * L) + (e->lb_splits > 1 ? (int64_t)12 * S * e->lb_splits : 0) +
-                        (e->fw_splits > 1 ? (int64_t)4 * S * e->fw_splits : 0);
-  int64_t tb = 0;
-  auto tab = [&](int64_t bytes) { char* o = e->ws + tb; tb = round_up(tb + bytes, 256); return o; };
-  e->d_scalars = (MemberScalars*)tab(sizeof(MemberScalars) * S);
-  e->d_counters = (iql_counters*)tab(sizeof(iql_counters) * S);
-  e->d_replay = (ReplayBinding*)tab(sizeof(ReplayBinding) * S);
-  e->d_probs = (GemmProb*)tab(sizeof(GemmProb) * nprob);
-  e->d_maps = tab(128 * 2 * nprob);
-  e->d_act_off = (int64_t*)tab(sizeof(int64_t) * 2 * (L + 1));
-  e->d_loss_ring = (float*)tab(sizeof(float) * 3 * (int64_t)S * e->cfg.max_steps_per_call);
-  e->d_adam_sc = (AdamScalars*)tab(sizeof(AdamScalars) * 3 * S);
-  if (e->cfg.math_mode == IQL_MATH_TF32_TCGEN05) {
-    e->d_wshadow = (float*)tab(sizeof(float) * (int64_t)S * e->layout.param_floats);
-    e->d_tshadow = (float*)tab(sizeof(float) * (int64_t)S * e->layout.q_floats);
-    e->d_wshadow_lo = (float*)tab(sizeof(float) * (int64_t)S * e->layout.param_floats);
-    e->d_tshadow_lo = (float*)tab(sizeof(float) * (int64_t)S * e->layout.q_floats);
-    e->d_maps_first = tab((int64_t)128 * 4 * S * N_PASS);
-    e->d_maps_store = tab((int64_t)128 * L * S * N_PASS);
-    e->d_maps_c = tab((int64_t)128 * nprob);
-    e->d_maps_chain = tab((int64_t)128 * 2 * 4 * S * (2 * L));
-    e->d_maps_pol = tab((int64_t)128 * 4 * S);
-  }
-  e->d_ws_f = (float*)(e->ws + e->tables_bytes);
+// The part of binding that depends on which members train: problem tables, tensor maps, the chained backward's task
+// list and every path choice made from the member count.  Run by iql_bind_state and again by iql_set_active_members;
+// the workspace split (lb_splits / fw_splits) stays as iql_create sized it.
+static int bind_tables(iql_engine* e) {
+  const int Sa = (int)e->active.size(), L = e->cfg.n_hidden;
+  const int64_t nprob = (int64_t)Sa * ((L + 1) * N_PASS + 4 * (L + 1) + 4 * L) + (e->lb_splits > 1 ? (int64_t)12 * Sa * e->lb_splits : 0) +
+                        (e->fw_splits > 1 ? (int64_t)4 * Sa * e->fw_splits : 0);
   build_problems(e);
   const bool tc_mode = e->cfg.math_mode == IQL_MATH_TF32_TCGEN05 && umma_phase_supported(0, e->cfg.batch_size, e->cfg.hidden_dim);
   // 3xTF32 input layer, and on top of it the fused forward (all hidden layers of a tile chained through TMEM)
@@ -782,7 +763,7 @@ extern "C" int iql_bind_state(iql_engine* e, float* params, float* exp_avg, floa
         }
     e->h_maps_store.clear();
     if (e->fused_fwd) {  // outputs H_1..H_L of every forward problem, stored by TMA from the fused kernel
-      const int L = e->cfg.n_hidden, np = e->fwd_phases[0].count;
+      const int np = e->fwd_phases[0].count;
       e->h_maps_store.assign((size_t)128 * L * np, 0);
       for (int l = 0; l < L; ++l)
         for (int i = 0; i < np; ++i) {
@@ -797,9 +778,8 @@ extern "C" int iql_bind_state(iql_engine* e, float* params, float* exp_avg, floa
   e->h_maps_pol.clear();
   if (tc_mode && e->fused_fwd && !fused_fwd_policy_head(e->cfg.action_dim) && e->cfg.action_dim <= 32 &&
       dbg_getenv("IQL_B200_NO_POL_UMMA") == nullptr) {
-    const int L = e->cfg.n_hidden;
     const Phase& pout = e->fwd_phases[L];
-    const int n_scalar = (N_PASS - 1) * S;
+    const int n_scalar = (N_PASS - 1) * Sa;
     std::vector<GemmProb> hi(e->h_probs.begin() + pout.first + n_scalar, e->h_probs.begin() + pout.first + pout.count), lo = hi;
     const int64_t P = e->layout.param_floats;
     for (size_t i = 0; i < hi.size(); ++i) {
@@ -809,7 +789,7 @@ extern "C" int iql_bind_state(iql_engine* e, float* params, float* exp_avg, floa
       lo[i].B = e->d_wshadow_lo + (int64_t)m * P + w_off;
     }
     e->h_maps_pol.assign((size_t)128 * 4 * hi.size(), 0);
-    if ((int)hi.size() == S &&
+    if ((int)hi.size() == Sa &&
         umma_encode_maps_split(hi.data(), lo.data(), (int)hi.size(), umma_tile_n(e->cfg.action_dim), e->h_maps_pol.data(), false) == 0)
       e->pol_umma = true;
     else
@@ -824,11 +804,11 @@ extern "C" int iql_bind_state(iql_engine* e, float* params, float* exp_avg, floa
   // follows.  "auto" takes 4 from CHAIN_GRADS_MIN_MEMBERS members on, or with 3+ hidden layers: below that the
   // per-phase kernels' narrow dgrad units spread a two-layer step of few tasks over more SMs (DESIGN.md section 8).
   const bool want_chain = e->step_path == 2 || e->step_path == 4 ||
-                          (e->step_path == 0 && (S >= CHAIN_GRADS_MIN_MEMBERS || e->cfg.n_hidden >= 3));
+                          (e->step_path == 0 && (Sa >= CHAIN_GRADS_MIN_MEMBERS || e->cfg.n_hidden >= 3));
   if (tc_mode && want_chain && e->fw_splits == 1 && last_bwd_skinny_ok(e->cfg.batch_size, e->cfg.action_dim) &&
       bwd_chain_supported(e->cfg.batch_size, e->cfg.hidden_dim, e->cfg.n_hidden, e->cfg.state_dim + e->cfg.action_dim,
                           e->fused_fwd)) {
-    const int L = e->cfg.n_hidden, ntask = 4 * S;
+    const int ntask = 4 * Sa;
     BwdChainArgs& ca = e->chain_args;
     memset(&ca, 0, sizeof(ca));
     e->h_maps_chain.assign((size_t)128 * 2 * ntask * (2 * L), 0);
@@ -883,6 +863,48 @@ extern "C" int iql_bind_state(iql_engine* e, float* params, float* exp_avg, floa
     return fail(e, IQL_ERR_INVALID, "iql_bind_state: IQL_OPT_STEP_PATH = chained backward, but this shape / math mode does not support it "
                                     "(needs tf32, hidden 256, batch 256, 2..4 hidden layers, action_dim <= 24, "
                                     "state_dim + action_dim <= 256)");
+  return IQL_OK;
+}
+
+extern "C" int iql_bind_state(iql_engine* e, float* params, float* exp_avg, float* exp_avg_sq, float* target,
+                              float* grads, void* workspace, size_t workspace_bytes) {
+  if (!e) return IQL_ERR_INVALID;
+  if (!params || !exp_avg || !exp_avg_sq || !target || !grads || !workspace)
+    return fail(e, IQL_ERR_INVALID, "iql_bind_state: null device pointer");
+  if ((int64_t)workspace_bytes < e->layout.workspace_bytes) return fail(e, IQL_ERR_INVALID, "iql_bind_state: workspace too small");
+  const uintptr_t all = (uintptr_t)params | (uintptr_t)exp_avg | (uintptr_t)exp_avg_sq | (uintptr_t)target |
+                        (uintptr_t)grads | (uintptr_t)workspace;
+  if (all & 127) return fail(e, IQL_ERR_INVALID, "iql_bind_state: pointers must be 128-byte aligned");
+  e->params = params; e->exp_avg = exp_avg; e->exp_avg_sq = exp_avg_sq; e->target = target; e->grads = grads;
+  e->ws = (char*)workspace; e->ws_bytes = workspace_bytes;
+  const int S = e->cfg.n_members, L = e->cfg.n_hidden;
+  const int64_t nprob = (int64_t)S * ((L + 1) * N_PASS + 4 * (L + 1) + 4 * L) + (e->lb_splits > 1 ? (int64_t)12 * S * e->lb_splits : 0) +
+                        (e->fw_splits > 1 ? (int64_t)4 * S * e->fw_splits : 0);
+  int64_t tb = 0;
+  auto tab = [&](int64_t bytes) { char* o = e->ws + tb; tb = round_up(tb + bytes, 256); return o; };
+  e->d_scalars = (MemberScalars*)tab(sizeof(MemberScalars) * S);
+  e->d_counters = (iql_counters*)tab(sizeof(iql_counters) * S);
+  e->d_replay = (ReplayBinding*)tab(sizeof(ReplayBinding) * S);
+  e->d_probs = (GemmProb*)tab(sizeof(GemmProb) * nprob);
+  e->d_maps = tab(128 * 2 * nprob);
+  e->d_act_off = (int64_t*)tab(sizeof(int64_t) * 2 * (L + 1));
+  e->d_loss_ring = (float*)tab(sizeof(float) * 3 * (int64_t)S * e->cfg.max_steps_per_call);
+  e->d_adam_sc = (AdamScalars*)tab(sizeof(AdamScalars) * 3 * S);
+  e->d_active = (int32_t*)tab(sizeof(int32_t) * S);
+  if (e->cfg.math_mode == IQL_MATH_TF32_TCGEN05) {
+    e->d_wshadow = (float*)tab(sizeof(float) * (int64_t)S * e->layout.param_floats);
+    e->d_tshadow = (float*)tab(sizeof(float) * (int64_t)S * e->layout.q_floats);
+    e->d_wshadow_lo = (float*)tab(sizeof(float) * (int64_t)S * e->layout.param_floats);
+    e->d_tshadow_lo = (float*)tab(sizeof(float) * (int64_t)S * e->layout.q_floats);
+    e->d_maps_first = tab((int64_t)128 * 4 * S * N_PASS);
+    e->d_maps_store = tab((int64_t)128 * L * S * N_PASS);
+    e->d_maps_c = tab((int64_t)128 * nprob);
+    e->d_maps_chain = tab((int64_t)128 * 2 * 4 * S * (2 * L));
+    e->d_maps_pol = tab((int64_t)128 * 4 * S);
+  }
+  e->d_ws_f = (float*)(e->ws + e->tables_bytes);
+  int rc = bind_tables(e);
+  if (rc != IQL_OK) return rc;
   if (!e->side) {  // optional: without it the backward simply stays on one stream
     if (cudaStreamCreateWithFlags(&e->side, cudaStreamNonBlocking) != cudaSuccess ||
         cudaEventCreateWithFlags(&e->ev_fork, cudaEventDisableTiming) != cudaSuccess ||
@@ -925,6 +947,11 @@ static int flush_tables(iql_engine* e, cudaStream_t st) {
       off[L + 1 + l] = e->b_off[IQL_NET_ACTOR][l];
     }
     CUDA_TRY(e, cudaMemcpyAsync(e->d_act_off, off.data(), sizeof(int64_t) * off.size(), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(e, cudaMemcpyAsync(e->d_active, e->active.data(), sizeof(int32_t) * e->active.size(), cudaMemcpyHostToDevice, st));
+    // loss rows of members that do not train read NaN (all-ones bytes) until they train again
+    const size_t ring_row = sizeof(float) * 3 * (size_t)e->cfg.max_steps_per_call;
+    for (int m = 0; m < S; ++m)
+      if (!e->is_active[m]) CUDA_TRY(e, cudaMemsetAsync((char*)e->d_loss_ring + ring_row * m, 0xFF, ring_row, st));
     CUDA_TRY(e, cudaStreamSynchronize(st));  // `off` is a stack temporary
     e->tables_dirty = false;
   }
@@ -949,7 +976,8 @@ static StepCtx make_ctx(const iql_engine* e) {
   c.B = e->cfg.batch_size;
   c.S_dim = e->cfg.state_dim; c.A_dim = e->cfg.action_dim; c.H = e->cfg.hidden_dim; c.L = e->cfg.n_hidden;
   c.deterministic = e->cfg.deterministic;
-  c.n_members = e->cfg.n_members;
+  c.n_active = (int)e->active.size();
+  c.active = (int)e->active.size() < e->cfg.n_members ? e->d_active : nullptr;
   c.P = e->layout.param_floats; c.PQ = e->layout.q_floats;
   c.v_begin = e->layout.v_begin; c.v_end = e->layout.v_end;
   c.a_begin = e->layout.actor_begin; c.a_end = e->layout.actor_end;
@@ -1042,7 +1070,7 @@ static void launch_chain(iql_engine* e, const StepCtx& ctx, cudaStream_t st, Ste
       }
     }
     if (!e->chain_grads)  // p, m, v in and out + shadows
-      by += e->cfg.n_members * 4.0 * ((6.0 + 1.0) * e->layout.param_floats + 3.0 * e->layout.q_floats);
+      by += e->active.size() * 4.0 * ((6.0 + 1.0) * e->layout.param_floats + 3.0 * e->layout.q_floats);
     tm->flops.back() = fl;
     tm->bytes.back() = by;
   }
@@ -1066,7 +1094,7 @@ static int enqueue_step(iql_engine* e, StepCtx& ctx, bool gather, cudaStream_t s
   int launches = 0;
   cudaStream_t st = st_main;  // the stream run_phase launches on (switched to e->side for the wgrad leaves)
   const bool tf32 = e->cfg.math_mode == IQL_MATH_TF32_TCGEN05;
-  const double S_d = e->cfg.n_members;
+  const double S_d = (double)e->active.size();
   if (gather) {
     if (tm) tm->mark("gather", 0, 2.0 * S_d * e->cfg.batch_size * e->layout.row.row_floats * 4);
     launch_gather(ctx, e->d_ws_f, e->wl.member_floats, e->wl.xrow, st);
@@ -1129,7 +1157,7 @@ static int enqueue_step(iql_engine* e, StepCtx& ctx, bool gather, cudaStream_t s
       // forward, last hidden layer: fuse the FP32 output Linear into the epilogue and skip the next phase
       const bool fuse = ph.mode == 0 && ph.epi == EPI_RELU && next && next->kind == PH_OUT_FWD && H == 256 &&
                         umma_can_fuse_out(A);
-      const int n_scalar = (N_PASS - 1) * e->cfg.n_members;  // problems with a scalar head (V, Q passes)
+      const int n_scalar = (N_PASS - 1) * (int)e->active.size();  // problems with a scalar head (V, Q passes)
       launch_umma_gemm(ph.mode, pp, split ? e->d_maps_first : e->d_maps + (size_t)256 * ph.first,
                        fuse ? e->d_probs + next->first : nullptr, ph.epi, ph.count, ph.maxM, ph.maxN, ctx, st, split,
                        n_scalar, ph.cta2, ph.maxK, ph.rowepi ? e->d_maps_c + (size_t)128 * ph.first : nullptr, ph.tile_n);
@@ -1182,7 +1210,7 @@ static int enqueue_step(iql_engine* e, StepCtx& ctx, bool gather, cudaStream_t s
   if (tf32 && e->fused_fwd) {
     // one launch for layers 0..L-1 + scalar heads; the policy head (N = act_dim) stays with the FP32 output kernel
     const int L = c.n_hidden;
-    const int n_scalar = (N_PASS - 1) * c.n_members;
+    const int n_scalar = (N_PASS - 1) * (int)e->active.size();
     const Phase& pout = e->fwd_phases[L];
     FusedFwdArgs fa;
     memset(&fa, 0, sizeof(fa));
@@ -1349,13 +1377,13 @@ extern "C" int iql_train_steps(iql_engine* e, int32_t k_steps, int32_t sample_mo
     if (!indices) return fail(e, IQL_ERR_INVALID, "iql_train_steps: IQL_SAMPLE_INDICES needs indices");
   } else if (sample_mode == IQL_SAMPLE_PRELOADED) {
     if (k_steps != 1) return fail(e, IQL_ERR_INVALID, "iql_train_steps: IQL_SAMPLE_PRELOADED runs exactly one step");
-    for (int m = 0; m < S; ++m)
+    for (const int m : e->active)
       if (!e->preloaded[m]) return fail(e, IQL_ERR_STATE, "iql_train_steps: no batch staged (call iql_load_batch)");
   } else if (sample_mode != IQL_SAMPLE_PHILOX) {
     return fail(e, IQL_ERR_INVALID, "iql_train_steps: unknown sample_mode");
   }
   if (sample_mode != IQL_SAMPLE_PRELOADED)
-    for (int m = 0; m < S; ++m) {
+    for (const int m : e->active) {
       if (!e->h_replay[m].rows) return fail(e, IQL_ERR_STATE, "iql_train_steps: replay buffer not bound");
       if (e->h_replay[m].size <= 0 && sample_mode == IQL_SAMPLE_PHILOX)
         return fail(e, IQL_ERR_INVALID, "iql_train_steps: cannot sample from an empty replay buffer");
@@ -1418,12 +1446,17 @@ extern "C" int iql_train_steps(iql_engine* e, int32_t k_steps, int32_t sample_mo
     if (ctx.advance_k != -1) { launch_advance(ctx, k_steps, st); ++launches; }
   }
   CUDA_TRY(e, cudaGetLastError());
-  for (int m = 0; m < S; ++m) {
+  for (const int m : e->active) {
     iql_counters& c = e->h_counters[m];
     c.v_step += k_steps; c.q_step += k_steps; c.actor_step += k_steps; c.total_it += k_steps; c.sample_step += k_steps;
     if (e->h_hparams[m].cosine_t_max > 0) c.sched_epoch += k_steps;
     e->preloaded[m] = 0;
   }
+  if (idx_out)  // the gather writes the rows of the members that trained; the others read -1 (all-ones bytes)
+    for (int m = 0; m < S; ++m)
+      if (!e->is_active[m])
+        CUDA_TRY(e, cudaMemsetAsync(idx_out + (size_t)m * k_steps * e->cfg.batch_size, 0xFF,
+                                    sizeof(int64_t) * (size_t)k_steps * e->cfg.batch_size, st));
   if (out_losses) {
     const size_t row = sizeof(float) * 3 * (size_t)k_steps;
     CUDA_TRY(e, cudaMemcpy2DAsync(out_losses, row, e->d_loss_ring, sizeof(float) * 3 * (size_t)e->cfg.max_steps_per_call, row, S,
@@ -1481,7 +1514,7 @@ extern "C" int iql_train_host_step(iql_engine* e, const int64_t* host_indices, f
   if (!st) return fail(e, IQL_ERR_INVALID, "iql_train_host_step: needs a non-default stream (graph capture)");
   const int S = e->cfg.n_members, B = e->cfg.batch_size;
   const bool gather = host_indices != nullptr;
-  for (int m = 0; m < S; ++m) {
+  for (const int m : e->active) {
     if (gather && !e->h_replay[m].rows) return fail(e, IQL_ERR_STATE, "iql_train_host_step: replay buffer not bound");
     if (!gather && !e->preloaded[m]) return fail(e, IQL_ERR_STATE, "iql_train_host_step: no batch staged (call iql_load_batch)");
   }
@@ -1505,7 +1538,7 @@ extern "C" int iql_train_host_step(iql_engine* e, const int64_t* host_indices, f
     if (rcw != IQL_OK) return rcw;
   }
   if (gather)
-    for (int m = 0; m < S; ++m) {
+    for (const int m : e->active) {  // rows of members that do not train are never read
       const int64_t cap = e->h_replay[m].capacity;
       for (int b = 0; b < e->h_scalars[m].batch; ++b) {  // entries past B_m are never read
         const int64_t i = host_indices[(size_t)m * B + b];
@@ -1513,7 +1546,7 @@ extern "C" int iql_train_host_step(iql_engine* e, const int64_t* host_indices, f
         mail_idx[(size_t)m * B + b] = i;
       }
     }
-  for (int m = 0; m < S; ++m) reinterpret_cast<volatile uint32_t*>(mail)[m * 4 + 3] = 0u;
+  for (const int m : e->active) reinterpret_cast<volatile uint32_t*>(mail)[m * 4 + 3] = 0u;
   std::atomic_thread_fence(std::memory_order_seq_cst);
   // The graph is captured on `stream` (capture needs a non-default stream) but LAUNCHED on the caller's stream: the
   // step is then ordered against everything the caller enqueues (inserted rows, a staged batch, later reads of the
@@ -1561,7 +1594,7 @@ extern "C" int iql_train_host_step(iql_engine* e, const int64_t* host_indices, f
   }
   CUDA_TRY(e, cudaGraphLaunch(it->second.first, run));
   e->last_launches = it->second.second;
-  for (int m = 0; m < S; ++m) {
+  for (const int m : e->active) {
     iql_counters& c = e->h_counters[m];
     c.v_step += 1; c.q_step += 1; c.actor_step += 1; c.total_it += 1; c.sample_step += 1;
     if (e->h_hparams[m].cosine_t_max > 0) c.sched_epoch += 1;
@@ -1580,14 +1613,59 @@ extern "C" int iql_host_step_wait(iql_engine* e, float* host_losses, void* strea
   cudaStream_t st = e->host_step_stream;  // the stream the step was launched on (a failed launch is noticed through it)
   const int S = e->cfg.n_members, B = e->cfg.batch_size;
   float* mail = (float*)(e->h_mail + sizeof(int64_t) * (size_t)S * B);
-  // wait for the flag words (bounded: a failed launch never raises them)
-  for (int m = 0; m < S; ++m) {
+  // wait for the flag words of the members the step trained (bounded: a failed launch never raises them); the active
+  // set cannot have changed since the launch, iql_set_active_members collects a pending step first
+  for (const int m : e->active) {
     int rc = spin_flag(e, reinterpret_cast<volatile uint32_t*>(mail) + m * 4 + 3, st, "iql_host_step_wait");
     if (rc != IQL_OK) return rc;
   }
   std::atomic_thread_fence(std::memory_order_acquire);
   for (int m = 0; m < S; ++m)
-    for (int j = 0; j < 3; ++j) host_losses[m * 3 + j] = reinterpret_cast<volatile float*>(mail)[m * 4 + j];
+    for (int j = 0; j < 3; ++j)
+      host_losses[m * 3 + j] = e->is_active[m] ? reinterpret_cast<volatile float*>(mail)[m * 4 + j] : NAN;
+  return IQL_OK;
+}
+
+// Members that train.  The problem tables, tensor maps and chain tasks are rebuilt over the active members only, so the
+// others launch no CTA and their arena rows, counters and batch sizes stay as they are; the path choices that depend on
+// the member count are re-made from the new count.  Host work (tensor-map encoding), paid once per change.
+extern "C" int iql_set_active_members(iql_engine* e, int32_t n, const int32_t* host_ids) {
+  if (!e) return IQL_ERR_INVALID;
+  const int S = e->cfg.n_members;
+  if (!host_ids || n <= 0) return fail(e, IQL_ERR_INVALID, "iql_set_active_members: need at least one member id");
+  std::vector<char> mask(S, 0);
+  for (int i = 0; i < n; ++i) {
+    const int32_t m = host_ids[i];
+    if (m < 0 || m >= S) return fail(e, IQL_ERR_INVALID, "iql_set_active_members: member " + std::to_string(m) + " out of range");
+    if (mask[m]) return fail(e, IQL_ERR_INVALID, "iql_set_active_members: member " + std::to_string(m) + " listed twice");
+    mask[m] = 1;
+  }
+  if (!e->bound) return fail(e, IQL_ERR_STATE, "iql_set_active_members: state not bound");
+  if (e->mail_pending) {  // the in-flight host step's flag words belong to the old set: collect it first
+    std::vector<float> sink(3 * (size_t)S);
+    const int rcw = iql_host_step_wait(e, sink.data(), e->host_step_stream);
+    if (rcw != IQL_OK) return rcw;
+  }
+  const std::vector<int32_t> old = e->active;
+  e->active.clear();
+  for (int m = 0; m < S; ++m)
+    if (mask[m]) e->active.push_back(m);
+  int rc = bind_tables(e);
+  if (rc != IQL_OK) {  // cannot happen for a set the old tables were built for; restore it anyway
+    e->active = old;
+    bind_tables(e);
+    return rc;
+  }
+  e->is_active = mask;
+  e->tables_dirty = true;
+  for (auto& kv : e->graphs) cudaGraphExecDestroy(kv.second.first);  // the tables' sizes are baked into the launches
+  e->graphs.clear();
+  return IQL_OK;
+}
+
+extern "C" int iql_get_active_members(iql_engine* e, int8_t* host_mask) {
+  if (!e || !host_mask) return fail(e, IQL_ERR_INVALID, "iql_get_active_members: null argument");
+  for (int m = 0; m < e->cfg.n_members; ++m) host_mask[m] = e->is_active[m];
   return IQL_OK;
 }
 
@@ -1896,7 +1974,7 @@ extern "C" int iql_profile_step(iql_engine* e, int32_t reps, int32_t max_slots, 
   if (!e || !n_slots || !avg_ms || !flops || !bytes || !labels || reps <= 0 || max_slots <= 0)
     return fail(e, IQL_ERR_INVALID, "iql_profile_step: null or non-positive argument");
   if (!e->bound) return fail(e, IQL_ERR_STATE, "iql_profile_step: state not bound");
-  for (int m = 0; m < e->cfg.n_members; ++m)
+  for (const int m : e->active)
     if (!e->h_replay[m].rows || e->h_replay[m].size <= 0) return fail(e, IQL_ERR_STATE, "iql_profile_step: replay buffer not bound");
   cudaStream_t st = (cudaStream_t)stream;
   int rc = flush_tables(e, st);
@@ -1913,7 +1991,7 @@ extern "C" int iql_profile_step(iql_engine* e, int32_t reps, int32_t max_slots, 
     enqueue_step(e, ctx, true, st, &tm);
     launch_advance(ctx, 1, st);
     CUDA_TRY(e, cudaStreamSynchronize(st));
-    for (int m = 0; m < e->cfg.n_members; ++m) {
+    for (const int m : e->active) {
       iql_counters& c = e->h_counters[m];
       c.v_step++; c.q_step++; c.actor_step++; c.total_it++; c.sample_step++;
       if (e->h_hparams[m].cosine_t_max > 0) c.sched_epoch++;

@@ -80,7 +80,10 @@ struct StepCtx {
   int B;
   int S_dim, A_dim, H, L;
   int deterministic;
-  int n_members;
+  // members this step trains (iql_set_active_members), ascending; the per-member kernels (gather, loss, optimizer,
+  // operand refresh, counter advance) run one CTA row per entry and take their member from active[blockIdx]
+  int n_active;
+  const int32_t* active;         // [n_active] device; null when every member trains (member i = CTA row i)
   int64_t P;                     // member block floats
   int64_t PQ;                    // q range [0, PQ)
   int64_t v_begin, v_end, a_begin, a_end;

@@ -172,12 +172,16 @@ void launch_simt_gemm(int mode, const GemmProb* probs, int nprob, int maxM, int 
   else simt_gemm_kernel<false, false><<<grid, 256, 0, st>>>(probs, ctx);
 }
 
+// member served by CTA row i of a per-member kernel (StepCtx::active; null when every member trains, which saves the
+// dependent load at the head of every per-member kernel of a full ensemble's step)
+__device__ __forceinline__ int member_of(const StepCtx& ctx, int i) { return ctx.active ? ctx.active[i] : i; }
+
 // ===========================================================================
 // replay gather into the step workspace: xrow[m][b][:] = rows_m[idx][:]
 // ===========================================================================
 __device__ __forceinline__ void gather_body(const StepCtx& ctx, float* __restrict__ ws, int64_t ws_member_floats, int64_t xrow_off,
                                             int bx) {
-  const int m = blockIdx.y;
+  const int m = member_of(ctx, blockIdx.y);
   const int RF = ctx.row.row_floats, Q = RF >> 2;
   const int t = bx * blockDim.x + threadIdx.x;
   stamp_begin(ctx.stamps, ST_GATHER);
@@ -215,7 +219,7 @@ __global__ void __launch_bounds__(256) gather_kernel(StepCtx ctx, float* __restr
 
 void launch_gather(const StepCtx& ctx, float* ws, int64_t ws_member_floats, int64_t xrow_off, cudaStream_t st) {
   const int threads = ctx.B * (ctx.row.row_floats >> 2);
-  dim3 grid((threads + 255) / 256, ctx.n_members);
+  dim3 grid((threads + 255) / 256, ctx.n_active);
   gather_kernel<<<grid, 256, 0, st>>>(ctx, ws, ws_member_floats, xrow_off);
 }
 
@@ -271,13 +275,14 @@ __global__ void __launch_bounds__(256) loss_kernel(StepCtx ctx, float* __restric
   // One shuffle tree per quantity and ONE block barrier; summation order is fixed (rows by lane, warps 0..7).
   __shared__ float red[8][4 + LOSS_MAX_A];
   stamp_begin(ctx.stamps, ST_LOSS);
-  if (blockIdx.x >= ctx.n_members) {
+  if (blockIdx.x >= ctx.n_active) {
     // Extra CTAs (idle SMs, next to the loss CTAs): the Adam scalars of this step for the optimizer kernel --
     // torch computes the bias corrections and the step size in Python floats, CosineAnnealingLR in closed form.
     // 6 threads per member: thread (o, which) takes one fp64 pow, the pair combines through a shuffle.
-    const int idx = (blockIdx.x - ctx.n_members) * 42 + threadIdx.x / 6;
+    const int slot = (blockIdx.x - ctx.n_active) * 42 + threadIdx.x / 6;
     const int o = (threadIdx.x % 6) >> 1, which = threadIdx.x & 1;  // o: 0 q, 1 v, 2 actor
-    const bool act = threadIdx.x < 252 && idx < ctx.n_members;
+    const bool act = threadIdx.x < 252 && slot < ctx.n_active;
+    const int idx = act ? member_of(ctx, slot) : 0;
     double pw = 0.0, lr = 0.0;
     if (act) {
       const MemberScalars sc = ctx.scalars[idx];
@@ -306,7 +311,7 @@ __global__ void __launch_bounds__(256) loss_kernel(StepCtx ctx, float* __restric
     stamp_end(ctx.stamps, ST_LOSS);
     return;
   }
-  const int m = blockIdx.x;
+  const int m = member_of(ctx, blockIdx.x);
   const int B = ctx.B, A = ctx.A_dim, RF = ctx.row.row_floats, Ald = wl.Ald;
   float* w = ws + m * ws_member_floats;
   const float* xrow = w + wl.xrow;
@@ -430,7 +435,7 @@ __global__ void __launch_bounds__(256) loss_kernel(StepCtx ctx, float* __restric
 
 void launch_loss(const StepCtx& ctx, float* ws, int64_t ws_member_floats, const WorkspaceLayout& wl,
                  const float* params, float* grads, cudaStream_t st) {
-  loss_kernel<<<ctx.n_members + (ctx.n_members + 41) / 42, 256, 0, st>>>(ctx, ws, ws_member_floats, wl, params, grads);
+  loss_kernel<<<ctx.n_active + (ctx.n_active + 41) / 42, 256, 0, st>>>(ctx, ws, ws_member_floats, wl, params, grads);
 }
 
 // ===========================================================================
@@ -448,7 +453,7 @@ __global__ void __launch_bounds__(256) adam_polyak_kernel(StepCtx ctx, float* __
                                                           float* __restrict__ exp_avg, float* __restrict__ exp_avg_sq,
                                                           float* __restrict__ target,
                                                           const float* __restrict__ grads) {
-  const int m = blockIdx.y;
+  const int m = member_of(ctx, blockIdx.y);
   const MemberScalars* sc = ctx.scalars + m;
   stamp_begin(ctx.stamps, ST_ADAM);
   pdl_wait();  // gradients, Adam scalars of the step: written by the launches before this one
@@ -493,7 +498,7 @@ __global__ void __launch_bounds__(256) adam_polyak_kernel(StepCtx ctx, float* __
 // TF32-rounded operand copies of params / target, rebuilt at the start of every engine call so that weights
 // written from outside (checkpoint loads, parameter surgery through the torch views) are always picked up.
 __device__ __forceinline__ void refresh_body(const StepCtx& ctx, float* __restrict__ params, float* __restrict__ target, int bx) {
-  const int m = blockIdx.y;
+  const int m = member_of(ctx, blockIdx.y);
   const int64_t i = ((int64_t)bx * blockDim.x + threadIdx.x) * 4;
   stamp_begin(ctx.stamps, ST_REFRESH);
   bool first_layer = false;
@@ -532,7 +537,7 @@ __global__ void __launch_bounds__(256) refresh_shadow_kernel(StepCtx ctx, float*
 }
 
 void launch_refresh_shadow(const StepCtx& ctx, float* params, float* target, cudaStream_t st) {
-  dim3 grid((unsigned)((ctx.P / 4 + 255) / 256), ctx.n_members);
+  dim3 grid((unsigned)((ctx.P / 4 + 255) / 256), ctx.n_active);
   refresh_shadow_kernel<<<grid, 256, 0, st>>>(ctx, params, target);
 }
 
@@ -551,20 +556,21 @@ __global__ void __launch_bounds__(256) gather_refresh_kernel(StepCtx ctx, float*
 void launch_gather_refresh(const StepCtx& ctx, float* ws, int64_t ws_member_floats, int64_t xrow_off, float* params, float* target,
                            cudaStream_t st) {
   const int n_gather = (ctx.B * (ctx.row.row_floats >> 2) + 255) / 256;
-  dim3 grid((unsigned)(n_gather + (ctx.P / 4 + 255) / 256), ctx.n_members);
+  dim3 grid((unsigned)(n_gather + (ctx.P / 4 + 255) / 256), ctx.n_active);
   gather_refresh_kernel<<<grid, 256, 0, st>>>(ctx, ws, ws_member_floats, xrow_off, params, target, n_gather);
 }
 
 void launch_adam(const StepCtx& ctx, float* params, float* exp_avg, float* exp_avg_sq, float* target,
                  const float* grads, cudaStream_t st) {
   const int64_t quads = (ctx.P + 3) / 4;
-  dim3 grid((unsigned)((quads + 256 * ADAM_UNROLL - 1) / (256 * ADAM_UNROLL)), ctx.n_members);
+  dim3 grid((unsigned)((quads + 256 * ADAM_UNROLL - 1) / (256 * ADAM_UNROLL)), ctx.n_active);
   launch_pdl(adam_polyak_kernel, grid, dim3(256), 0, st, 1, ctx, params, exp_avg, exp_avg_sq, target, grads);
 }
 
 __global__ void advance_kernel(StepCtx ctx, int K) {
-  const int m = blockIdx.x * blockDim.x + threadIdx.x;
-  if (m >= ctx.n_members) return;
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= ctx.n_active) return;
+  const int m = member_of(ctx, i);
   iql_counters c = ctx.counters[m];
   c.v_step += K;
   c.q_step += K;
@@ -576,7 +582,7 @@ __global__ void advance_kernel(StepCtx ctx, int K) {
 }
 
 void launch_advance(const StepCtx& ctx, int K, cudaStream_t st) {
-  advance_kernel<<<(ctx.n_members + 127) / 128, 128, 0, st>>>(ctx, K);
+  advance_kernel<<<(ctx.n_active + 127) / 128, 128, 0, st>>>(ctx, K);
 }
 
 // ===========================================================================

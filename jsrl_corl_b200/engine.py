@@ -98,10 +98,7 @@ class EnsembleEngine:
                                               self.workspace.data_ptr(), self.workspace.numel()), self._h, "iql_bind_state")
         # which kernels serve this shape: math_mode="tf32" outside the tcgen05 shapes (batch % 128, hidden % 256) runs the
         # FP32 CUDA-core kernels -- reported here, and refused when the caller insists on tensor cores
-        self.paths = {"tensor_cores": bool(self.info(_lib.INFO_TENSOR_CORE_PATH)),
-                      "fused_forward": bool(self.info(_lib.INFO_FUSED_FORWARD)),
-                      "chained_backward": bool(self.info(_lib.INFO_CHAINED_BACKWARD)),
-                      "chained_backward_grads": bool(self.info(_lib.INFO_CHAINED_BACKWARD_GRADS))}
+        self.paths = self._read_paths()
         if math_mode == "tf32" and strict_tf32 and not self.paths["tensor_cores"]:
             raise ValueError(f"math_mode='tf32' with strict_tf32: batch {batch_size} / hidden {hidden_dim} is outside the tcgen05 "
                              "kernels (batch % 128 == 0 and hidden % 256 == 0 required); the FP32 kernels would run")
@@ -128,6 +125,12 @@ class EnsembleEngine:
         return HParams(beta=3.0, iql_tau=0.7, discount=0.99, tau=0.005, vf_lr=3e-4, qf_lr=3e-4, actor_lr=3e-4,
                        actor_dropout=0.0, adam_beta1=0.9, adam_beta2=0.999, adam_eps=1e-8, lr_eta_min=0.0,
                        cosine_t_max=1000000, seed=m)
+
+    def _read_paths(self) -> Dict[str, bool]:
+        return {"tensor_cores": bool(self.info(_lib.INFO_TENSOR_CORE_PATH)),
+                "fused_forward": bool(self.info(_lib.INFO_FUSED_FORWARD)),
+                "chained_backward": bool(self.info(_lib.INFO_CHAINED_BACKWARD)),
+                "chained_backward_grads": bool(self.info(_lib.INFO_CHAINED_BACKWARD_GRADS))}
 
     def info(self, key: int) -> int:
         out = C.c_int64(0)
@@ -163,6 +166,26 @@ class EnsembleEngine:
     def batch_sizes(self) -> List[int]:
         """The members' batch sizes B_m (a copy; the per-step host loop reads it without a library call)."""
         return list(self._batch_sizes)
+
+    def set_active(self, members):
+        """Train only ``members`` (indices, any non-empty subset; `iql_set_active_members`).  The others launch no work
+        in later steps and keep their parameters, optimizer state, target and counters bit for bit; their loss rows
+        read NaN.  Calling it again with a member resumes it where it stopped.  Re-encodes the tensor maps (host
+        milliseconds) and drops the captured graphs, so call it at evaluation points rather than every step."""
+        ids = np.ascontiguousarray(sorted(int(m) for m in members), dtype=np.int32)
+        _lib.check(self._L.iql_set_active_members(self._h, int(ids.size), ids.ctypes.data if ids.size else None), self._h,
+                   "iql_set_active_members")
+        self._active = None
+        self.paths = self._read_paths()
+
+    @property
+    def active(self) -> np.ndarray:
+        """[n_members] bool: the members that train."""
+        if getattr(self, "_active", None) is None:
+            mask = np.zeros(self.n_members, dtype=np.int8)
+            _lib.check(self._L.iql_get_active_members(self._h, mask.ctypes.data), self._h, "iql_get_active_members")
+            self._active = mask.astype(bool)
+        return self._active.copy()
 
     def get_counters(self, member: int) -> Counters:
         c = Counters()
@@ -364,9 +387,10 @@ class EnsembleEngine:
     def train_steps(self, k_steps: int, mode: str = "philox", indices: Optional[torch.Tensor] = None,
                     dropout_masks: Optional[torch.Tensor] = None, return_indices: bool = False,
                     out: Optional[torch.Tensor] = None):
-        """Run K update steps for all members; returns losses [S, K, 3]
-        (value_loss, q_loss, actor_loss) on the device, asynchronously.  `indices` [S, K, B]: entries past a
-        member's batch size B_m are ignored; `return_indices` gives -1 there."""
+        """Run K update steps for the active members; returns losses [S, K, 3]
+        (value_loss, q_loss, actor_loss) on the device, asynchronously, NaN in the rows of inactive members.
+        `indices` [S, K, B]: entries past a member's batch size B_m, and the rows of inactive members, are ignored;
+        `return_indices` gives -1 there."""
         S, B = self.n_members, self.batch_size
         smode = {"philox": _lib.SAMPLE_PHILOX, "indices": _lib.SAMPLE_INDICES, "preloaded": _lib.SAMPLE_PRELOADED}[mode]
         idx_ptr = None

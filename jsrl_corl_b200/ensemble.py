@@ -114,12 +114,27 @@ class IQLEnsemble:
         e = self.engine
         if indices is None:
             indices = np.zeros((e.n_members, e.batch_size), dtype=np.int64)
-            for m, (rb, bm) in enumerate(zip(self._buffers, e._batch_sizes)):
-                indices[m, :bm] = np.random.randint(0, rb._high(), size=bm)
+            for m in np.flatnonzero(e.active):  # inactive members draw nothing; their losses come back NaN
+                indices[m, :e._batch_sizes[m]] = np.random.randint(0, self._buffers[m]._high(), size=e._batch_sizes[m])
         idx = np.ascontiguousarray(indices, dtype=np.int64)
         if idx.shape != (e.n_members, e.batch_size):
             raise ValueError(f"indices must be [{e.n_members}, {e.batch_size}]")
         return np.asarray(e.host_step(host_indices=idx.ctypes.data), dtype=np.float32).reshape(e.n_members, 3)
+
+    # ---- early stopping: members that no longer train ----------------------
+    @property
+    def active(self) -> np.ndarray:
+        """[n_members] bool: the members that train in ``train_steps`` / ``train_step_logged``."""
+        return self.engine.active
+
+    def retire(self, members):
+        """Stop training ``members`` (a stopped trial of a search): they cost no GPU time in later steps, keep their
+        state bit for bit, still act, insert and checkpoint, and read NaN losses.  At least one member must stay."""
+        self.engine.set_active(np.flatnonzero(self.active & ~_member_mask(members, self.n_members)))
+
+    def resume(self, members):
+        """Train ``members`` again from where they stopped (their counters, schedules and Philox streams continue)."""
+        self.engine.set_active(np.flatnonzero(self.active | _member_mask(members, self.n_members)))
 
     # ---- the online phase: guide, batched act, batched ring insert ------------
     def set_guide(self, other: Optional["IQLEnsemble"]):
@@ -254,6 +269,15 @@ class IQLEnsemble:
         e.set_hparams(m, **kw)
         e.set_counters(m, q_step=steps["qf"], v_step=steps["vf"], actor_step=steps["actor"],
                        sched_epoch=int(sched.get("last_epoch", 0)), total_it=int(sd["total_it"]))
+
+
+def _member_mask(members, n: int) -> np.ndarray:
+    ids = np.asarray(list(members), dtype=np.int64).reshape(-1)
+    if ids.size and (ids.min() < 0 or ids.max() >= n):
+        raise ValueError(f"member index out of range [0, {n}): {ids.tolist()}")
+    mask = np.zeros(n, dtype=bool)
+    mask[ids] = True
+    return mask
 
 
 def cosine_lr(base_lr: float, epoch: int, t_max: int, eta_min: float = 0.0) -> float:

@@ -215,22 +215,35 @@ def train_loop(config, env, eval_env, replay_buffer: Optional[ReplayBuffer], sta
 # ---------------------------------------------------------------------------
 # S members through the whole JSRL run at once (the reference's process-per-seed launchers, ray_trainer.py)
 # ---------------------------------------------------------------------------
-# fields every member of an ensemble run must share: the loop runs all members in lockstep (batch size, iteration
-# counts, evaluation points), `horizon_fn` is a module global of jsrl_utils, and the policy type / dropout / online
-# buffer rule fix the engine shape and the update gate
-ENSEMBLE_SHARED_FIELDS = ("batch_size", "offline_iterations", "online_iterations", "eval_freq", "n_episodes", "horizon_fn",
+# fields every member of an ensemble run must share: the loop runs all members in lockstep (iteration counts,
+# evaluation points), `horizon_fn` is a module global of jsrl_utils, and the policy type / dropout / online buffer rule
+# fix the engine shape and the update gate.  `batch_size` is checked on its own: it must be the same for every member
+# unless the caller asks for per-member batch sizes (`mixed_batch_sizes=True`); then the engine runs the largest,
+# member m trains on its own B_m rows (IQLEnsemble(batch_sizes=...)) and its gate `t >= B_m` keeps it inactive until it
+# opens.
+ENSEMBLE_SHARED_FIELDS = ("offline_iterations", "online_iterations", "eval_freq", "n_episodes", "horizon_fn",
                           "iql_deterministic", "actor_dropout", "new_online_buffer")
 
 
-def check_ensemble_configs(configs):
-    """Refuse (ValueError) configs whose shared fields differ, and (NotImplementedError) the options the ensemble
-    loop does not cover.  Touches no device."""
+def check_ensemble_configs(configs, scheduler=None, mixed_batch_sizes: bool = False):
+    """Refuse (ValueError) configs whose shared fields differ, whose batch sizes differ without ``mixed_batch_sizes``
+    or are not positive integers, a scheduler without ``on_result``, and (NotImplementedError) the options the
+    ensemble loop does not cover.  Touches no device."""
     if len(configs) == 0:
         raise ValueError("ensemble_train_loop needs at least one config")
     for f in ENSEMBLE_SHARED_FIELDS:
         vals = [getattr(c, f) for c in configs]
         if any(v != vals[0] for v in vals[1:]):
             raise ValueError(f"ensemble_train_loop: `{f}` must be the same for every member, got {vals}")
+    sizes = [c.batch_size for c in configs]
+    if any(not isinstance(b, (int, np.integer)) or isinstance(b, bool) or b < 1 for b in sizes):
+        raise ValueError(f"ensemble_train_loop: every `batch_size` must be a positive integer, got {sizes}")
+    if not mixed_batch_sizes and any(b != sizes[0] for b in sizes[1:]):
+        raise ValueError(f"ensemble_train_loop: `batch_size` must be the same for every member, got {sizes} (pass "
+                         "mixed_batch_sizes=True to train each member on its own batch size)")
+    if scheduler is not None and not callable(getattr(scheduler, "on_result", None)):
+        raise ValueError("ensemble_train_loop: the scheduler needs an on_result(member, t, score, total_it) method "
+                         "(jsrl_corl_b200.asha.ASHAScheduler)")
     c0 = configs[0]
     for c in configs:
         if getattr(c, "guide_heuristic_fn", None) is not None:
@@ -274,17 +287,26 @@ def _build_ensemble(configs, nets, state_dim, action_dim, t_max, device):
     from .ensemble import IQLEnsemble
 
     c0 = configs[0]
-    ens = IQLEnsemble(len(configs), state_dim, action_dim, 256, 2, c0.batch_size, deterministic=c0.iql_deterministic,
+    sizes = [int(c.batch_size) for c in configs]
+    ens = IQLEnsemble(len(configs), state_dim, action_dim, 256, 2, max(sizes), deterministic=c0.iql_deterministic,
                       device=device, max_steps_per_call=max(1, min(256, int(c0.eval_freq))), seeds=[c.seed for c in configs],
-                      hparams=[_member_hparams(c, t_max) for c in configs], init=False)
+                      hparams=[_member_hparams(c, t_max) for c in configs], init=False,
+                      batch_sizes=sizes if len(set(sizes)) > 1 else None)
     for m, (q, v, actor) in enumerate(nets):
         ens.engine.load_params(m, {"qf": q.state_dict(), "vf": v.state_dict(), "actor": actor.state_dict()})
     return ens
 
 
+def _sync_active(ens, want: np.ndarray):
+    """Make the members in ``want`` (bool [S], not all False) the ones that train; no call when nothing changes."""
+    if not np.array_equal(ens.active, want):
+        ens.engine.set_active(np.flatnonzero(want))
+
+
 @torch.no_grad()
-def ensemble_eval_actor(envs, ensemble, use_guide: bool, configs, max_action: float):
-    """``eval_actor`` for every member at once: member m plays ``n_episodes`` episodes on ``envs[m]`` with
+def ensemble_eval_actor(envs, ensemble, use_guide: bool, configs, max_action: float, members=None):
+    """``eval_actor`` for every member at once (for those whose ``members`` entry is true, when given; the others get
+    None): member m plays ``n_episodes`` episodes on ``envs[m]`` with
     ``ensemble``'s member m as the learner and, with ``use_guide``, the guide bound by ``set_guide`` as the guide.
     All members step in lockstep with one act launch per step; members whose episodes are over are skipped.  Each
     member's episodes are exactly those ``eval_actor`` plays for it alone (the horizon function reads and
@@ -297,7 +319,8 @@ def ensemble_eval_actor(envs, ensemble, use_guide: bool, configs, max_action: fl
     source = np.zeros(S, dtype=np.int8)
     out = np.zeros((S, ensemble.engine.action_dim), dtype=np.float32)
     ep = [0] * S
-    live = [n_ep > 0] * S
+    chosen = [True] * S if members is None else [bool(x) for x in members]
+    live = [n_ep > 0 and chosen[m] for m in range(S)]
     fresh = [True] * S
     raw_state = [None] * S
     acc = [dict(returns=[], successes=[], horizons=[], agent_types=[]) for _ in range(S)]
@@ -342,6 +365,9 @@ def ensemble_eval_actor(envs, ensemble, use_guide: bool, configs, max_action: fl
                 live[m] = ep[m] < n_ep
     results = []
     for m in range(S):
+        if not chosen[m]:
+            results.append(None)
+            continue
         a, c = acc[m], configs[m]
         horizon = np.max(a["horizons"]) if ((not use_guide) and c.max_init_horizon) else np.mean(a["horizons"])
         results.append((np.asarray(a["returns"]), float(np.mean(a["successes"])), horizon, float(np.mean(a["agent_types"]))))
@@ -350,9 +376,10 @@ def ensemble_eval_actor(envs, ensemble, use_guide: bool, configs, max_action: fl
 
 def ensemble_train_loop(configs, envs, eval_envs, replay_buffers, state_dim: int, action_dim: int, max_action: float,
                         max_steps: int, log: Optional[Callable[[int, Dict, int], None]] = None, reward_mod_dicts=None,
-                        is_env_with_goal: bool = False):
+                        is_env_with_goal: bool = False, scheduler=None, mixed_batch_sizes: bool = False):
     """``train_loop`` for S members at once, one ``JsrlTrainConfig`` per member (seed, IQL / Adam hyper-parameters,
-    curriculum, tolerance, noise and checkpoint path may differ; ``ENSEMBLE_SHARED_FIELDS`` may not).
+    curriculum, tolerance, noise and checkpoint path may differ; ``ENSEMBLE_SHARED_FIELDS`` may not; ``batch_size``
+    may differ with ``mixed_batch_sizes=True``, the batch-size axis of a search).
 
     Offline: one ``IQLEnsemble`` (cosine schedule with T_max = offline_iterations) trained in K-step calls that end at
     the evaluation points, on indices drawn from each member's own ``np.random.RandomState(seed)``.  Switch: a
@@ -361,10 +388,17 @@ def ensemble_train_loop(configs, envs, eval_envs, replay_buffers, state_dim: int
     guide's networks copied when there is a single curriculum stage), each member with its own online ring.  Online,
     per env step for all members: the horizon functions on the host, ONE act launch, exploration noise or the
     Gaussian sample from each member's own ``torch.Generator(seed)``, S env steps, ONE ring-insert launch and ONE
-    logged update.  ``train_loop``'s quirks are kept per member.  ``log(member, dict, step)`` receives what
-    ``train_loop``'s ``log`` receives.  Returns (learner ensemble, configs, one eval history per member); the guide
-    ensemble is ``learner.guide``."""
-    check_ensemble_configs(configs)
+    logged update.  ``train_loop``'s quirks are kept per member; a member whose update gate (``t >= batch_size`` with
+    a new online buffer) is still closed does not train (``IQLEnsemble.retire``).  ``log(member, dict, step)``
+    receives what ``train_loop``'s ``log`` receives.
+
+    ``scheduler`` (e.g. ``asha.ASHAScheduler``): every evaluation of both phases reports each evaluated member's score
+    (the value ``horizon_update_callback`` sees) as ``on_result(member, n_reports, score, total_it)``; a member it
+    stops gets no act, env step, insert, update, evaluation, log or checkpoint from then on and costs no GPU time.
+    Members stopped offline skip the guide probe and start the online phase retired.  The run ends when every member
+    has stopped.  Returns (learner ensemble, configs, one eval history per member); the guide ensemble is
+    ``learner.guide``."""
+    check_ensemble_configs(configs, scheduler, mixed_batch_sizes)
     S = len(configs)
     if not (len(envs) == len(eval_envs) == S):
         raise ValueError("need one env and one eval env per member")
@@ -380,7 +414,9 @@ def ensemble_train_loop(configs, envs, eval_envs, replay_buffers, state_dim: int
                              "other's transitions)")
     log = log or (lambda m, d, step: None)
     c0 = configs[0]
-    B, off, on, eval_freq = int(c0.batch_size), int(c0.offline_iterations), int(c0.online_iterations), int(c0.eval_freq)
+    Bm = [int(c.batch_size) for c in configs]
+    off, on, eval_freq = int(c0.offline_iterations), int(c0.online_iterations), int(c0.eval_freq)
+    gated = bool(c0.new_online_buffer)  # train_loop's update gate `t >= batch_size` on the global t
     gaussian = not c0.iql_deterministic
     jsrl.horizon_str = c0.horizon_fn
     device = c0.device
@@ -394,13 +430,16 @@ def ensemble_train_loop(configs, envs, eval_envs, replay_buffers, state_dim: int
     histories = [[] for _ in range(S)]
     eval_successes = [[] for _ in range(S)]
     states = [_reset(envs[m], configs[m].seed) for m in range(S)]
+    live = np.ones(S, dtype=bool)  # not stopped by the scheduler
+    reports = [0] * S
 
-    def evaluate(t, ens, use_guide, total_it):
+    def evaluate(t, ens, use_guide, total_it, members):
         if not use_guide:
-            for c in configs:
-                c.curriculum_stage = np.nan
-        results = ensemble_eval_actor(eval_envs, ens, use_guide, configs, max_action)
-        for m, c in enumerate(configs):
+            for m in np.flatnonzero(members):
+                configs[m].curriculum_stage = np.nan
+        results = ensemble_eval_actor(eval_envs, ens, use_guide, configs, max_action, members)
+        for m in np.flatnonzero(members):
+            c = configs[m]
             scores, success, c.mean_horizon_reached, c.eval_mean_agent_type = results[m]
             score = float(scores.mean())
             norm_fn = getattr(eval_envs[m], "get_normalized_score", None) if c.normalize_reward else None
@@ -420,49 +459,68 @@ def ensemble_train_loop(configs, envs, eval_envs, replay_buffers, state_dim: int
                 eval_log["eval/score"] = score
             if c.checkpoints_path is not None:
                 torch.save(ens.member_state_dict(m), os.path.join(c.checkpoints_path, f"checkpoint_{t}.pt"))
-            log(m, eval_log, total_it)
+            log(m, eval_log, total_it[m])
             histories[m].append(dict(eval_log, t=t))
+            if scheduler is not None:
+                reports[m] += 1
+                if scheduler.on_result(int(m), reports[m], score, int(total_it[m])) == "stop":
+                    live[m] = False
+        if live.any() and not np.array_equal(ens.active, ens.active & live):
+            _sync_active(ens, ens.active & live)  # stopped members are retired at once
 
-    # ---- offline phase: K-step calls between evaluation points ----
+    # ---- offline phase: K-step calls between evaluation points and gate openings ----
     offline = _build_ensemble(configs, [n[0] for n in nets], state_dim, action_dim, off, device)
     offline.bind_replay(list(replay_buffers))
-    first = 0 if not c0.new_online_buffer else min(B, off)  # train_loop's gate `t >= batch_size` on the global t
-    t, done_steps = first, 0
-    while t < off:
+    first = np.array([min(b, off) if gated else 0 for b in Bm])  # the first offline step of each member
+    done_steps = [0] * S
+    t = int(first.min())
+    while t < off and live.any():
         stop = min(off, (t // eval_freq + 1) * eval_freq, t + offline.engine.max_steps_per_call)
+        opening = first[first > t]
+        if opening.size:
+            stop = min(stop, int(opening.min()))
         K = stop - t
-        idx = np.empty((S, K, B), dtype=np.int64)
-        for m, rb in enumerate(replay_buffers):
-            high = rb._high()
+        train = live & (first <= t)
+        if not train.any():  # the members still running have not reached their gates yet
+            t = stop
+            continue
+        _sync_active(offline, train)
+        idx = np.zeros((S, K, max(Bm)), dtype=np.int64)
+        for m in np.flatnonzero(train):
+            high = replay_buffers[m]._high()
             for k in range(K):
-                idx[m, k] = index_rng[m].randint(0, high, size=B)
+                idx[m, k, :Bm[m]] = index_rng[m].randint(0, high, size=Bm[m])
         losses = offline.train_steps(K, mode="indices", indices=torch.from_numpy(idx)).cpu().numpy()
         for k in range(K):
-            done_steps += 1
-            for m in range(S):
+            for m in np.flatnonzero(train):
+                done_steps[m] += 1
                 log(m, {"value_loss": float(losses[m, k, 0]), "q_loss": float(losses[m, k, 1]),
-                        "actor_loss": float(losses[m, k, 2]), "offline_iter": t + k}, done_steps)
+                        "actor_loss": float(losses[m, k, 2]), "offline_iter": t + k}, done_steps[m])
         t = stop
         if t % eval_freq == 0:
-            evaluate(t - 1, offline, False, done_steps)
-    if on <= 0:
+            evaluate(t - 1, offline, False, done_steps, train)
+    if on <= 0 or not live.any():
         return offline, configs, histories
 
     # ---- switch to online: guide-only probe, guide binding, fresh learners, online rings ----
-    for c in configs:
-        c.curriculum_stage = np.nan
-    probe = ensemble_eval_actor(envs, offline, False, configs, max_action)
+    for m in np.flatnonzero(live):
+        configs[m].curriculum_stage = np.nan
+    probe = ensemble_eval_actor(envs, offline, False, configs, max_action, live)
     learner = _build_ensemble(configs, [n[1] for n in nets], state_dim, action_dim, 0, device)
     for m, c in enumerate(configs):
         if c.n_curriculum_stages == 1:  # the guide's trained networks, fresh optimizers (get_learning_agent)
             learner.engine.load_params(m, offline.engine.param_views(m))
         learner.engine.set_counters(m, total_it=off)
     learner.set_guide(offline)
-    for m, c in enumerate(configs):
-        configs[m] = jsrl.prepare_finetuning(probe[m][2], c)
-    online_buffers = [jsrl.get_online_buffer(c, replay_buffers[m], state_dim, action_dim) for m, c in enumerate(configs)]
+    for m in np.flatnonzero(live):
+        configs[m] = jsrl.prepare_finetuning(probe[m][2], configs[m])
+    # stopped members keep the offline buffer bound: they never sample from it
+    online_buffers = [jsrl.get_online_buffer(c, replay_buffers[m], state_dim, action_dim) if live[m] else replay_buffers[m]
+                      for m, c in enumerate(configs)]
     learner.bind_replay(online_buffers)
-    states = [_reset(envs[m]) for m in range(S)]
+    if not live.all():
+        _sync_active(learner, live)
+    states = [_reset(envs[m]) if live[m] else None for m in range(S)]
 
     hfn = jsrl.HORIZON_FNS[jsrl.horizon_str]["horizon_fn"]
     A = action_dim
@@ -479,10 +537,15 @@ def ensemble_train_loop(configs, envs, eval_envs, replay_buffers, state_dim: int
     ep_ret, ep_step, goal = [0.0] * S, [0] * S, [False] * S
     ep_types = [[] for _ in range(S)]
     train_successes = [[] for _ in range(S)]
-    total_it = off
+    total_it = [off] * S
+    idx = np.zeros((S, max(Bm)), dtype=np.int64)
     for t in range(off, off + on):
+        if not live.any():
+            break
+        members = np.flatnonzero(live)
         online_logs = [{} for _ in range(S)]
-        for m, c in enumerate(configs):
+        for m in members:
+            c = configs[m]
             if ep_step[m] == 0:
                 ep_types[m] = []
                 c.ep_agent_type = 0
@@ -491,8 +554,10 @@ def ensemble_train_loop(configs, envs, eval_envs, replay_buffers, state_dim: int
             use[m], _ = hfn(ep_step[m], states[m], envs[m], c)
             obs[m] = np.asarray(states[m], dtype=np.float32).reshape(-1)
             source[m] = learner_code if use[m] else _lib_codes.ACT_GUIDE
+        source[~live] = _lib_codes.ACT_SKIP
         learner.act(obs, source, max_action, out=act_out, std=act_std)
-        for m, c in enumerate(configs):
+        for m in members:
+            c = configs[m]
             ep_types[m].append(1 if use[m] else 0)
             a = act_out[m].copy()
             if use[m] and gaussian:  # GaussianPolicy.act in training mode: mean + std * N(0, 1), scaled and clipped
@@ -523,16 +588,20 @@ def ensemble_train_loop(configs, envs, eval_envs, replay_buffers, state_dim: int
                 lg.update({"train/episode_return": ep_ret[m], "train/mean_ep_agent_type": float(np.mean(ep_types[m])),
                            "train/episode_length": ep_step[m]})
                 ep_ret[m], ep_step[m], goal[m] = 0.0, 0, False
-        learner.add_transitions(obs, actions, rewards, next_obs, real_dones)
-        if t >= B or not c0.new_online_buffer:
-            idx = np.stack([index_rng[m].randint(0, online_buffers[m]._high(), size=B) for m in range(S)])
-            losses = learner.train_step_logged(idx)
-            total_it += 1
-            for m in range(S):
-                log_dict = {"value_loss": float(losses[m, 0]), "q_loss": float(losses[m, 1]), "actor_loss": float(losses[m, 2]),
-                            "online_iter": t - off}
-                log_dict.update(online_logs[m])
-                log(m, log_dict, total_it)
-            if (t + 1) % eval_freq == 0:
-                evaluate(t, learner, True, total_it)
+        learner.add_transitions(obs, actions, rewards, next_obs, real_dones, mask=live)
+        train = live & np.array([t >= b or not gated for b in Bm])
+        if not train.any():
+            continue
+        _sync_active(learner, train)
+        for m in np.flatnonzero(train):
+            idx[m, :Bm[m]] = index_rng[m].randint(0, online_buffers[m]._high(), size=Bm[m])
+        losses = learner.train_step_logged(idx)
+        for m in np.flatnonzero(train):
+            total_it[m] += 1
+            log_dict = {"value_loss": float(losses[m, 0]), "q_loss": float(losses[m, 1]), "actor_loss": float(losses[m, 2]),
+                        "online_iter": t - off}
+            log_dict.update(online_logs[m])
+            log(m, log_dict, total_it[m])
+        if (t + 1) % eval_freq == 0:
+            evaluate(t, learner, True, total_it, train)
     return learner, configs, histories
