@@ -291,6 +291,18 @@ int iql_act_host_gaussian(iql_engine* e, int32_t member, const float* host_state
 #define IQL_ACT_LEARNER 1      /* eval-mode action of the member's learner: clamp(max_action * tanh(MLP(s)))          */
 #define IQL_ACT_LEARNER_DIST 2 /* Gaussian learner: mean = tanh(MLP(s)) (unscaled) and std = exp(clamp(log_std, -20, 2)) */
 #define IQL_ACT_GUIDE 3        /* eval-mode action of the member's guide (the arena bound by iql_bind_guide)          */
+#define IQL_ACT_LEARNER_DROPOUT 4      /* training-mode deterministic act: clamp(max_action * tanh(MLP_drop(s)))        */
+#define IQL_ACT_LEARNER_DIST_DROPOUT 5 /* training-mode Gaussian act: mean = tanh(MLP_drop(s)) (unscaled) and std, as 2 */
+/* MLP_drop is the policy MLP with nn.Dropout(p = the member's iql_hparams.actor_dropout) after every hidden ReLU, the
+ * learner in training mode (GaussianPolicy.act's dist.sample(), DeterministicPolicy.act's self(state)).  Hidden unit j of
+ * hidden layer l (0 <= l < n_hidden) is kept iff
+ *     word (j & 3) of Philox4x32-10(counter = (j >> 2, act_step lo, act_step hi, 0x80000000 + l),
+ *                                   key = (seed lo, seed hi))  >=  floor(p * 2^32)
+ * (words x, y, z, w = 0..3), where seed is the member's iql_hparams.seed; a kept unit becomes relu(a) * (float)(1 / (1 - p)),
+ * a dropped unit exactly 0 -- the rule of the update's dropout masks, whose counter word 3 is 1 + l, so the act masks never
+ * repeat a training mask of the same key.  act_step is the member's act counter (iql_get_act_steps): every launched
+ * member with code 4 or 5 draws at its counter's current value, and the counter then advances by one, whatever p is
+ * (p = 0 gives codes 1 / 2 bit for bit).  No other code, no other call (iql_set_active_members included) touches it. */
 /* Bind a second [S][param_floats] parameter arena with this handle's layout as the members' guides (JSRL's guide
  * policy: in practice the frozen offline ensemble's parameter arena, zero-copy).  The engine only reads it.  NULL
  * unbinds.  16-byte aligned device memory. */
@@ -298,14 +310,18 @@ int iql_bind_guide(iql_engine* e, const float* guide_params);
 /* replaces: GaussianPolicy.act / DeterministicPolicy.act (iql.py:371-379, 403-413) behind jsrl_utils.learner_or_guide_action
  * (jsrl_utils.py:547-622), for every member of the ensemble in ONE launch: host_states [S][state_dim], host_source [S]
  * IQL_ACT_* codes.  host_out [S][action_dim] receives the action (or the mean of IQL_ACT_LEARNER_DIST), host_std
- * [S][action_dim] the std of IQL_ACT_LEARNER_DIST members (may be NULL when no member asks for it).  Skipped members
+ * [S][action_dim] the std of IQL_ACT_LEARNER_DIST / IQL_ACT_LEARNER_DIST_DROPOUT members (may be NULL when no member asks for it).  Skipped members
  * cost no CTA.  Every active member's result is bit-identical to iql_act_host / iql_act_host_gaussian on the same
  * weights.  Observations travel through an engine-owned pinned, device-mapped block (no state_dim limit), results
  * come back through pinned memory with one flag word per member: no copies, no stream synchronisation.  Launched on
  * `caller_stream`, ordered behind the host steps like iql_act_host.  Refused (IQL_ERR_INVALID): a guide code with no
- * guide bound, the distribution code on a deterministic policy, unknown codes. */
+ * guide bound, a distribution code on a deterministic policy, unknown codes (nothing is launched, no counter moves). */
 int iql_act_host_members(iql_engine* e, const float* host_states, const int8_t* host_source, float max_action,
                          float* host_out, float* host_std, void* stream, void* caller_stream);
+/* host_out[S]: the act counters of all members (start at 0; see IQL_ACT_LEARNER_DROPOUT). */
+int iql_get_act_steps(iql_engine* e, uint64_t* host_out);
+/* host_in[S]: set the act counters of all members (setting a counter back to k repeats the masks drawn at k). */
+int iql_set_act_steps(iql_engine* e, const uint64_t* host_in);
 /* replaces: ReplayBuffer.add_transition (iql.py:180-196) for every member in ONE launch: member m's transition
  * (host_states [S][state_dim], host_actions [S][action_dim], host_rewards [S], host_next_states [S][state_dim],
  * host_dones [S], all host memory) is packed in the iql_row_layout layout, padding zeroed, and written at row

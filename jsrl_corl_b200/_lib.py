@@ -23,8 +23,9 @@ KIND_WEIGHT, KIND_BIAS, KIND_LOG_STD = 0, 1, 2
 OPT_STEP_PATH, OPT_KEEP_GRADS = 1, 2
 INFO_TENSOR_CORE_PATH, INFO_FUSED_FORWARD, INFO_CHAINED_BACKWARD, INFO_CHAINED_BACKWARD_GRADS = 1, 2, 3, 4
 STEP_PATHS = {"auto": 0, "phases": 1, "chain": 2, "chain_grads": 4}
-ACT_SKIP, ACT_LEARNER, ACT_LEARNER_DIST, ACT_GUIDE = 0, 1, 2, 3
-ACT_SOURCES = {"skip": ACT_SKIP, "learner": ACT_LEARNER, "learner_dist": ACT_LEARNER_DIST, "guide": ACT_GUIDE}
+ACT_SKIP, ACT_LEARNER, ACT_LEARNER_DIST, ACT_GUIDE, ACT_LEARNER_DROPOUT, ACT_LEARNER_DIST_DROPOUT = 0, 1, 2, 3, 4, 5
+ACT_SOURCES = {"skip": ACT_SKIP, "learner": ACT_LEARNER, "learner_dist": ACT_LEARNER_DIST, "guide": ACT_GUIDE,
+               "learner_dropout": ACT_LEARNER_DROPOUT, "learner_dist_dropout": ACT_LEARNER_DIST_DROPOUT}
 
 
 class Config(C.Structure):
@@ -121,6 +122,8 @@ SYMBOLS = {
     "iql_act_host_gaussian": (C.c_int, [_P, C.c_int32, _P, _P, _P, _P, _P]),
     "iql_bind_guide": (C.c_int, [_P, _P]),
     "iql_act_host_members": (C.c_int, [_P, _P, _P, C.c_float, _P, _P, _P, _P]),
+    "iql_get_act_steps": (C.c_int, [_P, _P]),
+    "iql_set_act_steps": (C.c_int, [_P, _P]),
     "iql_replay_insert_members_host": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "iql_last_launch_count": (C.c_int64, [_P]),
     "iql_debug_fused_trace": (C.c_int, [_P, C.c_int32]),

@@ -19,6 +19,9 @@ namespace iql {
 
 #define IQL_STREAM_SAMPLE 0u        // counter word 3 for replay index sampling
 #define IQL_STREAM_DROPOUT_BASE 1u  // + hidden layer index, for dropout masks
+// + hidden layer index, for the dropout masks of the training-mode act (iql_act_host_members codes 4 / 5); the update
+// streams above use words 0 .. 1 + n_hidden, so the act masks never repeat a training mask of the same key
+#define IQL_STREAM_ACT_DROPOUT_BASE 0x80000000u
 
 struct Philox4 {
   uint32_t x, y, z, w;
@@ -70,6 +73,14 @@ __host__ __device__ __forceinline__ int64_t philox_index(uint64_t seed, uint64_t
 __host__ __device__ __forceinline__ Philox4 philox_dropout_quad(uint64_t seed, uint64_t step, uint32_t layer,
                                                                 uint32_t quad) {
   return philox4x32_10(quad, (uint32_t)step, (uint32_t)(step >> 32), IQL_STREAM_DROPOUT_BASE + layer,
+                       (uint32_t)seed, (uint32_t)(seed >> 32));
+}
+
+// The same for the act kernel: neurons 4 * quad .. 4 * quad + 3 of hidden layer `layer` at act counter `act_step`
+// (restated on the CPU in tests/act_mask_oracle.py).
+__host__ __device__ __forceinline__ Philox4 philox_act_dropout_quad(uint64_t seed, uint64_t act_step, uint32_t layer,
+                                                                    uint32_t quad) {
+  return philox4x32_10(quad, (uint32_t)act_step, (uint32_t)(act_step >> 32), IQL_STREAM_ACT_DROPOUT_BASE + layer,
                        (uint32_t)seed, (uint32_t)(seed >> 32));
 }
 

@@ -171,7 +171,8 @@ struct iql_engine {
   cudaEvent_t ev_in = nullptr, ev_out = nullptr;
   // online phase of an ensemble (iql_act_host_members / iql_replay_insert_members_host)
   const float* guide = nullptr;  // [S][P] guide parameter arena (iql_bind_guide), read only
-  char* h_actm = nullptr;        // pinned, device-mapped: states [S][state_dim] | ids [S] | codes [S] | results [S][2A] | flags [S]
+  char* h_actm = nullptr;        // pinned, device-mapped: states [S][state_dim] | ids [S] | codes [S] | steps [S] | results [S][2A] | flags [S]
+  std::vector<uint64_t> act_steps;  // [S] act counters of the dropout codes (IQL_ACT_LEARNER_DROPOUT)
   char* h_ins = nullptr;         // pinned, device-mapped: 2 slots of rows [S][RF] | ids [S] | pointers [S] | consumed [S]
   int ins_slot = 0;              // slot the next insert call fills
   int ins_n[2] = {0, 0};         // rows launched from each slot (their consumed words are awaited before the slot is refilled)
@@ -338,6 +339,7 @@ extern "C" int iql_create(const iql_config* cfg, iql_engine** out) {
   e->h_scalars.resize(S);
   e->h_hparams.resize(S);
   e->h_counters.assign(S, iql_counters{0, 0, 0, 0, 0, 0});
+  e->act_steps.assign(S, 0);
   e->h_replay.assign(S, ReplayBinding{nullptr, 0, 0});
   e->preloaded.assign(S, 0);
   e->active.resize(S);
@@ -1793,21 +1795,24 @@ extern "C" int iql_act_host_members(iql_engine* e, const float* host_states, con
                                     float* host_out, float* host_std, void* stream, void* caller_stream) {
   if (!e) return IQL_ERR_INVALID;
   if (!host_states || !host_source || !host_out) return fail(e, IQL_ERR_INVALID, "iql_act_host_members: null states, sources or output");
-  if (!e->bound) return fail(e, IQL_ERR_STATE, "iql_act_host_members: state not bound");
   const int S = e->cfg.n_members, Sd = e->cfg.state_dim, A = e->cfg.action_dim, L = e->cfg.n_hidden;
   int n = 0;
   for (int m = 0; m < S; ++m) {
     const int c = host_source[m];
-    if (c < IQL_ACT_SKIP || c > IQL_ACT_GUIDE) return fail(e, IQL_ERR_INVALID, "iql_act_host_members: unknown source code " + std::to_string(c));
+    if (c < IQL_ACT_SKIP || c > IQL_ACT_LEARNER_DIST_DROPOUT)
+      return fail(e, IQL_ERR_INVALID, "iql_act_host_members: unknown source code " + std::to_string(c));
     if (c == IQL_ACT_GUIDE && !e->guide) return fail(e, IQL_ERR_INVALID, "iql_act_host_members: a member asks for its guide, but no guide is bound (iql_bind_guide)");
-    if (c == IQL_ACT_LEARNER_DIST && e->cfg.deterministic)
+    const bool dist = c == IQL_ACT_LEARNER_DIST || c == IQL_ACT_LEARNER_DIST_DROPOUT;
+    if (dist && e->cfg.deterministic)
       return fail(e, IQL_ERR_INVALID, "iql_act_host_members: the distribution code needs a Gaussian policy; this one is deterministic");
-    if (c == IQL_ACT_LEARNER_DIST && !host_std) return fail(e, IQL_ERR_INVALID, "iql_act_host_members: null std with distribution members");
+    if (dist && !host_std) return fail(e, IQL_ERR_INVALID, "iql_act_host_members: null std with distribution members");
     n += c != IQL_ACT_SKIP;
   }
+  if (!e->bound) return fail(e, IQL_ERR_STATE, "iql_act_host_members: state not bound");
   if (n == 0) return IQL_OK;
   const size_t off_ids = align16(sizeof(float) * (size_t)S * Sd), off_codes = off_ids + align16(sizeof(int32_t) * S);
-  const size_t off_mail = off_codes + align16(sizeof(int32_t) * S), off_flags = off_mail + align16(sizeof(float) * (size_t)S * 2 * A);
+  const size_t off_steps = off_codes + align16(sizeof(int32_t) * S), off_mail = off_steps + align16(sizeof(uint64_t) * S);
+  const size_t off_flags = off_mail + align16(sizeof(float) * (size_t)S * 2 * A);
   if (!e->h_actm) {
     if (!host_events(e) || cudaHostAlloc((void**)&e->h_actm, off_flags + sizeof(uint32_t) * S, cudaHostAllocMapped) != cudaSuccess) {
       cudaGetLastError();
@@ -1818,16 +1823,20 @@ extern "C" int iql_act_host_members(iql_engine* e, const float* host_states, con
   float* states = (float*)e->h_actm;
   int32_t* ids = (int32_t*)(e->h_actm + off_ids);
   int32_t* codes = (int32_t*)(e->h_actm + off_codes);
+  uint64_t* steps = (uint64_t*)(e->h_actm + off_steps);
   float* mail = (float*)(e->h_actm + off_mail);
   volatile uint32_t* flags = (volatile uint32_t*)(e->h_actm + off_flags);
   // the previous call returned only after every flag of its launch was raised: the block is free to refill
   memcpy(states, host_states, sizeof(float) * (size_t)S * Sd);
   int j = 0;
+  bool drop_codes = false;
   for (int m = 0; m < S; ++m)
     if (host_source[m] != IQL_ACT_SKIP) {
       ids[j] = m;
       codes[j] = host_source[m];
+      steps[j] = e->act_steps[m];
       flags[m] = 0u;
+      drop_codes |= codes[j] == IQL_ACT_LEARNER_DROPOUT || codes[j] == IQL_ACT_LEARNER_DIST_DROPOUT;
       ++j;
     }
   std::atomic_thread_fence(std::memory_order_seq_cst);
@@ -1838,9 +1847,11 @@ extern "C" int iql_act_host_members(iql_engine* e, const float* host_states, con
   rc = flush_tables(e, cur);
   if (rc != IQL_OK) return rc;
   StepCtx ctx = make_ctx(e);
-  launch_act_members(ctx, e->params, e->guide, e->d_act_off, e->d_act_off + (L + 1), states, ids, codes, n, max_action, mail,
-                     (uint32_t*)flags, cur);
+  launch_act_members(ctx, e->params, e->guide, e->d_act_off, e->d_act_off + (L + 1), states, ids, codes, steps, drop_codes, n,
+                     max_action, mail, (uint32_t*)flags, cur);
   CUDA_TRY(e, cudaGetLastError());
+  for (int i = 0; i < n && drop_codes; ++i)  // the masks of the dropout codes are drawn: their counters move on, whatever p is
+    if (codes[i] == IQL_ACT_LEARNER_DROPOUT || codes[i] == IQL_ACT_LEARNER_DIST_DROPOUT) ++e->act_steps[ids[i]];
   for (int i = 0; i < n; ++i) {
     rc = spin_flag(e, flags + ids[i], cur, "iql_act_host_members");
     if (rc != IQL_OK) return rc;
@@ -1849,9 +1860,21 @@ extern "C" int iql_act_host_members(iql_engine* e, const float* host_states, con
     const int m = ids[i];
     const volatile float* row = mail + (size_t)m * 2 * A;
     for (int k = 0; k < A; ++k) host_out[(size_t)m * A + k] = row[k];
-    if (codes[i] == IQL_ACT_LEARNER_DIST)
+    if (codes[i] == IQL_ACT_LEARNER_DIST || codes[i] == IQL_ACT_LEARNER_DIST_DROPOUT)
       for (int k = 0; k < A; ++k) host_std[(size_t)m * A + k] = row[A + k];
   }
+  return IQL_OK;
+}
+
+extern "C" int iql_get_act_steps(iql_engine* e, uint64_t* host_out) {
+  if (!e || !host_out) return fail(e, IQL_ERR_INVALID, "iql_get_act_steps: null argument");
+  std::copy(e->act_steps.begin(), e->act_steps.end(), host_out);
+  return IQL_OK;
+}
+
+extern "C" int iql_set_act_steps(iql_engine* e, const uint64_t* host_in) {
+  if (!e || !host_in) return fail(e, IQL_ERR_INVALID, "iql_set_act_steps: null argument");
+  std::copy(host_in, host_in + e->cfg.n_members, e->act_steps.begin());
   return IQL_OK;
 }
 

@@ -200,10 +200,11 @@ void launch_act_host(const StepCtx& ctx, const float* actor_block, const int64_t
                      const float* host_state, float max_action, const float* log_std /* null: deterministic policy */, float* mail,
                      cudaStream_t st);
 // iql_act_host_members: one CTA per active member, the observations and the member list in a device-mapped pinned block
-// (`ids` [n] member indices, `codes` [n] IQL_ACT_* of those members); results [S][2A] + flag words [S] in pinned memory
+// (`ids` [n] member indices, `codes` [n] IQL_ACT_* of those members, `steps` [n] their act counters, read by codes 4 / 5;
+// `drop_codes`: some code is 4 or 5); results [S][2A] + flag words [S] in pinned memory
 void launch_act_members(const StepCtx& ctx, const float* params, const float* guide, const int64_t* w_off, const int64_t* b_off,
-                        const float* states, const int32_t* ids, const int32_t* codes, int n, float max_action, float* mail,
-                        uint32_t* flags, cudaStream_t st);
+                        const float* states, const int32_t* ids, const int32_t* codes, const uint64_t* steps, bool drop_codes,
+                        int n, float max_action, float* mail, uint32_t* flags, cudaStream_t st);
 // iql_replay_insert_members_host: one CTA per inserting member copies its packed row (device-mapped pinned block) to the
 // ring bound in `replay` and raises its consumed word
 void launch_insert_members(const ReplayBinding* replay, int RF, const float* rows, const int32_t* ids, const int64_t* pointers,

@@ -596,9 +596,21 @@ void launch_advance(const StepCtx& ctx, int K, cudaStream_t st) {
 constexpr int ACT_THREADS = 1024, ACT_NEURONS = 4, ACT_STATE_MAX = 512;
 struct ActState { float v[ACT_STATE_MAX]; };
 
+// Training-mode dropout of the act (iql_act_host_members codes 4 / 5): hidden unit j of layer l is kept iff word j & 3
+// of philox_act_dropout_quad(seed, step, l, j >> 2) is >= threshold, and a kept unit becomes relu(a) * scale -- the rule
+// of the update's forward epilogues, on the act's own Philox stream.
+struct ActDropout {
+  uint64_t seed, step;
+  uint32_t threshold;
+  float scale;
+};
+
+// DROP = false is the eval-mode body; `drop` is read only when DROP is true.
+template <bool DROP>
 __device__ __forceinline__ void act_body(int S, int A, int H, int L, const float* __restrict__ block,
                                          const int64_t* __restrict__ w_off, const int64_t* __restrict__ b_off,
-                                         const float* __restrict__ state, float max_action, float* __restrict__ out, float* sm) {
+                                         const float* __restrict__ state, float max_action, float* __restrict__ out, float* sm,
+                                         const ActDropout& drop = ActDropout{}) {
   const int width = ((H > S ? H : S) + 3) & ~3;
   float* cur = sm;
   float* nxt = sm + width;
@@ -636,8 +648,18 @@ __device__ __forceinline__ void act_body(int S, int A, int H, int L, const float
 #pragma unroll
         for (int u = 1; u < ACT_NEURONS; ++u) a = (lane == u) ? acc[u] : a;
         a += bias[j0 + lane];
-        if (l < L) nxt[j0 + lane] = fmaxf(a, 0.f);
-        else out[j0 + lane] = fminf(fmaxf(max_action * tanhf(a), -max_action), max_action);
+        if (l < L) {
+          float h = fmaxf(a, 0.f);
+          if constexpr (DROP) {
+            // j0 is a multiple of 4: the warp's four neurons are exactly one Philox quad
+            const Philox4 r = philox_act_dropout_quad(drop.seed, drop.step, (uint32_t)l, (uint32_t)(j0 >> 2));
+            const uint32_t w = lane == 0 ? r.x : lane == 1 ? r.y : lane == 2 ? r.z : r.w;
+            h = (w >= drop.threshold) ? h * drop.scale : 0.f;
+          }
+          nxt[j0 + lane] = h;
+        } else {
+          out[j0 + lane] = fminf(fmaxf(max_action * tanhf(a), -max_action), max_action);
+        }
       }
     }
     if (l < L)
@@ -656,7 +678,7 @@ __global__ void __launch_bounds__(ACT_THREADS) act_kernel(int S, int A, int H, i
   extern __shared__ float sm[];  // 2 * round_up(max(H, S), 4)
   // blockIdx.y = ensemble member (vectorised-env mode: every member's policy on its own rows), blockIdx.x = row
   const int64_t row = (int64_t)blockIdx.y * gridDim.x + blockIdx.x;
-  act_body(S, A, H, L, block0 + blockIdx.y * member_stride, w_off, b_off, states + row * S, max_action, out + row * A, sm);
+  act_body<false>(S, A, H, L, block0 + blockIdx.y * member_stride, w_off, b_off, states + row * S, max_action, out + row * A, sm);
 }
 
 // one observation from the kernel parameters, the action into pinned host memory + flag word (iql_act_host)
@@ -668,7 +690,7 @@ __global__ void __launch_bounds__(ACT_THREADS) act_host_kernel(int S, int A, int
   extern __shared__ float sm[];
   const int width = ((H > S ? H : S) + 3) & ~3;
   float* res = sm + 2 * width;  // [A]
-  act_body(S, A, H, L, block, w_off, b_off, state.v, max_action, res, sm);
+  act_body<false>(S, A, H, L, block, w_off, b_off, state.v, max_action, res, sm);
   __syncthreads();
   if (threadIdx.x < 32) {  // mailbox: [A] actions | [A] std = exp(clamp(log_std, -20, 2)) (Gaussian policies) | flag word
     for (int i = threadIdx.x; i < A; i += 32) {
@@ -691,21 +713,32 @@ void launch_act(const StepCtx& ctx, const float* actor_block, int n_members, con
 
 // every active member of an ensemble in one launch (iql_act_host_members): CTA i serves member ids[i] with the learner
 // arena or the guide arena; the observations are read from device-mapped pinned memory, the results go to the member's
-// mailbox row [2A] (action or mean | std) followed by the member's flag word.  act_body is the single-observation body
-// unchanged, so every member's result is bit-identical to act_host_kernel's.
+// mailbox row [2A] (action or mean | std) followed by the member's flag word.  For codes 0-3 act_body is the
+// single-observation body unchanged, so every member's result is bit-identical to act_host_kernel's; codes 4 / 5 add the
+// member's dropout (key and p from its MemberScalars) drawn at act counter steps[i].  DROP_CODES = false (no member of
+// the launch asks for dropout) compiles the kernel without the dropout body, so launches of codes 0-3 alone run the
+// instructions they ran before codes 4 / 5 existed.
+template <bool DROP_CODES>
 __global__ void __launch_bounds__(ACT_THREADS) act_members_kernel(int S, int A, int H, int L, const float* __restrict__ params,
                                                                   const float* __restrict__ guide, int64_t P,
                                                                   const int64_t* __restrict__ w_off,
                                                                   const int64_t* __restrict__ b_off, int64_t log_std_off,
                                                                   const float* states, const int32_t* ids, const int32_t* codes,
+                                                                  const uint64_t* steps, const MemberScalars* __restrict__ scalars,
                                                                   float max_action, float* mail, uint32_t* flags) {
   extern __shared__ float sm[];
   const int width = ((H > S ? H : S) + 3) & ~3;
   float* res = sm + 2 * width;  // [A]
   const int m = ids[blockIdx.x], code = codes[blockIdx.x];
   const float* block = (code == IQL_ACT_GUIDE ? guide : params) + (int64_t)m * P;
-  const bool dist = code == IQL_ACT_LEARNER_DIST;
-  act_body(S, A, H, L, block, w_off, b_off, states + (int64_t)m * S, dist ? 1.0f : max_action, res, sm);
+  const bool dist = code == IQL_ACT_LEARNER_DIST || (DROP_CODES && code == IQL_ACT_LEARNER_DIST_DROPOUT);
+  const bool drop = DROP_CODES && (code == IQL_ACT_LEARNER_DROPOUT || code == IQL_ACT_LEARNER_DIST_DROPOUT);
+  if (drop && scalars[m].drop_threshold != 0u) {  // p = 0: the eval-mode body, as in the update's epilogues
+    const ActDropout d{scalars[m].seed, steps[blockIdx.x], scalars[m].drop_threshold, scalars[m].drop_scale};
+    act_body<true>(S, A, H, L, block, w_off, b_off, states + (int64_t)m * S, dist ? 1.0f : max_action, res, sm, d);
+  } else {
+    act_body<false>(S, A, H, L, block, w_off, b_off, states + (int64_t)m * S, dist ? 1.0f : max_action, res, sm);
+  }
   __syncthreads();
   if (threadIdx.x < 32) {
     float* row = mail + (int64_t)m * 2 * A;
@@ -720,12 +753,12 @@ __global__ void __launch_bounds__(ACT_THREADS) act_members_kernel(int S, int A, 
 }
 
 void launch_act_members(const StepCtx& ctx, const float* params, const float* guide, const int64_t* w_off, const int64_t* b_off,
-                        const float* states, const int32_t* ids, const int32_t* codes, int n, float max_action, float* mail,
-                        uint32_t* flags, cudaStream_t st) {
+                        const float* states, const int32_t* ids, const int32_t* codes, const uint64_t* steps, bool drop_codes,
+                        int n, float max_action, float* mail, uint32_t* flags, cudaStream_t st) {
   const int width = ((ctx.H > ctx.S_dim ? ctx.H : ctx.S_dim) + 3) & ~3;
-  act_members_kernel<<<n, ACT_THREADS, (2 * width + ctx.A_dim) * sizeof(float), st>>>(
+  (drop_codes ? act_members_kernel<true> : act_members_kernel<false>)<<<n, ACT_THREADS, (2 * width + ctx.A_dim) * sizeof(float), st>>>(
       ctx.S_dim, ctx.A_dim, ctx.H, ctx.L, params, guide, ctx.P, w_off, b_off, ctx.deterministic ? 0 : ctx.log_std_off, states,
-      ids, codes, max_action, mail, flags);
+      ids, codes, steps, ctx.scalars, max_action, mail, flags);
 }
 
 int act_host_state_max() { return ACT_STATE_MAX; }

@@ -545,10 +545,13 @@ class EnsembleEngine:
     def act_members_host(self, states: np.ndarray, source, max_action: float = 1.0, out: Optional[np.ndarray] = None,
                          std: Optional[np.ndarray] = None):
         """One env step of every member's policy in one launch (`iql_act_host_members`).  ``states`` [S, state_dim],
-        ``source`` [S] IQL_ACT_* codes (int) or names ("skip", "learner", "learner_dist", "guide").  Returns
-        ``(out, std)``: out [S, action_dim] holds the eval-mode action of "learner" / "guide" members and the unscaled
-        mean of "learner_dist" members, std [S, action_dim] the std of the latter (None when there are none).  Rows of
-        skipped members are left as they were in ``out`` / ``std`` (NaN when the arrays are allocated here)."""
+        ``source`` [S] IQL_ACT_* codes (int) or names ("skip", "learner", "learner_dist", "guide", "learner_dropout",
+        "learner_dist_dropout").  Returns ``(out, std)``: out [S, action_dim] holds the eval-mode action of "learner" /
+        "guide" members, the training-mode action (actor dropout active) of "learner_dropout" members and the unscaled
+        mean of "learner_dist" / "learner_dist_dropout" members, std [S, action_dim] the std of the latter (None when
+        there are none).  Rows of skipped members are left as they were in ``out`` / ``std`` (NaN when the arrays are
+        allocated here).  Each dropout member draws its masks at its act counter (``act_steps``), which then advances
+        by one."""
         S, A = self.n_members, self.action_dim
         src = np.asarray([_lib.ACT_SOURCES[s] if isinstance(s, str) else int(s) for s in source], dtype=np.int8) \
             if not (isinstance(source, np.ndarray) and source.dtype == np.int8) else source
@@ -559,7 +562,7 @@ class EnsembleEngine:
             raise ValueError(f"states must be [{S}, {self.state_dim}]")
         if out is None:
             out = np.full((S, A), np.nan, dtype=np.float32)
-        if std is None and (src == _lib.ACT_LEARNER_DIST).any():
+        if std is None and ((src == _lib.ACT_LEARNER_DIST) | (src == _lib.ACT_LEARNER_DIST_DROPOUT)).any():
             std = np.full((S, A), np.nan, dtype=np.float32)
         for arr in (out, std):
             if arr is not None and (arr.shape != (S, A) or arr.dtype != np.float32 or not arr.flags.c_contiguous):
@@ -580,6 +583,24 @@ class EnsembleEngine:
                 guard.__exit__(None, None, None)
         self.act_calls += 1
         return out, std
+
+    @property
+    def act_steps(self) -> np.ndarray:
+        """[n_members] uint64: the act counters at which the members' next training-mode dropout acts draw their masks
+        (`iql_get_act_steps`; a copy)."""
+        out = np.zeros(self.n_members, dtype=np.uint64)
+        _lib.check(self._L.iql_get_act_steps(self._h, out.ctypes.data), self._h, "iql_get_act_steps")
+        return out
+
+    def set_act_steps(self, steps):
+        """Set every member's act counter (`iql_set_act_steps`): one non-negative integer per member."""
+        arr = np.asarray(steps).reshape(-1)
+        if arr.shape != (self.n_members,):
+            raise ValueError(f"need one act counter per member ({self.n_members}), got {arr.shape[0]}")
+        if arr.dtype.kind not in "ui" or (arr.dtype.kind == "i" and (arr < 0).any()):
+            raise ValueError("act counters must be non-negative integers")
+        arr = np.ascontiguousarray(arr, dtype=np.uint64)
+        _lib.check(self._L.iql_set_act_steps(self._h, arr.ctypes.data), self._h, "iql_set_act_steps")
 
     def insert_members_host(self, states: np.ndarray, actions: np.ndarray, rewards: np.ndarray, next_states: np.ndarray,
                             dones: np.ndarray, pointers: np.ndarray):

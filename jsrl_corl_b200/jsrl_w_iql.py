@@ -220,15 +220,16 @@ def train_loop(config, env, eval_env, replay_buffer: Optional[ReplayBuffer], sta
 # fix the engine shape and the update gate.  `batch_size` is checked on its own: it must be the same for every member
 # unless the caller asks for per-member batch sizes (`mixed_batch_sizes=True`); then the engine runs the largest,
 # member m trains on its own B_m rows (IQLEnsemble(batch_sizes=...)) and its gate `t >= B_m` keeps it inactive until it
-# opens.
+# opens.  `actor_dropout` > 0 needs `philox_act_dropout=True`: the learners' training-mode acts then draw their dropout
+# masks from the engine's Philox stream, not from torch's, so the loop asks the caller to say so.
 ENSEMBLE_SHARED_FIELDS = ("offline_iterations", "online_iterations", "eval_freq", "n_episodes", "horizon_fn",
                           "iql_deterministic", "actor_dropout", "new_online_buffer")
 
 
-def check_ensemble_configs(configs, scheduler=None, mixed_batch_sizes: bool = False):
+def check_ensemble_configs(configs, scheduler=None, mixed_batch_sizes: bool = False, philox_act_dropout: bool = False):
     """Refuse (ValueError) configs whose shared fields differ, whose batch sizes differ without ``mixed_batch_sizes``
     or are not positive integers, a scheduler without ``on_result``, and (NotImplementedError) the options the
-    ensemble loop does not cover.  Touches no device."""
+    ensemble loop does not cover, actor dropout without ``philox_act_dropout``.  Touches no device."""
     if len(configs) == 0:
         raise ValueError("ensemble_train_loop needs at least one config")
     for f in ENSEMBLE_SHARED_FIELDS:
@@ -256,9 +257,10 @@ def check_ensemble_configs(configs, scheduler=None, mixed_batch_sizes: bool = Fa
         raise NotImplementedError("ensemble_train_loop: the `variance` horizon needs a value network per member on the host")
     if c0.horizon_fn not in jsrl.HORIZON_FNS:
         raise ValueError(f"unknown horizon_fn {c0.horizon_fn!r}")
-    if c0.actor_dropout:
+    if c0.actor_dropout and not philox_act_dropout:
         raise NotImplementedError("ensemble_train_loop: training-mode act with active actor dropout has no engine kernel "
-                                  "(the single-learner path falls back to stock torch there)")
+                                  "(the single-learner path falls back to stock torch there); pass philox_act_dropout=True "
+                                  "to draw the learners' act masks in the engine's act kernel from its Philox stream")
 
 
 def member_networks(config, state_dim: int, action_dim: int, max_action: float):
@@ -283,17 +285,22 @@ def _member_hparams(c, t_max: int) -> Dict:
                 actor_lr=c.actor_lr, cosine_t_max=int(t_max))
 
 
-def _build_ensemble(configs, nets, state_dim, action_dim, t_max, device):
+def _build_ensemble(configs, nets, state_dim, action_dim, t_max, device, learner: bool = False):
+    """``learner`` (with actor dropout): the members' Philox keys get bit 63 set, so that a learner's masks -- of its
+    updates and of its training-mode acts -- never repeat those its guide (the offline member of the same seed) drew."""
     from .ensemble import IQLEnsemble
 
     c0 = configs[0]
     sizes = [int(c.batch_size) for c in configs]
+    p = float(c0.actor_dropout or 0.0)
+    keys = [int(c.seed) | (1 << 63) if learner and p > 0.0 else c.seed for c in configs]
     ens = IQLEnsemble(len(configs), state_dim, action_dim, 256, 2, max(sizes), deterministic=c0.iql_deterministic,
-                      device=device, max_steps_per_call=max(1, min(256, int(c0.eval_freq))), seeds=[c.seed for c in configs],
+                      actor_dropout=p, device=device, max_steps_per_call=max(1, min(256, int(c0.eval_freq))), seeds=keys,
                       hparams=[_member_hparams(c, t_max) for c in configs], init=False,
                       batch_sizes=sizes if len(set(sizes)) > 1 else None)
     for m, (q, v, actor) in enumerate(nets):
-        ens.engine.load_params(m, {"qf": q.state_dict(), "vf": v.state_dict(), "actor": actor.state_dict()})
+        ens.engine.load_params(m, {"qf": q.state_dict(), "vf": v.state_dict(), "actor": actor.state_dict()},
+                               dropout_keys=p > 0.0)
     return ens
 
 
@@ -376,7 +383,8 @@ def ensemble_eval_actor(envs, ensemble, use_guide: bool, configs, max_action: fl
 
 def ensemble_train_loop(configs, envs, eval_envs, replay_buffers, state_dim: int, action_dim: int, max_action: float,
                         max_steps: int, log: Optional[Callable[[int, Dict, int], None]] = None, reward_mod_dicts=None,
-                        is_env_with_goal: bool = False, scheduler=None, mixed_batch_sizes: bool = False):
+                        is_env_with_goal: bool = False, scheduler=None, mixed_batch_sizes: bool = False,
+                        philox_act_dropout: bool = False):
     """``train_loop`` for S members at once, one ``JsrlTrainConfig`` per member (seed, IQL / Adam hyper-parameters,
     curriculum, tolerance, noise and checkpoint path may differ; ``ENSEMBLE_SHARED_FIELDS`` may not; ``batch_size``
     may differ with ``mixed_batch_sizes=True``, the batch-size axis of a search).
@@ -397,8 +405,15 @@ def ensemble_train_loop(configs, envs, eval_envs, replay_buffers, state_dim: int
     stops gets no act, env step, insert, update, evaluation, log or checkpoint from then on and costs no GPU time.
     Members stopped offline skip the guide probe and start the online phase retired.  The run ends when every member
     has stopped.  Returns (learner ensemble, configs, one eval history per member); the guide ensemble is
-    ``learner.guide``."""
-    check_ensemble_configs(configs, scheduler, mixed_batch_sizes)
+    ``learner.guide``.
+
+    ``philox_act_dropout``: runs configs with ``actor_dropout`` > 0 (refused without it).  The learner's env steps act
+    in training mode as the reference's do, with dropout after every hidden ReLU, in the batched act kernel
+    (IQL_ACT_LEARNER_DIST_DROPOUT / IQL_ACT_LEARNER_DROPOUT): member m's masks come from the engine's Philox stream
+    keyed by ``seed | 1 << 63`` at its act counter (``learner.engine.act_steps[m]``, one per learner env step), so they
+    are reproducible but are not torch's ``nn.Dropout`` draws.  Guide acts and evaluations run without dropout.
+    Checkpoints carry the reference's dropout-policy keys."""
+    check_ensemble_configs(configs, scheduler, mixed_batch_sizes, philox_act_dropout)
     S = len(configs)
     if not (len(envs) == len(eval_envs) == S):
         raise ValueError("need one env and one eval env per member")
@@ -506,7 +521,7 @@ def ensemble_train_loop(configs, envs, eval_envs, replay_buffers, state_dim: int
     for m in np.flatnonzero(live):
         configs[m].curriculum_stage = np.nan
     probe = ensemble_eval_actor(envs, offline, False, configs, max_action, live)
-    learner = _build_ensemble(configs, [n[1] for n in nets], state_dim, action_dim, 0, device)
+    learner = _build_ensemble(configs, [n[1] for n in nets], state_dim, action_dim, 0, device, learner=True)
     for m, c in enumerate(configs):
         if c.n_curriculum_stages == 1:  # the guide's trained networks, fresh optimizers (get_learning_agent)
             learner.engine.load_params(m, offline.engine.param_views(m))
@@ -532,7 +547,10 @@ def ensemble_train_loop(configs, envs, eval_envs, replay_buffers, state_dim: int
     rewards = np.zeros(S, dtype=np.float32)
     real_dones = np.zeros(S, dtype=np.float32)
     source = np.zeros(S, dtype=np.int8)
-    learner_code = _lib_codes.ACT_LEARNER_DIST if gaussian else _lib_codes.ACT_LEARNER
+    if c0.actor_dropout:  # training mode: dropout active in the learner's act (checked: philox_act_dropout)
+        learner_code = _lib_codes.ACT_LEARNER_DIST_DROPOUT if gaussian else _lib_codes.ACT_LEARNER_DROPOUT
+    else:
+        learner_code = _lib_codes.ACT_LEARNER_DIST if gaussian else _lib_codes.ACT_LEARNER
     use = [False] * S
     ep_ret, ep_step, goal = [0.0] * S, [0] * S, [False] * S
     ep_types = [[] for _ in range(S)]
