@@ -15,6 +15,7 @@
 #include <map>
 #include <tuple>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "common.cuh"
@@ -68,14 +69,42 @@ struct Phase {
 };
 enum { PH_GENERIC = 0, PH_FIRST_FWD = 1, PH_OUT_FWD = 2, PH_LAST_WGRAD = 3, PH_LAST_DGRAD = 4, PH_FIRST_WGRAD = 5 };
 
+// The skinny-layer kernels keep one operand in shared memory; a layer whose operand does not fit takes the generic GEMM.
+static bool skinny_enabled() {
+  static const bool on = dbg_getenv("IQL_B200_NO_SKINNY") == nullptr;
+  return on;
+}
+
+// input-layer forward (first_fwd_kernel): K = state_dim + action_dim up to 72
+static bool first_fwd_skinny_ok(int k0) { return skinny_enabled() && k0 <= 72; }
+
+// input-layer weight gradient (first_wgrad_kernel): the batch's rows of X at the padded K
+static bool first_wgrad_skinny_ok(int batch, int k0) {
+  const int kpad = k0 <= 24 ? 24 : (k0 <= 40 ? 40 : 72);
+  return first_fwd_skinny_ok(k0) && ((size_t)batch * kpad + 512 * (kpad + 1)) * 4 <= 200 * 1024;
+}
+
+// output-layer forward (out_fwd_kernel): the padded head weights [apad][H]
+static bool out_fwd_skinny_ok(int hidden, int action_dim) {
+  const int apad = action_dim <= 1 ? 1 : (action_dim <= 8 ? 8 : (action_dim <= 24 ? 24 : 64));
+  return skinny_enabled() && action_dim <= 64 && (size_t)apad * hidden * 4 <= 200 * 1024;
+}
+
 // The output-layer backward runs on the skinny kernels (last_bwd_v4 / last_bwd_kernel<24>, the output-layer operand in
 // shared memory) up to 24 actions; wider heads take two generic GEMMs.  The chained backward starts from the skinny
 // kernels' outputs, so bind time and every step must agree on this rule.
 static bool last_bwd_skinny_ok(int batch, int action_dim) {
-  static const bool no_skinny = dbg_getenv("IQL_B200_NO_SKINNY") != nullptr;
   const int apad = action_dim <= 1 ? 1 : (action_dim <= 8 ? 8 : 24);
-  return !no_skinny && action_dim <= 24 && ((size_t)batch * apad + 256 * apad) * 4 <= 200 * 1024;
+  return skinny_enabled() && action_dim <= 24 && ((size_t)batch * apad + 256 * apad) * 4 <= 200 * 1024;
 }
+
+// The shape runs on the tcgen05 kernels.  TF32 math alone is not enough: outside the batch / hidden widths the tensor-core
+// kernels take, a TF32 engine runs the FP32 CUDA-core kernels.
+static bool tensor_core_path(const iql_config& c) {
+  return c.math_mode == IQL_MATH_TF32_TCGEN05 && umma_phase_supported(0, c.batch_size, c.hidden_dim);
+}
+
+using GraphKey = std::tuple<int, int, uintptr_t>;  // (sample mode or host-step variant, K, index pointer)
 
 struct iql_engine {
   iql_config cfg;
@@ -153,22 +182,22 @@ struct iql_engine {
   std::vector<char> is_active;   // [S]
   int64_t last_launches = 0;
   std::string err;
-  // CUDA graphs of the K-step sequence, keyed by K (Philox sampling mode only)
-  std::map<std::tuple<int, int, uintptr_t>, std::pair<cudaGraphExec_t, int64_t>> graphs;
+  // CUDA graphs of iql_train_steps and iql_train_host_step with their launch counts (launch_graph)
+  std::map<GraphKey, std::pair<cudaGraphExec_t, int64_t>> graphs;
   // the hidden-layer weight-gradient launches are leaves of the backward: they run on a side stream next to the
   // dgrad chain so that the partially filled last wave of one persistent kernel is covered by the other
   cudaStream_t side = nullptr;
   cudaEvent_t ev_fork = nullptr, ev_side = nullptr, ev_fork_g = nullptr, ev_gather = nullptr;
   bool use_graphs = true;
   // host-step path (iql_train_host_step): pinned, device-mapped host block = [S][B] int64 indices | [S][4] floats
-  // (losses + flag word, written by the loss kernel); events ordering the engine stream against the caller's stream
+  // (losses + flag word, written by the loss kernel); an event ordering a caller's stream behind the last host step
   unsigned long long* d_stamps = nullptr;  // IQL_STEP_TRACE: [ST_COUNT][2] globaltimer stamps (debug)
   float* h_act = nullptr;        // iql_act_host: pinned, device-mapped [action_dim floats | flag word]
   char* h_mail = nullptr;
   bool mail_pending = false;     // a host step has been launched and its losses not collected yet
   cudaStream_t host_step_stream = nullptr;  // the caller's stream the last host step was launched on
   bool host_step_stream_set = false;
-  cudaEvent_t ev_in = nullptr, ev_out = nullptr;
+  cudaEvent_t ev_in = nullptr;
   // online phase of an ensemble (iql_act_host_members / iql_replay_insert_members_host)
   const float* guide = nullptr;  // [S][P] guide parameter arena (iql_bind_guide), read only
   char* h_actm = nullptr;        // pinned, device-mapped: states [S][state_dim] | ids [S] | codes [S] | steps [S] | results [S][2A] | flags [S]
@@ -200,6 +229,48 @@ static int net_in_dim(const iql_config& c, int net) {
   return (net == IQL_NET_Q1 || net == IQL_NET_Q2) ? c.state_dim + c.action_dim : c.state_dim;
 }
 static int net_out_dim(const iql_config& c, int net) { return net == IQL_NET_ACTOR ? c.action_dim : 1; }
+
+// Problems in the tables of `members` training members: forward and backward phases, then the row-split copies of the
+// output-layer backward and the K-split copies of the input-layer weight gradient (build_problems)
+static int64_t problem_count(const iql_engine* e, int members) {
+  const int L = e->cfg.n_hidden;
+  return (int64_t)members * ((L + 1) * N_PASS + 4 * (L + 1) + 4 * L) +
+         (e->lb_splits > 1 ? (int64_t)12 * members * e->lb_splits : 0) + (e->fw_splits > 1 ? (int64_t)4 * members * e->fw_splits : 0);
+}
+
+// The device tables at the head of the workspace, in this order, each 256-byte aligned; sized for every member.  Returns
+// their size in bytes.  With the workspace `base` it also points the d_* tables into it; with base == nullptr it only
+// sizes them (iql_create), so the size and the pointers always come from the same list.
+static int64_t place_tables(iql_engine* e, char* base) {
+  const int S = e->cfg.n_members, L = e->cfg.n_hidden;
+  const int64_t nprob = problem_count(e, S);
+  int64_t tb = 0;
+  auto tab = [&](auto*& ptr, int64_t bytes) {
+    if (base) ptr = reinterpret_cast<std::remove_reference_t<decltype(ptr)>>(base + tb);
+    tb = round_up(tb + bytes, 256);
+  };
+  tab(e->d_scalars, sizeof(MemberScalars) * S);
+  tab(e->d_counters, sizeof(iql_counters) * S);
+  tab(e->d_replay, sizeof(ReplayBinding) * S);
+  tab(e->d_probs, sizeof(GemmProb) * nprob);
+  tab(e->d_maps, 128 * 2 * nprob);
+  tab(e->d_act_off, sizeof(int64_t) * 2 * (L + 1));
+  tab(e->d_loss_ring, sizeof(float) * 3 * (int64_t)S * e->cfg.max_steps_per_call);
+  tab(e->d_adam_sc, sizeof(AdamScalars) * 3 * S);
+  tab(e->d_active, sizeof(int32_t) * S);
+  if (e->cfg.math_mode == IQL_MATH_TF32_TCGEN05) {
+    tab(e->d_wshadow, sizeof(float) * (int64_t)S * e->layout.param_floats);
+    tab(e->d_tshadow, sizeof(float) * (int64_t)S * e->layout.q_floats);
+    tab(e->d_wshadow_lo, sizeof(float) * (int64_t)S * e->layout.param_floats);
+    tab(e->d_tshadow_lo, sizeof(float) * (int64_t)S * e->layout.q_floats);
+    tab(e->d_maps_first, (int64_t)128 * 4 * S * N_PASS);
+    tab(e->d_maps_store, (int64_t)128 * L * S * N_PASS);
+    tab(e->d_maps_c, (int64_t)128 * nprob);
+    tab(e->d_maps_chain, (int64_t)128 * 2 * 4 * S * (2 * L));  // chain maps: <= 2L - 1 phases x 4 S tasks x (A, B)
+    tab(e->d_maps_pol, (int64_t)128 * 4 * S);                   // policy-head maps: H_L, Wp hi, H_L, Wp lo
+  }
+  return tb;
+}
 
 static void build_layout(iql_engine* e) {
   const iql_config& c = e->cfg;
@@ -288,33 +359,8 @@ static void build_layout(iql_engine* e) {
   }
   wl.member_floats = w;
 
-  const int S = c.n_members;
-  const int64_t nprob = (int64_t)S * ((L + 1) * N_PASS + 4 * (L + 1) + 4 * L) + (e->lb_splits > 1 ? (int64_t)12 * S * e->lb_splits : 0) +
-                        (e->fw_splits > 1 ? (int64_t)4 * S * e->fw_splits : 0);
-  int64_t tb = 0;
-  auto tab = [&](int64_t bytes) { int64_t o = tb; tb = round_up(tb + bytes, 256); return o; };
-  tab(sizeof(MemberScalars) * S);
-  tab(sizeof(iql_counters) * S);
-  tab(sizeof(ReplayBinding) * S);
-  tab(sizeof(GemmProb) * nprob);
-  tab(128 * 2 * nprob);
-  tab(sizeof(int64_t) * 2 * (L + 1));
-  tab(sizeof(float) * 3 * (int64_t)S * c.max_steps_per_call);
-  tab(sizeof(AdamScalars) * 3 * S);
-  tab(sizeof(int32_t) * S);
-  if (c.math_mode == IQL_MATH_TF32_TCGEN05) {
-    tab(sizeof(float) * (int64_t)S * e->layout.param_floats);
-    tab(sizeof(float) * (int64_t)S * e->layout.q_floats);
-    tab(sizeof(float) * (int64_t)S * e->layout.param_floats);
-    tab(sizeof(float) * (int64_t)S * e->layout.q_floats);
-    tab((int64_t)128 * 4 * S * N_PASS);
-    tab((int64_t)128 * L * S * N_PASS);
-    tab((int64_t)128 * nprob);
-    tab((int64_t)128 * 2 * 4 * S * (2 * L));  // chain maps: <= 2L - 1 phases x 4 S tasks x (A, B)
-    tab((int64_t)128 * 4 * S);                // policy-head maps: H_L, Wp hi, H_L, Wp lo
-  }
-  e->tables_bytes = tb;
-  e->layout.workspace_bytes = tb + (int64_t)S * wl.member_floats * (int64_t)sizeof(float);
+  e->tables_bytes = place_tables(e, nullptr);
+  e->layout.workspace_bytes = e->tables_bytes + (int64_t)c.n_members * wl.member_floats * (int64_t)sizeof(float);
 }
 
 extern "C" int iql_create(const iql_config* cfg, iql_engine** out) {
@@ -362,16 +408,20 @@ extern "C" int iql_create(const iql_config* cfg, iql_engine** out) {
   return IQL_OK;
 }
 
+static void drop_graphs(iql_engine* e) {
+  for (auto& kv : e->graphs) cudaGraphExecDestroy(kv.second.first);
+  e->graphs.clear();
+}
+
 extern "C" void iql_destroy(iql_engine* e) {
   if (!e) return;
-  for (auto& kv : e->graphs) cudaGraphExecDestroy(kv.second.first);
+  drop_graphs(e);
   if (e->ev_fork) cudaEventDestroy(e->ev_fork);
   if (e->ev_side) cudaEventDestroy(e->ev_side);
   if (e->ev_fork_g) cudaEventDestroy(e->ev_fork_g);
   if (e->ev_gather) cudaEventDestroy(e->ev_gather);
   if (e->side) cudaStreamDestroy(e->side);
   if (e->ev_in) cudaEventDestroy(e->ev_in);
-  if (e->ev_out) cudaEventDestroy(e->ev_out);
   if (e->h_mail) cudaFreeHost(e->h_mail);
   if (e->h_act) cudaFreeHost(e->h_act);
   if (e->h_actm) cudaFreeHost(e->h_actm);
@@ -433,8 +483,7 @@ extern "C" int iql_set_option(iql_engine* e, int32_t key, int64_t value) {
   }
   if (key == IQL_OPT_KEEP_GRADS) {
     e->keep_grads = value != 0;
-    for (auto& kv : e->graphs) cudaGraphExecDestroy(kv.second.first);  // the flag is baked into captured launches
-    e->graphs.clear();
+    drop_graphs(e);  // the flag is baked into captured launches
     return IQL_OK;
   }
   return fail(e, IQL_ERR_INVALID, "iql_set_option: unknown key");
@@ -442,9 +491,8 @@ extern "C" int iql_set_option(iql_engine* e, int32_t key, int64_t value) {
 
 extern "C" int iql_get_info(const iql_engine* e, int32_t key, int64_t* out) {
   if (!e || !out) return IQL_ERR_INVALID;
-  const bool tc = e->cfg.math_mode == IQL_MATH_TF32_TCGEN05 && umma_phase_supported(0, e->cfg.batch_size, e->cfg.hidden_dim);
   switch (key) {
-    case IQL_INFO_TENSOR_CORE_PATH: *out = tc ? 1 : 0; return IQL_OK;   // 0: the FP32 CUDA-core kernels run this shape
+    case IQL_INFO_TENSOR_CORE_PATH: *out = tensor_core_path(e->cfg) ? 1 : 0; return IQL_OK;   // 0: the FP32 CUDA-core kernels run this shape
     case IQL_INFO_FUSED_FORWARD: *out = e->bound && e->fused_fwd ? 1 : 0; return IQL_OK;
     case IQL_INFO_CHAINED_BACKWARD: *out = e->bound && e->chain && !e->chain_grads ? 1 : 0; return IQL_OK;
     case IQL_INFO_CHAINED_BACKWARD_GRADS: *out = e->bound && e->chain && e->chain_grads ? 1 : 0; return IQL_OK;
@@ -490,7 +538,7 @@ static void build_problems(iql_engine* e) {
   const int ROW = e->layout.row.row_floats;
   const WorkspaceLayout& wl = e->wl;
   const int64_t P = e->layout.param_floats, PQ = e->layout.q_floats;
-  const bool use_shadow = c.math_mode == IQL_MATH_TF32_TCGEN05 && umma_phase_supported(0, B, H);
+  const bool use_shadow = tensor_core_path(c);
   // hidden-layer weights as tcgen05 operands: read from the arenas themselves (biased in place during a call) instead of
   // from a TF32-rounded shadow copy
   e->bias_hidden = use_shadow && L >= 2 && L <= 4 && dbg_getenv("IQL_B200_NO_BIASED_WEIGHTS") == nullptr;
@@ -684,10 +732,9 @@ static void build_problems(iql_engine* e) {
 // the workspace split (lb_splits / fw_splits) stays as iql_create sized it.
 static int bind_tables(iql_engine* e) {
   const int Sa = (int)e->active.size(), L = e->cfg.n_hidden;
-  const int64_t nprob = (int64_t)Sa * ((L + 1) * N_PASS + 4 * (L + 1) + 4 * L) + (e->lb_splits > 1 ? (int64_t)12 * Sa * e->lb_splits : 0) +
-                        (e->fw_splits > 1 ? (int64_t)4 * Sa * e->fw_splits : 0);
+  const int64_t nprob = problem_count(e, Sa);
   build_problems(e);
-  const bool tc_mode = e->cfg.math_mode == IQL_MATH_TF32_TCGEN05 && umma_phase_supported(0, e->cfg.batch_size, e->cfg.hidden_dim);
+  const bool tc_mode = tensor_core_path(e->cfg);
   // 3xTF32 input layer, and on top of it the fused forward (all hidden layers of a tile chained through TMEM)
   e->split_first = tc_mode && dbg_getenv("IQL_B200_NO_SPLIT_FIRST") == nullptr;
   e->fused_fwd = e->split_first && umma_can_fuse_out(e->cfg.action_dim) &&
@@ -879,31 +926,7 @@ extern "C" int iql_bind_state(iql_engine* e, float* params, float* exp_avg, floa
   if (all & 127) return fail(e, IQL_ERR_INVALID, "iql_bind_state: pointers must be 128-byte aligned");
   e->params = params; e->exp_avg = exp_avg; e->exp_avg_sq = exp_avg_sq; e->target = target; e->grads = grads;
   e->ws = (char*)workspace; e->ws_bytes = workspace_bytes;
-  const int S = e->cfg.n_members, L = e->cfg.n_hidden;
-  const int64_t nprob = (int64_t)S * ((L + 1) * N_PASS + 4 * (L + 1) + 4 * L) + (e->lb_splits > 1 ? (int64_t)12 * S * e->lb_splits : 0) +
-                        (e->fw_splits > 1 ? (int64_t)4 * S * e->fw_splits : 0);
-  int64_t tb = 0;
-  auto tab = [&](int64_t bytes) { char* o = e->ws + tb; tb = round_up(tb + bytes, 256); return o; };
-  e->d_scalars = (MemberScalars*)tab(sizeof(MemberScalars) * S);
-  e->d_counters = (iql_counters*)tab(sizeof(iql_counters) * S);
-  e->d_replay = (ReplayBinding*)tab(sizeof(ReplayBinding) * S);
-  e->d_probs = (GemmProb*)tab(sizeof(GemmProb) * nprob);
-  e->d_maps = tab(128 * 2 * nprob);
-  e->d_act_off = (int64_t*)tab(sizeof(int64_t) * 2 * (L + 1));
-  e->d_loss_ring = (float*)tab(sizeof(float) * 3 * (int64_t)S * e->cfg.max_steps_per_call);
-  e->d_adam_sc = (AdamScalars*)tab(sizeof(AdamScalars) * 3 * S);
-  e->d_active = (int32_t*)tab(sizeof(int32_t) * S);
-  if (e->cfg.math_mode == IQL_MATH_TF32_TCGEN05) {
-    e->d_wshadow = (float*)tab(sizeof(float) * (int64_t)S * e->layout.param_floats);
-    e->d_tshadow = (float*)tab(sizeof(float) * (int64_t)S * e->layout.q_floats);
-    e->d_wshadow_lo = (float*)tab(sizeof(float) * (int64_t)S * e->layout.param_floats);
-    e->d_tshadow_lo = (float*)tab(sizeof(float) * (int64_t)S * e->layout.q_floats);
-    e->d_maps_first = tab((int64_t)128 * 4 * S * N_PASS);
-    e->d_maps_store = tab((int64_t)128 * L * S * N_PASS);
-    e->d_maps_c = tab((int64_t)128 * nprob);
-    e->d_maps_chain = tab((int64_t)128 * 2 * 4 * S * (2 * L));
-    e->d_maps_pol = tab((int64_t)128 * 4 * S);
-  }
+  place_tables(e, e->ws);
   e->d_ws_f = (float*)(e->ws + e->tables_bytes);
   int rc = bind_tables(e);
   if (rc != IQL_OK) return rc;
@@ -923,8 +946,7 @@ extern "C" int iql_bind_state(iql_engine* e, float* params, float* exp_avg, floa
   }
   e->bound = true;
   e->tables_dirty = e->scalars_dirty = e->counters_dirty = e->replay_dirty = true;
-  for (auto& kv : e->graphs) cudaGraphExecDestroy(kv.second.first);
-  e->graphs.clear();
+  drop_graphs(e);
   return IQL_OK;
 }
 
@@ -989,7 +1011,7 @@ static StepCtx make_ctx(const iql_engine* e) {
   c.loss_ring = e->d_loss_ring;
   c.adam_sc = e->d_adam_sc;
   c.k_max = e->cfg.max_steps_per_call;
-  c.tf32 = (e->cfg.math_mode == IQL_MATH_TF32_TCGEN05) && umma_phase_supported(0, e->cfg.batch_size, e->cfg.hidden_dim);
+  c.tf32 = tensor_core_path(e->cfg);
   c.w_shadow = e->d_wshadow;
   c.t_shadow = e->d_tshadow;
   c.w_shadow_lo = e->d_wshadow_lo;
@@ -1095,7 +1117,8 @@ static int enqueue_step(iql_engine* e, StepCtx& ctx, bool gather, cudaStream_t s
                         bool gather_next = false) {
   int launches = 0;
   cudaStream_t st = st_main;  // the stream run_phase launches on (switched to e->side for the wgrad leaves)
-  const bool tf32 = e->cfg.math_mode == IQL_MATH_TF32_TCGEN05;
+  // the math mode only: on a shape outside the tcgen05 kernels (tensor_core_path false) it is still true
+  const bool tf32_math = e->cfg.math_mode == IQL_MATH_TF32_TCGEN05;
   const double S_d = (double)e->active.size();
   if (gather) {
     if (tm) tm->mark("gather", 0, 2.0 * S_d * e->cfg.batch_size * e->layout.row.row_floats * 4);
@@ -1104,12 +1127,9 @@ static int enqueue_step(iql_engine* e, StepCtx& ctx, bool gather, cudaStream_t s
   }
   const iql_config& c = e->cfg;
   const int B = c.batch_size, H = c.hidden_dim, A = c.action_dim, K0 = c.state_dim + c.action_dim;
-  // the skinny-layer kernels keep one operand in shared memory; fall back to the generic GEMM when it does not fit
-  static const bool no_skinny = dbg_getenv("IQL_B200_NO_SKINNY") != nullptr;
-  auto kpad = [](int k) { return k <= 24 ? 24 : (k <= 40 ? 40 : 72); };
-  const bool first_ok = !no_skinny && K0 <= 72;
-  const bool first_wgrad_ok = first_ok && ((size_t)B * kpad(K0) + 512 * (kpad(K0) + 1)) * 4 <= 200 * 1024;
-  const bool out_ok = !no_skinny && A <= 64 && (size_t)(A <= 1 ? 1 : (A <= 8 ? 8 : (A <= 24 ? 24 : 64))) * H * 4 <= 200 * 1024;
+  const bool first_ok = first_fwd_skinny_ok(K0);
+  const bool first_wgrad_ok = first_wgrad_skinny_ok(B, K0);
+  const bool out_ok = out_fwd_skinny_ok(H, A);
   const bool last_ok = last_bwd_skinny_ok(B, A);
   static const bool no_side = dbg_getenv("IQL_B200_NO_SIDE_STREAM") != nullptr;
   const bool loss_recomputed = last_ok && e->bwd_phases.size() >= 2 &&
@@ -1119,11 +1139,20 @@ static int enqueue_step(iql_engine* e, StepCtx& ctx, bool gather, cudaStream_t s
   bool skip_next = false, skip_colsum = false;
   // the reduction of the row-split output-layer backward (single learners) only feeds the optimizer: it leaves the
   // critical path last_bwd -> dgrad -> ... through the side stream (8 us of a 57 us single-learner step)
-  const bool lb_side = tf32 && !tm && !no_side && e->side != nullptr;
+  const bool lb_side = tf32_math && !tm && !no_side && e->side != nullptr;
   bool lb_on_side = false;
   auto run_phase = [&](const Phase& ph, const Phase* next, const Phase* next2) {
     if (skip_next) { skip_next = false; return; }
     const GemmProb* pp = e->d_probs + ph.first;
+    // Mixed precision: the input layer (observations, K = 11..69) and the output heads run in FP32 on CUDA
+    // cores; every hidden-layer GEMM and the first-layer weight gradient run as TF32 tcgen05 GEMMs.  TF32 on the
+    // input layer doubles the value-loss error (measured 1.2e-3 -> 2.6e-3) for < 10 % of the step time.
+    const bool split = ph.kind == PH_FIRST_FWD && e->split_first;  // 3xTF32: FP32-accurate on tensor cores
+    const bool umma = tf32_math && ph.umma_ok && umma_phase_supported(ph.mode, B, H) &&
+                      !(ph.kind == PH_FIRST_FWD && !split && first_ok);
+    // forward, last hidden layer on the tensor cores: the FP32 output Linear is fused into the epilogue, the next phase skipped
+    const bool fuse_out = umma && ph.mode == 0 && ph.epi == EPI_RELU && next && next->kind == PH_OUT_FWD && H == 256 &&
+                          umma_can_fuse_out(A);
     if (tm) {  // algorithmic work: 2MNK flops; each operand read once, the output written once
       double fl = 0, by = 0;
       auto add = [&](const Phase& q) {
@@ -1134,36 +1163,23 @@ static int enqueue_step(iql_engine* e, StepCtx& ctx, bool gather, cudaStream_t s
         }
       };
       add(ph);
-      const bool fuse_next = next && ((ph.kind == PH_LAST_WGRAD && next->kind == PH_LAST_DGRAD) ||
-                                      (next->kind == PH_OUT_FWD && ph.mode == 0 && ph.epi == EPI_RELU && tf32 && H == 256 &&
-                                       umma_can_fuse_out(A) && umma_phase_supported(0, B, H)));
-      if (fuse_next) add(*next);
+      if (fuse_out || (next && ph.kind == PH_LAST_WGRAD && next->kind == PH_LAST_DGRAD)) add(*next);
       static const char* kinds[] = {"gemm", "first_fwd", "out_fwd", "last_bwd", "last_dgrad", "first_wgrad"};
       static const char* modes[] = {"fwd", "dgrad", "wgrad"};
       char nm[32];
-      snprintf(nm, sizeof(nm), "%s_%s%s", ph.kind == PH_GENERIC ? "hidden" : kinds[ph.kind], modes[ph.mode],
-               (tf32 && ph.umma_ok && umma_phase_supported(ph.mode, B, H)) ? "" : "");
+      snprintf(nm, sizeof(nm), "%s_%s", ph.kind == PH_GENERIC ? "hidden" : kinds[ph.kind], modes[ph.mode]);
       tm->mark(nm, fl, by);
     }
-    // Mixed precision: the input layer (observations, K = 11..69) and the output heads run in FP32 on CUDA
-    // cores; every hidden-layer GEMM and the first-layer weight gradient run as TF32 tcgen05 GEMMs.  TF32 on the
-    // input layer doubles the value-loss error (measured 1.2e-3 -> 2.6e-3) for < 10 % of the step time.
-    const bool split = ph.kind == PH_FIRST_FWD && e->split_first;  // 3xTF32: FP32-accurate on tensor cores
-    const bool umma = tf32 && ph.umma_ok && umma_phase_supported(ph.mode, B, H) &&
-                      !(ph.kind == PH_FIRST_FWD && !split && first_ok);
     if (umma && ph.kind == PH_OUT_FWD) {
       // the heads stay in FP32: TF32 rounding of Q and V would be amplified by adv = q - v and exp(beta * adv)
       if (out_ok) launch_out_fwd(pp, ph.count, B, H, A, st);
       else launch_simt_gemm(ph.mode, pp, ph.count, ph.maxM, ph.maxN, ctx, st);
     } else if (umma && ph.kind != PH_LAST_WGRAD) {
-      // forward, last hidden layer: fuse the FP32 output Linear into the epilogue and skip the next phase
-      const bool fuse = ph.mode == 0 && ph.epi == EPI_RELU && next && next->kind == PH_OUT_FWD && H == 256 &&
-                        umma_can_fuse_out(A);
       const int n_scalar = (N_PASS - 1) * (int)e->active.size();  // problems with a scalar head (V, Q passes)
       launch_umma_gemm(ph.mode, pp, split ? e->d_maps_first : e->d_maps + (size_t)256 * ph.first,
-                       fuse ? e->d_probs + next->first : nullptr, ph.epi, ph.count, ph.maxM, ph.maxN, ctx, st, split,
+                       fuse_out ? e->d_probs + next->first : nullptr, ph.epi, ph.count, ph.maxM, ph.maxN, ctx, st, split,
                        n_scalar, ph.cta2, ph.maxK, ph.rowepi ? e->d_maps_c + (size_t)128 * ph.first : nullptr, ph.tile_n);
-      if (fuse) {  // the policy head (N = act_dim) stays with the FP32 output-layer kernel
+      if (fuse_out) {  // the policy head (N = act_dim) stays with the FP32 output-layer kernel
         const GemmProb* pa = e->d_probs + next->first + n_scalar;
         if (out_ok) launch_out_fwd(pa, ph.count - n_scalar, B, H, A, st);
         else launch_simt_gemm(0, pa, ph.count - n_scalar, B, A, ctx, st);
@@ -1182,7 +1198,7 @@ static int enqueue_step(iql_engine* e, StepCtx& ctx, bool gather, cudaStream_t s
     } else if (ph.kind == PH_LAST_WGRAD && last_ok && next && next->kind == PH_LAST_DGRAD) {
       // fused wgrad + dgrad of the output layer; it also emits db_{L-1} when layer L-1 is a hidden-layer
       // tcgen05 wgrad phase (whose kernel does not produce bias gradients)
-      const bool emit_db = next2 && tf32 && next2->umma_ok && umma_phase_supported(2, B, H);
+      const bool emit_db = next2 && tf32_math && next2->umma_ok && umma_phase_supported(2, B, H);
       if (e->lb_splits > 1 && e->bwd_phases.size() >= 3 && ph.first == e->bwd_phases[0].first) {
         const int sp = e->lb_splits, n = ph.count * sp;
         const GemmProb* t0 = e->d_probs + e->lb_first;
@@ -1209,7 +1225,7 @@ static int enqueue_step(iql_engine* e, StepCtx& ctx, bool gather, cudaStream_t s
     }
     ++launches;
   };
-  if (tf32 && e->fused_fwd) {
+  if (tf32_math && e->fused_fwd) {
     // one launch for layers 0..L-1 + scalar heads; the policy head (N = act_dim) stays with the FP32 output kernel
     const int L = c.n_hidden;
     const int n_scalar = (N_PASS - 1) * (int)e->active.size();
@@ -1278,7 +1294,7 @@ static int enqueue_step(iql_engine* e, StepCtx& ctx, bool gather, cudaStream_t s
   }
   ++launches;
   // per-kernel timing (tm) keeps everything on one stream
-  const bool two_streams = tf32 && !tm && !no_side && e->side != nullptr;
+  const bool two_streams = tf32_math && !tm && !no_side && e->side != nullptr;
   int forks = 0;
   // chained backward: the output-layer backward (phases 0, 1) runs as before, everything after it -- hidden dgrad /
   // wgrad chain, input-layer wgrad (+ Adam + Polyak unless gradient-only) -- is ONE launch on CTA pairs.  Bind time set
@@ -1291,7 +1307,7 @@ static int enqueue_step(iql_engine* e, StepCtx& ctx, bool gather, cudaStream_t s
     const Phase* n2 = i + 2 < e->bwd_phases.size() ? &e->bwd_phases[i + 2] : nullptr;
     const bool leaf = two_streams && ph.mode == 2 && ph.kind == PH_GENERIC && ph.umma_ok &&
                       umma_phase_supported(2, B, H) && !skip_next;
-    if (ph.kind == PH_FIRST_WGRAD && e->fw_splits > 1 && tf32 && ph.umma_ok && umma_phase_supported(2, B, H) && !skip_next) {
+    if (ph.kind == PH_FIRST_WGRAD && e->fw_splits > 1 && tf32_math && ph.umma_ok && umma_phase_supported(2, B, H) && !skip_next) {
       // few problems x a long batch: the tcgen05 kernel runs the K-split copies (enough tiles to fill the GPU), then the
       // partial dW_0 / db_0 are added up in split order
       run_phase(e->fw_phase, nullptr, nullptr);  // batch > 256: the phase also runs colsum_kernel (partial db_0)
@@ -1368,6 +1384,37 @@ static int enqueue_step(iql_engine* e, StepCtx& ctx, bool gather, cudaStream_t s
   return launches;
 }
 
+// Launch the graph cached under `key` on `run`.  On a miss, `body` (enqueues the launches on `capture`, returns how many)
+// is captured into a new graph first.  *launches receives the graph's launch count.
+template <class Body>
+static int launch_graph(iql_engine* e, const GraphKey& key, cudaStream_t capture, cudaStream_t run, const char* who, Body&& body,
+                        int64_t* launches) {
+  auto it = e->graphs.find(key);
+  if (it == e->graphs.end()) {
+    cudaGraph_t graph = nullptr;
+    CUDA_TRY(e, cudaStreamBeginCapture(capture, cudaStreamCaptureModeThreadLocal));
+    const int64_t n = body();
+    cudaError_t cerr = cudaStreamEndCapture(capture, &graph);
+    if (cerr != cudaSuccess) return fail(e, IQL_ERR_CUDA, std::string(who) + ": graph capture: " + cudaGetErrorString(cerr));
+    cudaGraphExec_t exec = nullptr;
+    CUDA_TRY(e, cudaGraphInstantiate(&exec, graph, 0));
+    cudaGraphDestroy(graph);
+    it = e->graphs.emplace(key, std::make_pair(exec, n)).first;
+  }
+  CUDA_TRY(e, cudaGraphLaunch(it->second.first, run));
+  *launches = it->second.second;
+  return IQL_OK;
+}
+
+// The host shadow of the counters moves with the device copy: a call of k steps advances every member that trained
+static void advance_counters(iql_engine* e, int k) {
+  for (const int m : e->active) {
+    iql_counters& c = e->h_counters[m];
+    c.v_step += k; c.q_step += k; c.actor_step += k; c.total_it += k; c.sample_step += k;
+    if (e->h_hparams[m].cosine_t_max > 0) c.sched_epoch += k;
+  }
+}
+
 extern "C" int iql_train_steps(iql_engine* e, int32_t k_steps, int32_t sample_mode, const int64_t* indices,
                                const uint8_t* dropout_masks, float* out_losses, int64_t* idx_out, void* stream) {
   if (!e) return IQL_ERR_INVALID;
@@ -1403,57 +1450,36 @@ extern "C" int iql_train_steps(iql_engine* e, int32_t k_steps, int32_t sample_mo
   static const bool no_overlap_gather = dbg_getenv("IQL_B200_NO_GATHER_AHEAD") != nullptr || dbg_getenv("IQL_B200_NO_SIDE_STREAM") != nullptr;
   // (not with the chained backward + optimizer: its last phase still reads the gathered rows, see enqueue_step)
   const bool overlap_gather = !no_overlap_gather && e->side != nullptr && st != nullptr && !(e->chain && !e->chain_grads);
+  auto k_step_loop = [&]() -> int64_t {
+    int64_t n = 0;
+    for (int k = 0; k < k_steps; ++k) {
+      ctx.k = k;
+      if (k == k_steps - 1) ctx.advance_k = k_steps;
+      const bool ahead = gather && overlap_gather && k + 1 < k_steps;  // step k+1's gather rides along step k's optimizer
+      n += enqueue_step(e, ctx, gather && (k == 0 || !overlap_gather), st, nullptr, ahead);
+    }
+    if (ctx.advance_k != -1) { launch_advance(ctx, k_steps, st); ++n; }
+    return n;
+  };
   // the legacy default stream cannot be captured; the facade runs the engine on its own stream
   // Graphs: the K-step Philox loop, and the single preloaded step of the drop-in `train(batch)` path (its ~11
-  // launches would otherwise be launch-latency bound).  Keyed by K, negative for the preloaded variant.
+  // launches would otherwise be launch-latency bound).  Keyed by sample mode and K.
   // (the index pointer is baked into the captured kernels, so the INDICES variant is keyed by it: callers that
   // reuse one staging buffer -- the Python facade does -- replay one graph; at most 16 graphs are kept)
   const bool graphable = e->use_graphs && st != nullptr && !dropout_masks && !idx_out &&
                          (k_steps > 1 || sample_mode == IQL_SAMPLE_PRELOADED);
-  const auto graph_key = std::make_tuple((int)sample_mode, (int)k_steps,
-                                         sample_mode == IQL_SAMPLE_INDICES ? (uintptr_t)indices : (uintptr_t)0);
-  if (graphable && e->graphs.size() >= 16 && e->graphs.find(graph_key) == e->graphs.end()) {
-    for (auto& kv : e->graphs) cudaGraphExecDestroy(kv.second.first);
-    e->graphs.clear();
-  }
+  const GraphKey graph_key((int)sample_mode, (int)k_steps, sample_mode == IQL_SAMPLE_INDICES ? (uintptr_t)indices : (uintptr_t)0);
+  if (graphable && e->graphs.size() >= 16 && e->graphs.find(graph_key) == e->graphs.end()) drop_graphs(e);
   int64_t launches = 0;
   if (graphable) {
-    auto it = e->graphs.find(graph_key);
-    if (it == e->graphs.end()) {
-      cudaGraph_t graph = nullptr;
-      CUDA_TRY(e, cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
-      for (int k = 0; k < k_steps; ++k) {
-        ctx.k = k;
-        if (k == k_steps - 1) ctx.advance_k = k_steps;
-        const bool ahead = gather && overlap_gather && k + 1 < k_steps;  // step k+1's gather rides along step k's optimizer
-        launches += enqueue_step(e, ctx, gather && (k == 0 || !overlap_gather), st, nullptr, ahead);
-      }
-      if (ctx.advance_k != -1) { launch_advance(ctx, k_steps, st); ++launches; }
-      cudaError_t cerr = cudaStreamEndCapture(st, &graph);
-      if (cerr != cudaSuccess) return fail(e, IQL_ERR_CUDA, std::string("graph capture: ") + cudaGetErrorString(cerr));
-      cudaGraphExec_t exec = nullptr;
-      CUDA_TRY(e, cudaGraphInstantiate(&exec, graph, 0));
-      cudaGraphDestroy(graph);
-      it = e->graphs.emplace(graph_key, std::make_pair(exec, launches)).first;
-    }
-    CUDA_TRY(e, cudaGraphLaunch(it->second.first, st));
-    launches = it->second.second;
+    rc = launch_graph(e, graph_key, st, st, "iql_train_steps", k_step_loop, &launches);
+    if (rc != IQL_OK) return rc;
   } else {
-    for (int k = 0; k < k_steps; ++k) {
-      ctx.k = k;
-      if (k == k_steps - 1) ctx.advance_k = k_steps;
-      const bool ahead = gather && overlap_gather && k + 1 < k_steps;
-      launches += enqueue_step(e, ctx, gather && (k == 0 || !overlap_gather), st, nullptr, ahead);
-    }
-    if (ctx.advance_k != -1) { launch_advance(ctx, k_steps, st); ++launches; }
+    launches = k_step_loop();
   }
   CUDA_TRY(e, cudaGetLastError());
-  for (const int m : e->active) {
-    iql_counters& c = e->h_counters[m];
-    c.v_step += k_steps; c.q_step += k_steps; c.actor_step += k_steps; c.total_it += k_steps; c.sample_step += k_steps;
-    if (e->h_hparams[m].cosine_t_max > 0) c.sched_epoch += k_steps;
-    e->preloaded[m] = 0;
-  }
+  advance_counters(e, k_steps);
+  for (const int m : e->active) e->preloaded[m] = 0;
   if (idx_out)  // the gather writes the rows of the members that trained; the others read -1 (all-ones bytes)
     for (int m = 0; m < S; ++m)
       if (!e->is_active[m])
@@ -1475,13 +1501,29 @@ extern "C" int iql_train_steps(iql_engine* e, int32_t k_steps, int32_t sample_mo
 // pinned memory, the whole step, counter advance).  The loss kernel stores its scalars into device-mapped pinned
 // memory and raises a flag word; this function spins on that word and returns as soon as the losses of the step are on
 // the host -- while the step's backward and optimizer launches are still running, so the caller's host work for the
-// next step (index draw, Python) overlaps them.  Everything the caller enqueues afterwards is stream-ordered behind
-// the step (ev_out), exactly as after iql_train_steps.
+// next step (index draw, Python) overlaps them.
 // ---------------------------------------------------------------------------
-static bool host_events(iql_engine* e) {  // events that order the engine stream against the caller's stream
-  if (e->ev_in && e->ev_out) return true;
-  return cudaEventCreateWithFlags(&e->ev_in, cudaEventDisableTiming) == cudaSuccess &&
-         cudaEventCreateWithFlags(&e->ev_out, cudaEventDisableTiming) == cudaSuccess;
+// Pinned, device-mapped host block of the host-driven entry points (kernels read and write it at its host address),
+// allocated zeroed on first use together with ev_in, the event order_behind_host_step records.
+static int pinned_block(iql_engine* e, void** block, size_t bytes, const char* who) {
+  if (*block) return IQL_OK;
+  if ((!e->ev_in && cudaEventCreateWithFlags(&e->ev_in, cudaEventDisableTiming) != cudaSuccess) ||
+      cudaHostAlloc(block, bytes, cudaHostAllocMapped) != cudaSuccess) {
+    cudaGetLastError();
+    *block = nullptr;
+    return fail(e, IQL_ERR_CUDA, std::string(who) + ": pinned block / event allocation failed");
+  }
+  memset(*block, 0, bytes);
+  return IQL_OK;
+}
+
+// The caller's stream waits for the stream of the last host step when the two differ
+static int order_behind_host_step(iql_engine* e, cudaStream_t cur) {
+  if (e->host_step_stream_set && e->host_step_stream != cur) {
+    CUDA_TRY(e, cudaEventRecord(e->ev_in, e->host_step_stream));
+    CUDA_TRY(e, cudaStreamWaitEvent(cur, e->ev_in, 0));
+  }
+  return IQL_OK;
 }
 
 // Spin until the device has raised `flag` (pinned host memory); bounded, and a failed launch is noticed through the stream.
@@ -1508,6 +1550,14 @@ static int spin_flag(iql_engine* e, volatile uint32_t* flag, cudaStream_t st, co
 }
 
 extern "C" int iql_host_step_wait(iql_engine* e, float* host_losses, void* stream);
+
+// Collect a host step still in flight (its losses are dropped), so that its flag words and index block can be reused
+static int collect_host_step(iql_engine* e) {
+  if (!e->mail_pending) return IQL_OK;
+  std::vector<float> sink(3 * (size_t)e->cfg.n_members);
+  return iql_host_step_wait(e, sink.data(), e->host_step_stream);
+}
+
 extern "C" int iql_train_host_step(iql_engine* e, const int64_t* host_indices, float* host_losses, void* stream,
                                    void* caller_stream) {
   if (!e) return IQL_ERR_INVALID;
@@ -1521,24 +1571,12 @@ extern "C" int iql_train_host_step(iql_engine* e, const int64_t* host_indices, f
     if (!gather && !e->preloaded[m]) return fail(e, IQL_ERR_STATE, "iql_train_host_step: no batch staged (call iql_load_batch)");
   }
   const size_t idx_bytes = sizeof(int64_t) * (size_t)S * B;
-  if (!e->h_mail) {
-    if (!host_events(e) || cudaHostAlloc((void**)&e->h_mail, idx_bytes + sizeof(float) * 4 * S, cudaHostAllocMapped) != cudaSuccess) {
-      cudaGetLastError();
-      e->h_mail = nullptr;
-      return fail(e, IQL_ERR_CUDA, "iql_train_host_step: pinned mailbox / event allocation failed");
-    }
-    memset(e->h_mail, 0, idx_bytes + sizeof(float) * 4 * S);
-  }
+  int rc = pinned_block(e, (void**)&e->h_mail, idx_bytes + sizeof(float) * 4 * S, "iql_train_host_step");
+  if (rc != IQL_OK) return rc;
   int64_t* mail_idx = (int64_t*)e->h_mail;
   float* mail = (float*)(e->h_mail + idx_bytes);
-  if (e->mail_pending) {  // one step in flight at a time: its gather may not have read the index block yet
-    float drop[3 * 64];
-    std::vector<float> big;
-    float* sink = drop;
-    if (S > 64) { big.resize(3 * (size_t)S); sink = big.data(); }
-    int rcw = iql_host_step_wait(e, sink, e->host_step_stream);
-    if (rcw != IQL_OK) return rcw;
-  }
+  rc = collect_host_step(e);  // one step in flight at a time: its gather may not have read the index block yet
+  if (rc != IQL_OK) return rc;
   if (gather)
     for (const int m : e->active) {  // rows of members that do not train are never read
       const int64_t cap = e->h_replay[m].capacity;
@@ -1556,52 +1594,37 @@ extern "C" int iql_train_host_step(iql_engine* e, const int64_t* host_indices, f
   // stream against the caller's (iql_act_host, the Python guard around iql_train_steps).  A caller that hops between
   // streams gets the two ordered by an event.
   cudaStream_t run = cur;
-  if (e->host_step_stream_set && e->host_step_stream != run) {
-    CUDA_TRY(e, cudaEventRecord(e->ev_in, e->host_step_stream));
-    CUDA_TRY(e, cudaStreamWaitEvent(run, e->ev_in, 0));
-  }
+  rc = order_behind_host_step(e, run);
+  if (rc != IQL_OK) return rc;
   e->host_step_stream = run;
   e->host_step_stream_set = true;
-  int rc = flush_tables(e, run);
+  rc = flush_tables(e, run);
   if (rc != IQL_OK) return rc;
-  const auto graph_key = std::make_tuple(gather ? 101 : 102, 1, (uintptr_t)0);
-  auto it = e->graphs.find(graph_key);
-  if (it == e->graphs.end()) {
+  auto one_step = [&]() -> int64_t {
     StepCtx ctx = make_ctx(e);
     ctx.K = 1;
     ctx.k = 0;
     ctx.indices = gather ? mail_idx : nullptr;  // unified addressing: the pinned block is device-visible at its host address
     ctx.host_mail = mail;
-    cudaGraph_t graph = nullptr;
-    int64_t launches = 0;
-    CUDA_TRY(e, cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
+    int64_t n = 0;
     // the TF32 operand refresh and the gather are independent: one launch, which releases the forward at once
     const bool fork_refresh = ctx.tf32 && gather;
     if (fork_refresh) {
       launch_gather_refresh(ctx, e->d_ws_f, e->wl.member_floats, e->wl.xrow, e->params, e->target, st);
-      ++launches;
+      ++n;
     } else if (ctx.tf32) {
       launch_refresh_shadow(ctx, e->params, e->target, st);
-      ++launches;
+      ++n;
     }
     ctx.advance_k = 1;
-    launches += enqueue_step(e, ctx, gather && !fork_refresh, st, nullptr, false);
-    if (ctx.advance_k != -1) { launch_advance(ctx, 1, st); ++launches; }
-    cudaError_t cerr = cudaStreamEndCapture(st, &graph);
-    if (cerr != cudaSuccess) return fail(e, IQL_ERR_CUDA, std::string("iql_train_host_step: graph capture: ") + cudaGetErrorString(cerr));
-    cudaGraphExec_t exec = nullptr;
-    CUDA_TRY(e, cudaGraphInstantiate(&exec, graph, 0));
-    cudaGraphDestroy(graph);
-    it = e->graphs.emplace(graph_key, std::make_pair(exec, launches)).first;
-  }
-  CUDA_TRY(e, cudaGraphLaunch(it->second.first, run));
-  e->last_launches = it->second.second;
-  for (const int m : e->active) {
-    iql_counters& c = e->h_counters[m];
-    c.v_step += 1; c.q_step += 1; c.actor_step += 1; c.total_it += 1; c.sample_step += 1;
-    if (e->h_hparams[m].cosine_t_max > 0) c.sched_epoch += 1;
-    e->preloaded[m] = 0;
-  }
+    n += enqueue_step(e, ctx, gather && !fork_refresh, st, nullptr, false);
+    if (ctx.advance_k != -1) { launch_advance(ctx, 1, st); ++n; }
+    return n;
+  };
+  rc = launch_graph(e, GraphKey(gather ? 101 : 102, 1, 0), st, run, "iql_train_host_step", one_step, &e->last_launches);
+  if (rc != IQL_OK) return rc;
+  advance_counters(e, 1);
+  for (const int m : e->active) e->preloaded[m] = 0;
   e->mail_pending = true;
   if (!host_losses) return IQL_OK;  // the caller collects the losses with iql_host_step_wait
   return iql_host_step_wait(e, host_losses, run);
@@ -1643,16 +1666,13 @@ extern "C" int iql_set_active_members(iql_engine* e, int32_t n, const int32_t* h
     mask[m] = 1;
   }
   if (!e->bound) return fail(e, IQL_ERR_STATE, "iql_set_active_members: state not bound");
-  if (e->mail_pending) {  // the in-flight host step's flag words belong to the old set: collect it first
-    std::vector<float> sink(3 * (size_t)S);
-    const int rcw = iql_host_step_wait(e, sink.data(), e->host_step_stream);
-    if (rcw != IQL_OK) return rcw;
-  }
+  int rc = collect_host_step(e);  // the in-flight host step's flag words belong to the old set
+  if (rc != IQL_OK) return rc;
   const std::vector<int32_t> old = e->active;
   e->active.clear();
   for (int m = 0; m < S; ++m)
     if (mask[m]) e->active.push_back(m);
-  int rc = bind_tables(e);
+  rc = bind_tables(e);
   if (rc != IQL_OK) {  // cannot happen for a set the old tables were built for; restore it anyway
     e->active = old;
     bind_tables(e);
@@ -1660,8 +1680,7 @@ extern "C" int iql_set_active_members(iql_engine* e, int32_t n, const int32_t* h
   }
   e->is_active = mask;
   e->tables_dirty = true;
-  for (auto& kv : e->graphs) cudaGraphExecDestroy(kv.second.first);  // the tables' sizes are baked into the launches
-  e->graphs.clear();
+  drop_graphs(e);  // the tables' sizes are baked into the launches
   return IQL_OK;
 }
 
@@ -1738,24 +1757,17 @@ static int act_host_impl(iql_engine* e, int32_t member, const float* host_state,
   if (e->cfg.state_dim > act_host_state_max()) return fail(e, IQL_ERR_INVALID, "iql_act_host: state_dim too large for the by-value path (use iql_act)");
   cudaStream_t st = (cudaStream_t)stream, cur = (cudaStream_t)caller_stream;
   const int A = e->cfg.action_dim, L = e->cfg.n_hidden;
-  if (!e->h_act) {
-    if (!host_events(e) || cudaHostAlloc((void**)&e->h_act, sizeof(float) * (2 * A + 1), cudaHostAllocMapped) != cudaSuccess) {
-      cudaGetLastError();
-      e->h_act = nullptr;
-      return fail(e, IQL_ERR_CUDA, "iql_act_host: pinned mailbox / event allocation failed");
-    }
-  }
+  int rc = pinned_block(e, (void**)&e->h_act, sizeof(float) * (2 * A + 1), "iql_act_host");
+  if (rc != IQL_OK) return rc;
   volatile uint32_t* flag = reinterpret_cast<volatile uint32_t*>(e->h_act + 2 * A);
   *flag = 0u;
   std::atomic_thread_fence(std::memory_order_seq_cst);
   // launched on the caller's stream, like the host step: ordered behind the last update by stream order (a K-step call
   // on the engine's stream is ordered against the caller's stream by the Python guard around iql_train_steps)
   (void)st;
-  if (e->host_step_stream_set && e->host_step_stream != cur) {
-    CUDA_TRY(e, cudaEventRecord(e->ev_in, e->host_step_stream));
-    CUDA_TRY(e, cudaStreamWaitEvent(cur, e->ev_in, 0));
-  }
-  int rc = flush_tables(e, cur);
+  rc = order_behind_host_step(e, cur);
+  if (rc != IQL_OK) return rc;
+  rc = flush_tables(e, cur);
   if (rc != IQL_OK) return rc;
   StepCtx ctx = make_ctx(e);
   const float* block = e->params + (int64_t)member * e->layout.param_floats;
@@ -1774,15 +1786,6 @@ static int act_host_impl(iql_engine* e, int32_t member, const float* host_state,
 // Online phase of an ensemble: one act launch and one ring-insert launch per env step for all members
 // ---------------------------------------------------------------------------
 static size_t align16(size_t n) { return (n + 15) & ~(size_t)15; }
-
-// the caller's stream waits for the stream of the last host step when the two differ (as in act_host_impl)
-static int order_behind_host_step(iql_engine* e, cudaStream_t cur) {
-  if (e->host_step_stream_set && e->host_step_stream != cur) {
-    CUDA_TRY(e, cudaEventRecord(e->ev_in, e->host_step_stream));
-    CUDA_TRY(e, cudaStreamWaitEvent(cur, e->ev_in, 0));
-  }
-  return IQL_OK;
-}
 
 extern "C" int iql_bind_guide(iql_engine* e, const float* guide_params) {
   if (!e) return IQL_ERR_INVALID;
@@ -1813,13 +1816,8 @@ extern "C" int iql_act_host_members(iql_engine* e, const float* host_states, con
   const size_t off_ids = align16(sizeof(float) * (size_t)S * Sd), off_codes = off_ids + align16(sizeof(int32_t) * S);
   const size_t off_steps = off_codes + align16(sizeof(int32_t) * S), off_mail = off_steps + align16(sizeof(uint64_t) * S);
   const size_t off_flags = off_mail + align16(sizeof(float) * (size_t)S * 2 * A);
-  if (!e->h_actm) {
-    if (!host_events(e) || cudaHostAlloc((void**)&e->h_actm, off_flags + sizeof(uint32_t) * S, cudaHostAllocMapped) != cudaSuccess) {
-      cudaGetLastError();
-      e->h_actm = nullptr;
-      return fail(e, IQL_ERR_CUDA, "iql_act_host_members: pinned block / event allocation failed");
-    }
-  }
+  int rc = pinned_block(e, (void**)&e->h_actm, off_flags + sizeof(uint32_t) * S, "iql_act_host_members");
+  if (rc != IQL_OK) return rc;
   float* states = (float*)e->h_actm;
   int32_t* ids = (int32_t*)(e->h_actm + off_ids);
   int32_t* codes = (int32_t*)(e->h_actm + off_codes);
@@ -1842,7 +1840,7 @@ extern "C" int iql_act_host_members(iql_engine* e, const float* host_states, con
   std::atomic_thread_fence(std::memory_order_seq_cst);
   cudaStream_t cur = (cudaStream_t)caller_stream;
   (void)stream;
-  int rc = order_behind_host_step(e, cur);
+  rc = order_behind_host_step(e, cur);
   if (rc != IQL_OK) return rc;
   rc = flush_tables(e, cur);
   if (rc != IQL_OK) return rc;
@@ -1908,14 +1906,8 @@ extern "C" int iql_replay_insert_members_host(iql_engine* e, const float* host_s
                                           std::to_string(rings[i].second) + " share one ring; members must not see each other's transitions");
   const size_t off_ids = align16(sizeof(float) * (size_t)S * RF), off_ptr = off_ids + align16(sizeof(int32_t) * S);
   const size_t off_cons = off_ptr + align16(sizeof(int64_t) * S), slot_bytes = align16(off_cons + sizeof(uint32_t) * S);
-  if (!e->h_ins) {
-    if (!host_events(e) || cudaHostAlloc((void**)&e->h_ins, 2 * slot_bytes, cudaHostAllocMapped) != cudaSuccess) {
-      cudaGetLastError();
-      e->h_ins = nullptr;
-      return fail(e, IQL_ERR_CUDA, "iql_replay_insert_members_host: pinned block / event allocation failed");
-    }
-    e->ins_n[0] = e->ins_n[1] = 0;
-  }
+  int rc = pinned_block(e, (void**)&e->h_ins, 2 * slot_bytes, "iql_replay_insert_members_host");
+  if (rc != IQL_OK) return rc;
   const int s = e->ins_slot;
   char* slot = e->h_ins + s * slot_bytes;
   float* rows = (float*)slot;
@@ -1925,7 +1917,7 @@ extern "C" int iql_replay_insert_members_host(iql_engine* e, const float* host_s
   // guard: the launch that last read this slot must have consumed every row of it (it was issued two calls ago, so
   // this almost never waits; it is a spin on pinned words, not a stream synchronisation)
   for (int i = 0; i < e->ins_n[s]; ++i) {
-    int rc = spin_flag(e, consumed + i, e->ins_stream[s], "iql_replay_insert_members_host");
+    rc = spin_flag(e, consumed + i, e->ins_stream[s], "iql_replay_insert_members_host");
     if (rc != IQL_OK) return rc;
   }
   int i = 0;
@@ -1946,7 +1938,7 @@ extern "C" int iql_replay_insert_members_host(iql_engine* e, const float* host_s
   std::atomic_thread_fence(std::memory_order_seq_cst);
   cudaStream_t cur = (cudaStream_t)caller_stream;
   (void)stream;
-  int rc = order_behind_host_step(e, cur);
+  rc = order_behind_host_step(e, cur);
   if (rc != IQL_OK) return rc;
   rc = flush_tables(e, cur);
   if (rc != IQL_OK) return rc;
@@ -2014,11 +2006,7 @@ extern "C" int iql_profile_step(iql_engine* e, int32_t reps, int32_t max_slots, 
     enqueue_step(e, ctx, true, st, &tm);
     launch_advance(ctx, 1, st);
     CUDA_TRY(e, cudaStreamSynchronize(st));
-    for (const int m : e->active) {
-      iql_counters& c = e->h_counters[m];
-      c.v_step++; c.q_step++; c.actor_step++; c.total_it++; c.sample_step++;
-      if (e->h_hparams[m].cosine_t_max > 0) c.sched_epoch++;
-    }
+    advance_counters(e, 1);
     if (acc.empty()) acc.assign(tm.label.size(), 0.0);
     for (size_t i = 0; i + 1 < tm.ev.size() && i < acc.size(); ++i) {
       float ms = 0.f;
