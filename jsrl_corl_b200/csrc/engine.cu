@@ -12,6 +12,7 @@
 #include <algorithm>
 #include <atomic>
 #include <chrono>
+#include <functional>
 #include <map>
 #include <tuple>
 #include <string>
@@ -30,20 +31,38 @@ static thread_local std::string g_create_error;
 // crossover against the per-phase backward on the B200 (profiles/r03_summary.md)
 static constexpr int CHAIN_GRADS_MIN_MEMBERS = 8;
 
+// The update step as plan_step lays it out for the bound shape: entries in launch order, one per profile slot, each a
+// few kernel launches with their arguments bound.  A launch runs on the main stream, on the side stream (forked from
+// main at that launch, joined before the optimizer), or as a hidden-layer wgrad leaf on the side stream (the fork first
+// waits for the previous leaf).  An entry's side launches come last in it; the entry records ev_side after them.
+enum StepLane { LANE_MAIN, LANE_SIDE, LANE_LEAF };
+using StepFn = std::function<int(StepCtx&, cudaStream_t)>;  // enqueues a launch, returns how many kernels it launched
+struct StepLaunch {
+  StepFn run;
+  int lane;
+};
+struct StepEntry {
+  std::string label;    // iql_profile_step slot
+  double flops, bytes;  // algorithmic work of the slot
+  std::vector<StepLaunch> launches;
+  bool gather = false;  // the step's own gather: only when the call asks for it
+  bool join = false;    // the optimizer: joins the side stream first; the next step's gather may run beside it
+};
+
 // Optional per-launch instrumentation of one update step (iql_profile_step).
 struct StepTimer {
   std::vector<cudaEvent_t> ev;       // ev[i] recorded BEFORE launch i; one extra at the end
   std::vector<std::string> label;
   std::vector<double> flops, bytes;  // algorithmic work of the launch
   cudaStream_t st = nullptr;
-  void mark(const char* name, double fl, double by) {
+  void mark(const StepEntry& s) {
     cudaEvent_t e;
     cudaEventCreate(&e);
     cudaEventRecord(e, st);
     ev.push_back(e);
-    label.push_back(name);
-    flops.push_back(fl);
-    bytes.push_back(by);
+    label.push_back(s.label);
+    flops.push_back(s.flops);
+    bytes.push_back(s.bytes);
   }
   void finish() {
     cudaEvent_t e;
@@ -92,7 +111,7 @@ static bool out_fwd_skinny_ok(int hidden, int action_dim) {
 
 // The output-layer backward runs on the skinny kernels (last_bwd_v4 / last_bwd_kernel<24>, the output-layer operand in
 // shared memory) up to 24 actions; wider heads take two generic GEMMs.  The chained backward starts from the skinny
-// kernels' outputs, so bind time and every step must agree on this rule.
+// kernels' outputs, so the chain's gate and the step plan both ask this rule.
 static bool last_bwd_skinny_ok(int batch, int action_dim) {
   const int apad = action_dim <= 1 ? 1 : (action_dim <= 8 ? 8 : 24);
   return skinny_enabled() && action_dim <= 24 && ((size_t)batch * apad + 256 * apad) * 4 <= 200 * 1024;
@@ -153,7 +172,9 @@ struct iql_engine {
   int step_path = 0;             // iql_set_option(IQL_OPT_STEP_PATH): 0 auto, 1 per-phase kernels, 2 chained backward +
                                  // optimizer, 4 chained backward (gradients) + adam_polyak_kernel (2 and 4 required)
   int keep_grads = 0;            // iql_set_option(IQL_OPT_KEEP_GRADS): the chained backward also stores the weight gradients
-  BwdChainArgs chain_args;
+  BwdChainArgs chain_args;       // all but keep_grads, filled when the chain is set up
+  std::vector<StepEntry> plan;   // the update step (plan_step, rebuilt by every bind_tables)
+  bool gather_ahead = false;     // the next step's gather may run on the side stream beside this step's optimizer
   char* d_maps_chain = nullptr;
   std::vector<char> h_maps_chain;
   // policy heads wider than the fused forward's epilogue handles (8 < act_dim <= 32): z = H_L Wp^T + b as a two-pass
@@ -727,6 +748,8 @@ static void build_problems(iql_engine* e) {
   }
 }
 
+static void plan_step(iql_engine* e);
+
 // The part of binding that depends on which members train: problem tables, tensor maps, the chained backward's task
 // list and every path choice made from the member count.  Run by iql_bind_state and again by iql_set_active_members;
 // the workspace split (lb_splits / fw_splits) stays as iql_create sized it.
@@ -906,12 +929,16 @@ static int bind_tables(iql_engine* e) {
     }
     e->chain = ok;
     e->chain_grads = ok && e->step_path != 2;
+    ca.probs = e->d_probs; ca.maps = e->d_maps_chain; ca.cmaps = e->d_maps_c;
+    ca.grads_only = e->chain_grads ? 1 : 0;
+    ca.params = e->params; ca.exp_avg = e->exp_avg; ca.exp_avg_sq = e->exp_avg_sq; ca.target = e->target; ca.grads = e->grads;
     if (!ok) e->h_maps_chain.clear();
   }
   if ((e->step_path == 2 || e->step_path == 4) && !e->chain)
     return fail(e, IQL_ERR_INVALID, "iql_bind_state: IQL_OPT_STEP_PATH = chained backward, but this shape / math mode does not support it "
                                     "(needs tf32, hidden 256, batch 256, 2..4 hidden layers, action_dim <= 24, "
                                     "state_dim + action_dim <= 256)");
+  plan_step(e);
   return IQL_OK;
 }
 
@@ -928,9 +955,7 @@ extern "C" int iql_bind_state(iql_engine* e, float* params, float* exp_avg, floa
   e->ws = (char*)workspace; e->ws_bytes = workspace_bytes;
   place_tables(e, e->ws);
   e->d_ws_f = (float*)(e->ws + e->tables_bytes);
-  int rc = bind_tables(e);
-  if (rc != IQL_OK) return rc;
-  if (!e->side) {  // optional: without it the backward simply stays on one stream
+  if (!e->side) {  // optional: without it the whole step runs on one stream; bind_tables reads it
     if (cudaStreamCreateWithFlags(&e->side, cudaStreamNonBlocking) != cudaSuccess ||
         cudaEventCreateWithFlags(&e->ev_fork, cudaEventDisableTiming) != cudaSuccess ||
         cudaEventCreateWithFlags(&e->ev_side, cudaEventDisableTiming) != cudaSuccess ||
@@ -940,6 +965,8 @@ extern "C" int iql_bind_state(iql_engine* e, float* params, float* exp_avg, floa
       e->side = nullptr;
     }
   }
+  int rc = bind_tables(e);
+  if (rc != IQL_OK) return rc;
   if (dbg_getenv("IQL_STEP_TRACE") && !e->d_stamps && cudaMalloc((void**)&e->d_stamps, sizeof(unsigned long long) * 2 * ST_COUNT) != cudaSuccess) {
     cudaGetLastError();
     e->d_stamps = nullptr;
@@ -1079,269 +1106,214 @@ extern "C" int iql_load_batch(iql_engine* e, int32_t member, const float* states
   return IQL_OK;
 }
 
-// The chained backward (bwd_chain.cu) after the output-layer backward: hidden dgrad / wgrad chain and input-layer wgrad,
-// plus Adam + Polyak in the wgrad epilogues unless the engine runs it gradient-only.  With `tm`, the work of the launch
-// goes to the timer's last slot.
-static void launch_chain(iql_engine* e, const StepCtx& ctx, cudaStream_t st, StepTimer* tm) {
-  if (tm) {  // operands read once; dZ written; the weight gradients written (gradient-only) or the optimizer state streamed
-    double fl = 0, by = 0;
-    for (size_t i = 2; i < e->bwd_phases.size(); ++i) {
-      const Phase& q = e->bwd_phases[i];
-      for (int j = 0; j < q.count; ++j) {
-        const GemmProb& g = e->h_probs[q.first + j];
-        fl += 2.0 * g.M * g.N * g.K;
-        by += 4.0 * ((double)g.M * g.K + (double)g.N * g.K + (q.mode == 1 || e->chain_grads ? (double)g.M * g.N : 0.0));
-      }
-    }
-    if (!e->chain_grads)  // p, m, v in and out + shadows
-      by += e->active.size() * 4.0 * ((6.0 + 1.0) * e->layout.param_floats + 3.0 * e->layout.q_floats);
-    tm->flops.back() = fl;
-    tm->bytes.back() = by;
+// Algorithmic work of a launch (iql_profile_step)
+struct Work {
+  double flops = 0, bytes = 0;
+  Work& operator+=(const Work& o) { flops += o.flops; bytes += o.bytes; return *this; }
+};
+
+// Work of problems [first, first + count) of the table: 2MNK flops each (per pass), every operand read once -- A only
+// with `read_a` -- and the output written once unless `store` is false or the problem skips its store; with `mask` the
+// FP32 ReLU mask of a dgrad problem is read too
+static Work gemm_work(const iql_engine* e, int first, int count, bool store = true, bool mask = true, bool read_a = true,
+                      double passes = 1.0) {
+  Work w;
+  for (int i = first; i < first + count; ++i) {
+    const GemmProb& g = e->h_probs[i];
+    const double mn = (double)g.M * g.N;
+    w.flops += 2.0 * mn * g.K * passes;
+    w.bytes += 4.0 * ((read_a ? (double)g.M * g.K : 0.0) + (double)g.N * g.K + (store && !g.no_store ? mn : 0.0) +
+                      (mask && g.mask ? mn : 0.0));
   }
-  BwdChainArgs ca = e->chain_args;
-  ca.probs = e->d_probs;
-  ca.maps = e->d_maps_chain;
-  ca.cmaps = e->d_maps_c;
-  ca.keep_grads = e->keep_grads;
-  ca.grads_only = e->chain_grads ? 1 : 0;
-  ca.params = e->params; ca.exp_avg = e->exp_avg; ca.exp_avg_sq = e->exp_avg_sq; ca.target = e->target; ca.grads = e->grads;
-  launch_bwd_chain(ca, ctx, st);
+  return w;
 }
 
-// one update step for all members; returns number of launches
-// gather: sample + gather this step's rows first.  gather_next: the NEXT step's gather (ctx.k + 1) runs on the side
-// stream next to this step's optimizer launch -- nothing after the input-layer weight gradient reads the row
-// buffers, the gather is pure latency and the optimizer pure bandwidth -- and the caller passes gather = false for
-// that next step.
-static int enqueue_step(iql_engine* e, StepCtx& ctx, bool gather, cudaStream_t st_main, StepTimer* tm = nullptr,
-                        bool gather_next = false) {
-  int launches = 0;
-  cudaStream_t st = st_main;  // the stream run_phase launches on (switched to e->side for the wgrad leaves)
-  // the math mode only: on a shape outside the tcgen05 kernels (tensor_core_path false) it is still true
-  const bool tf32_math = e->cfg.math_mode == IQL_MATH_TF32_TCGEN05;
-  const double S_d = (double)e->active.size();
-  if (gather) {
-    if (tm) tm->mark("gather", 0, 2.0 * S_d * e->cfg.batch_size * e->layout.row.row_floats * 4);
-    launch_gather(ctx, e->d_ws_f, e->wl.member_floats, e->wl.xrow, st);
-    ++launches;
-  }
+// The update step of the bound shape and active members: which kernel serves each phase, with what arguments, on which
+// stream lane, and the work of each profile slot.  Every kernel choice and debug switch of the step is read here, once
+// per bind_tables, so that enqueue_step only walks the list.
+static void plan_step(iql_engine* e) {
   const iql_config& c = e->cfg;
-  const int B = c.batch_size, H = c.hidden_dim, A = c.action_dim, K0 = c.state_dim + c.action_dim;
-  const bool first_ok = first_fwd_skinny_ok(K0);
-  const bool first_wgrad_ok = first_wgrad_skinny_ok(B, K0);
-  const bool out_ok = out_fwd_skinny_ok(H, A);
-  const bool last_ok = last_bwd_skinny_ok(B, A);
-  static const bool no_side = dbg_getenv("IQL_B200_NO_SIDE_STREAM") != nullptr;
-  const bool loss_recomputed = last_ok && e->bwd_phases.size() >= 2 &&
-                               last_bwd_recomputes_loss_grads(H, A, e->bwd_phases[0].count * e->lb_splits, B / e->lb_splits) &&
-                               e->bwd_phases[0].kind == PH_LAST_WGRAD && e->bwd_phases[1].kind == PH_LAST_DGRAD &&
-                               e->bwd_phases[0].count % 4 == 0;
+  const int B = c.batch_size, H = c.hidden_dim, A = c.action_dim, L = c.n_hidden, K0 = c.state_dim + c.action_dim;
+  const double S_d = (double)e->active.size();
+  const int n_scalar = (N_PASS - 1) * (int)e->active.size();  // problems with a scalar head (V, Q passes)
+  const std::vector<Phase>&fwd = e->fwd_phases, &bwd = e->bwd_phases;
+  // the math mode only: on a shape outside the tcgen05 kernels (tensor_core_path false) it is still true
+  const bool tf32_math = c.math_mode == IQL_MATH_TF32_TCGEN05;
+  const bool umma_shape = umma_phase_supported(0, B, H);
+  const bool first_ok = first_fwd_skinny_ok(K0), first_wgrad_ok = first_wgrad_skinny_ok(B, K0);
+  const bool out_ok = out_fwd_skinny_ok(H, A), last_ok = last_bwd_skinny_ok(B, A);
+  const bool side_ok = dbg_getenv("IQL_B200_NO_SIDE_STREAM") == nullptr;
+  // The output-layer backward derives the loss gradients of its rows itself, so loss_kernel (logged losses, log_std
+  // gradient, Adam scalars of the step: all needed by the optimizer launch only) leaves the critical path and runs on
+  // the side stream next to the backward.
+  const bool loss_recomputed = last_ok && bwd.size() >= 2 &&
+                               last_bwd_recomputes_loss_grads(H, A, bwd[0].count * e->lb_splits, B / e->lb_splits) &&
+                               bwd[0].kind == PH_LAST_WGRAD && bwd[1].kind == PH_LAST_DGRAD && bwd[0].count % 4 == 0;
+  std::vector<StepEntry>& plan = e->plan;
+  plan.clear();
+  auto entry = [&](const std::string& label, Work w) { plan.push_back(StepEntry{label, w.flops, w.bytes, {}}); };
+  auto add = [&](StepFn run, int lane = LANE_MAIN) { plan.back().launches.push_back({run, lane}); };
+  // launches of the per-phase kernels on problem table p
+  auto simt = [=](int mode, const GemmProb* p, int n, int maxM, int maxN) -> StepFn {
+    return [=](StepCtx& x, cudaStream_t st) { launch_simt_gemm(mode, p, n, maxM, maxN, x, st); return 1; };
+  };
+  auto out_fwd = [=](const GemmProb* p, int n) -> StepFn { return [=](StepCtx&, cudaStream_t st) { launch_out_fwd(p, n, B, H, A, st); return 1; }; };
+  auto lb_reduce = [=](const GemmProb* split, const GemmProb* prev_split, const GemmProb* pw, const GemmProb* prev, int n, int sp) -> StepFn {
+    return [=](StepCtx&, cudaStream_t st) { launch_lb_reduce(split, prev_split, pw, prev, n, sp, st); return 1; };
+  };
+  entry("gather", Work{0, 2.0 * S_d * B * e->layout.row.row_floats * 4});
+  add([e](StepCtx& x, cudaStream_t st) { launch_gather(x, e->d_ws_f, e->wl.member_floats, e->wl.xrow, st); return 1; });
+  plan.back().gather = true;
+  // One phase of the per-phase path.  A launch that also covers the next phase (fused output Linear, fused output-layer
+  // wgrad + dgrad) skips it; a tcgen05 weight gradient adds colsum_kernel for its bias gradient unless the dgrad or the
+  // output-layer backward before it wrote that already.
   bool skip_next = false, skip_colsum = false;
-  // the reduction of the row-split output-layer backward (single learners) only feeds the optimizer: it leaves the
-  // critical path last_bwd -> dgrad -> ... through the side stream (8 us of a 57 us single-learner step)
-  const bool lb_side = tf32_math && !tm && !no_side && e->side != nullptr;
-  bool lb_on_side = false;
-  auto run_phase = [&](const Phase& ph, const Phase* next, const Phase* next2) {
+  auto phase = [&](const Phase& ph, const Phase* next, const Phase* next2, int lane) {
     if (skip_next) { skip_next = false; return; }
     const GemmProb* pp = e->d_probs + ph.first;
+    const int n = ph.count;
     // Mixed precision: the input layer (observations, K = 11..69) and the output heads run in FP32 on CUDA
     // cores; every hidden-layer GEMM and the first-layer weight gradient run as TF32 tcgen05 GEMMs.  TF32 on the
     // input layer doubles the value-loss error (measured 1.2e-3 -> 2.6e-3) for < 10 % of the step time.
     const bool split = ph.kind == PH_FIRST_FWD && e->split_first;  // 3xTF32: FP32-accurate on tensor cores
-    const bool umma = tf32_math && ph.umma_ok && umma_phase_supported(ph.mode, B, H) &&
-                      !(ph.kind == PH_FIRST_FWD && !split && first_ok);
-    // forward, last hidden layer on the tensor cores: the FP32 output Linear is fused into the epilogue, the next phase skipped
+    const bool umma = tf32_math && ph.umma_ok && umma_shape && !(ph.kind == PH_FIRST_FWD && !split && first_ok);
+    // forward, last hidden layer on the tensor cores: the FP32 output Linear is fused into the epilogue
     const bool fuse_out = umma && ph.mode == 0 && ph.epi == EPI_RELU && next && next->kind == PH_OUT_FWD && H == 256 &&
                           umma_can_fuse_out(A);
-    if (tm) {  // algorithmic work: 2MNK flops; each operand read once, the output written once
-      double fl = 0, by = 0;
-      auto add = [&](const Phase& q) {
-        for (int i = 0; i < q.count; ++i) {
-          const GemmProb& g = e->h_probs[q.first + i];
-          fl += 2.0 * g.M * g.N * g.K;
-          by += 4.0 * ((double)g.M * g.K + (double)g.N * g.K + (g.no_store ? 0.0 : (double)g.M * g.N) + (g.mask ? (double)g.M * g.N : 0.0));
-        }
-      };
-      add(ph);
-      if (fuse_out || (next && ph.kind == PH_LAST_WGRAD && next->kind == PH_LAST_DGRAD)) add(*next);
-      static const char* kinds[] = {"gemm", "first_fwd", "out_fwd", "last_bwd", "last_dgrad", "first_wgrad"};
-      static const char* modes[] = {"fwd", "dgrad", "wgrad"};
-      char nm[32];
-      snprintf(nm, sizeof(nm), "%s_%s", ph.kind == PH_GENERIC ? "hidden" : kinds[ph.kind], modes[ph.mode]);
-      tm->mark(nm, fl, by);
-    }
+    Work w = gemm_work(e, ph.first, n);
+    if (fuse_out || (next && ph.kind == PH_LAST_WGRAD && next->kind == PH_LAST_DGRAD)) w += gemm_work(e, next->first, next->count);
+    static const char* kinds[] = {"gemm", "first_fwd", "out_fwd", "last_bwd", "last_dgrad", "first_wgrad"};
+    static const char* modes[] = {"fwd", "dgrad", "wgrad"};
+    entry(std::string(ph.kind == PH_GENERIC ? "hidden" : kinds[ph.kind]) + "_" + modes[ph.mode], w);
     if (umma && ph.kind == PH_OUT_FWD) {
       // the heads stay in FP32: TF32 rounding of Q and V would be amplified by adv = q - v and exp(beta * adv)
-      if (out_ok) launch_out_fwd(pp, ph.count, B, H, A, st);
-      else launch_simt_gemm(ph.mode, pp, ph.count, ph.maxM, ph.maxN, ctx, st);
+      add(out_ok ? out_fwd(pp, n) : simt(ph.mode, pp, n, ph.maxM, ph.maxN), lane);
     } else if (umma && ph.kind != PH_LAST_WGRAD) {
-      const int n_scalar = (N_PASS - 1) * (int)e->active.size();  // problems with a scalar head (V, Q passes)
-      launch_umma_gemm(ph.mode, pp, split ? e->d_maps_first : e->d_maps + (size_t)256 * ph.first,
-                       fuse_out ? e->d_probs + next->first : nullptr, ph.epi, ph.count, ph.maxM, ph.maxN, ctx, st, split,
-                       n_scalar, ph.cta2, ph.maxK, ph.rowepi ? e->d_maps_c + (size_t)128 * ph.first : nullptr, ph.tile_n);
+      const void* maps = split ? (const void*)e->d_maps_first : (const void*)(e->d_maps + (size_t)256 * ph.first);
+      const GemmProb* p_out = fuse_out ? e->d_probs + next->first : nullptr;
+      const void* cmaps = ph.rowepi ? e->d_maps_c + (size_t)128 * ph.first : nullptr;
+      add([=](StepCtx& x, cudaStream_t st) {
+        launch_umma_gemm(ph.mode, pp, maps, p_out, ph.epi, n, ph.maxM, ph.maxN, x, st, split, n_scalar, ph.cta2, ph.maxK, cmaps, ph.tile_n);
+        return 1;
+      }, lane);
       if (fuse_out) {  // the policy head (N = act_dim) stays with the FP32 output-layer kernel
-        const GemmProb* pa = e->d_probs + next->first + n_scalar;
-        if (out_ok) launch_out_fwd(pa, ph.count - n_scalar, B, H, A, st);
-        else launch_simt_gemm(0, pa, ph.count - n_scalar, B, A, ctx, st);
-        ++launches;
+        add(out_ok ? out_fwd(p_out + n_scalar, n - n_scalar) : simt(0, p_out + n_scalar, n - n_scalar, B, A), lane);
         skip_next = true;
       }
       if (ph.mode == 1 && umma_dgrad_writes_dbias(B)) skip_colsum = true;  // the dgrad epilogue wrote db of the layer below
       if (ph.mode == 2) {
         if (skip_colsum) skip_colsum = false;  // db already written by the fused output-layer backward
-        else { launch_colsum(pp, ph.count, ph.maxM, st); ++launches; }
+        else add([=, maxM = ph.maxM](StepCtx&, cudaStream_t st) { launch_colsum(pp, n, maxM, st); return 1; }, lane);
       }
     } else if (ph.kind == PH_FIRST_FWD && first_ok) {
-      launch_first_fwd(pp, ph.count, B, H, K0, ctx, st);
+      add([=](StepCtx& x, cudaStream_t st) { launch_first_fwd(pp, n, B, H, K0, x, st); return 1; }, lane);
     } else if (ph.kind == PH_OUT_FWD && out_ok) {
-      launch_out_fwd(pp, ph.count, B, H, A, st);
+      add(out_fwd(pp, n), lane);
     } else if (ph.kind == PH_LAST_WGRAD && last_ok && next && next->kind == PH_LAST_DGRAD) {
       // fused wgrad + dgrad of the output layer; it also emits db_{L-1} when layer L-1 is a hidden-layer
       // tcgen05 wgrad phase (whose kernel does not produce bias gradients)
-      const bool emit_db = next2 && tf32_math && next2->umma_ok && umma_phase_supported(2, B, H);
-      if (e->lb_splits > 1 && e->bwd_phases.size() >= 3 && ph.first == e->bwd_phases[0].first) {
-        const int sp = e->lb_splits, n = ph.count * sp;
-        const GemmProb* t0 = e->d_probs + e->lb_first;
-        launches += launch_last_bwd(t0, t0 + n, emit_db ? t0 + 2 * n : nullptr, n, B / sp, H, A, ctx, st,
-                                    loss_recomputed ? e->d_ws_f : nullptr, e->wl.member_floats, &e->wl, e->params);
-        if (lb_side) {
-          cudaEventRecord(e->ev_fork, st_main);
-          cudaStreamWaitEvent(e->side, e->ev_fork, 0);
-          launch_lb_reduce(t0 + n, emit_db ? t0 + 2 * n : nullptr, pp, emit_db ? e->d_probs + next2->first : nullptr, ph.count, sp, e->side);
-          cudaEventRecord(e->ev_side, e->side);
-          lb_on_side = true;
-        } else {
-          launch_lb_reduce(t0 + n, emit_db ? t0 + 2 * n : nullptr, pp, emit_db ? e->d_probs + next2->first : nullptr, ph.count, sp, st);
-        }
-      } else
-      launches += -1 + launch_last_bwd(e->d_probs + next->first, pp, emit_db ? e->d_probs + next2->first : nullptr, ph.count, B, H, A, ctx, st,
-                      loss_recomputed ? e->d_ws_f : nullptr, e->wl.member_floats, &e->wl, e->params);
+      const bool emit_db = next2 && tf32_math && next2->umma_ok && umma_shape;
+      const GemmProb* prev = emit_db ? e->d_probs + next2->first : nullptr;
+      const bool row_split = e->lb_splits > 1 && bwd.size() >= 3 && ph.first == bwd[0].first;
+      const int sp = row_split ? e->lb_splits : 1, ns = n * sp;
+      const GemmProb* t0 = e->d_probs + e->lb_first;  // row-split problems: [dgrad | wgrad | prev wgrad][split] (build_problems)
+      const GemmProb* dg = row_split ? t0 : e->d_probs + next->first;
+      const GemmProb* wg = row_split ? t0 + ns : pp;
+      const GemmProb* pv = row_split ? (emit_db ? t0 + 2 * ns : nullptr) : prev;
+      const float* ws = loss_recomputed ? e->d_ws_f : nullptr;
+      add([=](StepCtx& x, cudaStream_t st) {
+        return launch_last_bwd(dg, wg, pv, ns, B / sp, H, A, x, st, ws, e->wl.member_floats, &e->wl, e->params);
+      }, lane);
+      // the reduction of the row-split output-layer backward (single learners) only feeds the optimizer: it leaves the
+      // critical path last_bwd -> dgrad -> ... through the side stream (8 us of a 57 us single-learner step)
+      if (row_split) add(lb_reduce(wg, pv, pp, prev, n, sp), tf32_math && side_ok ? LANE_SIDE : lane);
       skip_next = true;
       skip_colsum = emit_db;
     } else if (ph.kind == PH_FIRST_WGRAD && first_wgrad_ok) {
-      launch_first_wgrad(pp, ph.count, B, H, K0, st);
+      add([=](StepCtx&, cudaStream_t st) { launch_first_wgrad(pp, n, B, H, K0, st); return 1; }, lane);
     } else {
-      launch_simt_gemm(ph.mode, pp, ph.count, ph.maxM, ph.maxN, ctx, st);
+      add(simt(ph.mode, pp, n, ph.maxM, ph.maxN), lane);
     }
-    ++launches;
   };
-  if (tf32_math && e->fused_fwd) {
-    // one launch for layers 0..L-1 + scalar heads; the policy head (N = act_dim) stays with the FP32 output kernel
-    const int L = c.n_hidden;
-    const int n_scalar = (N_PASS - 1) * (int)e->active.size();
-    const Phase& pout = e->fwd_phases[L];
+  if (e->fused_fwd) {
+    // one launch for layers 0..L-1 + scalar heads; the policy head (N = act_dim) too when it fits the fused epilogue,
+    // else a launch of its own
+    const Phase& pout = fwd[L];
+    const bool pol_fused = fused_fwd_policy_head(A);
     FusedFwdArgs fa;
     memset(&fa, 0, sizeof(fa));
     for (int l = 0; l < L; ++l) {
-      fa.probs[l] = e->d_probs + e->fwd_phases[l].first;
-      fa.maps[l] = (l == 0) ? (const void*)e->d_maps_first : (const void*)(e->d_maps + (size_t)256 * e->fwd_phases[l].first);
-      fa.store_maps[l] = e->d_maps_store + (size_t)128 * l * e->fwd_phases[0].count;
+      fa.probs[l] = e->d_probs + fwd[l].first;
+      fa.maps[l] = (l == 0) ? (const void*)e->d_maps_first : (const void*)(e->d_maps + (size_t)256 * fwd[l].first);
+      fa.store_maps[l] = e->d_maps_store + (size_t)128 * l * fwd[0].count;
     }
     fa.probs_out = e->d_probs + pout.first;
     fa.pair = e->fused_pair ? 1 : 0;
-    const bool pol_fused = fused_fwd_policy_head(A);
     fa.fuse_policy = pol_fused ? 1 : 0;
-    fa.L = L; fa.nprob = e->fwd_phases[0].count; fa.batch = B; fa.fuse_count = n_scalar; fa.k0_max = e->fwd_phases[0].maxK;
-    if (tm) {  // operands read once, the activations of the training passes written once
-      double fl = 0, by = 0;
-      for (int l = 0; l <= L; ++l) {
-        const Phase& q = e->fwd_phases[l];
-        for (int i = 0; i < q.count; ++i) {
-          const GemmProb& g = e->h_probs[q.first + i];
-          const bool kept = e->h_probs[e->fwd_phases[L - 1].first + i].no_store == 0;
-          fl += 2.0 * g.M * g.N * g.K * (l == 0 ? 3.0 : 1.0);
-          if (l == L && i >= n_scalar && !pol_fused) { fl -= 2.0 * g.M * g.N * g.K; continue; }  // policy head: its own launch
-          by += 4.0 * ((l == 0 ? (double)g.M * g.K : 0.0) + (double)g.N * g.K + ((l == L || kept) ? (double)g.M * g.N : 0.0));
-        }
-      }
-      tm->mark("fused_fwd", fl, by);
-    }
-    launch_fused_fwd(fa, ctx, st);
-    ++launches;
-    const GemmProb* pa = e->d_probs + pout.first + n_scalar;
+    fa.L = L; fa.nprob = fwd[0].count; fa.batch = B; fa.fuse_count = n_scalar; fa.k0_max = fwd[0].maxK;
+    // operands read once (the input layer in three passes), the activations of the training passes written once
+    Work w;
+    for (int l = 0; l <= L; ++l)
+      for (int i = 0; i < (l == L && !pol_fused ? n_scalar : fwd[l].count); ++i)
+        w += gemm_work(e, fwd[l].first + i, 1, l == L || !e->h_probs[fwd[L - 1].first + i].no_store, false, l == 0, l == 0 ? 3.0 : 1.0);
+    entry("fused_fwd", w);
+    add([=](StepCtx& x, cudaStream_t st) { launch_fused_fwd(fa, x, st); return 1; });
     if (!pol_fused) {
-    if (tm) {
-      double fl = 0, by = 0;
-      for (int i = n_scalar; i < pout.count; ++i) {
-        const GemmProb& g = e->h_probs[pout.first + i];
-        fl += 2.0 * g.M * g.N * g.K;
-        by += 4.0 * ((double)g.M * g.K + (double)g.N * g.K + (double)g.M * g.N);
-      }
-      tm->mark("policy_head", fl, by);
-    }
-    if (e->pol_umma)
-      launch_umma_gemm(0, pa, e->d_maps_pol, nullptr, EPI_LINEAR, pout.count - n_scalar, B, A, ctx, st, 2, 0, false, H);
-    else if (out_ok) launch_out_fwd(pa, pout.count - n_scalar, B, H, A, st);
-    else launch_simt_gemm(0, pa, pout.count - n_scalar, B, A, ctx, st);
-    ++launches;
+      const GemmProb* pa = e->d_probs + pout.first + n_scalar;
+      const int np = pout.count - n_scalar;
+      const void* maps = e->d_maps_pol;
+      entry("policy_head", gemm_work(e, pout.first + n_scalar, np));
+      if (e->pol_umma)
+        add([=](StepCtx& x, cudaStream_t st) { launch_umma_gemm(0, pa, maps, nullptr, EPI_LINEAR, np, B, A, x, st, 2, 0, false, H); return 1; });
+      else
+        add(out_ok ? out_fwd(pa, np) : simt(0, pa, np, B, A));
     }
   } else {
-    for (size_t i = 0; i < e->fwd_phases.size(); ++i)
-      run_phase(e->fwd_phases[i], i + 1 < e->fwd_phases.size() ? &e->fwd_phases[i + 1] : nullptr, nullptr);
+    for (size_t i = 0; i < fwd.size(); ++i) phase(fwd[i], i + 1 < fwd.size() ? &fwd[i + 1] : nullptr, nullptr, LANE_MAIN);
   }
-  // The output-layer backward derives the loss gradients of its rows itself, so loss_kernel (logged losses, log_std
-  // gradient, Adam scalars of the step: all needed by the optimizer launch only) leaves the critical path and
-  // runs on the side stream next to the backward.
-  const bool loss_on_side = loss_recomputed && !tm && !no_side && e->side != nullptr;
-  if (tm) tm->mark("loss", 0, S_d * e->cfg.batch_size * 4.0 * (8 + 3 * e->wl.Ald));
-  if (loss_on_side) {
-    cudaEventRecord(e->ev_fork, st_main);
-    cudaStreamWaitEvent(e->side, e->ev_fork, 0);
-    launch_loss(ctx, e->d_ws_f, e->wl.member_floats, e->wl, e->params, e->grads, e->side);
-    cudaEventRecord(e->ev_side, e->side);
-  } else {
-    launch_loss(ctx, e->d_ws_f, e->wl.member_floats, e->wl, e->params, e->grads, st);
-  }
-  ++launches;
-  // per-kernel timing (tm) keeps everything on one stream
-  const bool two_streams = tf32_math && !tm && !no_side && e->side != nullptr;
-  int forks = 0;
+  entry("loss", Work{0, S_d * B * 4.0 * (8 + 3 * e->wl.Ald)});
+  add([e](StepCtx& x, cudaStream_t st) { launch_loss(x, e->d_ws_f, e->wl.member_floats, e->wl, e->params, e->grads, st); return 1; },
+      loss_recomputed && side_ok ? LANE_SIDE : LANE_MAIN);
   // chained backward: the output-layer backward (phases 0, 1) runs as before, everything after it -- hidden dgrad /
   // wgrad chain, input-layer wgrad (+ Adam + Polyak unless gradient-only) -- is ONE launch on CTA pairs.  Bind time set
   // e->chain only for shapes it serves (tf32, skinny output-layer backward, 2L + 1 phases), so what it reports runs.
-  const bool chain = e->chain;
-  for (size_t i = 0; i < e->bwd_phases.size(); ++i) {
-    if (chain && i >= 2) break;
-    const Phase& ph = e->bwd_phases[i];
-    const Phase* n1 = i + 1 < e->bwd_phases.size() ? &e->bwd_phases[i + 1] : nullptr;
-    const Phase* n2 = i + 2 < e->bwd_phases.size() ? &e->bwd_phases[i + 2] : nullptr;
-    const bool leaf = two_streams && ph.mode == 2 && ph.kind == PH_GENERIC && ph.umma_ok &&
-                      umma_phase_supported(2, B, H) && !skip_next;
-    if (ph.kind == PH_FIRST_WGRAD && e->fw_splits > 1 && tf32_math && ph.umma_ok && umma_phase_supported(2, B, H) && !skip_next) {
+  for (size_t i = 0; i < bwd.size() && !(e->chain && i >= 2); ++i) {
+    const Phase& ph = bwd[i];
+    const Phase* n1 = i + 1 < bwd.size() ? &bwd[i + 1] : nullptr;
+    const Phase* n2 = i + 2 < bwd.size() ? &bwd[i + 2] : nullptr;
+    if (ph.kind == PH_FIRST_WGRAD && e->fw_splits > 1 && tf32_math && ph.umma_ok && umma_shape && !skip_next) {
       // few problems x a long batch: the tcgen05 kernel runs the K-split copies (enough tiles to fill the GPU), then the
       // partial dW_0 / db_0 are added up in split order
-      run_phase(e->fw_phase, nullptr, nullptr);  // batch > 256: the phase also runs colsum_kernel (partial db_0)
-      launch_lb_reduce(e->d_probs + e->fw_phase.first, nullptr, e->d_probs + ph.first, nullptr, ph.count, e->fw_splits, st);
-      ++launches;
+      phase(e->fw_phase, nullptr, nullptr, LANE_MAIN);  // batch > 256: the phase also runs colsum_kernel (partial db_0)
+      add(lb_reduce(e->d_probs + e->fw_phase.first, nullptr, e->d_probs + ph.first, nullptr, ph.count, e->fw_splits));
       continue;
     }
-    if (leaf) {
-      // G_l (written by the previous launch) -> side stream.  The previous leaf must be done first: the dgrad that
-      // follows on the main stream overwrites the ping-pong buffer that leaf was reading.
-      if (forks > 0) cudaStreamWaitEvent(st_main, e->ev_side, 0);
-      cudaEventRecord(e->ev_fork, st_main);
-      cudaStreamWaitEvent(e->side, e->ev_fork, 0);
-      st = e->side;
-      run_phase(ph, n1, n2);
-      st = st_main;
-      cudaEventRecord(e->ev_side, e->side);
-      ++forks;
-    } else {
-      run_phase(ph, n1, n2);
-    }
+    // the hidden-layer weight gradients are leaves of the backward: beside the dgrad chain on the side stream
+    const bool leaf = tf32_math && side_ok && ph.mode == 2 && ph.kind == PH_GENERIC && ph.umma_ok && umma_shape;
+    phase(ph, n1, n2, leaf ? LANE_LEAF : LANE_MAIN);
   }
-  // chained backward (gradients only): the chain reads nothing the side stream writes (loss kernel: logged losses,
-  // log_std gradient, Adam scalars; row-split reduction: dW_L, db_L), so it starts right after the output-layer backward
-  if (chain && e->chain_grads) {
-    if (tm) tm->mark("bwd_chain_grads", 0, 0);
-    launch_chain(e, ctx, st, tm);
-    ++launches;
+  // chained backward: gradient-only, it reads nothing the side stream writes (loss kernel: logged losses, log_std
+  // gradient, Adam scalars; row-split reduction: dW_L, db_L), so it starts right after the output-layer backward, before
+  // the join; with the optimizer in its epilogues it is the step's optimizer launch
+  if (e->chain) {
+    // operands read once; dZ written; the weight gradients written (gradient-only) or the optimizer state streamed
+    Work w;
+    for (size_t i = 2; i < bwd.size(); ++i) w += gemm_work(e, bwd[i].first, bwd[i].count, bwd[i].mode == 1 || e->chain_grads, false);
+    if (!e->chain_grads)  // p, m, v in and out + shadows
+      w.bytes += S_d * 4.0 * ((6.0 + 1.0) * e->layout.param_floats + 3.0 * e->layout.q_floats);
+    entry(e->chain_grads ? "bwd_chain_grads" : "bwd_chain", w);
+    add([e](StepCtx& x, cudaStream_t st) {
+      BwdChainArgs ca = e->chain_args;
+      ca.keep_grads = e->keep_grads;
+      launch_bwd_chain(ca, x, st);
+      return 1;
+    });
   }
-  if (forks > 0 || loss_on_side || lb_on_side) cudaStreamWaitEvent(st_main, e->ev_side, 0);  // join before the optimizer
-  // Adam: read g, p, m, v + target; write p, m, v + target (+ the TF32 shadow copies in tcgen05 mode)
-  if (tm) {
-    // TF32 operand copies the optimizer maintains: everything except the hidden-layer weights when those carry the
-    // rounding bias in place (no shadow), plus the lo parts of the first-layer (and wide policy-head) ranges
+  if (!e->chain || e->chain_grads) {
+    // Adam: read g, p, m, v + target; write p, m, v + target (+ the TF32 shadow copies in tcgen05 mode): everything
+    // except the hidden-layer weights when those carry the rounding bias in place (no shadow), plus the lo parts of the
+    // first-layer (and wide policy-head) ranges
+    const StepCtx ctx = make_ctx(e);
     double shadow_p = 0, shadow_t = 0;
     if (ctx.tf32) {
       double hid_p = 0, hid_q = 0, lo_p = 0, lo_q = 0;
@@ -1356,29 +1328,58 @@ static int enqueue_step(iql_engine* e, StepCtx& ctx, bool gather, cudaStream_t s
       shadow_p = (double)e->layout.param_floats - hid_p + lo_p;
       shadow_t = (double)e->layout.q_floats - hid_q + lo_q;
     }
-    tm->mark("adam_polyak", 0, S_d * 4.0 * (7.0 * e->layout.param_floats + 2.0 * e->layout.q_floats + shadow_p + shadow_t));
+    entry("adam_polyak", Work{0, S_d * 4.0 * (7.0 * e->layout.param_floats + 2.0 * e->layout.q_floats + shadow_p + shadow_t)});
+    add([e](StepCtx& x, cudaStream_t st) {
+      launch_adam(x, e->params, e->exp_avg, e->exp_avg_sq, e->target, e->grads, st);
+      if (x.advance_k > 0) x.advance_k = -1;  // consumed: the optimizer launch advanced the counters
+      return 1;
+    });
   }
+  plan.back().join = true;
   // (chained backward + optimizer: its input-layer weight-gradient phase still reads the gathered rows, so the next
   // step's gather cannot run beside it; the caller then gathers at the top of every step)
-  const bool fork_gather = gather_next && !tm && e->side != nullptr && !(chain && !e->chain_grads);
-  if (fork_gather) {
-    StepCtx next = ctx;
-    next.k = ctx.k + 1;
-    cudaEventRecord(e->ev_fork_g, st_main);
-    cudaStreamWaitEvent(e->side, e->ev_fork_g, 0);
-    launch_gather(next, e->d_ws_f, e->wl.member_floats, e->wl.xrow, e->side);
-    cudaEventRecord(e->ev_gather, e->side);
-    ++launches;
+  e->gather_ahead = e->side != nullptr && side_ok && dbg_getenv("IQL_B200_NO_GATHER_AHEAD") == nullptr && !(e->chain && !e->chain_grads);
+}
+
+// One update step for all members: the plan of plan_step.  Returns the number of launches.
+// gather: sample + gather this step's rows first.  gather_next (only with e->gather_ahead): the NEXT step's gather
+// (ctx.k + 1) runs on the side stream next to this step's optimizer launch -- nothing after the input-layer weight
+// gradient reads the row buffers, the gather is pure latency and the optimizer pure bandwidth -- and the caller passes
+// gather = false for that next step.  Per-kernel timing (tm) keeps every launch on the main stream.
+static int enqueue_step(iql_engine* e, StepCtx& ctx, bool gather, cudaStream_t st_main, StepTimer* tm = nullptr,
+                        bool gather_next = false) {
+  const bool two_streams = !tm && e->side != nullptr;
+  const bool fork_gather = gather_next && !tm;
+  int launches = 0, forks = 0;
+  bool side_used = false;
+  for (const StepEntry& s : e->plan) {
+    if (s.gather && !gather) continue;
+    if (s.join && side_used) cudaStreamWaitEvent(st_main, e->ev_side, 0);  // join before the optimizer
+    if (tm) tm->mark(s);
+    if (s.join && fork_gather) {
+      StepCtx next = ctx;
+      next.k = ctx.k + 1;
+      cudaEventRecord(e->ev_fork_g, st_main);
+      cudaStreamWaitEvent(e->side, e->ev_fork_g, 0);
+      launch_gather(next, e->d_ws_f, e->wl.member_floats, e->wl.xrow, e->side);
+      cudaEventRecord(e->ev_gather, e->side);
+      ++launches;
+    }
+    if (s.join) ctx.unbias_out = (ctx.k == ctx.K - 1) ? 1 : 0;  // the call's last optimizer launch leaves plain fp32 in the arenas
+    bool on_side = false;
+    for (const StepLaunch& l : s.launches) {
+      if (two_streams && l.lane != LANE_MAIN && !on_side) {
+        // a leaf waits for the previous leaf: the dgrad that follows on the main stream overwrites the ping-pong buffer
+        // that leaf was reading
+        if (l.lane == LANE_LEAF && forks++ > 0) cudaStreamWaitEvent(st_main, e->ev_side, 0);
+        cudaEventRecord(e->ev_fork, st_main);
+        cudaStreamWaitEvent(e->side, e->ev_fork, 0);
+        on_side = side_used = true;
+      }
+      launches += l.run(ctx, on_side ? e->side : st_main);
+    }
+    if (on_side) cudaEventRecord(e->ev_side, e->side);
   }
-  ctx.unbias_out = (ctx.k == ctx.K - 1) ? 1 : 0;  // the call's last optimizer launch leaves plain fp32 in the arenas
-  if (chain && !e->chain_grads) {
-    if (tm) tm->label.back() = "bwd_chain";
-    launch_chain(e, ctx, st, tm);
-  } else {
-    launch_adam(ctx, e->params, e->exp_avg, e->exp_avg_sq, e->target, e->grads, st);
-    if (ctx.advance_k > 0) ctx.advance_k = -1;  // consumed: the optimizer launch advanced the counters
-  }
-  ++launches;
   if (fork_gather) cudaStreamWaitEvent(st_main, e->ev_gather, 0);
   if (tm) tm->finish();
   return launches;
@@ -1447,9 +1448,7 @@ extern "C" int iql_train_steps(iql_engine* e, int32_t k_steps, int32_t sample_mo
   ctx.dropout_masks = dropout_masks;
   ctx.idx_out = idx_out;
   const bool gather = sample_mode != IQL_SAMPLE_PRELOADED;
-  static const bool no_overlap_gather = dbg_getenv("IQL_B200_NO_GATHER_AHEAD") != nullptr || dbg_getenv("IQL_B200_NO_SIDE_STREAM") != nullptr;
-  // (not with the chained backward + optimizer: its last phase still reads the gathered rows, see enqueue_step)
-  const bool overlap_gather = !no_overlap_gather && e->side != nullptr && st != nullptr && !(e->chain && !e->chain_grads);
+  const bool overlap_gather = e->gather_ahead && st != nullptr;
   auto k_step_loop = [&]() -> int64_t {
     int64_t n = 0;
     for (int k = 0; k < k_steps; ++k) {
