@@ -40,6 +40,11 @@ extern "C" {
 #define IQL_SAMPLE_PHILOX 0    /* indices drawn in-kernel (Philox4x32-10)     */
 #define IQL_SAMPLE_INDICES 1   /* caller-supplied int64 indices [S][K][B]     */
 #define IQL_SAMPLE_PRELOADED 2 /* batch already staged by iql_load_batch (K=1) */
+#define IQL_SAMPLE_MT19937 3   /* numpy's RandomState.randint stream per member, drawn on the device (iql_bind_index_streams) */
+
+/* One member's numpy index stream: uint32 words [key[624] | pos | pad], the ('MT19937', key, pos, ...) tuple of
+ * RandomState.get_state() copied word for word (pos in [0, 624]; the pad word is not read). */
+#define IQL_MT_STATE_WORDS 626
 
 #define IQL_NET_Q1 0
 #define IQL_NET_Q2 1
@@ -233,6 +238,13 @@ int iql_replay_sample_host(const float* rows, const iql_row_layout* lay, int64_t
                            const int64_t* host_indices, float* states, float* actions, float* rewards,
                            float* next_states, float* dones, void* stream);
 
+/* The sampler of IQL_SAMPLE_MT19937 without a handle (the np.random.randint draw of iql.py:172 for n independent
+ * streams): stream i draws host_count[i] values of RandomState.randint(0, host_high[i]) from states + i *
+ * IQL_MT_STATE_WORDS into out + i * stride (stride >= every count) and advances its state.  host_high / host_count are
+ * host arrays, 1 <= high <= 2^32 (else IQL_ERR_INVALID, nothing drawn). */
+int iql_mt19937_randint(uint32_t* states, int32_t n, const int64_t* host_high, const int64_t* host_count, int64_t* out,
+                        int64_t stride, void* stream);
+
 /* ---- the update ----------------------------------------------------------- */
 /* Attach member's replay rows (several members may share one buffer). */
 int iql_bind_replay(iql_engine* e, int32_t member, const float* rows, int64_t capacity, int64_t size);
@@ -251,6 +263,17 @@ int iql_load_batch(iql_engine* e, int32_t member, const float* states, const flo
 int iql_train_steps(iql_engine* e, int32_t k_steps, int32_t sample_mode, const int64_t* indices,
                     const uint8_t* dropout_masks, float* out_losses, int64_t* idx_out,
                     void* stream);
+/* The numpy index streams of IQL_SAMPLE_MT19937 (replaces: the host draw np.random.randint(0, high, size=B) of
+ * ReplayBuffer.sample, iql.py:172, made with each member's own RandomState as ensemble_train_loop does).  Both buffers
+ * are caller-allocated device memory, borrowed for the handle's lifetime: states [S][IQL_MT_STATE_WORDS] uint32 (8-byte
+ * aligned), indices [S][max_steps_per_call][batch_size] int64 (16-byte aligned; a K-step call uses its first S * K * B
+ * entries as [S][K][B]).  Member m's draws in a call are exactly RandomState.randint(0, high_m, size=K * B_m) (int64):
+ * step k gets draws [k B_m, (k + 1) B_m) in rows b < B_m; pad rows draw nothing.  high_m is the member's replay size
+ * (iql_set_replay_size) at the call, read by the sampler at run time, so a size change needs no new graph.  A stream
+ * continues across calls, graph replays and host steps; write a state to restart it.  Members that do not train draw
+ * nothing and their state words keep every bit.  Refusals, with nothing drawn: IQL_ERR_STATE when no streams are bound;
+ * IQL_ERR_INVALID for an active member whose size is 0 or above 2^32 (numpy's 64-bit path).  NULL, NULL unbinds. */
+int iql_bind_index_streams(iql_engine* e, uint32_t* states, int64_t* indices);
 /* replaces: ONE iteration of the reference's training loop as a host caller sees it --
  * `batch = replay_buffer.sample(B); log_dict = trainer.train(batch)` (offline/iql.py:631-635, finetune/iql.py:542-563),
  * whose log_dict holds the three losses as host floats every step.
@@ -262,6 +285,11 @@ int iql_train_steps(iql_engine* e, int32_t k_steps, int32_t sample_mode, const i
  * they have landed, while the step's backward / optimizer launches are still in flight. */
 int iql_train_host_step(iql_engine* e, const int64_t* host_indices, float* host_losses, void* stream,
                         void* caller_stream);
+/* iql_train_host_step with the indices drawn on the device from the streams of iql_bind_index_streams (one step,
+ * B_m draws per active member at its replay size).  Same graph launch, pinned loss mailbox and host_losses == NULL /
+ * iql_host_step_wait contract; the members' bounds travel in the pinned block where the host indices would go, so the
+ * step uploads nothing from pageable memory. */
+int iql_train_host_step_mt19937(iql_engine* e, float* host_losses, void* stream, void* caller_stream);
 /* host_losses == NULL above returns right after the launch; this collects the losses of that step (spins on the
  * flag words, bounded; `stream` as above).  Lets the caller do its per-step host bookkeeping while the GPU works. */
 int iql_host_step_wait(iql_engine* e, float* host_losses, void* stream);

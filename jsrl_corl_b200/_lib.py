@@ -17,7 +17,8 @@ if os.environ.get("IQL_B200_DEBUG") and os.environ.get("IQL_B200_LIB"):  # A/B b
 
 IQL_OK, IQL_ERR_INVALID, IQL_ERR_CUDA, IQL_ERR_STATE, IQL_ERR_SHAPE = 0, 1, 2, 3, 4
 MATH_FP32_SIMT, MATH_TF32_TCGEN05 = 0, 1
-SAMPLE_PHILOX, SAMPLE_INDICES, SAMPLE_PRELOADED = 0, 1, 2
+SAMPLE_PHILOX, SAMPLE_INDICES, SAMPLE_PRELOADED, SAMPLE_MT19937 = 0, 1, 2, 3
+MT_STATE_WORDS = 626  # IQL_MT_STATE_WORDS: key[624] | pos | pad
 NET_Q1, NET_Q2, NET_V, NET_ACTOR = 0, 1, 2, 3
 KIND_WEIGHT, KIND_BIAS, KIND_LOG_STD = 0, 1, 2
 OPT_STEP_PATH, OPT_KEEP_GRADS = 1, 2
@@ -116,6 +117,9 @@ SYMBOLS = {
     "iql_load_batch": (C.c_int, [_P, C.c_int32, _P, _P, _P, _P, _P, _P]),
     "iql_train_steps": (C.c_int, [_P, C.c_int32, C.c_int32, _P, _P, _P, _P, _P]),
     "iql_train_host_step": (C.c_int, [_P, _P, _P, _P, _P]),
+    "iql_train_host_step_mt19937": (C.c_int, [_P, _P, _P, _P]),
+    "iql_bind_index_streams": (C.c_int, [_P, _P, _P]),
+    "iql_mt19937_randint": (C.c_int, [_P, C.c_int32, _P, _P, _P, C.c_int64, _P]),
     "iql_host_step_wait": (C.c_int, [_P, _P, _P]),
     "iql_act": (C.c_int, [_P, C.c_int32, _P, C.c_int64, C.c_float, _P, _P]),
     "iql_act_host": (C.c_int, [_P, C.c_int32, _P, C.c_float, _P, _P, _P]),

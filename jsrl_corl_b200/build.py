@@ -12,7 +12,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libiql_b200.so")
-SOURCES = ["engine.cu", "kernels_simt.cu", "kernels_skinny.cu", "replay.cu", "umma_gemm.cu", "fused_fwd.cu", "bwd_chain.cu"]
+SOURCES = ["engine.cu", "kernels_simt.cu", "kernels_skinny.cu", "replay.cu", "umma_gemm.cu", "fused_fwd.cu", "bwd_chain.cu", "mt19937.cu"]
 HEADERS = ["engine.h", "common.cuh", "umma_gemm.h", "tcgen05.cuh", "adam.cuh", os.path.join("..", "..", "include", "iql_b200.h")]
 NVCC_FLAGS = [
     "-O3", "-std=c++17", "-lineinfo",

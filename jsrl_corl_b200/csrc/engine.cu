@@ -196,6 +196,12 @@ struct iql_engine {
   std::vector<GemmProb> h_probs;
   std::vector<Phase> fwd_phases, bwd_phases;
   bool bound = false, tables_dirty = true, scalars_dirty = true, counters_dirty = true, replay_dirty = true;
+  // only replay sizes changed since the last upload (iql_set_replay_size): the host steps read no size on the device, so
+  // they leave the upload to the next call that does
+  bool sizes_dirty = false;
+  // numpy index streams (iql_bind_index_streams): [S][IQL_MT_STATE_WORDS] generator states, [S][Kmax][B] drawn indices
+  uint32_t* mt_states = nullptr;
+  int64_t* mt_indices = nullptr;
   std::vector<char> preloaded;
   // members that train (iql_set_active_members), ascending.  The problem tables, tensor maps and chain tasks hold these
   // members only, and every bind-time choice that depends on the member count is made from active.size().
@@ -977,7 +983,8 @@ extern "C" int iql_bind_state(iql_engine* e, float* params, float* exp_avg, floa
   return IQL_OK;
 }
 
-static int flush_tables(iql_engine* e, cudaStream_t st) {
+// sizes: the call reads the replay sizes on the device (K-step calls: the Philox and MT19937 samplers)
+static int flush_tables(iql_engine* e, cudaStream_t st, bool sizes = true) {
   const int S = e->cfg.n_members, L = e->cfg.n_hidden;
   if (e->tables_dirty) {
     CUDA_TRY(e, cudaMemcpyAsync(e->d_probs, e->h_probs.data(), sizeof(GemmProb) * e->h_probs.size(), cudaMemcpyHostToDevice, st));
@@ -1014,9 +1021,9 @@ static int flush_tables(iql_engine* e, cudaStream_t st) {
     CUDA_TRY(e, cudaMemcpyAsync(e->d_counters, e->h_counters.data(), sizeof(iql_counters) * S, cudaMemcpyHostToDevice, st));
     e->counters_dirty = false;
   }
-  if (e->replay_dirty) {
+  if (e->replay_dirty || (sizes && e->sizes_dirty)) {
     CUDA_TRY(e, cudaMemcpyAsync(e->d_replay, e->h_replay.data(), sizeof(ReplayBinding) * S, cudaMemcpyHostToDevice, st));
-    e->replay_dirty = false;
+    e->replay_dirty = e->sizes_dirty = false;
   }
   return IQL_OK;
 }
@@ -1087,7 +1094,30 @@ extern "C" int iql_set_replay_size(iql_engine* e, int32_t member, int64_t size) 
   if (!e || member < 0 || member >= e->cfg.n_members) return fail(e, IQL_ERR_INVALID, "iql_set_replay_size: bad member");
   if (size < 0 || size > e->h_replay[member].capacity) return fail(e, IQL_ERR_INVALID, "iql_set_replay_size: size out of range");
   e->h_replay[member].size = size;
-  e->replay_dirty = true;
+  e->sizes_dirty = true;
+  return IQL_OK;
+}
+
+extern "C" int iql_bind_index_streams(iql_engine* e, uint32_t* states, int64_t* indices) {
+  if (!e) return IQL_ERR_INVALID;
+  if (!states != !indices) return fail(e, IQL_ERR_INVALID, "iql_bind_index_streams: bind both buffers or neither");
+  if (((uintptr_t)states & 7) || ((uintptr_t)indices & 15))
+    return fail(e, IQL_ERR_INVALID, "iql_bind_index_streams: states must be 8-byte and indices 16-byte aligned");
+  e->mt_states = states;
+  e->mt_indices = indices;
+  drop_graphs(e);  // the buffers are baked into captured launches
+  return IQL_OK;
+}
+
+// IQL_SAMPLE_MT19937 refusals: no streams bound, or an active member whose bound is outside numpy's 32-bit path
+static int check_index_streams(iql_engine* e, const char* who) {
+  if (!e->mt_states) return fail(e, IQL_ERR_STATE, std::string(who) + ": no index streams bound (iql_bind_index_streams)");
+  for (const int m : e->active) {
+    const int64_t high = e->h_replay[m].size;
+    if (high < 1 || high > ((int64_t)1 << 32))
+      return fail(e, IQL_ERR_INVALID, std::string(who) + ": member " + std::to_string(m) + " has replay size " + std::to_string(high) +
+                                          "; the numpy stream needs 1 <= size <= 2^32");
+  }
   return IQL_OK;
 }
 
@@ -1429,7 +1459,7 @@ extern "C" int iql_train_steps(iql_engine* e, int32_t k_steps, int32_t sample_mo
     if (k_steps != 1) return fail(e, IQL_ERR_INVALID, "iql_train_steps: IQL_SAMPLE_PRELOADED runs exactly one step");
     for (const int m : e->active)
       if (!e->preloaded[m]) return fail(e, IQL_ERR_STATE, "iql_train_steps: no batch staged (call iql_load_batch)");
-  } else if (sample_mode != IQL_SAMPLE_PHILOX) {
+  } else if (sample_mode != IQL_SAMPLE_PHILOX && sample_mode != IQL_SAMPLE_MT19937) {
     return fail(e, IQL_ERR_INVALID, "iql_train_steps: unknown sample_mode");
   }
   if (sample_mode != IQL_SAMPLE_PRELOADED)
@@ -1438,19 +1468,28 @@ extern "C" int iql_train_steps(iql_engine* e, int32_t k_steps, int32_t sample_mo
       if (e->h_replay[m].size <= 0 && sample_mode == IQL_SAMPLE_PHILOX)
         return fail(e, IQL_ERR_INVALID, "iql_train_steps: cannot sample from an empty replay buffer");
     }
+  const bool mt = sample_mode == IQL_SAMPLE_MT19937;
+  if (mt) {
+    const int rc = check_index_streams(e, "iql_train_steps");
+    if (rc != IQL_OK) return rc;
+  }
   int rc = flush_tables(e, st);
   if (rc != IQL_OK) return rc;
 
   StepCtx ctx = make_ctx(e);
   ctx.K = k_steps;
   if (ctx.tf32) launch_refresh_shadow(ctx, e->params, e->target, st);
-  ctx.indices = (sample_mode == IQL_SAMPLE_INDICES) ? indices : nullptr;
+  ctx.indices = (sample_mode == IQL_SAMPLE_INDICES) ? indices : (mt ? e->mt_indices : nullptr);
   ctx.dropout_masks = dropout_masks;
   ctx.idx_out = idx_out;
   const bool gather = sample_mode != IQL_SAMPLE_PRELOADED;
   const bool overlap_gather = e->gather_ahead && st != nullptr;
   auto k_step_loop = [&]() -> int64_t {
     int64_t n = 0;
+    if (mt) {  // all K steps' indices in one launch; the gathers read them as caller indices
+      launch_mt19937_members(ctx, e->mt_states, e->mt_indices, nullptr, st);
+      ++n;
+    }
     for (int k = 0; k < k_steps; ++k) {
       ctx.k = k;
       if (k == k_steps - 1) ctx.advance_k = k_steps;
@@ -1557,17 +1596,23 @@ static int collect_host_step(iql_engine* e) {
   return iql_host_step_wait(e, sink.data(), e->host_step_stream);
 }
 
-extern "C" int iql_train_host_step(iql_engine* e, const int64_t* host_indices, float* host_losses, void* stream,
-                                   void* caller_stream) {
+// mt: the indices are drawn on the device from the bound index streams (iql_train_host_step_mt19937); host_indices is
+// then null and the members' bounds go to the pinned block instead
+static int host_step_impl(iql_engine* e, const int64_t* host_indices, bool mt, float* host_losses, void* stream,
+                          void* caller_stream, const char* who) {
   if (!e) return IQL_ERR_INVALID;
-  if (!e->bound) return fail(e, IQL_ERR_STATE, "iql_train_host_step: state not bound");
+  if (!e->bound) return fail(e, IQL_ERR_STATE, std::string(who) + ": state not bound");
   cudaStream_t st = (cudaStream_t)stream, cur = (cudaStream_t)caller_stream;
-  if (!st) return fail(e, IQL_ERR_INVALID, "iql_train_host_step: needs a non-default stream (graph capture)");
+  if (!st) return fail(e, IQL_ERR_INVALID, std::string(who) + ": needs a non-default stream (graph capture)");
   const int S = e->cfg.n_members, B = e->cfg.batch_size;
-  const bool gather = host_indices != nullptr;
+  const bool gather = host_indices != nullptr || mt;
   for (const int m : e->active) {
-    if (gather && !e->h_replay[m].rows) return fail(e, IQL_ERR_STATE, "iql_train_host_step: replay buffer not bound");
-    if (!gather && !e->preloaded[m]) return fail(e, IQL_ERR_STATE, "iql_train_host_step: no batch staged (call iql_load_batch)");
+    if (gather && !e->h_replay[m].rows) return fail(e, IQL_ERR_STATE, std::string(who) + ": replay buffer not bound");
+    if (!gather && !e->preloaded[m]) return fail(e, IQL_ERR_STATE, std::string(who) + ": no batch staged (call iql_load_batch)");
+  }
+  if (mt) {
+    const int rc = check_index_streams(e, who);
+    if (rc != IQL_OK) return rc;
   }
   const size_t idx_bytes = sizeof(int64_t) * (size_t)S * B;
   int rc = pinned_block(e, (void**)&e->h_mail, idx_bytes + sizeof(float) * 4 * S, "iql_train_host_step");
@@ -1576,7 +1621,9 @@ extern "C" int iql_train_host_step(iql_engine* e, const int64_t* host_indices, f
   float* mail = (float*)(e->h_mail + idx_bytes);
   rc = collect_host_step(e);  // one step in flight at a time: its gather may not have read the index block yet
   if (rc != IQL_OK) return rc;
-  if (gather)
+  if (mt)
+    for (const int m : e->active) mail_idx[m] = e->h_replay[m].size;  // the sampler's bounds: [m] of the index block
+  else if (gather)
     for (const int m : e->active) {  // rows of members that do not train are never read
       const int64_t cap = e->h_replay[m].capacity;
       for (int b = 0; b < e->h_scalars[m].batch; ++b) {  // entries past B_m are never read
@@ -1597,15 +1644,20 @@ extern "C" int iql_train_host_step(iql_engine* e, const int64_t* host_indices, f
   if (rc != IQL_OK) return rc;
   e->host_step_stream = run;
   e->host_step_stream_set = true;
-  rc = flush_tables(e, run);
+  rc = flush_tables(e, run, false);
   if (rc != IQL_OK) return rc;
   auto one_step = [&]() -> int64_t {
     StepCtx ctx = make_ctx(e);
     ctx.K = 1;
     ctx.k = 0;
-    ctx.indices = gather ? mail_idx : nullptr;  // unified addressing: the pinned block is device-visible at its host address
+    // unified addressing: the pinned block is device-visible at its host address
+    ctx.indices = mt ? e->mt_indices : (gather ? mail_idx : nullptr);
     ctx.host_mail = mail;
     int64_t n = 0;
+    if (mt) {
+      launch_mt19937_members(ctx, e->mt_states, e->mt_indices, mail_idx, st);
+      ++n;
+    }
     // the TF32 operand refresh and the gather are independent: one launch, which releases the forward at once
     const bool fork_refresh = ctx.tf32 && gather;
     if (fork_refresh) {
@@ -1620,13 +1672,22 @@ extern "C" int iql_train_host_step(iql_engine* e, const int64_t* host_indices, f
     if (ctx.advance_k != -1) { launch_advance(ctx, 1, st); ++n; }
     return n;
   };
-  rc = launch_graph(e, GraphKey(gather ? 101 : 102, 1, 0), st, run, "iql_train_host_step", one_step, &e->last_launches);
+  rc = launch_graph(e, GraphKey(mt ? 103 : (gather ? 101 : 102), 1, 0), st, run, who, one_step, &e->last_launches);
   if (rc != IQL_OK) return rc;
   advance_counters(e, 1);
   for (const int m : e->active) e->preloaded[m] = 0;
   e->mail_pending = true;
   if (!host_losses) return IQL_OK;  // the caller collects the losses with iql_host_step_wait
   return iql_host_step_wait(e, host_losses, run);
+}
+
+extern "C" int iql_train_host_step(iql_engine* e, const int64_t* host_indices, float* host_losses, void* stream,
+                                   void* caller_stream) {
+  return host_step_impl(e, host_indices, false, host_losses, stream, caller_stream, "iql_train_host_step");
+}
+
+extern "C" int iql_train_host_step_mt19937(iql_engine* e, float* host_losses, void* stream, void* caller_stream) {
+  return host_step_impl(e, nullptr, true, host_losses, stream, caller_stream, "iql_train_host_step_mt19937");
 }
 
 extern "C" int iql_host_step_wait(iql_engine* e, float* host_losses, void* stream) {
@@ -1766,7 +1827,7 @@ static int act_host_impl(iql_engine* e, int32_t member, const float* host_state,
   (void)st;
   rc = order_behind_host_step(e, cur);
   if (rc != IQL_OK) return rc;
-  rc = flush_tables(e, cur);
+  rc = flush_tables(e, cur, false);
   if (rc != IQL_OK) return rc;
   StepCtx ctx = make_ctx(e);
   const float* block = e->params + (int64_t)member * e->layout.param_floats;
@@ -1841,7 +1902,7 @@ extern "C" int iql_act_host_members(iql_engine* e, const float* host_states, con
   (void)stream;
   rc = order_behind_host_step(e, cur);
   if (rc != IQL_OK) return rc;
-  rc = flush_tables(e, cur);
+  rc = flush_tables(e, cur, false);
   if (rc != IQL_OK) return rc;
   StepCtx ctx = make_ctx(e);
   launch_act_members(ctx, e->params, e->guide, e->d_act_off, e->d_act_off + (L + 1), states, ids, codes, steps, drop_codes, n,
@@ -1939,7 +2000,7 @@ extern "C" int iql_replay_insert_members_host(iql_engine* e, const float* host_s
   (void)stream;
   rc = order_behind_host_step(e, cur);
   if (rc != IQL_OK) return rc;
-  rc = flush_tables(e, cur);
+  rc = flush_tables(e, cur, false);
   if (rc != IQL_OK) return rc;
   launch_insert_members(e->d_replay, RF, rows, ids, ptrs, n, (uint32_t*)consumed, cur);
   CUDA_TRY(e, cudaGetLastError());

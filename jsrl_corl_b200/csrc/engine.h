@@ -174,6 +174,9 @@ void launch_gather_refresh(const StepCtx& ctx, float* ws, int64_t ws_member_floa
                            cudaStream_t st);
 void launch_load_batch(const StepCtx& ctx, int member, float* xrow, const float* s, const float* a, const float* r,
                        const float* s2, const float* d, cudaStream_t st);
+// numpy index streams (mt19937.cu): CTA i draws the K x B_m indices of active member i at its bound high (replay table, or
+// host_high[m] when not null) into indices [S][K][B]
+void launch_mt19937_members(const StepCtx& ctx, uint32_t* states, int64_t* indices, const int64_t* host_high, cudaStream_t st);
 // skinny-layer kernels (kernels_skinny.cu)
 void launch_first_fwd(const GemmProb* probs, int nprob, int B, int H, int kmax, const StepCtx& ctx, cudaStream_t st);
 void launch_out_fwd(const GemmProb* probs, int nprob, int B, int H, int amax, cudaStream_t st);

@@ -51,6 +51,29 @@ def query_layout(n_members, state_dim, action_dim, hidden_dim, n_hidden, batch_s
     return lay, tensors
 
 
+def index_state_rows(rngs) -> np.ndarray:
+    """[len(rngs), IQL_MT_STATE_WORDS] uint32: each ``np.random.RandomState``'s generator in the device layout of
+    ``iql_bind_index_streams`` -- the key and pos of ``get_state()``, then a pad word."""
+    rows = np.zeros((len(rngs), _lib.MT_STATE_WORDS), dtype=np.uint32)
+    for i, rng in enumerate(rngs):
+        if not isinstance(rng, np.random.RandomState):
+            raise ValueError(f"index streams are np.random.RandomState objects, got {type(rng).__name__}")
+        name, key, pos, _, _ = rng.get_state()
+        if name != "MT19937":
+            raise ValueError(f"index stream {i} is a {name} generator, not MT19937")
+        rows[i, :624] = key
+        rows[i, 624] = pos
+    return rows
+
+
+def load_index_state_rows(rngs, rows: np.ndarray) -> None:
+    """Inverse of ``index_state_rows``: key and pos go back into each RandomState (``set_state``); its cached Gaussian
+    (``has_gauss`` / ``cached_gaussian``), which the index draws never touch, is kept."""
+    for rng, row in zip(rngs, rows):
+        _, _, _, has_gauss, cached = rng.get_state()
+        rng.set_state(("MT19937", np.array(row[:624], dtype=np.uint32), int(row[624]), has_gauss, cached))
+
+
 class EnsembleEngine:
     """S-member IQL update engine bound to one CUDA device."""
 
@@ -110,6 +133,7 @@ class EnsembleEngine:
         self._idx_stage: Dict[int, torch.Tensor] = {}
         self._host_losses = None
         self._dev_index = self.device.index
+        self._mt_states = self._mt_indices = None  # numpy index streams, allocated by the first set_index_states
 
     # ------------------------------------------------------------------
     def __del__(self):
@@ -277,6 +301,36 @@ class EnsembleEngine:
     def set_replay_size(self, member: int, size: int):
         _lib.check(self._L.iql_set_replay_size(self._h, member, int(size)), self._h)
 
+    def _bind_index_streams(self):
+        if self._mt_states is None:
+            S, K, B = self.n_members, self.max_steps_per_call, self.batch_size
+            self._mt_states = torch.zeros(S, _lib.MT_STATE_WORDS, dtype=torch.int32, device=self.device)
+            self._mt_indices = torch.zeros(S, K, B, dtype=torch.int64, device=self.device)
+            _lib.check(self._L.iql_bind_index_streams(self._h, self._mt_states.data_ptr(), self._mt_indices.data_ptr()),
+                       self._h, "iql_bind_index_streams")
+
+    def set_index_states(self, rngs):
+        """Start every member's numpy index stream (``mode="numpy"`` / ``host_step(numpy_streams=True)``) where the
+        ``np.random.RandomState`` ``rngs[m]`` stands: the next draws of member m are ``rngs[m].randint(0, high_m, ...)``.
+        The objects are read, not kept or advanced."""
+        if len(rngs) != self.n_members:
+            raise ValueError(f"need one RandomState per member ({self.n_members}), got {len(rngs)}")
+        rows = torch.from_numpy(index_state_rows(rngs).view(np.int32))
+        self._bind_index_streams()
+        with self._on_stream():
+            self._mt_states.copy_(rows.to(self.device))
+
+    def get_index_states(self, rngs):
+        """Write every member's device stream back into ``rngs[m]`` (key and pos; the cached Gaussian is kept), so that
+        ``rngs[m].randint`` continues where the device left off.  Waits for the engine's queued work."""
+        if self._mt_states is None:
+            raise RuntimeError("no index streams: call set_index_states first")
+        if len(rngs) != self.n_members:
+            raise ValueError(f"need one RandomState per member ({self.n_members}), got {len(rngs)}")
+        with self._on_stream():
+            rows = self._mt_states.cpu().numpy().view(np.uint32)
+        load_index_state_rows(rngs, rows)
+
     def load_batch(self, member: int, batch):
         s, a, r, s2, d = [self._dense(b) for b in batch]
         B = self.batch_size
@@ -319,10 +373,12 @@ class EnsembleEngine:
             _lib.check(rc, self._h, "iql_host_step_wait")
         return self._host_losses.tolist()
 
-    def host_step(self, batch=None, host_indices: Optional[int] = None, wait: bool = True) -> Optional[List[float]]:
+    def host_step(self, batch=None, host_indices: Optional[int] = None, wait: bool = True,
+                  numpy_streams: bool = False) -> Optional[List[float]]:
         """One update step for a host-driven loop (`iql_train_host_step`): `host_indices` is the ADDRESS of S x B int64
         indices in host memory (rows of the bound replay buffers), or `batch` the five dense tensors of an externally
-        built batch (S = 1).  One CUDA-graph launch; returns the step's [S * 3] losses as Python floats as soon as the
+        built batch (S = 1), or `numpy_streams` draws each member's B_m indices on the device from its numpy index
+        stream (`set_index_states`) at its replay size (`iql_train_host_step_mt19937`).  One CUDA-graph launch; returns the step's [S * 3] losses as Python floats as soon as the
         loss kernel has written them to pinned host memory -- the backward / optimizer launches of the step are still
         running then, stream-ordered before anything the caller enqueues next."""
         if self._host_losses is None:
@@ -335,6 +391,11 @@ class EnsembleEngine:
             guard.__enter__()
         try:
             cur = torch._C._cuda_getCurrentRawStream(self._dev_index)
+            if numpy_streams:
+                rc = self._L.iql_train_host_step_mt19937(self._h, self._host_losses_ptr if wait else None, self._stream_raw, cur)
+                if rc:
+                    _lib.check(rc, self._h, "iql_train_host_step_mt19937")
+                return self._host_losses.tolist() if wait else None
             if host_indices is None:
                 s, a, r, s2, d = [self._dense(b) for b in batch]
                 B = self.batch_size
@@ -390,9 +451,11 @@ class EnsembleEngine:
         """Run K update steps for the active members; returns losses [S, K, 3]
         (value_loss, q_loss, actor_loss) on the device, asynchronously, NaN in the rows of inactive members.
         `indices` [S, K, B]: entries past a member's batch size B_m, and the rows of inactive members, are ignored;
-        `return_indices` gives -1 there."""
+        `return_indices` gives -1 there.  ``mode="numpy"``: member m draws ``randint(0, size_m, size=K * B_m)`` from its
+        numpy index stream (`set_index_states`) on the device, step k taking draws [k B_m, (k + 1) B_m)."""
         S, B = self.n_members, self.batch_size
-        smode = {"philox": _lib.SAMPLE_PHILOX, "indices": _lib.SAMPLE_INDICES, "preloaded": _lib.SAMPLE_PRELOADED}[mode]
+        smode = {"philox": _lib.SAMPLE_PHILOX, "indices": _lib.SAMPLE_INDICES, "preloaded": _lib.SAMPLE_PRELOADED,
+                 "numpy": _lib.SAMPLE_MT19937}[mode]
         idx_ptr = None
         if smode == _lib.SAMPLE_INDICES:
             if indices is None:

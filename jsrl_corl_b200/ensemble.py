@@ -95,23 +95,47 @@ class IQLEnsemble:
         self._buffers = list(buffers)
         for m, rb in enumerate(buffers):
             self.engine.bind_replay(m, rb.rows, rb._high())
+        self._sizes = [rb._high() for rb in buffers]  # the replay sizes the engine holds
+        self._sharing = {}  # buffer -> the members bound to it
+        for m, rb in enumerate(buffers):
+            self._sharing.setdefault(id(rb), []).append(m)
 
     def refresh_replay_sizes(self):
         for m, rb in enumerate(self._buffers):
             self.engine.set_replay_size(m, rb._high())
+            self._sizes[m] = rb._high()
+
+    # ---- numpy index streams drawn on the device ----------------------------
+    def set_index_streams(self, rngs):
+        """Draw member m's batch indices from the ``np.random.RandomState`` ``rngs[m]`` -- ``rngs[m].randint(0,
+        buffer._high(), size=B_m)`` per step, the reference's ``ReplayBuffer.sample`` draw (iql.py:172) on a per-member
+        generator -- on the device, bit for bit, in ``train_steps(K, mode="numpy")`` and
+        ``train_step_logged(numpy_streams=True)``.  The generators' states are copied to the device; the objects are
+        kept (``index_streams``) and brought up to date by ``sync_index_streams``."""
+        rngs = list(rngs)
+        self.engine.set_index_states(rngs)
+        self.index_streams = rngs
+
+    def sync_index_streams(self):
+        """Write the device streams back into the ``RandomState`` objects of ``set_index_streams`` (key and pos; their
+        cached Gaussians are kept), so that host draws continue the device stream."""
+        self.engine.get_index_states(self.index_streams)
 
     def train_steps(self, k_steps: int, **kw) -> torch.Tensor:
         """K fused sample+update steps for every member; losses [S, K, 3] on device."""
         return self.engine.train_steps(k_steps, **kw)
 
-    def train_step_logged(self, indices: Optional[np.ndarray] = None) -> np.ndarray:
+    def train_step_logged(self, indices: Optional[np.ndarray] = None, numpy_streams: bool = False) -> np.ndarray:
         """ONE update step of every member with the losses on the host when it returns ([S, 3] float32:
         value_loss, q_loss, actor_loss) -- the ensemble form of the reference's `log_dict = trainer.train(batch)`
         (offline/iql.py:631-635), for loops that log or branch on the losses every step.  ``indices``: [S, B] int64 rows of
         the bound buffers (member m's first B_m drawn here with numpy, like `ReplayBuffer.sample(B_m)`, when omitted;
         entries past B_m are ignored).  Runs through `iql_train_host_step`: one graph launch, the call returns while the
-        backward of the step is still running."""
+        backward of the step is still running.  ``numpy_streams``: the indices come from the members' index streams
+        (``set_index_streams``), drawn on the device inside the same launch at each buffer's current size."""
         e = self.engine
+        if numpy_streams:
+            return np.asarray(e.host_step(numpy_streams=True), dtype=np.float32).reshape(e.n_members, 3)
         if indices is None:
             indices = np.zeros((e.n_members, e.batch_size), dtype=np.int64)
             for m in np.flatnonzero(e.active):  # inactive members draw nothing; their losses come back NaN
@@ -170,7 +194,8 @@ class IQLEnsemble:
         """``ReplayBuffer.add_transition`` (iql.py:180-196) for every member whose ``mask`` entry is true (all when
         None), into the member's own bound buffer, in one launch.  Advances each buffer's ``_pointer`` / ``_size`` as
         ``add_transition`` does and raises its IndexError for a buffer loaded to the brim -- before anything is
-        written.  Members sharing one buffer cannot insert in the same call."""
+        written.  Members sharing one buffer cannot insert in the same call.  The engine's replay size of every member
+        bound to a buffer that grew follows the buffer's ``_high()`` (the bound of the next draws)."""
         S = self.n_members
         bufs = getattr(self, "_buffers", None)
         if bufs is None:
@@ -187,6 +212,12 @@ class IQLEnsemble:
             rb = bufs[m]
             rb._pointer = (rb._pointer + 1) % rb._buffer_size
             rb._size = min(rb._size + 1, rb._buffer_size)
+        for i in np.flatnonzero(mask):  # a host-only call, and only while a ring fills
+            for m in self._sharing[id(bufs[i])]:
+                high = bufs[m]._high()
+                if high != self._sizes[m]:
+                    self.engine.set_replay_size(m, high)
+                    self._sizes[m] = high
 
     # ---- checkpoints in the reference layout --------------------------------
     def member_state_dict(self, m: int) -> Dict[str, Any]:

@@ -384,7 +384,7 @@ def ensemble_eval_actor(envs, ensemble, use_guide: bool, configs, max_action: fl
 def ensemble_train_loop(configs, envs, eval_envs, replay_buffers, state_dim: int, action_dim: int, max_action: float,
                         max_steps: int, log: Optional[Callable[[int, Dict, int], None]] = None, reward_mod_dicts=None,
                         is_env_with_goal: bool = False, scheduler=None, mixed_batch_sizes: bool = False,
-                        philox_act_dropout: bool = False):
+                        philox_act_dropout: bool = False, device_index_streams: bool = False):
     """``train_loop`` for S members at once, one ``JsrlTrainConfig`` per member (seed, IQL / Adam hyper-parameters,
     curriculum, tolerance, noise and checkpoint path may differ; ``ENSEMBLE_SHARED_FIELDS`` may not; ``batch_size``
     may differ with ``mixed_batch_sizes=True``, the batch-size axis of a search).
@@ -412,7 +412,14 @@ def ensemble_train_loop(configs, envs, eval_envs, replay_buffers, state_dim: int
     (IQL_ACT_LEARNER_DIST_DROPOUT / IQL_ACT_LEARNER_DROPOUT): member m's masks come from the engine's Philox stream
     keyed by ``seed | 1 << 63`` at its act counter (``learner.engine.act_steps[m]``, one per learner env step), so they
     are reproducible but are not torch's ``nn.Dropout`` draws.  Guide acts and evaluations run without dropout.
-    Checkpoints carry the reference's dropout-policy keys."""
+    Checkpoints carry the reference's dropout-policy keys.
+
+    ``device_index_streams``: each member's ``RandomState(seed)`` index stream runs on the device (numpy's MT19937 and
+    bounded-integer rule, bit for bit; ``IQLEnsemble.set_index_streams``) instead of on the host -- the same indices, so
+    the same results, without S ``randint`` calls and an index upload per update.  The offline ensemble's streams are
+    handed to the learner at the switch and written back to the generators at the end (``learner.index_streams``).
+    Off by default: the host form passes every call's indices through ``IQLEnsemble.train_steps`` /
+    ``train_step_logged``, where callers can see them."""
     check_ensemble_configs(configs, scheduler, mixed_batch_sizes, philox_act_dropout)
     S = len(configs)
     if not (len(envs) == len(eval_envs) == S):
@@ -486,6 +493,8 @@ def ensemble_train_loop(configs, envs, eval_envs, replay_buffers, state_dim: int
     # ---- offline phase: K-step calls between evaluation points and gate openings ----
     offline = _build_ensemble(configs, [n[0] for n in nets], state_dim, action_dim, off, device)
     offline.bind_replay(list(replay_buffers))
+    if device_index_streams:
+        offline.set_index_streams(index_rng)
     first = np.array([min(b, off) if gated else 0 for b in Bm])  # the first offline step of each member
     done_steps = [0] * S
     t = int(first.min())
@@ -500,12 +509,15 @@ def ensemble_train_loop(configs, envs, eval_envs, replay_buffers, state_dim: int
             t = stop
             continue
         _sync_active(offline, train)
-        idx = np.zeros((S, K, max(Bm)), dtype=np.int64)
-        for m in np.flatnonzero(train):
-            high = replay_buffers[m]._high()
-            for k in range(K):
-                idx[m, k, :Bm[m]] = index_rng[m].randint(0, high, size=Bm[m])
-        losses = offline.train_steps(K, mode="indices", indices=torch.from_numpy(idx)).cpu().numpy()
+        if device_index_streams:  # K x B_m draws per training member at its buffer's size, inside the call
+            losses = offline.train_steps(K, mode="numpy").cpu().numpy()
+        else:
+            idx = np.zeros((S, K, max(Bm)), dtype=np.int64)
+            for m in np.flatnonzero(train):
+                high = replay_buffers[m]._high()
+                for k in range(K):
+                    idx[m, k, :Bm[m]] = index_rng[m].randint(0, high, size=Bm[m])
+            losses = offline.train_steps(K, mode="indices", indices=torch.from_numpy(idx)).cpu().numpy()
         for k in range(K):
             for m in np.flatnonzero(train):
                 done_steps[m] += 1
@@ -514,6 +526,8 @@ def ensemble_train_loop(configs, envs, eval_envs, replay_buffers, state_dim: int
         t = stop
         if t % eval_freq == 0:
             evaluate(t - 1, offline, False, done_steps, train)
+    if device_index_streams:
+        offline.sync_index_streams()
     if on <= 0 or not live.any():
         return offline, configs, histories
 
@@ -533,6 +547,8 @@ def ensemble_train_loop(configs, envs, eval_envs, replay_buffers, state_dim: int
     online_buffers = [jsrl.get_online_buffer(c, replay_buffers[m], state_dim, action_dim) if live[m] else replay_buffers[m]
                       for m, c in enumerate(configs)]
     learner.bind_replay(online_buffers)
+    if device_index_streams:
+        learner.set_index_streams(index_rng)
     if not live.all():
         _sync_active(learner, live)
     states = [_reset(envs[m]) if live[m] else None for m in range(S)]
@@ -611,9 +627,12 @@ def ensemble_train_loop(configs, envs, eval_envs, replay_buffers, state_dim: int
         if not train.any():
             continue
         _sync_active(learner, train)
-        for m in np.flatnonzero(train):
-            idx[m, :Bm[m]] = index_rng[m].randint(0, online_buffers[m]._high(), size=Bm[m])
-        losses = learner.train_step_logged(idx)
+        if device_index_streams:  # B_m draws per training member at its ring's size, inside the step's launch
+            losses = learner.train_step_logged(numpy_streams=True)
+        else:
+            for m in np.flatnonzero(train):
+                idx[m, :Bm[m]] = index_rng[m].randint(0, online_buffers[m]._high(), size=Bm[m])
+            losses = learner.train_step_logged(idx)
         for m in np.flatnonzero(train):
             total_it[m] += 1
             log_dict = {"value_loss": float(losses[m, 0]), "q_loss": float(losses[m, 1]), "actor_loss": float(losses[m, 2]),
@@ -622,4 +641,6 @@ def ensemble_train_loop(configs, envs, eval_envs, replay_buffers, state_dim: int
             log(m, log_dict, total_it[m])
         if (t + 1) % eval_freq == 0:
             evaluate(t, learner, True, total_it, train)
+    if device_index_streams:
+        learner.sync_index_streams()
     return learner, configs, histories
