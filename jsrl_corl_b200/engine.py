@@ -39,15 +39,21 @@ def query_layout(n_members, state_dim, action_dim, hidden_dim, n_hidden, batch_s
     h = C.c_void_p()
     _lib.check(L.iql_create(C.byref(cfg), C.byref(h)), None, "iql_create")
     try:
-        lay = Layout()
-        _lib.check(L.iql_get_layout(h, C.byref(lay)), h)
-        tensors = []
-        for i in range(lay.n_tensors):
-            t = TensorInfo()
-            _lib.check(L.iql_tensor_at(h, i, C.byref(t)), h)
-            tensors.append((t.net, t.layer, t.kind, t.rows, t.cols, t.offset, t.ld))
+        lay, tensors = _read_layout(L, h)
     finally:
         L.iql_destroy(h)
+    return lay, [(t.net, t.layer, t.kind, t.rows, t.cols, t.offset, t.ld) for t in tensors]
+
+
+def _read_layout(L, h):
+    """The handle's arena layout and its tensor table ([TensorInfo], in table order)."""
+    lay = Layout()
+    _lib.check(L.iql_get_layout(h, C.byref(lay)), h)
+    tensors = []
+    for i in range(lay.n_tensors):
+        t = TensorInfo()
+        _lib.check(L.iql_tensor_at(h, i, C.byref(t)), h)
+        tensors.append(t)
     return lay, tensors
 
 
@@ -96,13 +102,7 @@ class EnsembleEngine:
             raise ValueError(f"step_path must be one of {sorted(_lib.STEP_PATHS)}")
         _lib.check(self._L.iql_set_option(self._h, _lib.OPT_STEP_PATH, _lib.STEP_PATHS[step_path]), self._h, "iql_set_option")
         self.step_path = step_path
-        self.layout = Layout()
-        _lib.check(self._L.iql_get_layout(self._h, C.byref(self.layout)), self._h)
-        self.tensors = []
-        for i in range(self.layout.n_tensors):
-            t = TensorInfo()
-            _lib.check(self._L.iql_tensor_at(self._h, i, C.byref(t)), self._h)
-            self.tensors.append(t)
+        self.layout, self.tensors = _read_layout(self._L, self._h)
         P, PQ = self.layout.param_floats, self.layout.q_floats
         with torch.cuda.device(self.device):
             f32 = dict(dtype=torch.float32, device=self.device)
@@ -126,13 +126,18 @@ class EnsembleEngine:
             raise ValueError(f"math_mode='tf32' with strict_tf32: batch {batch_size} / hidden {hidden_dim} is outside the tcgen05 "
                              "kernels (batch % 128 == 0 and hidden % 256 == 0 required); the FP32 kernels would run")
         self.act_calls = 0
-        self._act_in = self._act_out = self._act_in_dev = self._act_std = None
+        # host buffers of act_host / act_host_gaussian (observation in; action or mean, std out)
+        self._act_in = np.zeros(state_dim, dtype=np.float32)
+        self._act_out = np.zeros(action_dim, dtype=np.float32)
+        self._act_std = np.zeros(action_dim, dtype=np.float32)
+        self._act_ptrs = (self._act_in.ctypes.data, self._act_out.ctypes.data, self._act_std.ctypes.data)
         self._hparams = [self._default_hparams(m) for m in range(n_members)]
         self._batch_sizes = [batch_size] * n_members
         self._replay_refs: Dict[int, torch.Tensor] = {}
         self._idx_stage: Dict[int, torch.Tensor] = {}
         self._host_losses = None
         self._dev_index = self.device.index
+        self._stream_raw = self.stream.cuda_stream
         self._mt_states = self._mt_indices = None  # numpy index streams, allocated by the first set_index_states
 
     # ------------------------------------------------------------------
@@ -332,14 +337,7 @@ class EnsembleEngine:
         load_index_state_rows(rngs, rows)
 
     def load_batch(self, member: int, batch):
-        s, a, r, s2, d = [self._dense(b) for b in batch]
-        B = self.batch_size
-        if s.shape != (B, self.state_dim) or s2.shape != (B, self.state_dim):
-            raise ValueError(f"states must be [{B}, {self.state_dim}]")
-        if a.shape != (B, self.action_dim):
-            raise RuntimeError("Actions shape missmatch")  # iql.py:530
-        if r.numel() != B or d.numel() != B:
-            raise ValueError("rewards / dones must have batch_size elements")
+        s, a, r, s2, d = self._dense_batch(batch)
         with self._on_stream() as st:
             _lib.check(self._L.iql_load_batch(self._h, member, s.data_ptr(), a.data_ptr(), r.data_ptr(), s2.data_ptr(),
                                               d.data_ptr(), st.cuda_stream), self._h)
@@ -348,14 +346,7 @@ class EnsembleEngine:
     def train_on_batch(self, batch, out: Optional[torch.Tensor] = None) -> torch.Tensor:
         """S = 1 drop-in step: stage an externally sampled batch and run one update, under a single stream
         hand-over (the `ImplicitQLearning.train(batch)` path).  Returns losses [1, 1, 3] on the device."""
-        s, a, r, s2, d = [self._dense(b) for b in batch]
-        B = self.batch_size
-        if s.shape != (B, self.state_dim) or s2.shape != (B, self.state_dim):
-            raise ValueError(f"states must be [{B}, {self.state_dim}]")
-        if a.shape != (B, self.action_dim):
-            raise RuntimeError("Actions shape missmatch")  # iql.py:530
-        if r.numel() != B or d.numel() != B:
-            raise ValueError("rewards / dones must have batch_size elements")
+        s, a, r, s2, d = self._dense_batch(batch)
         if out is None:
             out = torch.empty(self.n_members, 1, 3, dtype=torch.float32, device=self.device)
         with self._on_stream() as st:
@@ -384,61 +375,52 @@ class EnsembleEngine:
         if self._host_losses is None:
             self._host_losses = np.zeros(3 * self.n_members, dtype=np.float32)
             self._host_losses_ptr = self._host_losses.ctypes.data
-            self._stream_raw = self.stream.cuda_stream
-        switch = torch._C._cuda_getDevice() != self._dev_index  # (torch.cuda.current_device() costs ~1.5 us of Python)
-        if switch:
-            guard = torch.cuda.device(self.device)
-            guard.__enter__()
-        try:
-            cur = torch._C._cuda_getCurrentRawStream(self._dev_index)
-            if numpy_streams:
-                rc = self._L.iql_train_host_step_mt19937(self._h, self._host_losses_ptr if wait else None, self._stream_raw, cur)
-                if rc:
-                    _lib.check(rc, self._h, "iql_train_host_step_mt19937")
-                return self._host_losses.tolist() if wait else None
-            if host_indices is None:
-                s, a, r, s2, d = [self._dense(b) for b in batch]
-                B = self.batch_size
-                if s.shape != (B, self.state_dim) or s2.shape != (B, self.state_dim):
-                    raise ValueError(f"states must be [{B}, {self.state_dim}]")
-                if a.shape != (B, self.action_dim):
-                    raise RuntimeError("Actions shape missmatch")  # iql.py:530
-                if r.numel() != B or d.numel() != B:
-                    raise ValueError("rewards / dones must have batch_size elements")
-                # staged on the caller's stream: the previous step made it wait for the engine stream (ev_out), and
-                # iql_train_host_step orders the engine stream behind it again (ev_in)
-                rc = self._L.iql_load_batch(self._h, 0, s.data_ptr(), a.data_ptr(), r.data_ptr(), s2.data_ptr(), d.data_ptr(), cur)
-                if rc:
-                    _lib.check(rc, self._h, "iql_load_batch")
-                self._keep = (s, a, r, s2, d)
-            rc = self._L.iql_train_host_step(self._h, host_indices, self._host_losses_ptr if wait else None, self._stream_raw, cur)
-            if rc:
-                _lib.check(rc, self._h, "iql_train_host_step")
-        finally:
-            if switch:
-                guard.__exit__(None, None, None)
+        losses = self._host_losses_ptr if wait else None
+        if numpy_streams:
+            _lib.call_on_device(self._dev_index, self.device, self._h, "iql_train_host_step_mt19937",
+                                self._L.iql_train_host_step_mt19937, self._h, losses, self._stream_raw)
+        elif host_indices is not None:
+            _lib.call_on_device(self._dev_index, self.device, self._h, "iql_train_host_step", self._L.iql_train_host_step,
+                                self._h, host_indices, losses, self._stream_raw)
+        else:
+            _lib.call_on_device(self._dev_index, self.device, self._h, "iql_train_host_step", self._load_and_step,
+                                self._dense_batch(batch), losses)
         return self._host_losses.tolist() if wait else None
+
+    def _load_and_step(self, batch, losses, cur) -> int:
+        # the batch is staged on the caller's stream, the stream the step runs on: plain stream order
+        s, a, r, s2, d = batch
+        rc = self._L.iql_load_batch(self._h, 0, s.data_ptr(), a.data_ptr(), r.data_ptr(), s2.data_ptr(), d.data_ptr(), cur)
+        if rc:
+            _lib.check(rc, self._h, "iql_load_batch")
+        self._keep = batch
+        return self._L.iql_train_host_step(self._h, None, losses, self._stream_raw, cur)
 
     def _dense(self, t: torch.Tensor) -> torch.Tensor:
         if t.device == self.device and t.dtype == torch.float32 and t.is_contiguous():
             return t
         return t.to(device=self.device, dtype=torch.float32).contiguous()
 
+    def _dense_batch(self, batch):
+        """The five tensors of an externally built batch (S = 1), dense float32 on the engine's device, shapes checked."""
+        s, a, r, s2, d = [self._dense(b) for b in batch]
+        B = self.batch_size
+        if s.shape != (B, self.state_dim) or s2.shape != (B, self.state_dim):
+            raise ValueError(f"states must be [{B}, {self.state_dim}]")
+        if a.shape != (B, self.action_dim):
+            raise RuntimeError("Actions shape missmatch")  # iql.py:530
+        if r.numel() != B or d.numel() != B:
+            raise ValueError("rewards / dones must have batch_size elements")
+        return s, a, r, s2, d
+
     @contextlib.contextmanager
     def _on_stream(self):
         """Every C-ABI call that launches runs inside this: the engine's device is made current (the engine may
         live on cuda:N while the process's current device is another) and the engine stream is ordered after / before
         the caller's current stream on that device."""
-        if torch.cuda.current_device() == self.device.index:  # common case: no device switch needed
+        switch = torch.cuda.current_device() != self.device.index
+        with torch.cuda.device(self.device) if switch else contextlib.nullcontext():
             cur = torch.cuda.current_stream()
-            self.stream.wait_stream(cur)
-            try:
-                yield self.stream
-            finally:
-                cur.wait_stream(self.stream)
-            return
-        with torch.cuda.device(self.device):
-            cur = torch.cuda.current_stream(self.device)
             self.stream.wait_stream(cur)
             try:
                 yield self.stream
@@ -536,51 +518,20 @@ class EnsembleEngine:
         rides in the kernel parameters, the kernel reads the policy weights straight from the parameter arena, the
         action comes back through pinned host memory the host spins on (`iql_act_host`: one launch, no copies, no
         stream synchronisation).  Returns the flat numpy action (scaled and clamped by max_action)."""
-        if self._act_in is None:
-            self._act_in = np.zeros(self.state_dim, dtype=np.float32)
-            self._act_out = np.zeros(self.action_dim, dtype=np.float32)
-            self._act_ptrs = (self._act_in.ctypes.data, self._act_out.ctypes.data)
-            self._stream_raw = self.stream.cuda_stream
         self._act_in[:] = np.asarray(state, dtype=np.float32).reshape(-1)
-        switch = torch._C._cuda_getDevice() != self._dev_index
-        if switch:
-            guard = torch.cuda.device(self.device)
-            guard.__enter__()
-        try:
-            rc = self._L.iql_act_host(self._h, member, self._act_ptrs[0], float(max_action), self._act_ptrs[1], self._stream_raw,
-                                      torch._C._cuda_getCurrentRawStream(self._dev_index))
-            if rc:
-                _lib.check(rc, self._h, "iql_act_host")
-        finally:
-            if switch:
-                guard.__exit__(None, None, None)
+        p_in, p_out, _ = self._act_ptrs
+        _lib.call_on_device(self._dev_index, self.device, self._h, "iql_act_host", self._L.iql_act_host,
+                            self._h, member, p_in, float(max_action), p_out, self._stream_raw)
         self.act_calls += 1
         return self._act_out.copy()
 
     def act_host_gaussian(self, member: int, state: np.ndarray):
         """(mean, std) of the Gaussian policy's action distribution for one host observation (`iql_act_host_gaussian`):
         mean = tanh(MLP(state)) unscaled, std = exp(clamp(log_std)); the caller samples on the host."""
-        if self._act_in is None:
-            self._act_in = np.zeros(self.state_dim, dtype=np.float32)
-            self._act_out = np.zeros(self.action_dim, dtype=np.float32)
-            self._act_ptrs = (self._act_in.ctypes.data, self._act_out.ctypes.data)
-            self._stream_raw = self.stream.cuda_stream
-        if self._act_std is None:
-            self._act_std = np.zeros(self.action_dim, dtype=np.float32)
-            self._act_std_ptr = self._act_std.ctypes.data
         self._act_in[:] = np.asarray(state, dtype=np.float32).reshape(-1)
-        switch = torch._C._cuda_getDevice() != self._dev_index
-        if switch:
-            guard = torch.cuda.device(self.device)
-            guard.__enter__()
-        try:
-            rc = self._L.iql_act_host_gaussian(self._h, member, self._act_ptrs[0], self._act_ptrs[1], self._act_std_ptr, self._stream_raw,
-                                               torch._C._cuda_getCurrentRawStream(self._dev_index))
-            if rc:
-                _lib.check(rc, self._h, "iql_act_host_gaussian")
-        finally:
-            if switch:
-                guard.__exit__(None, None, None)
+        p_in, p_out, p_std = self._act_ptrs
+        _lib.call_on_device(self._dev_index, self.device, self._h, "iql_act_host_gaussian", self._L.iql_act_host_gaussian,
+                            self._h, member, p_in, p_out, p_std, self._stream_raw)
         self.act_calls += 1
         return self._act_out.copy(), self._act_std.copy()
 
@@ -600,10 +551,6 @@ class EnsembleEngine:
                              "tensor on the engine's device")
         _lib.check(self._L.iql_bind_guide(self._h, params.data_ptr()), self._h, "iql_bind_guide")
         self._guide_ref = params
-
-    def _ensure_stream_raw(self):
-        if getattr(self, "_stream_raw", None) is None:
-            self._stream_raw = self.stream.cuda_stream
 
     def act_members_host(self, states: np.ndarray, source, max_action: float = 1.0, out: Optional[np.ndarray] = None,
                          std: Optional[np.ndarray] = None):
@@ -630,20 +577,9 @@ class EnsembleEngine:
         for arr in (out, std):
             if arr is not None and (arr.shape != (S, A) or arr.dtype != np.float32 or not arr.flags.c_contiguous):
                 raise ValueError(f"out / std must be C-contiguous float32 [{S}, {A}]")
-        self._ensure_stream_raw()
-        switch = torch._C._cuda_getDevice() != self._dev_index
-        if switch:
-            guard = torch.cuda.device(self.device)
-            guard.__enter__()
-        try:
-            rc = self._L.iql_act_host_members(self._h, st.ctypes.data, src.ctypes.data, float(max_action), out.ctypes.data,
-                                              std.ctypes.data if std is not None else None, self._stream_raw,
-                                              torch._C._cuda_getCurrentRawStream(self._dev_index))
-            if rc:
-                _lib.check(rc, self._h, "iql_act_host_members")
-        finally:
-            if switch:
-                guard.__exit__(None, None, None)
+        _lib.call_on_device(self._dev_index, self.device, self._h, "iql_act_host_members", self._L.iql_act_host_members,
+                            self._h, st.ctypes.data, src.ctypes.data, float(max_action), out.ctypes.data,
+                            std.ctypes.data if std is not None else None, self._stream_raw)
         self.act_calls += 1
         return out, std
 
@@ -676,17 +612,6 @@ class EnsembleEngine:
         s, a = f(states, (S, self.state_dim)), f(actions, (S, self.action_dim))
         r, s2, d = f(rewards, (S,)), f(next_states, (S, self.state_dim)), f(dones, (S,))
         p = np.ascontiguousarray(pointers, dtype=np.int64).reshape(S)
-        self._ensure_stream_raw()
-        switch = torch._C._cuda_getDevice() != self._dev_index
-        if switch:
-            guard = torch.cuda.device(self.device)
-            guard.__enter__()
-        try:
-            rc = self._L.iql_replay_insert_members_host(self._h, s.ctypes.data, a.ctypes.data, r.ctypes.data, s2.ctypes.data,
-                                                        d.ctypes.data, p.ctypes.data, self._stream_raw,
-                                                        torch._C._cuda_getCurrentRawStream(self._dev_index))
-            if rc:
-                _lib.check(rc, self._h, "iql_replay_insert_members_host")
-        finally:
-            if switch:
-                guard.__exit__(None, None, None)
+        _lib.call_on_device(self._dev_index, self.device, self._h, "iql_replay_insert_members_host",
+                            self._L.iql_replay_insert_members_host, self._h, s.ctypes.data, a.ctypes.data, r.ctypes.data,
+                            s2.ctypes.data, d.ctypes.data, p.ctypes.data, self._stream_raw)

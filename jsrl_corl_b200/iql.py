@@ -288,29 +288,25 @@ class ReplayBuffer:
     def row_layout(self) -> _lib.RowLayout:
         return self._lay
 
-    def _to_tensor(self, data: np.ndarray) -> torch.Tensor:
-        return torch.tensor(data, dtype=torch.float32, device=self._device)
-
-    def _stream(self) -> int:
-        # raw handle of torch's current stream on the buffer's device (torch.cuda.current_stream() costs ~7 us of Python)
-        return torch._C._cuda_getCurrentRawStream(self._dev_index)
-
-    def load_d4rl_dataset(self, data: Dict[str, np.ndarray]):
+    def _dataset_tensors(self, data: Dict[str, np.ndarray]):
+        """The five arrays of a D4RL-style dataset as float32 device tensors, once it is known to fit this buffer."""
         if self._size != 0:
             raise ValueError("Trying to load data into non-empty replay buffer")
-        n = data["observations"].shape[0]
-        if n > self._buffer_size:
+        if data["observations"].shape[0] > self._buffer_size:
             raise ValueError("Replay buffer is smaller than the dataset you are trying to load!")
-        s = self._to_tensor(data["observations"]).contiguous()
-        a = self._to_tensor(data["actions"]).contiguous()
-        r = self._to_tensor(data["rewards"]).reshape(-1).contiguous()
-        s2 = self._to_tensor(data["next_observations"]).contiguous()
-        d = self._to_tensor(data["terminals"]).reshape(-1).contiguous()
+        # torch.tensor keeps the strides of a non-C-order array (Fortran order, a transposed view); the pack reads row-major
+        s, a, r, s2, d = [torch.tensor(data[k], dtype=torch.float32, device=self._device).contiguous()
+                          for k in ("observations", "actions", "rewards", "next_observations", "terminals")]
         if s.shape[1] != self._state_dim or a.shape[1] != self._action_dim:
             raise ValueError("dataset dims do not match the buffer")
-        with torch.cuda.device(self._device):
-            _lib.check(self._L.iql_replay_pack(self._rows.data_ptr(), C.byref(self._lay), 0, n, s.data_ptr(), a.data_ptr(),
-                                               r.data_ptr(), s2.data_ptr(), d.data_ptr(), self._stream()), None, "iql_replay_pack")
+        return s, a, r.reshape(-1), s2, d.reshape(-1)
+
+    def load_d4rl_dataset(self, data: Dict[str, np.ndarray]):
+        s, a, r, s2, d = self._dataset_tensors(data)
+        n = s.shape[0]
+        _lib.call_on_device(self._dev_index, self._device, None, "iql_replay_pack", self._L.iql_replay_pack,
+                            self._rows.data_ptr(), self._lay_ref, 0, n, s.data_ptr(), a.data_ptr(), r.data_ptr(),
+                            s2.data_ptr(), d.data_ptr())
         torch.cuda.current_stream(self._device).synchronize()  # inputs are temporaries
         self._size += n
         self._pointer = min(self._size, n)
@@ -324,29 +320,18 @@ class ReplayBuffer:
         value for locomotion tasks; ``reward_shift=1`` for antmaze), then the pack.  ``data`` is NOT modified.
         Returns ``(state_mean, state_std)`` as numpy arrays (``(0, 1)`` when ``normalize`` is off), which the caller
         hands to ``wrap_env`` exactly as with the reference functions."""
-        if self._size != 0:
-            raise ValueError("Trying to load data into non-empty replay buffer")
-        n = data["observations"].shape[0]
-        if n > self._buffer_size:
-            raise ValueError("Replay buffer is smaller than the dataset you are trying to load!")
-        s = self._to_tensor(data["observations"]).contiguous()
-        a = self._to_tensor(data["actions"]).contiguous()
-        r = self._to_tensor(data["rewards"]).reshape(-1).contiguous()
-        s2 = self._to_tensor(data["next_observations"]).contiguous()
-        d = self._to_tensor(data["terminals"]).reshape(-1).contiguous()
-        if s.shape[1] != self._state_dim or a.shape[1] != self._action_dim:
-            raise ValueError("dataset dims do not match the buffer")
+        s, a, r, s2, d = self._dataset_tensors(data)
+        n = s.shape[0]
         mean = torch.zeros(self._state_dim, dtype=torch.float32, device=self._device)
         std = torch.ones(self._state_dim, dtype=torch.float32, device=self._device)
         rdiv = rmul = 1.0
         if reward_mod:
             rdiv = float(np.float32(reward_mod["max_ret"] - reward_mod["min_ret"]))
             rmul = float(reward_mod["max_episode_steps"])
-        with torch.cuda.device(self._device):
-            _lib.check(self._L.iql_replay_ingest(self._rows.data_ptr(), C.byref(self._lay), 0, n, s.data_ptr(), a.data_ptr(),
-                                                 r.data_ptr(), s2.data_ptr(), d.data_ptr(), int(bool(normalize)), float(eps),
-                                                 mean.data_ptr(), std.data_ptr(), rdiv, rmul, float(reward_shift),
-                                                 self._stream()), None, "iql_replay_ingest")
+        _lib.call_on_device(self._dev_index, self._device, None, "iql_replay_ingest", self._L.iql_replay_ingest,
+                            self._rows.data_ptr(), self._lay_ref, 0, n, s.data_ptr(), a.data_ptr(), r.data_ptr(),
+                            s2.data_ptr(), d.data_ptr(), int(bool(normalize)), float(eps), mean.data_ptr(), std.data_ptr(),
+                            rdiv, rmul, float(reward_shift))
         torch.cuda.current_stream(self._device).synchronize()
         self._size += n
         self._pointer = min(self._size, n)
@@ -376,39 +361,26 @@ class ReplayBuffer:
 
     def sample(self, batch_size: int) -> TensorBatch:
         B = int(batch_size)
-        dev = self._device
         high = self._high()
-        switch = torch._C._cuda_getDevice() != self._dev_index
-        if switch:
-            ctx = torch.cuda.device(dev)
-            ctx.__enter__()
-        try:
-            if self._sampler == "numpy":
-                idx_host = np.random.randint(0, high, size=B)  # raises ValueError on an empty buffer, like the reference
-                if self._fresh_outputs:
-                    sl = _SampleSlot(self, B)
-                else:
-                    sl = self._out_slot(B)
-                # the indices ride in the kernel parameters: no staging buffer, no host->device copy
-                rc = self._L.iql_replay_sample_host(self._rows.data_ptr(), self._lay_ref, high, B, idx_host.__array_interface__["data"][0],
-                                                    *sl.ptrs, self._stream())
-                if rc:
-                    _lib.check(rc, None, "iql_replay_sample_host")
-                sl.idx_host, sl.high = idx_host, high
-                self._last_indices = idx_host
-            else:
-                if high <= 0:
-                    raise ValueError("low >= high")
-                sl = _SampleSlot(self, B) if self._fresh_outputs else self._out_slot(B)
-                sl.idx_host = None
-                rc = self._L.iql_replay_sample(self._rows.data_ptr(), self._lay_ref, high, B, None, self._seed, self._sample_calls,
-                                               *sl.ptrs, None, self._stream())
-                if rc:
-                    _lib.check(rc, None, "iql_replay_sample")
-            self._sample_calls += 1
-        finally:
-            if switch:
-                ctx.__exit__(None, None, None)
+        if self._sampler == "numpy":
+            idx_host = np.random.randint(0, high, size=B)  # raises ValueError on an empty buffer, like the reference
+        elif high <= 0:
+            raise ValueError("low >= high")
+        sl = _SampleSlot(self, B) if self._fresh_outputs else self._out_slot(B)
+        s, a, r, s2, d = sl.ptrs
+        if self._sampler == "numpy":
+            # the indices ride in the kernel parameters: no staging buffer, no host->device copy
+            _lib.call_on_device(self._dev_index, self._device, None, "iql_replay_sample_host", self._L.iql_replay_sample_host,
+                                self._rows.data_ptr(), self._lay_ref, high, B, idx_host.__array_interface__["data"][0],
+                                s, a, r, s2, d)
+            sl.idx_host, sl.high = idx_host, high
+            self._last_indices = idx_host
+        else:
+            sl.idx_host = None
+            _lib.call_on_device(self._dev_index, self._device, None, "iql_replay_sample", self._L.iql_replay_sample,
+                                self._rows.data_ptr(), self._lay_ref, high, B, None, self._seed, self._sample_calls,
+                                s, a, r, s2, d, None)
+        self._sample_calls += 1
         out = sl.out
         sl.ver = (out[0]._version, out[1]._version, out[2]._version, out[3]._version, out[4]._version)
         return list(out)
@@ -424,41 +396,36 @@ class ReplayBuffer:
             # a buffer loaded to the brim leaves _pointer == buffer_size (iql.py:168); the reference's
             # `self._states[self._pointer] = ...` raises IndexError there too
             raise IndexError(f"index {self._pointer} is out of bounds for dimension 0 with size {self._buffer_size}")
-        switch = torch._C._cuda_getDevice() != self._dev_index
-        if switch:
-            ctx = torch.cuda.device(self._device)
-            ctx.__enter__()
-        try:
-            if lay.row_floats <= 960:
-                # the packed row rides in the kernel parameters: one launch, no staging row, no copy
-                rc = self._L.iql_replay_insert_host(self._rows.data_ptr(), self._lay_ref, self._pointer, st.ctypes.data, ac.ctypes.data,
-                                                    float(reward), ns.ctypes.data, float(done), self._stream())
-                if rc:
-                    _lib.check(rc, None, "iql_replay_insert_host")
-            else:
-                # two pinned staging rows used alternately, each guarded by an event recorded after its host->device copy
-                i = self._stage_i
-                self._stage_i = i ^ 1
-                if self._stage_ev[i] is not None:
-                    self._stage_ev[i].synchronize()  # this slot's previous host->device copy (two inserts ago) has run
-                h = self._stage_host[i].numpy()
-                h[:] = 0.0
-                h[lay.off_state:lay.off_state + self._state_dim] = st
-                h[lay.off_action:lay.off_action + self._action_dim] = ac
-                h[lay.off_reward] = float(reward)
-                h[lay.off_next_state:lay.off_next_state + self._state_dim] = ns
-                h[lay.off_done] = float(done)
-                self._stage[i].copy_(self._stage_host[i], non_blocking=True)
-                ev = torch.cuda.Event()
-                ev.record(torch.cuda.current_stream(self._device))
-                self._stage_ev[i] = ev
-                _lib.check(self._L.iql_replay_insert(self._rows.data_ptr(), self._lay_ref, self._pointer, self._stage[i].data_ptr(),
-                                                     self._stream()), None, "iql_replay_insert")
-        finally:
-            if switch:
-                ctx.__exit__(None, None, None)
+        if lay.row_floats <= 960:
+            # the packed row rides in the kernel parameters: one launch, no staging row, no copy
+            _lib.call_on_device(self._dev_index, self._device, None, "iql_replay_insert_host", self._L.iql_replay_insert_host,
+                                self._rows.data_ptr(), self._lay_ref, self._pointer, st.ctypes.data, ac.ctypes.data,
+                                float(reward), ns.ctypes.data, float(done))
+        else:
+            _lib.call_on_device(self._dev_index, self._device, None, "iql_replay_insert", self._insert_staged,
+                                st, ac, reward, ns, done)
         self._pointer = (self._pointer + 1) % self._buffer_size
         self._size = min(self._size + 1, self._buffer_size)
+
+    def _insert_staged(self, st, ac, reward, ns, done, cur) -> int:
+        # two pinned staging rows used alternately, each guarded by an event recorded after its host->device copy
+        lay = self._lay
+        i = self._stage_i
+        self._stage_i = i ^ 1
+        if self._stage_ev[i] is not None:
+            self._stage_ev[i].synchronize()  # this slot's previous host->device copy (two inserts ago) has run
+        h = self._stage_host[i].numpy()
+        h[:] = 0.0
+        h[lay.off_state:lay.off_state + self._state_dim] = st
+        h[lay.off_action:lay.off_action + self._action_dim] = ac
+        h[lay.off_reward] = float(reward)
+        h[lay.off_next_state:lay.off_next_state + self._state_dim] = ns
+        h[lay.off_done] = float(done)
+        self._stage[i].copy_(self._stage_host[i], non_blocking=True)
+        ev = torch.cuda.Event()
+        ev.record(torch.cuda.current_stream(self._device))
+        self._stage_ev[i] = ev
+        return self._L.iql_replay_insert(self._rows.data_ptr(), self._lay_ref, self._pointer, self._stage[i].data_ptr(), cur)
 
 
 # ---------------------------------------------------------------------------
@@ -505,6 +472,14 @@ class MLP(nn.Module):
         return self.net(x)
 
 
+def _aliases_arena(eng: EnsembleEngine, weight: torch.Tensor, log_std: Optional[torch.Tensor] = None) -> bool:
+    """The parameters an engine act reads still point into ``eng.params``; False once they were re-pointed (module
+    moved / re-initialised), and the stock torch path serves the call."""
+    lo = eng.params.data_ptr()
+    hi = lo + eng.params.numel() * 4
+    return weight.device == eng.device and lo <= weight.data_ptr() < hi and (log_std is None or lo <= log_std.data_ptr() < hi)
+
+
 class _PolicyBase(nn.Module):
     def __init__(self, state_dim, act_dim, max_action, hidden_dim, n_hidden, dropout, dropout_when_not_none):
         super().__init__()
@@ -522,10 +497,8 @@ class _PolicyBase(nn.Module):
         if ref is None:
             return None
         eng, member = ref
-        p = self.net.net[0].weight
-        if p.device != eng.device or p.data_ptr() < eng.params.data_ptr() or \
-                p.data_ptr() >= eng.params.data_ptr() + eng.params.numel() * 4:
-            return None  # parameters were re-pointed (module moved / re-initialised): stock torch path
+        if not _aliases_arena(eng, self.net.net[0].weight):
+            return None
         return eng.act_host(member, state, float(self.max_action))
 
     def __deepcopy__(self, memo):
@@ -580,11 +553,8 @@ class GaussianPolicy(_PolicyBase):
         if ref is None:
             return None
         eng, member = ref
-        p = self.net.net[0].weight
-        if p.device != eng.device or p.data_ptr() < eng.params.data_ptr() or \
-                p.data_ptr() >= eng.params.data_ptr() + eng.params.numel() * 4 or \
-                self.log_std.data_ptr() < eng.params.data_ptr() or self.log_std.data_ptr() >= eng.params.data_ptr() + eng.params.numel() * 4:
-            return None  # parameters were re-pointed (module moved / re-initialised): stock torch path
+        if not _aliases_arena(eng, self.net.net[0].weight, self.log_std):
+            return None
         return eng.act_host_gaussian(member, state)
 
 
@@ -636,6 +606,9 @@ class ValueFunction(nn.Module):
 # ---------------------------------------------------------------------------
 # the learner
 # ---------------------------------------------------------------------------
+_COUNTER_OF = {"qf": "q", "vf": "v", "actor": "actor"}  # module group -> its optimizer's step counter in `_steps`
+
+
 def _adam_group(opt: torch.optim.Optimizer) -> dict:
     if not isinstance(opt, torch.optim.Adam) or len(opt.param_groups) != 1:
         raise NotImplementedError("the engine implements torch.optim.Adam with a single param group")
@@ -730,7 +703,7 @@ class ImplicitQLearning:
                     if st and "exp_avg" in st:
                         m_views[grp][name].copy_(st["exp_avg"])
                         v_views[grp][name].copy_(st["exp_avg_sq"])
-                        self._steps[{"qf": "q", "vf": "v", "actor": "actor"}[grp]] = int(float(st["step"]))
+                        self._steps[_COUNTER_OF[grp]] = int(float(st["step"]))
                     p.data = view  # module parameters now alias the engine arena
             for name, view in eng.target_views(0).items():
                 p = self.q_target.get_parameter(name)
@@ -765,7 +738,7 @@ class ImplicitQLearning:
         attached = 0
         for grp, mod in self._modules().items():
             opt = self._optimizers()[grp]
-            steps = self._steps[{"qf": "q", "vf": "v", "actor": "actor"}[grp]]
+            steps = self._steps[_COUNTER_OF[grp]]
             if steps == 0:
                 continue  # torch creates Adam state lazily at the first step
             # one CPU step tensor per optimizer, shared by its parameters and updated in place after every
@@ -884,7 +857,7 @@ class ImplicitQLearning:
     def _absorb_optimizer(self, grp: str):
         """After optimizer.load_state_dict: copy its moments into the arena."""
         opt, mod = self._optimizers()[grp], self._modules()[grp]
-        key = {"qf": "q", "vf": "v", "actor": "actor"}[grp]
+        key = _COUNTER_OF[grp]
         step = 0
         if self._engine is None:
             for st in opt.state.values():

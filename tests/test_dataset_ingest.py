@@ -80,3 +80,44 @@ def test_device_ingest_bit_exact_against_numpy_pipeline(env, normalize, normaliz
         assert (gmean, gstd) == (0, 1)
     assert got._size == want._size == 20011 and got._pointer == want._pointer
     assert torch.equal(got.rows, want.rows)
+
+
+def _fortran(d):
+    """The same dataset with every 2-D array in Fortran order and the 1-D ones as strided column views."""
+    out = {k: np.asfortranarray(v) for k, v in d.items()}
+    for k in ("rewards", "terminals"):
+        out[k] = np.asfortranarray(np.stack([d[k], d[k]], 1))[:, :1]
+    return out
+
+
+def test_dataset_tensors_are_dense_for_non_c_order_arrays():
+    import torch
+
+    from jsrl_corl_b200.iql import ReplayBuffer
+
+    rb = object.__new__(ReplayBuffer)  # the host-side part of a buffer; no device is touched
+    rb._device, rb._size, rb._buffer_size, rb._state_dim, rb._action_dim = torch.device("cpu"), 0, 100, 7, 3
+    data = _episodic(n=50)
+    got = rb._dataset_tensors(_fortran(data))
+    for t, k in zip(got, ("observations", "actions", "rewards", "next_observations", "terminals")):
+        assert t.is_contiguous(), k
+        np.testing.assert_array_equal(t.numpy().reshape(data[k].shape), data[k].astype(np.float32))
+
+
+@pytest.mark.gpu
+def test_non_c_order_dataset_loads_like_c_order():
+    import torch
+
+    from jsrl_corl_b200 import ReplayBuffer
+
+    data = _episodic(n=3001, S=11, A=3, seed=5)
+    want, got = ReplayBuffer(11, 3, 4000, "cuda"), ReplayBuffer(11, 3, 4000, "cuda")
+    want.load_d4rl_dataset(data)
+    got.load_d4rl_dataset(_fortran(data))
+    assert torch.equal(got.rows, want.rows)
+    want, got = ReplayBuffer(11, 3, 4000, "cuda"), ReplayBuffer(11, 3, 4000, "cuda")
+    m1, s1 = want.ingest_d4rl_dataset(data)
+    m2, s2 = got.ingest_d4rl_dataset(_fortran(data))
+    np.testing.assert_array_equal(m1, m2)
+    np.testing.assert_array_equal(s1, s2)
+    assert torch.equal(got.rows, want.rows)
